@@ -2,6 +2,7 @@
 """Benchmark of the waveFEniCS hot path on B200 (see the contract in DESIGN.md section 5).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--scaling weak|strong]
+                  [--dump-outputs DIR]
 
 N = 1 workload: BASELINE.json configs[1] -- single-B200 stiffness + mass operator apply,
 64^3 hex cells, P4 (16 974 593 dofs), fp64.  One "step" = one fused apply
@@ -11,11 +12,18 @@ N > 1 (weak, the default): the same per-GPU block on every rank of a cartesian p
 interface dofs of K u reduced with the halo exchange before the mass inverse.
 --scaling strong: BASELINE configs[3], a fixed 128^3-cell global mesh split over the N ranks.
 
-Timing: R windows of K applies each, every window bracketed by barrier + synchronize on both
-sides and timed with CUDA events on the launching stream, max over ranks per window; `value`
-comes from the MEDIAN window (all windows are reported).  A second, >= 0.6 s window gives the
-sustained (power-capped) figure with its own clock record.  The nvidia-smi sampler starts
-before the first barrier, so no rank does host work inside another rank's window.
+Timing: the K timed applies run back to back, split by CUDA events on the launching stream into
+R = min(--windows, K // MIN_WINDOW_STEPS) windows (at least one), with barrier + synchronize before the
+first and after the last; max over ranks per window; `value` comes from the MEDIAN window's time per
+apply (all windows are reported).  The default K = 140 is 7 windows of 20 applies.  A second,
+>= 0.6 s window gives the sustained (power-capped) figure with its own clock record.  The nvidia-smi
+sampler starts before the first barrier and the warm-up, so no rank does host work inside another
+rank's window.
+
+--dump-outputs DIR writes what the last timed step computed, kv (rank 0's vector when N > 1), to
+DIR/kv.npy in float64: all of it, or the entries at a fixed, seeded sample of DUMP_MAX_VALUES dof
+indices (sorted) when it is longer.  The inputs are seeded, so two builds run with the same arguments
+can be compared output for output.
 
 --impl reference times the CPU restatement of the reference operator (oracle/, built with the
 reference's own compiler flags) on the box's host cores, on a bounded sample of the workload;
@@ -37,6 +45,21 @@ sys.path.insert(0, ROOT)
 METRIC = "GDoF/s stiffness+mass apply (P4 hex, fp64)"
 UNIT = "GDoF/s"
 L = 0.1
+DUMP_MAX_VALUES = 1 << 22  # 32 MiB of float64 per dumped array
+MIN_WINDOW_STEPS = 20  # ~9 ms at the default size: the window length of the recorded measurements (profiles/)
+
+
+def dump_sample_index(n):
+    """None (the whole vector) or the sorted dof indices of the fixed sample that --dump-outputs writes."""
+    if n <= DUMP_MAX_VALUES:
+        return None
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_VALUES, replace=False))
+
+
+def dump_outputs(d, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def measured_peak():
@@ -110,7 +133,8 @@ def reference_operator_sample(mesh, P, G, m, x, threads, repeats):
     """The REFERENCE's own StiffnessOperator::operator() / skernel (oracle/_ref/libwfref_cpu_fast.so, cut out of
     common/operators.hpp and compiled at the reference's -Ofast) followed by b / m.  The reference is serial per
     MPI rank; the ranks are host threads here, each applying the operator to its own range of cells into a
-    private vector (ghost contributions), summed afterwards like scatter_rev(add).  None: library not built."""
+    private vector (ghost contributions), summed afterwards like scatter_rev(add).  -> (seconds, kv); None: library
+    not built."""
     import ctypes as C
     from concurrent.futures import ThreadPoolExecutor
     from oracle import oracle
@@ -148,12 +172,13 @@ def reference_operator_sample(mesh, P, G, m, x, threads, repeats):
             if it:
                 best = min(best, time.perf_counter() - t0)
     assert np.isfinite(kv).all()
-    return best
+    return best, kv
 
 
 def cpu_operator_sample(cells, P, threads, repeats=1):
     """Times the reference CPU operator (dense skernel + b/m) on a cells^3 sample mesh: the reference's own
-    code when oracle/_ref holds it (kind "reference"), else the oracle's restatement (kind "port")."""
+    code when oracle/_ref holds it (kind "reference"), else the oracle's restatement (kind "port").
+    -> (ndofs, seconds, kv)"""
     from oracle import oracle, refmesh
     mesh = refmesh.box(cells, P, (L, L, L))
     G, detJ = oracle.precompute_geometric_data(mesh, P)
@@ -164,7 +189,7 @@ def cpu_operator_sample(cells, P, threads, repeats=1):
     if t_ref is not None:
         CPU_KIND.update(kind="reference", how="the reference's own StiffnessOperator::operator() / skernel (oracle/_ref, "
                         "-Ofast -march=x86-64-v3) + b/m, {t} ranks = host threads over cell ranges, private vectors summed")
-        return mesh.ndofs, t_ref
+        return (mesh.ndofs, *t_ref)
     y = np.zeros(mesh.ndofs)
     oracle.stiffness_apply(mesh, P, G, x, y, dense=True, nthreads=threads, fast=True)  # warm-up
     best = 1e300
@@ -175,7 +200,7 @@ def cpu_operator_sample(cells, P, threads, repeats=1):
         kv = y / m
         best = min(best, time.perf_counter() - t0)
     assert np.isfinite(kv).all()
-    return mesh.ndofs, best
+    return mesh.ndofs, best, kv
 
 
 def run_reference(args):
@@ -187,16 +212,20 @@ def run_reference(args):
     for _ in range(args.warmup):
         cpu_operator_sample(min(cells, 8), args.P, threads)
     # bounded: if K steps of the requested sample would not end within ~2.5 minutes, shrink the sample
-    # mesh (the cost is proportional to the number of cells; the rate in DoF/s is what is reported)
-    ndofs, dt = cpu_operator_sample(cells, args.P, threads)
+    # mesh (the cost is proportional to the number of cells; the rate in DoF/s is what is reported) -- except
+    # under --dump-outputs, whose output must depend on the arguments only, not on the speed of the host
+    ndofs, dt, kv = cpu_operator_sample(cells, args.P, threads)
     budget = 150.0
-    if dt * args.steps > budget and cells > 8:
+    if dt * args.steps > budget and cells > 8 and not args.dump_outputs:
         cells = max(8, int(cells * (budget / (dt * args.steps)) ** (1.0 / 3.0)))
-        ndofs, dt = cpu_operator_sample(cells, args.P, threads)
+        ndofs, dt, kv = cpu_operator_sample(cells, args.P, threads)
     t = [dt]
     for _ in range(args.steps - 1):
-        ndofs, dt = cpu_operator_sample(cells, args.P, threads)
+        ndofs, dt, kv = cpu_operator_sample(cells, args.P, threads)
         t.append(dt)
+    if args.dump_outputs:
+        idx = dump_sample_index(kv.size)
+        dump_outputs(args.dump_outputs, {"kv": kv if idx is None else kv[idx]})
     ms = 1e3 * float(np.mean(t))
     value = ndofs / (ms * 1e-3) / 1e9
     sample = f"{cells}^3 cells P{args.P} ({ndofs} dofs) " + CPU_KIND["how"].format(t=threads)
@@ -300,29 +329,38 @@ def run_b200(args):
 
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
 
-    def window(k):
-        """k steps, barrier + synchronize on both sides, device time of this rank in ms"""
+    def windows(fn, sizes):
+        """sum(sizes) calls of fn back to back, an event after each window of sizes[i] calls, barrier +
+        synchronize before the first and after the last: device time of each window on this rank in ms"""
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(len(sizes) + 1)]
         sync_all()
-        ev0.record()
-        for _ in range(k):
-            step()
-        ev1.record()
+        ev[0].record()
+        for i, k in enumerate(sizes):
+            for _ in range(k):
+                fn()
+            ev[i + 1].record()
         sync_all()
-        return ev0.elapsed_time(ev1)
+        return [ev[i].elapsed_time(ev[i + 1]) for i in range(len(sizes))]
 
-    for _ in range(args.warmup):
-        step()
-    # the sampler (a forked nvidia-smi) starts BEFORE the first barrier of the timed windows
+    win_steps = [len(s) for s in np.array_split(np.arange(args.steps), args.windows)]
+    # the sampler (a forked nvidia-smi) starts BEFORE the first barrier of the timed windows, the warm-up after
+    # it, directly before the timed applies: with the warm-up first, the first window measured slower than the
+    # next (DESIGN.md section 5)
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
     sync_all()
+    for _ in range(args.warmup):
+        step()
     tw0 = time.time()
-    win_local = [window(args.steps) for _ in range(args.windows)]
+    win_local = windows(step, win_steps)
     tw1 = time.time()
+    if args.dump_outputs and rank == 0:
+        idx = dump_sample_index(mesh.ndofs)
+        kv = y if idx is None else y[torch.from_numpy(idx).to(dev)]
+        dump_outputs(args.dump_outputs, {"kv": kv.cpu().numpy()})
     win_ms = max_over_ranks(win_local)
-    ms_total = float(np.median(win_ms))
-    ms = ms_total / args.steps
+    ms = float(np.median([w / k for w, k in zip(win_ms, win_steps)]))
     ndofs_global = mesh.ndofs_global
     value = ndofs_global / (ms * 1e-3) / 1e9
 
@@ -331,7 +369,7 @@ def run_b200(args):
     if args.sustain_s > 0:
         k_sus = max(args.steps, int(np.ceil(args.sustain_s * 1e3 / ms)))
         ts0 = time.time()
-        ms_sus = max_over_ranks([window(k_sus)])[0] / k_sus
+        ms_sus = max_over_ranks(windows(step, [k_sus]))[0] / k_sus
         ts1 = time.time()
         sustained = {"ms_per_step": ms_sus, "steps": k_sus, "value": ndofs_global / (ms_sus * 1e-3) / 1e9}
     if rank == 0:
@@ -382,15 +420,7 @@ def run_b200(args):
         ki_a, info_a = stiff_a.kernel_info(), stiff_a.info()
         for _ in range(args.warmup):
             stiff_a.apply_scaled(x, minv_a, y)
-        wa = []
-        for _ in range(args.windows):
-            sync_all()
-            ev0.record()
-            for _ in range(args.steps):
-                stiff_a.apply_scaled(x, minv_a, y)
-            ev1.record()
-            sync_all()
-            wa.append(ev0.elapsed_time(ev1) / args.steps)
+        wa = [w / k for w, k in zip(windows(lambda: stiff_a.apply_scaled(x, minv_a, y), win_steps), win_steps)]
         ms_a = float(np.median(wa))
         # parity of the fast path inside the run: against the per-cell kernel on the per-point G
         simple_a = wfx.StiffnessOperator(mesh_a, P, ctx=ctx, geometry=geo_a, mode=wfx.capi.STIFF_CELL_COLOUR)
@@ -583,7 +613,7 @@ def run_b200(args):
     cpu = None
     if world == 1 and not args.no_cpu_baseline:
         threads = host_threads()
-        nd_cpu, t_cpu = cpu_operator_sample(args.ref_cells, P, threads)
+        nd_cpu, t_cpu, _ = cpu_operator_sample(args.ref_cells, P, threads)
         cpu = {"value": nd_cpu / t_cpu / 1e9, "unit": UNIT, "cores": threads, "kind": CPU_KIND["kind"],
                "sample": f"{args.ref_cells}^3 cells P{P} ({nd_cpu} dofs), " + CPU_KIND["how"].format(t=threads)}
     s = 8
@@ -598,15 +628,16 @@ def run_b200(args):
                        "l2_policy": f"inputs larger than L2 (G {g_bytes / 1e9:.2f} GB + vectors {vec_bytes / 1e9:.2f} GB per apply "
                                     f"vs 126 MB L2); no flush needed",
                        "dofmap": "brick-implicit (one int32 per brick dof, no per-point dofmap is read): see roofline.frac_no_dofmap",
-                       "timing": f"median of {args.windows} windows of {args.steps} applies, max over ranks per window",
+                       "timing": f"{args.steps} applies back to back in {len(win_steps)} windows of {win_steps} applies, "
+                                 "median window time per apply, max over ranks per window",
                        "partition": "x".join(map(str, grid)), "setup_s": round(t_setup, 2),
                        "kernel": kernel_info, "halo_transport": halo_transport},
-            "windows_ms": win_ms, "window_ms_min": min(win_ms), "window_ms_max": max(win_ms),
+            "windows_ms": win_ms, "window_steps": win_steps, "window_ms_min": min(win_ms), "window_ms_max": max(win_ms),
             "clocks": clocks, "sustained": sustained, "parity": parity, "affine_fast_path": affine,
             "e2e": e2e,
             # per apply: the colour launches of the brick kernel + the ghost reduction (one fused kernel over
             # peer memory; pack, unpack-add, pack, unpack around two NCCL groups otherwise)
-            "gpu_launches": (args.windows * args.steps) * (info["nlaunches"] + (0 if halo is None else (1 if halo_transport == "p2p" else 4))),
+            "gpu_launches": args.steps * (info["nlaunches"] + (0 if halo is None else (1 if halo_transport == "p2p" else 4))),
             "roofline": roofline, "cpu_baseline": cpu, "rk4": rk4, "strong_scaling": strong}
     print(json.dumps(line))
     if world > 1:
@@ -616,9 +647,11 @@ def run_b200(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=None, help="applies per timed window; default 20 (b200 arm), 5 (reference arm)")
+    ap.add_argument("--steps", type=int, default=None, help="timed applies; default 140 (b200 arm), 5 (reference arm)")
     ap.add_argument("--warmup", type=int, default=5)
-    ap.add_argument("--windows", type=int, default=7, help="timed windows; the median is reported")
+    ap.add_argument("--windows", type=int, default=7,
+                    help=f"windows the timed applies are split into, each of at least {MIN_WINDOW_STEPS} applies "
+                         "(one when --steps is smaller); the median is reported")
     ap.add_argument("--sustain-s", type=float, default=0.6, help="length of the sustained window in seconds (0 = skip)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
@@ -632,11 +665,13 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-affine", action="store_true")
     ap.add_argument("--no-strong", action="store_true", help="skip the 128^3 strong-scaling RK4 sub-measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output kv to DIR/kv.npy")
     args = ap.parse_args()
     if args.steps is None:
-        args.steps = 20 if args.impl == "b200" else 5
-    args.steps = max(1, args.steps)
-    args.windows = max(5, args.windows)
+        args.steps = 140 if args.impl == "b200" else 5
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    args.windows = max(1, min(args.windows, args.steps // MIN_WINDOW_STEPS))
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

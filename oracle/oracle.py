@@ -5,10 +5,13 @@ cpu_baseline / --impl reference legs of bench.py.  Never imported by the product
 PARITY UNPINNED for the C restatement (see the header of wave_oracle.c); the reference's own CUDA
 primitives, the one part of the path that compiles here, are available through ref_cuda().
 """
+import atexit
 import ctypes as C
 import hashlib
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -16,6 +19,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = os.path.join(HERE, "wave_oracle.c")
 OUT = os.path.join(HERE, "_build")
 GCC = os.environ.get("ORACLE_GCC", "/usr/bin/gcc")
+_tmp_out = []
 
 _i32p = C.POINTER(C.c_int32)
 _f64p = C.POINTER(C.c_double)
@@ -32,10 +36,23 @@ def _cpu_tag():
     return "unknown"
 
 
+def _out_dir():
+    """oracle/_build, or a private temporary directory (removed at exit) when the checkout is read-only."""
+    try:
+        os.makedirs(OUT, exist_ok=True)
+        if os.access(OUT, os.W_OK):
+            return OUT
+    except OSError:
+        pass
+    if not _tmp_out:
+        _tmp_out.append(tempfile.mkdtemp(prefix="wfx_oracle_"))
+        atexit.register(shutil.rmtree, _tmp_out[0], True)
+    return _tmp_out[0]
+
+
 def build(fast=False, force=False):
     """strict: IEEE build for parity.  fast: the reference's -Ofast -march=native flags
     (demo/cpu_planar3d/CMakeLists.txt:27) for CPU-baseline timing; rebuilt per host CPU."""
-    os.makedirs(OUT, exist_ok=True)
     with open(SRC, "rb") as fh:
         dig = hashlib.sha256(fh.read()).hexdigest()[:12]
     if fast:
@@ -43,6 +60,8 @@ def build(fast=False, force=False):
     else:
         name, flags = f"liboracle_{dig}.so", ["-O2", "-march=x86-64-v3", "-ffp-contract=off"]
     path = os.path.join(OUT, name)
+    if force or not os.path.exists(path):
+        path = os.path.join(_out_dir(), name)
     if force or not os.path.exists(path):
         cmd = [GCC, *flags, "-fopenmp", "-shared", "-fPIC", "-o", path + ".tmp", SRC, "-lm"]
         subprocess.run(cmd, check=True)

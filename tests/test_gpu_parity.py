@@ -824,7 +824,7 @@ def test_stiffness_repeatable_under_concurrent_load(wfx, torch):
         side.synchronize()
 
 
-# ---- the reference's own CUDA primitives (oracle/_ref, compiled from /root/reference) ----------------
+# ---- the reference's own CUDA primitives (oracle/_ref, compiled from the reference sources) -----------
 @pytest.mark.gpu
 @pytest.mark.parametrize("dtype", [np.float64, np.float32])
 def test_primitives_against_the_reference_cuda_kernels(wfx, orc, torch, dtype):
@@ -834,7 +834,7 @@ def test_primitives_against_the_reference_cuda_kernels(wfx, orc, torch, dtype):
     import ctypes as C
     ref = orc.ref_cuda()
     if ref is None:
-        pytest.skip("oracle/_ref/libwfref_cuda.so was not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libwfref_cuda.so was not built (needs the reference sources, WFX_REFERENCE, at build time)")
     sfx = "f64" if dtype == np.float64 else "f32"
     tdt = torch.float64 if dtype == np.float64 else torch.float32
     code = wfx.capi.dtype_code(dtype)
@@ -884,7 +884,7 @@ def test_primitives_against_the_reference_cuda_kernels(wfx, orc, torch, dtype):
     assert float((y - y_ref).norm() / y_ref.norm()) < (1e-14 if dtype == np.float64 else 2e-6)
 
 
-# ---- the reference's own CPU code (oracle/_ref/libwfref_cpu.so, cut out of /root/reference's headers) -----
+# ---- the reference's own CPU code (oracle/_ref/libwfref_cpu.so, cut out of the reference's headers) -------
 @pytest.mark.gpu
 @pytest.mark.parametrize("P,shape,perturb", [(4, (4, 3, 2), 0.15), (2, (5, 4, 3), 0.15), (5, (2, 2, 2), 0.1)])
 def test_cuda_operators_against_the_reference_cpu_code(wfx, orc, torch, P, shape, perturb):
@@ -892,7 +892,7 @@ def test_cuda_operators_against_the_reference_cpu_code(wfx, orc, torch, P, shape
     skernel and MassOperatorCPU::operator() / mkernel (common/operators.hpp), compiled from the reference
     sources (tests/test_reference_pins.py has the bit-for-bit pin of the oracle to the same code)."""
     if orc.ref_cpu() is None:
-        pytest.skip("oracle/_ref/libwfref_cpu.so was not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libwfref_cpu.so was not built (needs the reference sources, WFX_REFERENCE, at build time)")
     mesh = wfx.create_box_hex(shape, P, (L, 0.7 * L, 1.3 * L), perturb=perturb)
     geo = wfx.Geometry(mesh, P)
     Go, detJ = orc.precompute_geometric_data(mesh, P)
@@ -916,7 +916,7 @@ def test_cuda_rk4_against_the_reference_time_stepper(wfx, orc, torch, capfd, sha
     """The CUDA time stepper against the REFERENCE's own LinearGLLOpt::rk4 / f0 / f1 / kernels::axpy / copy
     (common/LinearGLL.hpp) over whole trajectories, including a shorter last step."""
     if orc.ref_cpu() is None:
-        pytest.skip("oracle/_ref/libwfref_cpu.so was not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libwfref_cpu.so was not built (needs the reference sources, WFX_REFERENCE, at build time)")
     P, c0, f0, p0 = 4, 1500.0, 0.5e6, 6e4
     mesh = wfx.create_box_hex(shape, P, (L * shape[0] / 8, L * shape[1] / 8, L * shape[2] / 8), perturb=perturb)
     Go, detJ = orc.precompute_geometric_data(mesh, P)

@@ -1,11 +1,13 @@
-"""The oracle pinned to REFERENCE CODE where the reference compiles.  Cut out of the headers where they lie
-under /root/reference and compiled into oracle/_ref/libwfref_cpu.so (oracle/build_ref.py) against the small
+"""The oracle pinned to REFERENCE CODE where the reference compiles.  Cut out of the headers of the reference sources
+(WFX_REFERENCE at build time) and compiled into oracle/_ref/libwfref_cpu.so (oracle/build_ref.py) against the small
 container stand-ins of oracle/ref_cpu_shim.cpp: the cell kernels `skernel` / `mkernel`, the call loops
 StiffnessOperator::operator() / MassOperatorCPU::operator() (common/operators.hpp), kernels::copy / axpy and
 LinearGLLOpt::init / f0 / f1 / rk4 (common/LinearGLL.hpp).  The oracle's restatements must reproduce them BIT
 FOR BIT (same flags: -O2 -ffp-contract=off) -- operators, right-hand side and whole RK4 trajectories.  What
 stays restated (third-party arithmetic, absent here): Basix tables, DOLFINx geometry, the FFCx facet kernel.
-The GPU box uses the prebuilt library (it travels with the snapshot)."""
+Without the reference sources the library is not built and the tests that call it skip; the reference outputs
+stored in tests/golden/reference_*.npz are compared in every checkout (test_oracle_reproduces_the_reference_golden_vectors,
+test_cuda_path_matches_the_reference_golden_vectors)."""
 import importlib.util
 import os
 
@@ -27,7 +29,7 @@ CASES = [(2, (3, 2, 2), 0.15), (3, (2, 2, 3), 0.15), (4, (2, 2, 2), 0.15), (4, (
 def ref(orc):
     L = orc.ref_cpu()
     if L is None:
-        pytest.skip("oracle/_ref/libwfref_cpu.so was not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libwfref_cpu.so was not built (needs the reference sources, WFX_REFERENCE, at build time)")
     return L
 
 
@@ -185,7 +187,7 @@ def test_rank_grid_is_the_reference_decompose3d(wfx, orc):
     import ctypes as C
     L = orc.ref_mesh()
     if L is None:
-        pytest.skip("oracle/_ref/libwfref_mesh.so was not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libwfref_mesh.so was not built (needs the reference sources, WFX_REFERENCE, at build time)")
     from wave_fenics_b200 import partition
     for x in range(0, 10):                                # 1 .. 512 ranks (powers of two: all the reference handles)
         out = (C.c_int * 3)()
@@ -205,7 +207,7 @@ def test_reorder_dofmap_is_the_reference_loop(wfx, orc, P):
     the oracle's and the product's host function equal the reference's own loop."""
     L = orc.ref_mesh()
     if L is None:
-        pytest.skip("oracle/_ref/libwfref_mesh.so was not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libwfref_mesh.so was not built (needs the reference sources, WFX_REFERENCE, at build time)")
     nd = (P + 1) ** 3
     rng = np.random.default_rng(P)
     dm = rng.integers(0, 10 ** 6, size=(11, nd)).astype(np.int32)
@@ -222,7 +224,7 @@ def test_time_step_is_the_reference_demos(wfx, orc):
     import ctypes as C
     L = orc.ref_mesh()
     if L is None:
-        pytest.skip("oracle/_ref/libwfref_mesh.so was not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libwfref_mesh.so was not built (needs the reference sources, WFX_REFERENCE, at build time)")
     rng = np.random.default_rng(2)
     for P in (2, 3, 4, 5, 7):
         for h in list(rng.uniform(1e-4, 5e-2, 6)) + [np.sqrt(3.0) * 0.1 / 16]:
@@ -238,7 +240,7 @@ def test_general_point_jacobian_and_factor_use_the_reference_dot(wfx, orc):
     equal the reference's own `dot` bit for bit (row a9)."""
     L = orc.ref_mesh()
     if L is None:
-        pytest.skip("oracle/_ref/libwfref_mesh.so was not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libwfref_mesh.so was not built (needs the reference sources, WFX_REFERENCE, at build time)")
     mesh = wfx.create_box_hex((2, 2, 1), 2, (1.0, 0.7, 1.3), perturb=0.2)
     pts = np.random.default_rng(4).uniform(0, 1, size=(5, 3))
     wts = np.random.default_rng(5).uniform(0.1, 1, size=5)
