@@ -43,10 +43,15 @@ enum {
   WFX_STIFF_NO_SPLIT = 2,    /* (or-ed in) distributed meshes: do not schedule the interface batches as
                                 a part of their own; the apply is then one pass and the ghost reduction
                                 follows it (best when the reduction is cheap: NVLink peer memory) */
-  WFX_STIFF_CELL_STREAM = 4  /* streamed-cell kernel: coloured cells, software-pipelined gather, FIRST / LAST
+  WFX_STIFF_CELL_STREAM = 4, /* streamed-cell kernel: coloured cells, software-pipelined gather, FIRST / LAST
                                 flags in the per-point dofmap (fused scaling, no memset); single-rank meshes.
                                 WFX_STIFF_AUTO takes it by itself at the degrees where it measured faster */
+  WFX_STIFF_ENSEMBLE = 8     /* (or-ed in) also build the ensemble path (wfx_stiffness_apply_ensemble); costs
+                                at most one more per-point dofmap (4 B per cell point), no copy of G */
 };
+
+/* most fields of one ensemble */
+#define WFX_ENSEMBLE_MAX 8
 
 typedef struct wfx_ctx wfx_ctx;
 typedef struct wfx_geom wfx_geom;
@@ -168,6 +173,16 @@ int wfx_stiffness_apply_part(wfx_stiffness* op, const void* x_dev, const void* s
  * Replaces stiff_op(u_n, b) followed by b/m (common/LinearGLL.hpp:173-191). */
 int wfx_stiffness_apply_scaled(wfx_stiffness* op, const void* x_dev, const void* scale_dev,
                                void* y_dev, void* stream);
+/* Ensemble apply: nv fields (1 <= nv <= WFX_ENSEMBLE_MAX) that share the mesh, the operator and c0, in
+ * one pass over G and the dofmap.  Vectors are member-interleaved, [ndofs][nv]: entry (dof i, member m)
+ * at i*nv + m -- the DOLFINx blocked la::Vector with block size bs = nv.  For every member m
+ *   y[:,m] (+)= scale .* (-c0^2 K x[:,m])
+ * scale_dev: [ndofs] (one value per dof for all members, e.g. 1/m) or NULL; a scale needs beta == 0 (as
+ * wfx_stiffness_apply_scaled).  Needs an operator created with WFX_STIFF_ENSEMBLE and without rank-shared
+ * dofs.  Deterministic: results repeat bit for bit, and a member's result does not depend on the others
+ * or on its position in the ensemble. */
+int wfx_stiffness_apply_ensemble(wfx_stiffness* op, int nv, const void* x_dev, const void* scale_dev,
+                                 void* y_dev, int beta, void* stream);
 /* Same call shape as the reference functor on host la::Vector arrays: copies x (and y
  * when beta != 0) to the GPU, applies, copies y back.  Synchronous. */
 int wfx_stiffness_apply_host(wfx_stiffness* op, const void* x_host, void* y_host, int beta);
@@ -294,6 +309,16 @@ int wfx_halo_destroy(wfx_halo* halo);
 int wfx_wave_create(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass, wfx_boundary* bnd,
                     wfx_halo* halo, int64_t size_local, double c0, double f0, double p0,
                     wfx_wave** wave);
+/* Ensemble model: nv members (1 <= nv <= WFX_ENSEMBLE_MAX) on one rank that share the mesh, the operators
+ * and c0; member m is the model LinearGLLOpt(..., c0, f0_host[m], p0_host[m]) with its own source
+ * g_m(t) = window_m(t) p0_m w_m / c0 cos(w_m t), w_m = 2 pi f0_m, and its own four-period Hann ramp.
+ * stiff must have been created with WFX_STIFF_ENSEMBLE.  init, set_state, get_state, state_ptrs, f0, f1,
+ * rk4, set_probes, get_probe_series and destroy accept the model; their vectors are then
+ * member-interleaved [ndofs][nv] (see wfx_stiffness_apply_ensemble), probe values [nrecords][nprobes][nv].
+ * set_snapshot refuses an ensemble model. */
+int wfx_wave_create_ensemble(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass, wfx_boundary* bnd, int nv,
+                             int64_t size_local, double c0, const double* f0_host, const double* p0_host,
+                             wfx_wave** wave);
 int wfx_wave_init(wfx_wave* wave);                                   /* :131-134 */
 /* Copies the state to the device; on a distributed mesh the ghost entries are then overwritten by
  * their owners' values (u->scatter_fwd(), v->scatter_fwd(), :164,167). */

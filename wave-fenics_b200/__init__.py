@@ -7,5 +7,5 @@ package is the Python host-side mirror of the reference's operator interface.
 from . import capi  # noqa: F401  (raises when libwavefx.so is missing: no CPU fallback)
 from .capi import WfxError  # noqa: F401
 from .mesh import HexMesh, create_box_hex, cfl_timestep, dof_coordinates  # noqa: F401
-from .operators import (BoundaryOperator, Context, Geometry, LinearGLLOpt, MassOperator,  # noqa: F401
-                        MassOperatorCPU, StiffnessOperator, compute_jacobian_data)
+from .operators import (BoundaryOperator, Context, Geometry, LinearGLLEnsemble, LinearGLLOpt,  # noqa: F401
+                        MassOperator, MassOperatorCPU, StiffnessOperator, compute_jacobian_data)

@@ -12,7 +12,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("WFX_LIB") or os.path.join(HERE, "libwavefx.so")
 
 F64, F32 = 0, 1
-STIFF_AUTO, STIFF_CELL_COLOUR, STIFF_NO_SPLIT, STIFF_CELL_STREAM = 0, 1, 2, 4
+STIFF_AUTO, STIFF_CELL_COLOUR, STIFF_NO_SPLIT, STIFF_CELL_STREAM, STIFF_ENSEMBLE = 0, 1, 2, 4, 8
+ENSEMBLE_MAX = 8
 
 _c_i32p = C.POINTER(C.c_int32)
 _c_i64p = C.POINTER(C.c_int64)
@@ -68,6 +69,7 @@ _SIG = {
     "wfx_halo_update_rev_fwd_scaled": [_vp, _vp, _vp, _vp],
     "wfx_boundary_assemble": [_vp, _vp],
     "wfx_stiffness_apply_scaled": [_vp, _vp, _vp, _vp, _vp],
+    "wfx_stiffness_apply_ensemble": [_vp, C.c_int, _vp, _vp, _vp, C.c_int, _vp],
     "wfx_stiffness_apply_host": [_vp, _vp, _vp, C.c_int],
     "wfx_stiffness_mass_apply_host": [_vp, _vp, _vp, _vp],
     "wfx_stiffness_mass_apply_host_batch": [_vp, _vp, C.c_int, _vpp, _vpp],
@@ -104,6 +106,7 @@ _SIG = {
     "wfx_halo_update_rev_fwd": [_vp, _vp, _vp],
     "wfx_halo_destroy": [_vp],
     "wfx_wave_create": [_vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_double, C.c_double, C.c_double, _vpp],
+    "wfx_wave_create_ensemble": [_vp, _vp, _vp, _vp, C.c_int, C.c_int64, C.c_double, _c_f64p, _c_f64p, _vpp],
     "wfx_wave_init": [_vp],
     "wfx_wave_set_state": [_vp, _vp, _vp],
     "wfx_wave_get_state": [_vp, _vp, _vp],

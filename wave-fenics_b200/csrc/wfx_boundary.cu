@@ -38,7 +38,46 @@ __global__ void boundary_kernel(int64_t nb, const int32_t* __restrict__ idx,
   const int32_t i = idx[t];
   b[i] = (T)((double)b[i] + c02g * m1[t] - c0 * m2[t] * (double)vn[i]);
 }
+
+// the same for nv member-interleaved fields, one thread per (boundary dof, member); c02 = c0^2 and the
+// product c0^2 * g_m is rounded once as in boundary_kernel
+struct EnsAmp
+{
+  double g[WFX_ENSEMBLE_MAX];
+};
+template <typename T>
+__global__ void boundary_ens_kernel(int64_t nb, int nv, const int32_t* __restrict__ idx,
+                                    const double* __restrict__ m1, const double* __restrict__ m2, double c02,
+                                    double c0, const EnsAmp gh, const double* __restrict__ g_dev,
+                                    const T* __restrict__ vn, T* __restrict__ b)
+{
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t >= nb * nv) return;
+  const int64_t p = t / nv;
+  const int m = (int)(t % nv);
+  const double c02g = __dmul_rn(c02, g_dev ? g_dev[m] : gh.g[m]);
+  const int64_t i = (int64_t)idx[p] * nv + m;
+  b[i] = (T)((double)b[i] + c02g * m1[p] - c0 * m2[p] * (double)vn[i]);
+}
 } // namespace
+
+void wfx::boundary_apply_ens(wfx_boundary* op, int nv, double c0, const double* g_host, const double* g_dev,
+                             const void* vn, void* b, cudaStream_t stream)
+{
+  if (!op || op->nb == 0) return;
+  if (nv < 1 || nv > WFX_ENSEMBLE_MAX) fail("boundary: nv = %d outside [1, %d]", nv, WFX_ENSEMBLE_MAX);
+  EnsAmp gh{};
+  if (!g_dev)
+    for (int m = 0; m < nv; ++m) gh.g[m] = g_host[m];
+  const unsigned grid = (unsigned)((op->nb * nv + 255) / 256);
+  if (op->dtype == WFX_F64)
+    boundary_ens_kernel<double><<<grid, 256, 0, stream>>>(op->nb, nv, op->d_idx.p, op->d_m1.p, op->d_m2.p, c0 * c0,
+                                                           c0, gh, g_dev, (const double*)vn, (double*)b);
+  else
+    boundary_ens_kernel<float><<<grid, 256, 0, stream>>>(op->nb, nv, op->d_idx.p, op->d_m1.p, op->d_m2.p, c0 * c0,
+                                                          c0, gh, g_dev, (const float*)vn, (float*)b);
+  WFX_CUDA(cudaGetLastError());
+}
 
 extern "C" int wfx_boundary_create(wfx_ctx* ctx, int P, int dtype, int64_t nfacets,
                                    const int32_t* fcell, const int32_t* flocal,

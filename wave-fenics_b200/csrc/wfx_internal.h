@@ -112,6 +112,12 @@ int boundary_dtype(const struct ::wfx_boundary* op);
 // replays of a time step change g without touching the graph), wfx_boundary.cu
 void boundary_apply_dev(struct ::wfx_boundary* op, double c0, const double* g_dev, const void* vn, void* b,
                         cudaStream_t stream);
+// ensemble models (member-interleaved vectors [ndofs][nv]): the operator has the ensemble path
+// (wfx_stiffness.cu); boundary term of every member, b[i,m] += c0^2 g_m m1_i - c0 m2_i vn[i,m], with the nv
+// amplitudes from g_dev when it is not NULL (graph replays), else from g_host (wfx_boundary.cu)
+bool stiffness_has_ensemble(const struct ::wfx_stiffness* op);
+void boundary_apply_ens(struct ::wfx_boundary* op, int nv, double c0, const double* g_host, const double* g_dev,
+                        const void* vn, void* b, cudaStream_t stream);
 
 // NVTX ranges around the phases of a time step (the reference marks its profiled regions the same
 // way: demo/gpu_scatter_mpi/main.cpp:101-121, demo/gpu_cg/CUDA/cg.hpp:74-113).  nvtx3 is header-only

@@ -783,6 +783,108 @@ stiff_cell2_kernel(const Cell2Args<T> a, const DMat<T, N> Dm, int cell0, int ncl
   if (!waited) pdl_wait();
 }
 
+// ---- ensemble kernel: nv fields per pass over G and the dofmap -------------------------------
+// Vectors are member-interleaved (entry (dof i, member m) at i*nv + m: DOLFINx's blocked layout with
+// bs = nv).  Cells run in colour order as in stiff_cell2_kernel -- no dof arrays in shared memory,
+// FIRST / LAST flags in the per-point dofmap -- one cell per slot.  The slot loads the cell's dof
+// indices and its whole G (N planes, GW = N) into registers once and then runs the sum-factorised
+// kernel once per member, so G and the dofmap stream from HBM once for all members while a dof's nv
+// values are one contiguous span of nv*sizeof(T) bytes: the gather / update of member m + 1 hits the
+// sectors member m brought into L1 / L2.  The next member's x values are gathered while the current
+// member finishes part 2.  nv is a run-time value: one instantiation serves every nv.
+template <typename T>
+struct EnsArgs
+{
+  const int32_t* cells;  // cell ids sorted by colour
+  const uint32_t* tdmf;  // [ncells][ND] k-major point order: global dof | BD_FIRST | BD_LAST
+  const T* G6;
+  const T* x;            // [ndofs][nv]
+  T* y;                  // [ndofs][nv]
+  const T* scale;        // [ndofs], nullable: applied on the LAST touch of a dof
+  T coeff;
+  int beta;    // 0: FIRST touch overwrites y; 1: accumulates into y
+  int g_order; // column order of G6 (see g_column)
+  int nv;
+  int64_t ndofs, ncells;
+};
+
+template <typename T, int N, int SLOT, int CPB, int MINB>
+__global__ void __launch_bounds__(SLOT* CPB, MINB)
+stiff_ens_kernel(const EnsArgs<T> a, const DMat<T, N> Dm, int cell0, int ncl)
+{
+  constexpr int N2 = N * N, ND = N2 * N;
+  using V2 = typename Vec2<T>::type;
+  using L = LayoutStd<N, sizeof(T)>;
+  static_assert(SLOT <= 32 ? (32 % SLOT == 0) : (SLOT % 32 == 0), "a slot is a fraction or a multiple of a warp");
+  static_assert(SLOT <= 32 || CPB <= 15, "one named barrier per slot");
+  __shared__ __align__(16) T s_w[CPB][L::SLOT_ELEMS];
+  pdl_launch_dependents(); // the next colour may start gathering; it waits before touching y
+  const int slot = threadIdx.x / SLOT, col = threadIdx.x % SLOT;
+  const bool lane_ok = col < N2;
+  const RoleOff ro = L::offsets(lane_ok ? col : 0);
+  const int gcol = g_column<L, N>(ro, lane_ok ? col : 0, a.g_order);
+  const int ci = (int)blockIdx.x * CPB + slot;
+  const int cell = ci < ncl ? __ldg(a.cells + cell0 + ci) : -1;
+  WFX_DEV_ASSERT(cell < a.ncells);
+  const bool active = lane_ok && cell >= 0;
+  const int nv = a.nv;
+  auto sync = [&]() {
+    if constexpr (SLOT <= 32) __syncwarp();
+    else SlotBarSync{slot + 1, SLOT}();
+  };
+  uint32_t dof[N];
+  T u[N];
+  V2 g[N][3];
+#pragma unroll
+  for (int k = 0; k < N; ++k)
+  {
+    dof[k] = active ? ld_once(a.tdmf + (int64_t)cell * ND + k * N2 + col) : BD_HOLE;
+    WFX_DEV_ASSERT(dof[k] == BD_HOLE || (int64_t)(dof[k] & BD_MASK) < a.ndofs);
+  }
+  if (active) load_G<T, N, N>(a.G6 + (int64_t)cell * (6 * ND), gcol, g);
+  auto gather = [&](int m) {
+#pragma unroll
+    for (int k = 0; k < N; ++k)
+      u[k] = dof[k] != BD_HOLE ? __ldg(a.x + (int64_t)(dof[k] & BD_MASK) * nv + m) : T(0);
+  };
+  gather(0);
+  bool waited = false;
+  T* tiles = s_w[slot];
+  PhaseTimer tm;
+  tm.start(false);
+  for (int m = 0; m < nv; ++m)
+  {
+    T f2[N], yv[N];
+    // G stays in its registers for every member (no window refill: gcur / gnext are null)
+    if constexpr (SLOT <= 32) cell_part1<T, N, L, N>(u, g, tiles, ro, Dm, a.coeff, active, WarpSync(), f2, tm);
+    else cell_part1<T, N, L, N>(u, g, tiles, ro, Dm, a.coeff, active, SlotBarSync{slot + 1, SLOT}, f2, tm);
+    // u is consumed: its registers take the next member's x values, in flight during part 2
+    if (m + 1 < nv) gather(m + 1);
+    if constexpr (SLOT <= 32) cell_part2<T, N, L>(f2, tiles, ro, Dm, active, WarpSync(), yv, tm);
+    else cell_part2<T, N, L>(f2, tiles, ro, Dm, active, SlotBarSync{slot + 1, SLOT}, yv, tm);
+    if (!waited)
+    {
+      pdl_wait(); // earlier colours have finished their writes to y
+      waited = true;
+    }
+    if (active)
+    {
+      T yo[N], sc[N];
+#pragma unroll
+      for (int k = 0; k < N; ++k)
+      {
+        const uint32_t e = dof[k];
+        yo[k] = (!(e & BD_FIRST) || a.beta) ? __ldcg(a.y + (int64_t)(e & BD_MASK) * nv + m) : T(0);
+        sc[k] = ((e & BD_LAST) && a.scale) ? __ldg(a.scale + (e & BD_MASK)) : T(1);
+      }
+#pragma unroll
+      for (int k = 0; k < N; ++k) a.y[(int64_t)(dof[k] & BD_MASK) * nv + m] = (yo[k] + yv[k]) * sc[k];
+    }
+    sync(); // part 2's reads of the tiles precede the next member's writes
+  }
+  if (!waited) pdl_wait();
+}
+
 // ---- product kernel: one CTA per batch ------------------------------------------------
 template <typename T>
 struct BrickArgs
@@ -1507,6 +1609,13 @@ __global__ void zero_entries_kernel(const int32_t* __restrict__ idx, int n, T* _
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t < n) y[idx[t]] = T(0);
 }
+// the same for member-interleaved vectors: all nv members of the listed dofs
+template <typename T>
+__global__ void zero_entries_ens_kernel(const int32_t* __restrict__ idx, int64_t n, int nv, T* __restrict__ y)
+{
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t < n) y[(int64_t)idx[t / nv] * nv + t % nv] = T(0);
+}
 
 // One-time in-place reordering of the columns of a degree-4 G6 (rows of 25 2-vectors, one warp
 // per row): the row's column q moves to position c_p4d_colpos[q].
@@ -1827,6 +1936,14 @@ struct wfx_stiffness
   int axis_perm[3] = {0, 1, 2}; // kernel axis a' is the mesh's tensor axis axis_perm[a'] (see detect_axis_perm)
   DevBuf<uint32_t> d_tdmf;
   DevBuf<unsigned char> d_G6perm; // private copy of G6 in the permuted axis order (empty: identity)
+  // ensemble path (WFX_STIFF_ENSEMBLE): streamed cells in colour order over member-interleaved vectors.
+  // An operator whose own path is the colour-ordered streamed kernel shares its plan and G; any other
+  // builds its own plan (identity axes: G6 is read as stored, through its column order)
+  bool ens = false;
+  int64_t nshared = 0;
+  CellColourPlan ens_plan; // cell ids live in d_ens_cells
+  DevBuf<int32_t> d_ens_cells, d_ens_untouched;
+  DevBuf<uint32_t> d_ens_tdmf;
   // brick path
   int ncolours = 0, nloc_pad = 0, W = 0, rounds_max = 0;
   int part_split = 0; // first execution colour of the interior part (distributed meshes)
@@ -1967,6 +2084,67 @@ void launch_cell2(wfx_stiffness* op, const T* x, const T* scale, T* y, int beta,
     const int per_cta = C2::CPB * op->cell2_cps;
     launch(stiff_cell2_kernel<T, N, C::SLOT, C2::CPB, MINB2, GW, false>, C::SLOT * C2::CPB,
            (ncl + per_cta - 1) / per_cta, beg, ncl);
+  }
+}
+
+// ensemble kernel: the streamed kernel's slot width, 256 threads per CTA.  A slot holds its cell's whole G
+// in registers; at fp64 from P5 up that does not fit 128 registers per thread next to the rest, so those
+// instantiations take up to 255 (one 256-thread CTA per SM less)
+template <typename T, int N>
+struct CfgE
+{
+  static constexpr int SLOT = Cell2Slot<N>::SLOT;
+  static constexpr int CPB = 256 / SLOT;
+  static constexpr int MINB = (sizeof(T) == 8 && N >= 6) ? 1 : 2;
+};
+
+template <typename T, int N>
+void launch_ens(wfx_stiffness* op, int nv, const T* x, const T* scale, T* y, int beta, cudaStream_t st)
+{
+  using C = CfgE<T, N>;
+  DMat<T, N> Dm;
+  for (int q = 0; q < N * N; ++q) Dm.d[q] = (T)op->Dhost[q];
+  for (int q = 0; q < N; ++q) Dm.w[q] = (T)op->Whost[q];
+  const bool share = op->cell2 && !op->cell2_brick; // the operator's own colour-ordered streamed plan
+  const CellColourPlan& cp = share ? op->cplan : op->ens_plan;
+  const DevBuf<int32_t>& untouched = share ? op->d_untouched : op->d_ens_untouched;
+  EnsArgs<T> a;
+  a.cells = share ? op->d_cells.p : op->d_ens_cells.p;
+  a.tdmf = share ? op->d_tdmf.p : op->d_ens_tdmf.p;
+  a.G6 = (share && op->d_G6perm.n) ? (const T*)op->d_G6perm.p : (const T*)op->geom->G6;
+  a.x = x;
+  a.y = y;
+  a.scale = scale;
+  a.coeff = (T)(-1.0 * op->c0 * op->c0);
+  a.beta = beta;
+  a.g_order = op->geom->g_colpos.empty() ? 0 : 1;
+  a.nv = nv;
+  a.ndofs = op->ndofs;
+  a.ncells = op->ncells;
+  if (!beta && untouched.n)
+  {
+    const int64_t n = (int64_t)untouched.n * nv;
+    zero_entries_ens_kernel<T><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(untouched.p, n, nv, y);
+  }
+  // the first launch sees everything earlier in the stream; later colours chain by programmatic
+  // dependent launch and wait before their first access to y
+  bool first = true;
+  for (int k = 0; k < cp.ncolours; ++k)
+  {
+    const int beg = cp.colour_off[k], ncl = cp.colour_off[k + 1] - beg;
+    if (ncl == 0) continue;
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3((ncl + C::CPB - 1) / C::CPB);
+    cfg.blockDim = dim3(C::SLOT * C::CPB);
+    cfg.dynamicSmemBytes = 0;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = (op->use_pdl && !first) ? 1 : 0;
+    WFX_CUDA(cudaLaunchKernelEx(&cfg, stiff_ens_kernel<T, N, C::SLOT, C::CPB, C::MINB>, a, Dm, beg, ncl));
+    first = false;
   }
 }
 
@@ -2212,6 +2390,22 @@ void apply_any(wfx_stiffness* op, const void* x, const void* scale, void* y, int
   else
     dispatch_apply<float>(op, (const float*)x, (const float*)scale, (float*)y, beta, part, (cudaStream_t)stream);
 }
+
+template <typename T>
+void dispatch_ens(wfx_stiffness* op, int nv, const T* x, const T* scale, T* y, int beta, cudaStream_t st)
+{
+  switch (op->N)
+  {
+  case 3: launch_ens<T, 3>(op, nv, x, scale, y, beta, st); break;
+  case 4: launch_ens<T, 4>(op, nv, x, scale, y, beta, st); break;
+  case 5: launch_ens<T, 5>(op, nv, x, scale, y, beta, st); break;
+  case 6: launch_ens<T, 6>(op, nv, x, scale, y, beta, st); break;
+  case 7: launch_ens<T, 7>(op, nv, x, scale, y, beta, st); break;
+  case 8: launch_ens<T, 8>(op, nv, x, scale, y, beta, st); break;
+  default: fail("stiffness: degree %d not supported", op->P);
+  }
+  WFX_CUDA(cudaGetLastError());
+}
 } // namespace
 
 // shared with the mass / boundary operators
@@ -2221,6 +2415,7 @@ int stiffness_dtype(const wfx_stiffness* op) { return op->dtype; }
 bool stiffness_has_split(const wfx_stiffness* op) { return op->part_split > 0; }
 // the single-launch form passes a per-apply epoch as a kernel argument: not replayable from a graph
 bool stiffness_graph_safe(const wfx_stiffness* op) { return !op->persistent; }
+bool stiffness_has_ensemble(const wfx_stiffness* op) { return op->ens; }
 
 // tensor-ordered dofmap in the kernels' k-major point order
 void build_tensor_dofmap(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap,
@@ -2284,7 +2479,8 @@ extern "C" int wfx_stiffness_create_partitioned(wfx_ctx* ctx, wfx_geom* geom, in
   if (ndofs < 0) fail("negative ndofs");
   if (ndofs >= (1ll << 31)) fail("more than 2^31 local dofs");
   bool split_parts = !(flags & WFX_STIFF_NO_SPLIT);
-  flags &= ~WFX_STIFF_NO_SPLIT;
+  const bool ensemble = (flags & WFX_STIFF_ENSEMBLE) != 0;
+  flags &= ~(WFX_STIFF_NO_SPLIT | WFX_STIFF_ENSEMBLE);
   if (flags != WFX_STIFF_AUTO && flags != WFX_STIFF_CELL_COLOUR && flags != WFX_STIFF_CELL_STREAM)
     fail("unknown stiffness flags %d", flags);
   if (const char* e = std::getenv("WFX_SPLIT")) split_parts = std::atoi(e) != 0;
@@ -2507,7 +2703,24 @@ extern "C" int wfx_stiffness_create_partitioned(wfx_ctx* ctx, wfx_geom* geom, in
       else configure_any<float>(op.get());
       timer.lap("uploads + configure");
     }
+    // ensemble path: single-rank operators only (a blocked ghost exchange does not exist); it reuses the
+    // operator's colour-ordered streamed plan when there is one
+    if (ensemble && nshared == 0 && !(op->cell2 && !op->cell2_brick))
+    {
+      StreamPlan sp;
+      build_stream_plan(op->P, op->ncells, ndofs, tdm.data(), nullptr, nullptr, false, BrickShape(1), 1, nullptr,
+                        false, false, sp);
+      timer.lap("ensemble plan");
+      if (std::getenv("WFX_VERIFY_PLAN")) verify_stream_plan(sp, tdm.data());
+      op->ens_plan.ncolours = sp.ncolours;
+      op->ens_plan.colour_off = sp.colour_off;
+      op->d_ens_cells.upload(sp.cells);
+      op->d_ens_tdmf.upload(sp.tdmf);
+      if (!sp.untouched.empty()) op->d_ens_untouched.upload(sp.untouched);
+    }
   }
+  op->nshared = nshared;
+  op->ens = ensemble && nshared == 0;
   *out = op.release();
   WFX_API_END
 }
@@ -2537,6 +2750,33 @@ extern "C" int wfx_stiffness_apply_scaled(wfx_stiffness* op, const void* x, cons
   WFX_API_BEGIN
   if (!scale) fail("stiffness: scale vector is NULL");
   apply_any(op, x, scale, y, 0, stream);
+  WFX_API_END
+}
+
+extern "C" int wfx_stiffness_apply_ensemble(wfx_stiffness* op, int nv, const void* x, const void* scale, void* y,
+                                            int beta, void* stream)
+{
+  WFX_API_BEGIN
+  if (!op) fail("stiffness operator is NULL");
+  if (op->nshared > 0)
+    fail("stiffness ensemble apply: the operator has %lld rank-shared dofs (ensembles are single-rank)",
+         (long long)op->nshared);
+  if (!op->ens) fail("stiffness ensemble apply: the operator was created without WFX_STIFF_ENSEMBLE");
+  if (nv < 1 || nv > WFX_ENSEMBLE_MAX) fail("stiffness ensemble apply: nv = %d outside [1, %d]", nv, WFX_ENSEMBLE_MAX);
+  if (scale && beta) fail("stiffness ensemble apply: a scale needs beta == 0");
+  if (!x || !y) fail("stiffness: NULL vector");
+  if (x == y) fail("stiffness: x and y must not alias");
+  if (op->ncells == 0)
+  {
+    if (!beta)
+      WFX_CUDA(cudaMemsetAsync(y, 0, (size_t)op->ndofs * nv * (op->dtype == WFX_F64 ? 8 : 4), (cudaStream_t)stream));
+    return 0;
+  }
+  ScopedDevice sd(op->ctx->device);
+  if (op->dtype == WFX_F64)
+    dispatch_ens<double>(op, nv, (const double*)x, (const double*)scale, (double*)y, beta, (cudaStream_t)stream);
+  else
+    dispatch_ens<float>(op, nv, (const float*)x, (const float*)scale, (float*)y, beta, (cudaStream_t)stream);
   WFX_API_END
 }
 

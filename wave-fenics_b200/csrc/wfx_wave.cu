@@ -26,6 +26,10 @@ struct wfx_wave
   int dtype = WFX_F64;
   int64_t n = 0, size_local = 0;
   double c0 = 0, f0 = 0, p0 = 0;
+  // ensemble model (wfx_wave_create_ensemble): nv members, vectors [n][nv], member m's source (f0s[m], p0s[m])
+  bool ens = false;
+  int nv = 1;
+  std::vector<double> f0s, p0s;
   const void* minv = nullptr;
   // u_, v_: solution; u0, v0: start of step; un, vn: stage state; b: right-hand side
   DevBuf<unsigned char> u_, v_, u0, v0, un, vn, b;
@@ -34,6 +38,7 @@ struct wfx_wave
   cudaEvent_t ev_iface = nullptr, ev_halo = nullptr;
   // one-rank runs: a full time step (4 stages, ~40 launches) is captured once per step size
   // into a CUDA graph and replayed; the four source amplitudes of the step live in g_dev
+  // ([stage][member] for an ensemble)
   bool use_graph = true;
   cudaGraphExec_t step_graph = nullptr;
   double graph_dt = 0;
@@ -141,11 +146,86 @@ void launch_stage(int stage, int64_t n, const void* b, const void* minv, void* u
 #undef WFX_STAGE
   WFX_CUDA(cudaGetLastError());
 }
+// rk_stage_kernel on member-interleaved vectors, one thread per entry: the nv threads of a dof are adjacent
+// lanes, so every access of a warp is contiguous and minv[i] is one broadcast load for all members of dof i
+template <typename T, int STAGE>
+__global__ void __launch_bounds__(256)
+rk_stage_ens_kernel(int64_t n, int nv, const T* __restrict__ b, const T* __restrict__ minv, T* __restrict__ u_,
+                    T* __restrict__ v_, T* __restrict__ u0, T* __restrict__ v0, T* __restrict__ un,
+                    T* __restrict__ vn, T bdt, T adt_next)
+{
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k >= n * nv) return;
+  const T kv = b[k] * minv[k / nv];
+  T us = u_[k], vs = v_[k];
+  T ku, ub, vb;
+  if (STAGE == 0)
+  {
+    ku = vs;
+    ub = us;
+    vb = vs;
+    u0[k] = ub;
+    v0[k] = vb;
+  }
+  else
+  {
+    ku = vn[k];
+    if (STAGE < 3)
+    {
+      ub = u0[k];
+      vb = v0[k];
+    }
+  }
+  u_[k] = ku * bdt + us;
+  v_[k] = kv * bdt + vs;
+  if (STAGE < 3)
+  {
+    un[k] = ku * adt_next + ub;
+    vn[k] = kv * adt_next + vb;
+  }
+}
+
+template <typename T>
+void launch_stage_ens(int stage, int64_t n, int nv, const void* b, const void* minv, void* u_, void* v_, void* u0,
+                      void* v0, void* un, void* vn, double bdt, double adt_next, cudaStream_t st)
+{
+  const unsigned grid = (unsigned)((n * nv + 255) / 256);
+#define WFX_STAGE(S)                                                                                        \
+  rk_stage_ens_kernel<T, S><<<grid, 256, 0, st>>>(n, nv, (const T*)b, (const T*)minv, (T*)u_, (T*)v_,     \
+                                                   (T*)u0, (T*)v0, (T*)un, (T*)vn, (T)bdt, (T)adt_next)
+  switch (stage)
+  {
+  case 0: WFX_STAGE(0); break;
+  case 1: WFX_STAGE(1); break;
+  case 2: WFX_STAGE(2); break;
+  default: WFX_STAGE(3); break;
+  }
+#undef WFX_STAGE
+  WFX_CUDA(cudaGetLastError());
+}
+
+// result[i,m] = b[i,m] * minv[i]: the b/m of f1 for an ensemble
+template <typename T>
+__global__ void scale_rows_kernel(int64_t n, int nv, const T* __restrict__ b, const T* __restrict__ minv,
+                                  T* __restrict__ out)
+{
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k < n * nv) out[k] = b[k] * minv[k / nv];
+}
+
 template <typename T>
 __global__ void probe_kernel(int64_t n, const int32_t* __restrict__ idx, const T* __restrict__ u, T* __restrict__ out)
 {
   const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (i < n) out[i] = u[idx[i]];
+}
+// ensemble models: out[p][m] = u[idx[p]][m]
+template <typename T>
+__global__ void probe_ens_kernel(int64_t n, int nv, const int32_t* __restrict__ idx, const T* __restrict__ u,
+                                 T* __restrict__ out)
+{
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t < n * nv) out[t] = u[(int64_t)idx[t / nv] * nv + t % nv];
 }
 
 // the pending snapshot's copy has landed: hand it to the callback
@@ -163,9 +243,13 @@ void after_step(wfx_wave* w, cudaStream_t ws)
   const size_t esz = w->dtype == WFX_F64 ? 8 : 4;
   if (w->nprobes && w->probe_rec < w->probe_cap)
   {
-    const unsigned grid = (unsigned)((w->nprobes + 255) / 256);
-    unsigned char* out = w->d_probe_val.p + (size_t)w->probe_rec * w->nprobes * esz;
-    if (w->dtype == WFX_F64)
+    const unsigned grid = (unsigned)((w->nprobes * w->nv + 255) / 256);
+    unsigned char* out = w->d_probe_val.p + (size_t)w->probe_rec * w->nprobes * w->nv * esz;
+    if (w->ens && w->dtype == WFX_F64)
+      probe_ens_kernel<double><<<grid, 256, 0, ws>>>(w->nprobes, w->nv, w->d_probe_idx.p, (const double*)w->u_.p, (double*)out);
+    else if (w->ens)
+      probe_ens_kernel<float><<<grid, 256, 0, ws>>>(w->nprobes, w->nv, w->d_probe_idx.p, (const float*)w->u_.p, (float*)out);
+    else if (w->dtype == WFX_F64)
       probe_kernel<double><<<grid, 256, 0, ws>>>(w->nprobes, w->d_probe_idx.p, (const double*)w->u_.p, (double*)out);
     else
       probe_kernel<float><<<grid, 256, 0, ws>>>(w->nprobes, w->d_probe_idx.p, (const float*)w->u_.p, (float*)out);
@@ -195,9 +279,18 @@ __global__ void set_source_kernel(double* g_dev, double g0, double g1, double g2
 {
   g_dev[0] = g0, g_dev[1] = g1, g_dev[2] = g2, g_dev[3] = g3;
 }
+// ensemble models: the 4 x nv amplitudes of a step, [stage][member], passed by value
+struct StepAmp
+{
+  double g[4 * WFX_ENSEMBLE_MAX];
+};
+__global__ void set_source_ens_kernel(double* g_dev, const StepAmp a, int n)
+{
+  if ((int)threadIdx.x < n) g_dev[threadIdx.x] = a.g[threadIdx.x];
+}
 
-// One time step of size dt on stream st: the four stages of LinearGLL.hpp:244-270.  g[i] is the
-// source amplitude of stage i; with g_from_dev the boundary kernels read it from w->g_dev
+// One time step of size dt on stream st: the four stages of LinearGLL.hpp:244-270.  g[i*nv + m] is the
+// source amplitude of stage i (of member m); with g_from_dev the boundary kernels read it from w->g_dev
 // instead (graph capture).
 void enqueue_step(wfx_wave* w, double dt, const double* g, bool g_from_dev, cudaStream_t st)
 {
@@ -205,7 +298,10 @@ void enqueue_step(wfx_wave* w, double dt, const double* g, bool g_from_dev, cuda
   const double b_runge[4] = {1.0 / 6.0, 1.0 / 3.0, 1.0 / 3.0, 1.0 / 6.0};
   auto boundary = [&](int i, const void* vn) {
     if (!w->bnd) return;
-    if (g_from_dev) boundary_apply_dev(w->bnd, w->c0, w->g_dev.p + i, vn, w->b.p, st);
+    if (w->ens)
+      boundary_apply_ens(w->bnd, w->nv, w->c0, g_from_dev ? nullptr : g + i * w->nv,
+                         g_from_dev ? w->g_dev.p + i * w->nv : nullptr, vn, w->b.p, st);
+    else if (g_from_dev) boundary_apply_dev(w->bnd, w->c0, w->g_dev.p + i, vn, w->b.p, st);
     else if (wfx_boundary_apply(w->bnd, w->c0, g[i], vn, w->b.p, st)) fail("%s", wfx_last_error()); // :175
   };
   static const char* const stage_name[4] = {"wfx rk4 stage 0", "wfx rk4 stage 1", "wfx rk4 stage 2", "wfx rk4 stage 3"};
@@ -220,7 +316,9 @@ void enqueue_step(wfx_wave* w, double dt, const double* g, bool g_from_dev, cuda
     {
       {
         NvtxRange r("wfx stiffness apply");
-        if (wfx_stiffness_apply(w->stiff, un, w->b.p, 0, st)) fail("%s", wfx_last_error()); // :173-174
+        const int rc = w->ens ? wfx_stiffness_apply_ensemble(w->stiff, w->nv, un, nullptr, w->b.p, 0, st)
+                              : wfx_stiffness_apply(w->stiff, un, w->b.p, 0, st); // :173-174
+        if (rc) fail("%s", wfx_last_error());
       }
       boundary(i, vn);
     }
@@ -251,7 +349,13 @@ void enqueue_step(wfx_wave* w, double dt, const double* g, bool g_from_dev, cuda
       boundary(i, vn);
     }
     NvtxRange update_range("wfx fused stage update");
-    if (w->dtype == WFX_F64)
+    if (w->ens && w->dtype == WFX_F64)
+      launch_stage_ens<double>(i, w->n, w->nv, w->b.p, w->minv, w->u_.p, w->v_.p, w->u0.p, w->v0.p, w->un.p,
+                               w->vn.p, dt * b_runge[i], dt * a_runge[i + 1], st);
+    else if (w->ens)
+      launch_stage_ens<float>(i, w->n, w->nv, w->b.p, w->minv, w->u_.p, w->v_.p, w->u0.p, w->v0.p, w->un.p,
+                              w->vn.p, dt * b_runge[i], dt * a_runge[i + 1], st);
+    else if (w->dtype == WFX_F64)
       launch_stage<double>(i, w->n, w->b.p, w->minv, w->u_.p, w->v_.p, w->u0.p, w->v0.p, w->un.p,
                            w->vn.p, dt * b_runge[i], dt * a_runge[i + 1], st);
     else
@@ -328,6 +432,37 @@ extern "C" int wfx_wave_create(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mas
   WFX_API_END
 }
 
+extern "C" int wfx_wave_create_ensemble(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass, wfx_boundary* bnd,
+                                        int nv, int64_t size_local, double c0, const double* f0_host,
+                                        const double* p0_host, wfx_wave** out)
+{
+  WFX_API_BEGIN
+  if (!ctx || !stiff || !mass || !out || !f0_host || !p0_host) fail("NULL argument");
+  if (nv < 1 || nv > WFX_ENSEMBLE_MAX) fail("wave ensemble: nv = %d outside [1, %d]", nv, WFX_ENSEMBLE_MAX);
+  if (!stiffness_has_ensemble(stiff))
+    fail("wave ensemble: the stiffness operator needs WFX_STIFF_ENSEMBLE and no rank-shared dofs");
+  for (int m = 0; m < nv; ++m)
+    if (!(f0_host[m] > 0)) fail("wave ensemble: source frequency of member %d must be positive", m);
+  wfx_wave* w = nullptr;
+  if (wfx_wave_create(ctx, stiff, mass, bnd, nullptr, size_local, c0, f0_host[0], p0_host[0], &w))
+    fail("%s", wfx_last_error());
+  std::unique_ptr<wfx_wave> guard(w);
+  ScopedDevice sd(ctx->device);
+  w->ens = true;
+  w->nv = nv;
+  w->f0s.assign(f0_host, f0_host + nv);
+  w->p0s.assign(p0_host, p0_host + nv);
+  w->g_dev.alloc(4 * WFX_ENSEMBLE_MAX);
+  const size_t nb = (size_t)w->n * nv * (w->dtype == WFX_F64 ? 8 : 4);
+  for (auto* v : {&w->u_, &w->v_, &w->u0, &w->v0, &w->un, &w->vn, &w->b})
+  {
+    v->alloc(nb);
+    if (nb) WFX_CUDA(cudaMemset(v->p, 0, nb));
+  }
+  *out = guard.release();
+  WFX_API_END
+}
+
 extern "C" int wfx_wave_init(wfx_wave* w)
 {
   WFX_API_BEGIN
@@ -389,11 +524,17 @@ extern "C" int wfx_wave_state_ptrs(wfx_wave* w, void** u, void** v)
 namespace
 {
 // g(t) of LinearGLL.hpp:155-162: Hann ramp over the first alpha periods
-double source_amplitude(const wfx_wave* w, double tn)
+double source_amplitude(double f0, double p0, double c0, double tn)
 {
-  const double w0 = 2.0 * M_PI * w->f0, T = 1.0 / w->f0, alpha = 4.0; // :96-99
-  const double window = tn < T * alpha ? 0.5 * (1.0 - std::cos(w->f0 * M_PI * tn / alpha)) : 1.0;
-  return window * w->p0 * w0 / w->c0 * std::cos(w0 * tn);
+  const double w0 = 2.0 * M_PI * f0, T = 1.0 / f0, alpha = 4.0; // :96-99
+  const double window = tn < T * alpha ? 0.5 * (1.0 - std::cos(f0 * M_PI * tn / alpha)) : 1.0;
+  return window * p0 * w0 / c0 * std::cos(w0 * tn);
+}
+double source_amplitude(const wfx_wave* w, double tn) { return source_amplitude(w->f0, w->p0, w->c0, tn); }
+// g_m(t) of every member (ensemble models): g[m], m < nv
+void source_amplitudes(const wfx_wave* w, double tn, double* g)
+{
+  for (int m = 0; m < w->nv; ++m) g[m] = source_amplitude(w->f0s[m], w->p0s[m], w->c0, tn);
 }
 } // namespace
 
@@ -403,7 +544,7 @@ extern "C" int wfx_wave_f0(wfx_wave* w, double, const void* u, const void* v, vo
   if (!w) fail("wave model is NULL");
   if (!u || !v || !result) fail("f0: NULL vector");
   ScopedDevice sd(w->ctx->device);
-  const size_t nb = (size_t)w->n * (w->dtype == WFX_F64 ? 8 : 4);
+  const size_t nb = (size_t)w->n * w->nv * (w->dtype == WFX_F64 ? 8 : 4);
   if (result != v) WFX_CUDA(cudaMemcpyAsync(result, v, nb, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   WFX_API_END
 }
@@ -416,6 +557,22 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
   if (result == u || result == v) fail("f1: result must not alias u or v");
   ScopedDevice sd(w->ctx->device);
   cudaStream_t st = (cudaStream_t)stream;
+  if (w->ens)
+  {
+    double g[WFX_ENSEMBLE_MAX];
+    source_amplitudes(w, t, g);
+    if (wfx_stiffness_apply_ensemble(w->stiff, w->nv, u, nullptr, w->b.p, 0, st)) fail("%s", wfx_last_error());
+    boundary_apply_ens(w->bnd, w->nv, w->c0, g, nullptr, v, w->b.p, st);
+    const int64_t n = w->n * w->nv;
+    if (n == 0) return 0;
+    const unsigned grid = (unsigned)((n + 255) / 256);
+    if (w->dtype == WFX_F64)
+      scale_rows_kernel<double><<<grid, 256, 0, st>>>(w->n, w->nv, (const double*)w->b.p, (const double*)w->minv, (double*)result);
+    else
+      scale_rows_kernel<float><<<grid, 256, 0, st>>>(w->n, w->nv, (const float*)w->b.p, (const float*)w->minv, (float*)result);
+    WFX_CUDA(cudaGetLastError());
+    return 0;
+  }
   const double g = source_amplitude(w, t);
   if (wfx_stiffness_apply(w->stiff, u, w->b.p, 0, st)) fail("%s", wfx_last_error());                     // :173-174
   if (w->halo && wfx_halo_update_rev_fwd(w->halo, w->b.p, st)) fail("%s", wfx_last_error());             // :176
@@ -451,11 +608,12 @@ extern "C" int wfx_wave_rk4(wfx_wave* w, double t0, double tf, double dt, int64_
     if (max_steps > 0 && step >= max_steps) break;
     NvtxRange step_range("wfx rk4 step");
     dt = std::min(dt, tf - t); // :242
-    double g[4];
+    double g[4 * WFX_ENSEMBLE_MAX]; // [stage][member]
     for (int i = 0; i < 4; ++i)
     {
       const double tn = t + c_runge[i] * dt; // :257
-      g[i] = source_amplitude(w, tn); // :155-162
+      if (w->ens) source_amplitudes(w, tn, g + i * w->nv);
+      else g[i] = source_amplitude(w, tn); // :155-162
     }
     if (graph_ok && dt == dt_nominal)
     {
@@ -481,7 +639,13 @@ extern "C" int wfx_wave_rk4(wfx_wave* w, double t0, double tf, double dt, int64_
         WFX_CUDA(ie);
         w->graph_dt = dt;
       }
-      set_source_kernel<<<1, 1, 0, ws>>>(w->g_dev.p, g[0], g[1], g[2], g[3]);
+      if (w->ens)
+      {
+        StepAmp a{};
+        for (int q = 0; q < 4 * w->nv; ++q) a.g[q] = g[q];
+        set_source_ens_kernel<<<1, 4 * WFX_ENSEMBLE_MAX, 0, ws>>>(w->g_dev.p, a, 4 * w->nv);
+      }
+      else set_source_kernel<<<1, 1, 0, ws>>>(w->g_dev.p, g[0], g[1], g[2], g[3]);
       WFX_CUDA(cudaGraphLaunch(w->step_graph, ws));
     }
     else enqueue_step(w, dt, g, false, ws);
@@ -526,7 +690,7 @@ extern "C" int wfx_wave_set_probes(wfx_wave* w, int64_t nprobes, const int32_t* 
   if (nprobes)
   {
     w->d_probe_idx.upload(dofs_host, (size_t)nprobes);
-    w->d_probe_val.alloc((size_t)nprobes * (size_t)max_records * (w->dtype == WFX_F64 ? 8 : 4));
+    w->d_probe_val.alloc((size_t)nprobes * (size_t)max_records * w->nv * (w->dtype == WFX_F64 ? 8 : 4));
   }
   WFX_API_END
 }
@@ -543,7 +707,7 @@ extern "C" int wfx_wave_get_probe_series(wfx_wave* w, int64_t* nrecords, double*
   {
     WFX_CUDA(cudaDeviceSynchronize());
     WFX_CUDA(cudaMemcpy(values_host, w->d_probe_val.p,
-                        (size_t)w->probe_rec * w->nprobes * (w->dtype == WFX_F64 ? 8 : 4), cudaMemcpyDeviceToHost));
+                        (size_t)w->probe_rec * w->nprobes * w->nv * (w->dtype == WFX_F64 ? 8 : 4), cudaMemcpyDeviceToHost));
   }
   WFX_API_END
 }
@@ -553,6 +717,7 @@ extern "C" int wfx_wave_set_snapshot(wfx_wave* w, int64_t every, wfx_snapshot_fn
   WFX_API_BEGIN
   if (!w) fail("wave model is NULL");
   if (every < 0) fail("snapshot interval must not be negative");
+  if (w->ens) fail("wave: snapshots are not available for ensemble models");
   ScopedDevice sd(w->ctx->device);
   flush_snapshot(w);
   w->snap_every = fn ? every : 0;

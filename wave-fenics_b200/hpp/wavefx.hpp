@@ -120,13 +120,15 @@ public:
   // shared_dofs (distributed meshes): the local dofs that also live on another rank (the union of
   // HaloSpec::send_indices and recv_indices).  Cells touching them are scheduled first so that the
   // ghost exchange overlaps the interior cells.
+  // flags: WFX_STIFF_ENSEMBLE adds the ensemble path (apply_ensemble_device)
   StiffnessOperator(std::shared_ptr<Geometry<T>> geom, const SpaceView& V, int bdegree,
-                    std::map<std::string, double>& params, const std::vector<std::int32_t>& shared_dofs = {})
+                    std::map<std::string, double>& params, const std::vector<std::int32_t>& shared_dofs = {},
+                    int flags = WFX_STIFF_AUTO)
       : _geom(std::move(geom)), _ndofs(V.ndofs), _params(params)
   {
     if (bdegree != V.degree) throw std::runtime_error("wavefx: degree mismatch");
     check(wfx_stiffness_create_partitioned(_geom->context()->get(), _geom->get(), V.ndofs, V.dofmap, 1500.0,
-                                           WFX_STIFF_AUTO, (std::int64_t)shared_dofs.size(),
+                                           flags, (std::int64_t)shared_dofs.size(),
                                            shared_dofs.empty() ? nullptr : shared_dofs.data(), &_h));
   }
   ~StiffnessOperator() { wfx_stiffness_destroy(_h); }
@@ -149,6 +151,12 @@ public:
   void apply_scaled_device(const T* x, const T* scale, T* y, void* stream = nullptr)
   {
     check(wfx_stiffness_apply_scaled(_h, x, scale, y, stream));
+  }
+  // nv member-interleaved fields ([ndofs][nv], the blocked la::Vector with bs = nv) in one pass over G:
+  // y[:,m] (+)= scale .* (-c0^2 K x[:,m]); scale (ndofs entries, e.g. 1/m) may be null and needs beta == 0
+  void apply_ensemble_device(int nv, const T* x, const T* scale, T* y, int beta = 0, void* stream = nullptr)
+  {
+    check(wfx_stiffness_apply_ensemble(_h, nv, x, scale, y, beta, stream));
   }
   std::size_t num_cells() const { return (std::size_t)info().ncells; }
   std::size_t num_dofs() const { return (std::size_t)info().nd; }
@@ -403,6 +411,95 @@ private:
   std::shared_ptr<VectorUpdater<double>> _halo;
   std::shared_ptr<Geometry<double>> _geom;
   std::int64_t _ndofs;
+  wfx_boundary* _bnd = nullptr;
+  wfx_wave* _wave = nullptr;
+};
+// nv wave models on one mesh (1 <= nv <= WFX_ENSEMBLE_MAX), one rank, fp64: member m is
+// LinearGLLOpt(V, degree, c0, f0[m], p0[m]); the stiffness apply of a stage reads G once for all members.
+// States are member-interleaved [ndofs][nv] (entry (dof i, member m) at i*nv + m), probe values
+// [nrec][nprobes][nv].  Snapshots are not available for ensembles.
+class LinearGLLEnsemble
+{
+public:
+  LinearGLLEnsemble(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
+                    const std::vector<double>& sourceFrequencies, const std::vector<double>& pressureAmplitudes)
+      : _ctx(std::move(ctx)), _ndofs(V.ndofs), _nv((int)sourceFrequencies.size())
+  {
+    if (pressureAmplitudes.size() != sourceFrequencies.size())
+      throw std::runtime_error("wavefx: one source frequency and one pressure amplitude per member expected");
+    _geom = std::make_shared<Geometry<double>>(_ctx, V);
+    mass_op = std::make_shared<MassOperator<double>>(_geom, V, degreeOfBasis);
+    std::map<std::string, double> params{{"c0", speedOfSound}};
+    stiff_op = std::make_shared<StiffnessOperator<double>>(_geom, V, degreeOfBasis, params, std::vector<std::int32_t>{},
+                                                           WFX_STIFF_ENSEMBLE);
+    check(wfx_boundary_create(_ctx->get(), V.degree, WFX_F64, V.nfacets, V.facet_cell, V.facet_local, V.facet_tag,
+                              V.npoints, V.x, V.xdofs, V.ndofs, V.dofmap, &_bnd));
+    check(wfx_wave_create_ensemble(_ctx->get(), stiff_op->get(), mass_op->get(), _bnd, _nv, V.size_local, speedOfSound,
+                                   sourceFrequencies.data(), pressureAmplitudes.data(), &_wave));
+  }
+  ~LinearGLLEnsemble()
+  {
+    wfx_wave_destroy(_wave);
+    wfx_boundary_destroy(_bnd);
+  }
+  LinearGLLEnsemble(const LinearGLLEnsemble&) = delete;
+  LinearGLLEnsemble& operator=(const LinearGLLEnsemble&) = delete;
+
+  int size() const { return _nv; }
+  void init() { check(wfx_wave_init(_wave)); }
+  // device arrays of ndofs * nv entries
+  void f0(double t, const double* u_dev, const double* v_dev, double* result_dev, void* stream = nullptr)
+  {
+    check(wfx_wave_f0(_wave, t, u_dev, v_dev, result_dev, stream));
+  }
+  void f1(double t, const double* u_dev, const double* v_dev, double* result_dev, void* stream = nullptr)
+  {
+    check(wfx_wave_f1(_wave, t, u_dev, v_dev, result_dev, stream));
+  }
+  std::int64_t rk4(double startTime, double finalTime, double timeStep)
+  {
+    std::int64_t steps = 0;
+    double t_end = 0;
+    check(wfx_wave_rk4(_wave, startTime, finalTime, timeStep, 0, &steps, &t_end, nullptr));
+    _ctx->synchronize();
+    return steps;
+  }
+  void set_probes(const std::vector<std::int32_t>& dofs, std::int64_t max_records)
+  {
+    _nprobes = (std::int64_t)dofs.size();
+    check(wfx_wave_set_probes(_wave, _nprobes, dofs.data(), max_records));
+  }
+  // times [nrec] and values [nrec][nprobes][nv] recorded so far
+  void probe_series(std::vector<double>& t, std::vector<double>& values) const
+  {
+    std::int64_t n = 0;
+    check(wfx_wave_get_probe_series(_wave, &n, nullptr, nullptr));
+    t.resize((std::size_t)n);
+    values.resize((std::size_t)(n * _nprobes * _nv));
+    check(wfx_wave_get_probe_series(_wave, &n, t.data(), values.data()));
+  }
+  void set_state(const std::vector<double>& u, const std::vector<double>& v)
+  {
+    if ((std::int64_t)u.size() != _ndofs * _nv || (std::int64_t)v.size() != _ndofs * _nv)
+      throw std::runtime_error("wavefx: ensemble state must hold ndofs * nv entries");
+    check(wfx_wave_set_state(_wave, u.data(), v.data()));
+  }
+  void solution(std::vector<double>& u_n, std::vector<double>& v_n) const
+  {
+    u_n.resize((std::size_t)(_ndofs * _nv));
+    v_n.resize((std::size_t)(_ndofs * _nv));
+    check(wfx_wave_get_state(_wave, u_n.data(), v_n.data()));
+  }
+
+  std::shared_ptr<MassOperator<double>> mass_op;
+  std::shared_ptr<StiffnessOperator<double>> stiff_op;
+
+private:
+  std::shared_ptr<Context> _ctx;
+  std::shared_ptr<Geometry<double>> _geom;
+  std::int64_t _ndofs;
+  int _nv;
+  std::int64_t _nprobes = 0;
   wfx_boundary* _bnd = nullptr;
   wfx_wave* _wave = nullptr;
 };

@@ -6,6 +6,8 @@ Same names, argument meaning and call shape as the reference classes:
   StiffnessOperator(V, degree, params)(x, y)    common/operators.hpp:136-201
   LinearGLLOpt(mesh, meshtags, degree, c0, f0, p0).init() / .rk4(t0, tf, dt)
                                                 common/LinearGLL.hpp:37-287
+  LinearGLLEnsemble(mesh, meshtags, degree, c0, f0s, p0s)
+                                                nv LinearGLLOpt models on one mesh, stepped together
 
 `V` is a HexMesh (mesh.py): it carries what the reference pulls out of the DOLFINx
 FunctionSpace (geometry, geometry dofmap, cell dofmap, index-map sizes).  Vectors are
@@ -141,7 +143,7 @@ class StiffnessOperator(_Operator):
     honour_params=True."""
 
     def __init__(self, V, degree, params=None, dtype=np.float64, ctx=None, geometry=None,
-                 mode=capi.STIFF_AUTO, honour_params=False, split=True):
+                 mode=capi.STIFF_AUTO, honour_params=False, split=True, ensemble=False):
         self.ctx = ctx or Context.get()
         self.P = int(degree)
         self.dtype = np.dtype(dtype)
@@ -160,7 +162,8 @@ class StiffnessOperator(_Operator):
             shared = np.unique(np.concatenate([halo["send_indices"], halo["recv_indices"]])).astype(np.int32)
         self.nshared = 0 if shared is None else len(shared)
         capi.call("wfx_stiffness_create_partitioned", self.ctx.handle, self.geometry.handle, self.ndofs,
-                  capi.i32p(dm.reshape(-1)), c0, mode | (0 if split else capi.STIFF_NO_SPLIT), self.nshared,
+                  capi.i32p(dm.reshape(-1)), c0,
+                  mode | (0 if split else capi.STIFF_NO_SPLIT) | (capi.STIFF_ENSEMBLE if ensemble else 0), self.nshared,
                   capi.i32p(shared), C.byref(self.handle))
         self.split = bool(split) and self.nshared > 0
 
@@ -188,6 +191,22 @@ class StiffnessOperator(_Operator):
         self._check(x, y)
         capi.call("wfx_stiffness_apply_scaled", self.handle, C.c_void_p(x.data_ptr()),
                   C.c_void_p(scale_ptr), C.c_void_p(y.data_ptr()), _stream_ptr())
+
+    def apply_ensemble(self, X, Y, beta=0, scale_ptr=None):
+        """Y[:, m] (+)= scale .* (-c0^2 K X[:, m]) for every member m, in one pass over the geometric
+        factors: X, Y contiguous CUDA tensors of shape (ndofs, nv), 1 <= nv <= 8 (member-interleaved, the
+        DOLFINx blocked layout with bs = nv).  scale_ptr: device pointer to ndofs values (e.g. 1/m) or None;
+        a scale needs beta == 0.  Needs ensemble=True at construction."""
+        import torch
+        want = torch.float64 if self.dtype == np.float64 else torch.float32
+        for v in (X, Y):
+            if (not _is_torch(v) or not v.is_cuda or v.dtype != want or not v.is_contiguous() or v.dim() != 2
+                    or v.shape[0] != self.ndofs):
+                raise capi.WfxError("ensemble vectors must be contiguous (ndofs, nv) CUDA tensors of the operator's dtype")
+        if X.shape != Y.shape:
+            raise capi.WfxError("ensemble vectors X and Y differ in shape")
+        capi.call("wfx_stiffness_apply_ensemble", self.handle, int(X.shape[1]), C.c_void_p(X.data_ptr()),
+                  C.c_void_p(scale_ptr) if scale_ptr else None, C.c_void_p(Y.data_ptr()), int(beta), _stream_ptr())
 
     def info(self):
         nc, nd, ndofs = C.c_int64(), C.c_int(), C.c_int64()
@@ -426,3 +445,68 @@ class LinearGLLOpt:
         if getattr(self, "handle", None) and getattr(capi, "lib", None) is not None:
             capi.lib.wfx_wave_destroy(self.handle)
             self.handle = None
+
+
+class LinearGLLEnsemble(LinearGLLOpt):
+    """nv wave models (1 <= nv <= 8) on one mesh with one speed of sound, stepped together: member m is
+    LinearGLLOpt(mesh, meshtags, degree, c0, f0s[m], p0s[m]).  One rank.  The stiffness apply of a stage
+    reads the geometric factors once for all members.  States are (ndofs, nv) arrays (member-interleaved,
+    entry (dof i, member m) at i*nv + m); probe values come as (nrecords, nprobes, nv).  Snapshots are not
+    available for ensembles."""
+
+    def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequencies, pressureAmplitudes,
+                 dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO):
+        self.ctx = ctx or Context.get()
+        self.V = mesh
+        if meshtags is not None:
+            import copy
+            mesh = copy.copy(mesh)
+            mesh.facet_cells, mesh.facet_local, mesh.facet_tags = meshtags
+        f0s = np.ascontiguousarray(sourceFrequencies, dtype=np.float64).reshape(-1)
+        p0s = np.ascontiguousarray(pressureAmplitudes, dtype=np.float64).reshape(-1)
+        if f0s.shape != p0s.shape:
+            raise capi.WfxError("one source frequency and one pressure amplitude per member expected")
+        self.nv = len(f0s)
+        self.k_ = int(degreeOfBasis)
+        self.c0_ = float(speedOfSound)
+        self.freq0s_, self.p0s_ = f0s, p0s
+        self.dtype = np.dtype(dtype)
+        self.geometry = Geometry(mesh, self.k_, dtype, self.ctx)
+        self.mass_op = MassOperator(mesh, self.k_, dtype, self.ctx, self.geometry)
+        self.stiff_op = StiffnessOperator(mesh, self.k_, {"c0": self.c0_}, dtype, self.ctx, self.geometry,
+                                          mode=stiffness_mode, ensemble=True)
+        self.bnd_op = BoundaryOperator(mesh, self.k_, dtype, self.ctx)
+        self.halo = None
+        self.handle = C.c_void_p()
+        capi.call("wfx_wave_create_ensemble", self.ctx.handle, self.stiff_op.handle, self.mass_op.handle,
+                  self.bnd_op.handle, self.nv, int(mesh.size_local), self.c0_, capi.f64p(f0s), capi.f64p(p0s),
+                  C.byref(self.handle))
+        self.ndofs = int(mesh.ndofs)
+
+    def _state(self, a):
+        a = np.ascontiguousarray(a, dtype=self.dtype)
+        if a.shape != (self.ndofs, self.nv):
+            raise capi.WfxError(f"ensemble state must have shape ({self.ndofs}, {self.nv})")
+        return a
+
+    def set_state(self, u, v):
+        u, v = self._state(u), self._state(v)
+        capi.call("wfx_wave_set_state", self.handle, C.c_void_p(u.ctypes.data), C.c_void_p(v.ctypes.data))
+
+    def get_state(self):
+        u = np.empty((self.ndofs, self.nv), dtype=self.dtype)
+        v = np.empty((self.ndofs, self.nv), dtype=self.dtype)
+        capi.call("wfx_wave_get_state", self.handle, C.c_void_p(u.ctypes.data), C.c_void_p(v.ctypes.data))
+        return u, v
+
+    def probe_series(self):
+        """(t [nrec], u [nrec, nprobes, nv]) recorded so far."""
+        n = C.c_int64()
+        capi.call("wfx_wave_get_probe_series", self.handle, C.byref(n), None, None)
+        t = np.empty(n.value)
+        vals = np.empty((n.value, getattr(self, "_nprobes", 0), self.nv), dtype=self.dtype)
+        capi.call("wfx_wave_get_probe_series", self.handle, C.byref(n), capi.f64p(t), C.c_void_p(vals.ctypes.data))
+        return t, vals
+
+    def set_snapshot(self, every, fn):
+        capi.call("wfx_wave_set_snapshot", self.handle, int(every), None, None)
