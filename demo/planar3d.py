@@ -4,10 +4,12 @@
 Same physical set-up and control flow as the reference driver: speed of sound 1500 m/s, source
 0.5 MHz, amplitude 60 kPa, domain length 0.1 m, degree 4, CFL time step snapped to whole steps
 per period, final time L/c0 + 8/f0, LinearGLLOpt.init() then .rk4(t0, tf, dt), "Solve time".
+--model lossy / westervelt runs the lossy or Westervelt model instead (DESIGN.md section 4.5a) with water-like
+defaults: diffusivity of sound 4.33e-6 m^2/s, coefficient of nonlinearity 3.5, density 1000 kg/m^3.
 The reference reads `../mesh.xdmf` (not in its repository); here the mesh is a structured
 n x m x m hexahedral box with tag 1 on x = 0 (source) and tag 2 on x = L (absorbing).
 
-    python demo/planar3d.py [--nx 32] [--nyz 4] [--steps N] [--check]
+    python demo/planar3d.py [--nx 32] [--nyz 4] [--steps N] [--check] [--model linear|lossy|westervelt]
 """
 import argparse
 import os
@@ -26,6 +28,10 @@ def main():
     ap.add_argument("--nyz", type=int, default=4, help="cells across")
     ap.add_argument("--steps", type=int, default=0, help="stop after this many steps (0: run to the final time)")
     ap.add_argument("--check", action="store_true", help="compare with the CPU oracle (small meshes)")
+    ap.add_argument("--model", choices=("linear", "lossy", "westervelt"), default="linear")
+    ap.add_argument("--delta", type=float, default=4.33e-6, help="diffusivity of sound [m^2/s] (lossy, westervelt)")
+    ap.add_argument("--beta", type=float, default=3.5, help="coefficient of nonlinearity (westervelt)")
+    ap.add_argument("--rho0", type=float, default=1000.0, help="density [kg/m^3] (westervelt)")
     args = ap.parse_args()
 
     speedOfSound, sourceFrequency, pressureAmplitude = 1500.0, 0.5e6, 60000.0   # main.cpp:25-30
@@ -40,7 +46,13 @@ def main():
     print(f"Number of step per period: {int(round(period / timeStepSize))}")
     print(f"dt = {timeStepSize:.15g}")
     nstep = int((finalTime - startTime) / timeStepSize + 1)
-    eqn = wfx.LinearGLLOpt(mesh, None, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude)  # :75
+    delta = 0.0 if args.model == "linear" else args.delta
+    beta = args.beta if args.model == "westervelt" else 0.0
+    if args.model == "linear":
+        eqn = wfx.LinearGLLOpt(mesh, None, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude)  # :75
+    else:
+        eqn = wfx.WesterveltGLLOpt(mesh, None, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
+                                   delta, beta, args.rho0)
     print(f"Number of steps: {nstep}")
     print(f"Degrees of freedom: {mesh.ndofs_global}")
     eqn.init()                                                                   # :83
@@ -59,9 +71,16 @@ def main():
         oracle.mass_apply(mesh, degreeOfBasis, detJ, np.ones(mesh.ndofs), m)
         m1, m2 = oracle.boundary_facet_mass(mesh, degreeOfBasis)
         uo, vo = np.zeros(mesh.ndofs), np.zeros(mesh.ndofs)
-        oracle.rk4(mesh, degreeOfBasis, G, m, m1, m2, speedOfSound, sourceFrequency, pressureAmplitude,
-                   startTime, finalTime, timeStepSize, uo, vo, max_steps=args.steps, sumfact=True,
-                   nthreads=oracle.max_threads())
+        if args.model == "linear":
+            oracle.rk4(mesh, degreeOfBasis, G, m, m1, m2, speedOfSound, sourceFrequency, pressureAmplitude,
+                       startTime, finalTime, timeStepSize, uo, vo, max_steps=args.steps, sumfact=True,
+                       nthreads=oracle.max_threads())
+        else:
+            from model_oracle import model_oracle
+            model_oracle.rk4_westervelt(mesh, degreeOfBasis, G, m, m1, m2, speedOfSound, sourceFrequency,
+                                        pressureAmplitude, delta, beta, args.rho0, startTime, finalTime,
+                                        timeStepSize, uo, vo, max_steps=args.steps, sumfact=True,
+                                        nthreads=oracle.max_threads())
         print(f"relative L2 difference to the CPU oracle: u {np.linalg.norm(u - uo) / np.linalg.norm(uo):.3e}"
               f"  v {np.linalg.norm(v - vo) / np.linalg.norm(vo):.3e}")
 

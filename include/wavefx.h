@@ -319,6 +319,21 @@ int wfx_wave_create(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass, wfx_boun
 int wfx_wave_create_ensemble(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass, wfx_boundary* bnd, int nv,
                              int64_t size_local, double c0, const double* f0_host, const double* p0_host,
                              wfx_wave** wave);
+/* Lossy (beta == 0) and Westervelt (beta > 0) models on one rank (DESIGN.md section 4.5a).  Pressure p:
+ *   (1 - kappa p) p_tt - c0^2 lap p - delta lap p_t = kappa p_t^2,   kappa = 2 beta / (rho0 c0^2)
+ *   dp/dn = g(t) on tag 1 (g as in wfx_wave_create), dp/dn = -p_t / c0 on tag 2.
+ * Lumped GLL system per dof i, with s = delta / c0^2 and q = (delta / c0) m2:
+ *   (m_i (1 - kappa p_i) + q_i) p_tt,i = [-c0^2 K (p + s p_t)]_i + kappa m_i p_t,i^2
+ *                                        + (c0^2 g + delta g') m1_i - c0 m2_i p_t,i
+ * (the stiffness term uses the operator's own c0: -delta K p_t exactly).  delta = beta = 0 is
+ * wfx_wave_create's model, bit for bit.  With wfx_geometry_scale_cells the per-cell coefficient multiplies
+ * the delta term too: delta_eff(x) = delta coeff(x).
+ * delta >= 0 [m^2/s], beta >= 0, rho0 > 0 [kg/m^3] when beta > 0, f0 > 0, all finite; the stiffness operator
+ * must have no rank-shared dofs.  init / set_state / get_state / state_ptrs / f0 / f1 / rk4 / probes /
+ * snapshots / destroy accept the model (single-field vectors). */
+int wfx_wave_create_westervelt(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass, wfx_boundary* bnd,
+                               int64_t size_local, double c0, double f0, double p0, double delta, double beta,
+                               double rho0, wfx_wave** wave);
 int wfx_wave_init(wfx_wave* wave);                                   /* :131-134 */
 /* Copies the state to the device; on a distributed mesh the ghost entries are then overwritten by
  * their owners' values (u->scatter_fwd(), v->scatter_fwd(), :164,167). */

@@ -1,0 +1,124 @@
+/*
+ * model_oracle.c -- CPU restatement of the lossy and Westervelt wave models (DESIGN.md section 4.5a).
+ *
+ * TEST INFRASTRUCTURE ONLY, like oracle/wave_oracle.c, which it includes unchanged: the stiffness applies,
+ * the stage loop and the source below are that oracle's, so that with delta = beta = 0 wo_rk4_westervelt
+ * reproduces wo_rk4 bit for bit (tests/test_models.py).  Its linear part is thereby pinned to the oracle,
+ * which is pinned to the reference's own code.  The new terms are written out plainly and independently of
+ * the CUDA path: un is kept explicitly, -c0^2 K un and -c0^2 K vn are two separate applies (not one apply
+ * on un + s vn), kv is the plain quotient of the lumped system, g' is analytic.
+ *
+ * Lumped system per dof i (kappa = 2 beta / (rho0 c0^2), q = (delta / c0) m2):
+ *   (m_i (1 - kappa p_i) + q_i) p_tt,i = [A p]_i + (delta / 1500^2) [A p_t]_i + kappa m_i p_t,i^2
+ *                                        + (c0^2 g + delta g') m1_i - c0 m2_i p_t,i
+ * with A = -1500^2 K the oracle's stiffness (c0 = 1500 hard-coded in skernel, as in the reference), so
+ * that the second term is -delta K p_t.
+ */
+#include "../oracle/wave_oracle.c"
+
+/* g(t) exactly as wo_rk4 forms it (LinearGLL.hpp:155-162) and its analytic derivative
+ *   g'(t) = A (W' cos(w0 t) - W w0 sin(w0 t)),  W' = (f0 pi / 8) sin(f0 pi t / 4) inside the ramp, else 0 */
+void wo_source(double t, double freq0, double p0, double c0, double* g, double* gdot)
+{
+  const double w0 = 2.0 * M_PI * freq0, T = 1.0 / freq0, alpha = 4.0;
+  const int ramp = t < T * alpha;
+  const double window = ramp ? 0.5 * (1.0 - cos(freq0 * M_PI * t / alpha)) : 1.0;
+  const double wdot = ramp ? 0.5 * sin(freq0 * M_PI * t / alpha) * (freq0 * M_PI / alpha) : 0.0;
+  *g = window * p0 * w0 / c0 * cos(w0 * t);
+  *gdot = p0 * w0 / c0 * (wdot * cos(w0 * t) - window * w0 * sin(w0 * t));
+}
+
+static void model_stiffness(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                            const double* x, double* y, int sumfact, int nthreads)
+{
+  if (sumfact) wo_stiffness_apply_sumfact(P, ncells, ndofs, dofmap, G, x, y, nthreads);
+  else wo_stiffness_apply_dense(P, ncells, ndofs, dofmap, G, x, y, nthreads);
+}
+
+/* kv = p_tt of the lumped system at time t for state (un, vn); b, bv: scratch vectors */
+static void model_rhs(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                      const double* m, const double* m1, const double* m2, double c0, double freq0, double p0,
+                      double delta, double beta, double rho0, double t, const double* un, const double* vn,
+                      double* kv, double* b, double* bv, int sumfact, int nthreads)
+{
+  const size_t nb = sizeof(double) * ndofs;
+  const double kappa = beta > 0 ? 2.0 * beta / (rho0 * c0 * c0) : 0.0;
+  const double s = delta / (1500.0 * 1500.0);
+  double g, gdot;
+  wo_source(t, freq0, p0, c0, &g, &gdot);
+  memset(b, 0, nb);
+  memset(bv, 0, nb);
+  model_stiffness(P, ncells, ndofs, dofmap, G, un, b, sumfact, nthreads);  /* A un */
+  model_stiffness(P, ncells, ndofs, dofmap, G, vn, bv, sumfact, nthreads); /* A vn */
+  for (int64_t k = 0; k < ndofs; ++k)
+  {
+    double r = b[k] + s * bv[k];
+    r += (c0 * c0 * g + delta * gdot) * m1[k] - c0 * m2[k] * vn[k];
+    r += kappa * m[k] * vn[k] * vn[k];
+    kv[k] = r / (m[k] * (1.0 - kappa * un[k]) + delta / c0 * m2[k]);
+  }
+}
+
+/* dv/dt = f1(t, u, v) of the lossy / Westervelt model */
+void wo_f1_westervelt(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                      const double* m, const double* m1, const double* m2, double c0, double freq0, double p0,
+                      double delta, double beta, double rho0, double t, const double* u, const double* v,
+                      double* out, int sumfact, int nthreads)
+{
+  const size_t nb = sizeof(double) * ndofs;
+  double *b = malloc(nb), *bv = malloc(nb);
+  model_rhs(P, ncells, ndofs, dofmap, G, m, m1, m2, c0, freq0, p0, delta, beta, rho0, t, u, v, out, b, bv,
+            sumfact, nthreads);
+  free(b);
+  free(bv);
+}
+
+/* rk4 of the lossy / Westervelt model: wo_rk4's stage loop (LinearGLL.hpp:241-270) with model_rhs as f1.
+ * u_n, v_n: in = initial state, out = final state.  Returns the number of steps; *t_end the final time. */
+int64_t wo_rk4_westervelt(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                          const double* m, const double* m1, const double* m2, double c0, double freq0, double p0,
+                          double delta, double beta, double rho0, double t0, double tf, double dt,
+                          int64_t max_steps, double* u_n, double* v_n, int sumfact, int nthreads, double* t_end)
+{
+  const double a_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  const double b_runge[4] = {1.0 / 6.0, 1.0 / 3.0, 1.0 / 3.0, 1.0 / 6.0};
+  const double c_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  const size_t nb = sizeof(double) * ndofs;
+  double *u_ = malloc(nb), *v_ = malloc(nb), *un = malloc(nb), *vn = malloc(nb);
+  double *u0 = malloc(nb), *v0 = malloc(nb), *ku = malloc(nb), *kv = malloc(nb), *b = malloc(nb), *bv = malloc(nb);
+  memcpy(u_, u_n, nb);
+  memcpy(v_, v_n, nb);
+  memcpy(ku, u_, nb);
+  memcpy(kv, v_, nb);
+  double t = t0;
+  int64_t step = 0;
+  while (t < tf)
+  {
+    if (max_steps > 0 && step >= max_steps) break;
+    dt = dt < tf - t ? dt : tf - t;
+    memcpy(u0, u_, nb);
+    memcpy(v0, v_, nb);
+    for (int i = 0; i < 4; ++i)
+    {
+      memcpy(un, u0, nb);
+      memcpy(vn, v0, nb);
+      const double adt = dt * a_runge[i];
+      for (int64_t k = 0; k < ndofs; ++k) un[k] = ku[k] * adt + un[k];
+      for (int64_t k = 0; k < ndofs; ++k) vn[k] = kv[k] * adt + vn[k];
+      const double tn = t + c_runge[i] * dt;
+      memcpy(ku, vn, nb);
+      model_rhs(P, ncells, ndofs, dofmap, G, m, m1, m2, c0, freq0, p0, delta, beta, rho0, tn, un, vn, kv, b, bv,
+                sumfact, nthreads);
+      const double bdt = dt * b_runge[i];
+      for (int64_t k = 0; k < ndofs; ++k) u_[k] = ku[k] * bdt + u_[k];
+      for (int64_t k = 0; k < ndofs; ++k) v_[k] = kv[k] * bdt + v_[k];
+    }
+    t += dt;
+    step += 1;
+  }
+  memcpy(u_n, u_, nb);
+  memcpy(v_n, v_, nb);
+  if (t_end) *t_end = t;
+  free(u_); free(v_); free(un); free(vn); free(u0); free(v0); free(ku); free(kv); free(b); free(bv);
+  return step;
+}

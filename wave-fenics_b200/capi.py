@@ -107,6 +107,8 @@ _SIG = {
     "wfx_halo_destroy": [_vp],
     "wfx_wave_create": [_vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_double, C.c_double, C.c_double, _vpp],
     "wfx_wave_create_ensemble": [_vp, _vp, _vp, _vp, C.c_int, C.c_int64, C.c_double, _c_f64p, _c_f64p, _vpp],
+    "wfx_wave_create_westervelt": [_vp, _vp, _vp, _vp, C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double,
+                                   C.c_double, C.c_double, _vpp],
     "wfx_wave_init": [_vp],
     "wfx_wave_set_state": [_vp, _vp, _vp],
     "wfx_wave_get_state": [_vp, _vp, _vp],

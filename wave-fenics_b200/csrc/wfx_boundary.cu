@@ -59,7 +59,39 @@ __global__ void boundary_ens_kernel(int64_t nb, int nv, const int32_t* __restric
   const int64_t i = (int64_t)idx[p] * nv + m;
   b[i] = (T)((double)b[i] + c02g * m1[p] - c0 * m2[p] * (double)vn[i]);
 }
+
+// Lossy / Westervelt models: the Gamma2 mass term q = qc m2 on the absorbing dofs only, so that the dense
+// stage update needs nothing beyond 1/m (see boundary_absorbing_mass in wfx_internal.h).  p is formed in T
+// exactly as the stage kernel forms it.
+template <typename T>
+__global__ void absorbing_mass_kernel(int64_t nb, const int32_t* __restrict__ idx, const double* __restrict__ m2,
+                                      const double* __restrict__ m, double qc, double kappa, T s,
+                                      const T* __restrict__ pw, const T* __restrict__ pd, T* __restrict__ b)
+{
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t >= nb || m2[t] == 0.0) return;
+  const int32_t i = idx[t];
+  const T pdt = pd[i];
+  const double p = (double)(pw[i] - s * pdt);
+  const double mi = m[i], a = 1.0 - kappa * p, kp2 = kappa * (double)pdt * (double)pdt;
+  const double kv = ((double)b[i] + mi * kp2) / (mi * a + qc * m2[t]);
+  b[i] = (T)(mi * (kv * a - kp2));
+}
 } // namespace
+
+void wfx::boundary_absorbing_mass(wfx_boundary* op, const double* m64, double qc, double kappa, double s,
+                                  const void* pw, const void* pd, void* b, cudaStream_t stream)
+{
+  if (!op || op->nb == 0) return;
+  const unsigned grid = (unsigned)((op->nb + 255) / 256);
+  if (op->dtype == WFX_F64)
+    absorbing_mass_kernel<double><<<grid, 256, 0, stream>>>(op->nb, op->d_idx.p, op->d_m2.p, m64, qc, kappa, s,
+                                                             (const double*)pw, (const double*)pd, (double*)b);
+  else
+    absorbing_mass_kernel<float><<<grid, 256, 0, stream>>>(op->nb, op->d_idx.p, op->d_m2.p, m64, qc, kappa, (float)s,
+                                                            (const float*)pw, (const float*)pd, (float*)b);
+  WFX_CUDA(cudaGetLastError());
+}
 
 void wfx::boundary_apply_ens(wfx_boundary* op, int nv, double c0, const double* g_host, const double* g_dev,
                              const void* vn, void* b, cudaStream_t stream)

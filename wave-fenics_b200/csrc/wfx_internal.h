@@ -118,6 +118,15 @@ void boundary_apply_dev(struct ::wfx_boundary* op, double c0, const double* g_de
 bool stiffness_has_ensemble(const struct ::wfx_stiffness* op);
 void boundary_apply_ens(struct ::wfx_boundary* op, int nv, double c0, const double* g_host, const double* g_dev,
                         const void* vn, void* b, cudaStream_t stream);
+// lossy / Westervelt models (wfx_wave_create_westervelt)
+double stiffness_c0(const struct ::wfx_stiffness* op);       // the c0 of y = -c0^2 K x
+int64_t stiffness_nshared(const struct ::wfx_stiffness* op); // rank-shared dofs (0 on one rank)
+const double* mass_diagonal64(const struct ::wfx_mass* op);   // m on the device, fp64 whatever the dtype
+// On the absorbing (tag 2) dofs: b_i -> m_i [kv_i (1 - kappa p_i) - kappa pd_i^2] with the exact
+// kv_i = (b_i + kappa m_i pd_i^2) / (m_i (1 - kappa p_i) + qc m2_i), so that the dense stage update
+// kv = (b minv + kappa pd^2) / (1 - kappa p) yields it; p = pw - s pd (s = 0: pw is p itself)
+void boundary_absorbing_mass(struct ::wfx_boundary* op, const double* m64, double qc, double kappa, double s,
+                             const void* pw, const void* pd, void* b, cudaStream_t stream);
 
 // NVTX ranges around the phases of a time step (the reference marks its profiled regions the same
 // way: demo/gpu_scatter_mpi/main.cpp:101-121, demo/gpu_cg/CUDA/cg.hpp:74-113).  nvtx3 is header-only

@@ -2416,6 +2416,8 @@ bool stiffness_has_split(const wfx_stiffness* op) { return op->part_split > 0; }
 // the single-launch form passes a per-apply epoch as a kernel argument: not replayable from a graph
 bool stiffness_graph_safe(const wfx_stiffness* op) { return !op->persistent; }
 bool stiffness_has_ensemble(const wfx_stiffness* op) { return op->ens; }
+double stiffness_c0(const wfx_stiffness* op) { return op->c0; }
+int64_t stiffness_nshared(const wfx_stiffness* op) { return op->nshared; }
 
 // tensor-ordered dofmap in the kernels' k-major point order
 void build_tensor_dofmap(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap,

@@ -30,6 +30,13 @@ struct wfx_wave
   bool ens = false;
   int nv = 1;
   std::vector<double> f0s, p0s;
+  // lossy (model 1) and Westervelt (model 2) models (wfx_wave_create_westervelt).  The stiffness input
+  // w = u + s_stiff v lives in `un` (nothing else reads un in these models); the source passed to the
+  // boundary term is g + s_src g'; q = qc m2 is the Gamma2 mass term; f1 builds its w in f1_w.
+  int model = 0;
+  double kappa = 0, s_stiff = 0, s_src = 0, qc = 0;
+  const double* m64 = nullptr;
+  DevBuf<unsigned char> f1_w;
   const void* minv = nullptr;
   // u_, v_: solution; u0, v0: start of step; un, vn: stage state; b: right-hand side
   DevBuf<unsigned char> u_, v_, u0, v0, un, vn, b;
@@ -204,6 +211,111 @@ void launch_stage_ens(int stage, int64_t n, int nv, const void* b, const void* m
   WFX_CUDA(cudaGetLastError());
 }
 
+// Stage update of the lossy (NL = false) and Westervelt (NL = true) models: rk_stage_kernel, and
+//   kv = b / m                                          (lossy)
+//   kv = (b / m + kappa pd^2) / (1 - kappa p)           (Westervelt; pd = ku = the stage's v)
+//   w' = un' + s vn'  written where rk_stage_kernel writes un'; STAGE 3 writes w = u_ + s v_ for the next step.
+// p is u_ at stage 0; at stages 1-3 it is rebuilt as w - s vn (one read of w, no un vector).
+// On the absorbing dofs b has been replaced beforehand (boundary_absorbing_mass) so that this
+// quotient is the exact kv of the lumped system with the Gamma2 mass term.
+template <typename T, int STAGE, bool NL>
+__global__ void __launch_bounds__(256)
+rk_stage_westervelt_kernel(int64_t n, const T* __restrict__ b, const T* __restrict__ minv, T* __restrict__ u_,
+                           T* __restrict__ v_, T* __restrict__ u0, T* __restrict__ v0, T* __restrict__ w,
+                           T* __restrict__ vn, T bdt, T adt_next, T s, T kappa)
+{
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  T kv = b[k] * minv[k];
+  T us = u_[k], vs = v_[k];
+  T ku, ub, vb, p;
+  if (STAGE == 0)
+  {
+    ku = vs;
+    ub = us;
+    vb = vs;
+    p = us;
+    u0[k] = ub;
+    v0[k] = vb;
+  }
+  else
+  {
+    ku = vn[k];
+    if (NL) p = w[k] - s * ku;
+    if (STAGE < 3)
+    {
+      ub = u0[k];
+      vb = v0[k];
+    }
+  }
+  if (NL) kv = (kv + kappa * ku * ku) / (T(1) - kappa * p);
+  const T un_ = ku * bdt + us, vn_ = kv * bdt + vs;
+  u_[k] = un_;
+  v_[k] = vn_;
+  if (STAGE < 3)
+  {
+    const T ui = ku * adt_next + ub, vi = kv * adt_next + vb;
+    w[k] = ui + s * vi;
+    vn[k] = vi;
+  }
+  else w[k] = un_ + s * vn_;
+}
+
+template <typename T>
+void launch_stage_westervelt(int stage, bool nl, int64_t n, const void* b, const void* minv, void* u_, void* v_,
+                             void* u0, void* v0, void* w, void* vn, double bdt, double adt_next, double s,
+                             double kappa, cudaStream_t st)
+{
+  const unsigned grid = (unsigned)((n + 255) / 256);
+#define WFX_STAGE(S, NL)                                                                                    \
+  rk_stage_westervelt_kernel<T, S, NL><<<grid, 256, 0, st>>>(n, (const T*)b, (const T*)minv, (T*)u_, (T*)v_, \
+                                                              (T*)u0, (T*)v0, (T*)w, (T*)vn, (T)bdt,          \
+                                                              (T)adt_next, (T)s, (T)kappa)
+  switch (stage * 2 + (nl ? 1 : 0))
+  {
+  case 0: WFX_STAGE(0, false); break;
+  case 1: WFX_STAGE(0, true); break;
+  case 2: WFX_STAGE(1, false); break;
+  case 3: WFX_STAGE(1, true); break;
+  case 4: WFX_STAGE(2, false); break;
+  case 5: WFX_STAGE(2, true); break;
+  case 6: WFX_STAGE(3, false); break;
+  default: WFX_STAGE(3, true); break;
+  }
+#undef WFX_STAGE
+  WFX_CUDA(cudaGetLastError());
+}
+
+// w = u + s v: the stiffness input of the lossy / Westervelt models
+template <typename T>
+__global__ void axpy_kernel(int64_t n, const T* __restrict__ u, const T* __restrict__ v, T s, T* __restrict__ w)
+{
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k < n) w[k] = u[k] + s * v[k];
+}
+
+// f1 of the lossy / Westervelt models: out = (b / m + kappa v^2) / (1 - kappa u), the stage kernel's kv
+template <typename T>
+__global__ void westervelt_rhs_kernel(int64_t n, const T* __restrict__ b, const T* __restrict__ minv,
+                                      const T* __restrict__ u, const T* __restrict__ v, T kappa, T* __restrict__ out)
+{
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const T vk = v[k];
+  out[k] = (b[k] * minv[k] + kappa * vk * vk) / (T(1) - kappa * u[k]);
+}
+
+void launch_axpy(const wfx_wave* w, const void* u, const void* v, double s, void* out, cudaStream_t st)
+{
+  if (w->n == 0) return;
+  const unsigned grid = (unsigned)((w->n + 255) / 256);
+  if (w->dtype == WFX_F64)
+    axpy_kernel<double><<<grid, 256, 0, st>>>(w->n, (const double*)u, (const double*)v, s, (double*)out);
+  else
+    axpy_kernel<float><<<grid, 256, 0, st>>>(w->n, (const float*)u, (const float*)v, (float)s, (float*)out);
+  WFX_CUDA(cudaGetLastError());
+}
+
 // result[i,m] = b[i,m] * minv[i]: the b/m of f1 for an ensemble
 template <typename T>
 __global__ void scale_rows_kernel(int64_t n, int nv, const T* __restrict__ b, const T* __restrict__ minv,
@@ -308,8 +420,9 @@ void enqueue_step(wfx_wave* w, double dt, const double* g, bool g_from_dev, cuda
   for (int i = 0; i < 4; ++i)
   {
     NvtxRange stage_range(stage_name[i]);
-    // stage state: the solution itself at stage 0 (a_0 = 0), else un/vn
-    const void* un = i == 0 ? w->u_.p : w->un.p;
+    // stage state: the solution itself at stage 0 (a_0 = 0), else un/vn.  Lossy / Westervelt models:
+    // the stiffness input is w = un + s vn, kept in `un` at every stage
+    const void* un = i == 0 && !w->model ? w->u_.p : w->un.p;
     const void* vn = i == 0 ? w->v_.p : w->vn.p;
     // f1 (:151-192)
     if (!w->halo)
@@ -347,6 +460,21 @@ void enqueue_step(wfx_wave* w, double dt, const double* g, bool g_from_dev, cuda
       }
       WFX_CUDA(cudaStreamWaitEvent(st, w->ev_halo, 0));
       boundary(i, vn);
+    }
+    if (w->model)
+    {
+      // Gamma2 mass term (compact, absorbing dofs), then the fused update; p = u_ at stage 0, else w - s vn
+      if (w->qc != 0)
+        boundary_absorbing_mass(w->bnd, w->m64, w->qc, w->kappa, i == 0 ? 0.0 : w->s_stiff,
+                                i == 0 ? w->u_.p : w->un.p, vn, w->b.p, st);
+      NvtxRange update_range("wfx fused stage update");
+      if (w->dtype == WFX_F64)
+        launch_stage_westervelt<double>(i, w->model == 2, w->n, w->b.p, w->minv, w->u_.p, w->v_.p, w->u0.p, w->v0.p,
+                                        w->un.p, w->vn.p, dt * b_runge[i], dt * a_runge[i + 1], w->s_stiff, w->kappa, st);
+      else
+        launch_stage_westervelt<float>(i, w->model == 2, w->n, w->b.p, w->minv, w->u_.p, w->v_.p, w->u0.p, w->v0.p,
+                                       w->un.p, w->vn.p, dt * b_runge[i], dt * a_runge[i + 1], w->s_stiff, w->kappa, st);
+      continue;
     }
     NvtxRange update_range("wfx fused stage update");
     if (w->ens && w->dtype == WFX_F64)
@@ -463,6 +591,35 @@ extern "C" int wfx_wave_create_ensemble(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_
   WFX_API_END
 }
 
+extern "C" int wfx_wave_create_westervelt(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass, wfx_boundary* bnd,
+                                          int64_t size_local, double c0, double f0, double p0, double delta,
+                                          double beta, double rho0, wfx_wave** out)
+{
+  WFX_API_BEGIN
+  if (!ctx || !stiff || !mass || !out) fail("NULL argument");
+  for (double x : {c0, f0, p0, delta, beta, rho0})
+    if (!std::isfinite(x)) fail("wave westervelt: non-finite parameter");
+  if (!(c0 > 0)) fail("wave westervelt: speed of sound must be positive");
+  if (!(f0 > 0)) fail("wave westervelt: source frequency must be positive");
+  if (delta < 0) fail("wave westervelt: diffusivity of sound delta must not be negative");
+  if (beta < 0) fail("wave westervelt: coefficient of nonlinearity beta must not be negative");
+  if (beta > 0 && !(rho0 > 0)) fail("wave westervelt: density rho0 must be positive when beta > 0");
+  if (stiffness_nshared(stiff) > 0) fail("wave westervelt: one rank only (the stiffness operator has rank-shared dofs)");
+  wfx_wave* w = nullptr;
+  if (wfx_wave_create(ctx, stiff, mass, bnd, nullptr, size_local, c0, f0, p0, &w)) fail("%s", wfx_last_error());
+  std::unique_ptr<wfx_wave> guard(w);
+  w->model = beta > 0 ? 2 : 1;
+  w->kappa = beta > 0 ? 2.0 * beta / (rho0 * c0 * c0) : 0.0;
+  // -delta K v = (delta / cK^2) (-cK^2 K v) with cK the operator's c0; c0^2 (g + s_src g') = c0^2 g + delta g'
+  const double cK = stiffness_c0(stiff);
+  w->s_stiff = delta / (cK * cK);
+  w->s_src = delta / (c0 * c0);
+  w->qc = bnd ? delta / c0 : 0.0;
+  w->m64 = mass_diagonal64(mass);
+  *out = guard.release();
+  WFX_API_END
+}
+
 extern "C" int wfx_wave_init(wfx_wave* w)
 {
   WFX_API_BEGIN
@@ -530,7 +687,21 @@ double source_amplitude(double f0, double p0, double c0, double tn)
   const double window = tn < T * alpha ? 0.5 * (1.0 - std::cos(f0 * M_PI * tn / alpha)) : 1.0;
   return window * p0 * w0 / c0 * std::cos(w0 * tn);
 }
-double source_amplitude(const wfx_wave* w, double tn) { return source_amplitude(w->f0, w->p0, w->c0, tn); }
+// its time derivative g'(t) = A (W' cos(w0 t) - W w0 sin(w0 t)), A = p0 w0 / c0
+double source_rate(double f0, double p0, double c0, double tn)
+{
+  const double w0 = 2.0 * M_PI * f0, T = 1.0 / f0, alpha = 4.0;
+  const bool ramp = tn < T * alpha;
+  const double window = ramp ? 0.5 * (1.0 - std::cos(f0 * M_PI * tn / alpha)) : 1.0;
+  const double rate = ramp ? f0 * M_PI / (2.0 * alpha) * std::sin(f0 * M_PI * tn / alpha) : 0.0;
+  return p0 * w0 / c0 * (rate * std::cos(w0 * tn) - window * w0 * std::sin(w0 * tn));
+}
+// the amplitude the boundary term receives: g, or g + (delta / c0^2) g' for the lossy / Westervelt models
+double source_amplitude(const wfx_wave* w, double tn)
+{
+  const double g = source_amplitude(w->f0, w->p0, w->c0, tn);
+  return w->model ? g + w->s_src * source_rate(w->f0, w->p0, w->c0, tn) : g;
+}
 // g_m(t) of every member (ensemble models): g[m], m < nv
 void source_amplitudes(const wfx_wave* w, double tn, double* g)
 {
@@ -574,6 +745,26 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
     return 0;
   }
   const double g = source_amplitude(w, t);
+  if (w->model)
+  {
+    // w = u + s v in a scratch vector of its own (the rk4 one carries the state of the next step)
+    const size_t nb = (size_t)w->n * (w->dtype == WFX_F64 ? 8 : 4);
+    if (w->f1_w.n != nb) w->f1_w.alloc(nb);
+    launch_axpy(w, u, v, w->s_stiff, w->f1_w.p, st);
+    if (wfx_stiffness_apply(w->stiff, w->f1_w.p, w->b.p, 0, st)) fail("%s", wfx_last_error());
+    if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());
+    if (w->qc != 0) boundary_absorbing_mass(w->bnd, w->m64, w->qc, w->kappa, 0.0, u, v, w->b.p, st);
+    if (w->n == 0) return 0;
+    const unsigned grid = (unsigned)((w->n + 255) / 256);
+    if (w->dtype == WFX_F64)
+      westervelt_rhs_kernel<double><<<grid, 256, 0, st>>>(w->n, (const double*)w->b.p, (const double*)w->minv,
+                                                           (const double*)u, (const double*)v, w->kappa, (double*)result);
+    else
+      westervelt_rhs_kernel<float><<<grid, 256, 0, st>>>(w->n, (const float*)w->b.p, (const float*)w->minv,
+                                                          (const float*)u, (const float*)v, (float)w->kappa, (float*)result);
+    WFX_CUDA(cudaGetLastError());
+    return 0;
+  }
   if (wfx_stiffness_apply(w->stiff, u, w->b.p, 0, st)) fail("%s", wfx_last_error());                     // :173-174
   if (w->halo && wfx_halo_update_rev_fwd(w->halo, w->b.p, st)) fail("%s", wfx_last_error());             // :176
   if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());       // :175
@@ -600,6 +791,10 @@ extern "C" int wfx_wave_rk4(wfx_wave* w, double t0, double tf, double dt, int64_
     WFX_CUDA(cudaEventRecord(w->ev_in, st));
     WFX_CUDA(cudaStreamWaitEvent(ws, w->ev_in, 0));
   }
+  // lossy / Westervelt models: the stiffness input w = u_ + s v_ of the first stage, rebuilt on every call so
+  // that it follows init, set_state, a restart or writes through wfx_wave_state_ptrs (later steps get it
+  // from stage 3 of the step before)
+  if (w->model) launch_axpy(w, w->u_.p, w->v_.p, w->s_stiff, w->un.p, ws);
   double t = t0;
   int64_t step = 0;
   const double dt_nominal = dt;

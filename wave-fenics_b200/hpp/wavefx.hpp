@@ -399,6 +399,22 @@ public:
   std::shared_ptr<MassOperator<double>> mass_op;
   std::shared_ptr<StiffnessOperator<double>> stiff_op;
 
+protected:
+  // the lossy / Westervelt models (wfx_wave_create_westervelt, one rank): see WesterveltGLLOpt
+  LinearGLLOpt(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
+               double sourceFrequency, double pressureAmplitude, double delta, double beta, double rho0)
+      : _ctx(std::move(ctx)), _ndofs(V.ndofs)
+  {
+    _geom = std::make_shared<Geometry<double>>(_ctx, V);
+    mass_op = std::make_shared<MassOperator<double>>(_geom, V, degreeOfBasis);
+    std::map<std::string, double> params{{"c0", speedOfSound}};
+    stiff_op = std::make_shared<StiffnessOperator<double>>(_geom, V, degreeOfBasis, params);
+    check(wfx_boundary_create(_ctx->get(), V.degree, WFX_F64, V.nfacets, V.facet_cell, V.facet_local,
+                              V.facet_tag, V.npoints, V.x, V.xdofs, V.ndofs, V.dofmap, &_bnd));
+    check(wfx_wave_create_westervelt(_ctx->get(), stiff_op->get(), mass_op->get(), _bnd, V.size_local, speedOfSound,
+                                     sourceFrequency, pressureAmplitude, delta, beta, rho0, &_wave));
+  }
+
 private:
   static void snapshot_trampoline(void* self, std::int64_t step, double t, const void* u, const void* v)
   {
@@ -414,6 +430,32 @@ private:
   wfx_boundary* _bnd = nullptr;
   wfx_wave* _wave = nullptr;
 };
+// The Westervelt model, one rank, fp64, with the interface of LinearGLLOpt (wavefx.h, DESIGN.md section 4.5a):
+//   (1 - kappa p) p_tt - c0^2 lap p - delta lap p_t = kappa p_t^2,  kappa = 2 beta / (rho0 c0^2),
+// dp/dn = g(t) on tag 1, dp/dn = -p_t / c0 on tag 2.  delta [m^2/s] >= 0, beta >= 0, rho0 > 0 when beta > 0.
+class WesterveltGLLOpt : public LinearGLLOpt
+{
+public:
+  WesterveltGLLOpt(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
+                   double sourceFrequency, double pressureAmplitude, double diffusivityOfSound,
+                   double coefficientOfNonlinearity, double density)
+      : LinearGLLOpt(std::move(ctx), V, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
+                     diffusivityOfSound, coefficientOfNonlinearity, density)
+  {
+  }
+};
+// The lossy model: WesterveltGLLOpt with beta = 0,  p_tt - c0^2 lap p - delta lap p_t = 0
+class LossyGLLOpt : public WesterveltGLLOpt
+{
+public:
+  LossyGLLOpt(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
+              double sourceFrequency, double pressureAmplitude, double diffusivityOfSound)
+      : WesterveltGLLOpt(std::move(ctx), V, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
+                         diffusivityOfSound, 0.0, 1.0)
+  {
+  }
+};
+
 // nv wave models on one mesh (1 <= nv <= WFX_ENSEMBLE_MAX), one rank, fp64: member m is
 // LinearGLLOpt(V, degree, c0, f0[m], p0[m]); the stiffness apply of a stage reads G once for all members.
 // States are member-interleaved [ndofs][nv] (entry (dof i, member m) at i*nv + m), probe values

@@ -8,6 +8,8 @@ Same names, argument meaning and call shape as the reference classes:
                                                 common/LinearGLL.hpp:37-287
   LinearGLLEnsemble(mesh, meshtags, degree, c0, f0s, p0s)
                                                 nv LinearGLLOpt models on one mesh, stepped together
+  WesterveltGLLOpt(mesh, meshtags, degree, c0, f0, p0, delta, beta, rho0), LossyGLLOpt (beta = 0)
+                                                lossy and nonlinear (Westervelt) models, DESIGN.md 4.5a
 
 `V` is a HexMesh (mesh.py): it carries what the reference pulls out of the DOLFINx
 FunctionSpace (geometry, geometry dofmap, cell dofmap, index-map sizes).  Vectors are
@@ -510,3 +512,49 @@ class LinearGLLEnsemble(LinearGLLOpt):
 
     def set_snapshot(self, every, fn):
         capi.call("wfx_wave_set_snapshot", self.handle, int(every), None, None)
+
+
+class WesterveltGLLOpt(LinearGLLOpt):
+    """The Westervelt model on one rank, with the surface of LinearGLLOpt (DESIGN.md section 4.5a):
+
+        (1 - kappa p) p_tt - c0^2 lap p - delta lap p_t = kappa p_t^2,   kappa = 2 beta / (rho0 c0^2)
+
+    dp/dn = g(t) on tag 1 (the source of LinearGLLOpt), dp/dn = -p_t / c0 on tag 2.  diffusivityOfSound
+    delta [m^2/s] >= 0, coefficientOfNonlinearity beta >= 0, density rho0 [kg/m^3] > 0 when beta > 0.
+    delta = beta = 0 is LinearGLLOpt bit for bit.  A per-cell coefficient set with Geometry.scale_cells
+    multiplies the delta term too (delta_eff = delta * coeff)."""
+
+    def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
+                 diffusivityOfSound, coefficientOfNonlinearity, density, dtype=np.float64, ctx=None,
+                 stiffness_mode=capi.STIFF_AUTO):
+        self.ctx = ctx or Context.get()
+        self.V = mesh
+        if meshtags is not None:
+            import copy
+            mesh = copy.copy(mesh)
+            mesh.facet_cells, mesh.facet_local, mesh.facet_tags = meshtags
+        self.k_ = int(degreeOfBasis)
+        self.c0_, self.freq0_, self.p0_ = float(speedOfSound), float(sourceFrequency), float(pressureAmplitude)
+        self.delta_, self.beta_, self.rho0_ = (float(diffusivityOfSound), float(coefficientOfNonlinearity),
+                                               float(density))
+        self.dtype = np.dtype(dtype)
+        self.geometry = Geometry(mesh, self.k_, dtype, self.ctx)
+        self.mass_op = MassOperator(mesh, self.k_, dtype, self.ctx, self.geometry)
+        self.stiff_op = StiffnessOperator(mesh, self.k_, {"c0": self.c0_}, dtype, self.ctx, self.geometry,
+                                          mode=stiffness_mode)
+        self.bnd_op = BoundaryOperator(mesh, self.k_, dtype, self.ctx)
+        self.halo = None
+        self.handle = C.c_void_p()
+        capi.call("wfx_wave_create_westervelt", self.ctx.handle, self.stiff_op.handle, self.mass_op.handle,
+                  self.bnd_op.handle, int(mesh.size_local), self.c0_, self.freq0_, self.p0_, self.delta_,
+                  self.beta_, self.rho0_, C.byref(self.handle))
+        self.ndofs = int(mesh.ndofs)
+
+
+class LossyGLLOpt(WesterveltGLLOpt):
+    """The lossy wave model (WesterveltGLLOpt with beta = 0):  p_tt - c0^2 lap p - delta lap p_t = 0."""
+
+    def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
+                 diffusivityOfSound, dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO):
+        super().__init__(mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
+                         diffusivityOfSound, 0.0, 1.0, dtype=dtype, ctx=ctx, stiffness_mode=stiffness_mode)
