@@ -6,10 +6,16 @@ Same physical set-up and control flow as the reference driver: speed of sound 15
 per period, final time L/c0 + 8/f0, LinearGLLOpt.init() then .rk4(t0, tf, dt), "Solve time".
 --model lossy / westervelt runs the lossy or Westervelt model instead (DESIGN.md section 4.5a) with water-like
 defaults: diffusivity of sound 4.33e-6 m^2/s, coefficient of nonlinearity 3.5, density 1000 kg/m^3.
+--stats-periods K accumulates field statistics on the device over the last K periods of the run (DESIGN.md
+section 4.5b) and prints, along the x axis, the peak positive and negative pressure and, at the absorbing end, the
+fundamental's amplitude and the second harmonic's share of it.  The harmonics are exact Fourier components only
+over whole periods of whole steps, so the run then stops on the last whole step before the final time (a shortened
+last step would be a sample off the uniform grid) and exactly K * (steps per period) steps are sampled.
 The reference reads `../mesh.xdmf` (not in its repository); here the mesh is a structured
 n x m x m hexahedral box with tag 1 on x = 0 (source) and tag 2 on x = L (absorbing).
 
     python demo/planar3d.py [--nx 32] [--nyz 4] [--steps N] [--check] [--model linear|lossy|westervelt]
+                            [--stats-periods K]
 """
 import argparse
 import os
@@ -22,6 +28,18 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import wave_fenics_b200 as wfx  # noqa: E402
 
 
+def stats_window(t0, tf, dt, k, periods, max_steps=0):
+    """(run_tf, run_steps, t_start) for field statistics over the last `periods` periods of k steps each: the run
+    takes nw whole steps (the last whole step at or before tf, or max_steps) and stops there, and the last
+    periods * k of them are sampled.  t_start - dt/2, the threshold of the sampling rule, lies half a step past
+    the step before the window, so rounding in the accumulated time cannot move the window's edge."""
+    nw = int(np.floor((tf - t0) / dt + 1e-9))
+    if max_steps > 0:
+        nw = min(nw, max_steps)
+    nsamples = min(periods * k, nw)
+    return t0 + (nw + 0.5) * dt, nw, t0 + (nw - nsamples + 1) * dt
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--nx", type=int, default=32, help="cells along the propagation direction")
@@ -32,6 +50,8 @@ def main():
     ap.add_argument("--delta", type=float, default=4.33e-6, help="diffusivity of sound [m^2/s] (lossy, westervelt)")
     ap.add_argument("--beta", type=float, default=3.5, help="coefficient of nonlinearity (westervelt)")
     ap.add_argument("--rho0", type=float, default=1000.0, help="density [kg/m^3] (westervelt)")
+    ap.add_argument("--stats-periods", type=int, default=0,
+                    help="field statistics (peaks, harmonics) over the last K periods of the run (0: off)")
     args = ap.parse_args()
 
     speedOfSound, sourceFrequency, pressureAmplitude = 1500.0, 0.5e6, 60000.0   # main.cpp:25-30
@@ -56,14 +76,35 @@ def main():
     print(f"Number of steps: {nstep}")
     print(f"Degrees of freedom: {mesh.ndofs_global}")
     eqn.init()                                                                   # :83
+    run_tf, run_steps = finalTime, args.steps
+    if args.stats_periods > 0:
+        k = int(round(period / timeStepSize))
+        run_tf, run_steps, t_start = stats_window(startTime, finalTime, timeStepSize, k, args.stats_periods, args.steps)
+        eqn.set_field_stats(t_start, harmonics=2)
     eqn.ctx.synchronize()
     t0 = time.perf_counter()
-    steps, t_end = eqn.rk4(startTime, finalTime, timeStepSize, max_steps=args.steps)  # :88
+    steps, t_end = eqn.rk4(startTime, run_tf, timeStepSize, max_steps=run_steps)  # :88
     eqn.ctx.synchronize()
     print(f"Solve time: {time.perf_counter() - t0:.6f}  ({steps} steps, t = {t_end:.6e})")   # :92
     u, v = eqn.get_state()
     X = wfx.dof_coordinates(mesh)
-    print(f"max |p| = {np.abs(u).max():.6e} at x = {X[np.abs(u).argmax(), 0]:.4f}")
+    if args.stats_periods > 0:
+        fs = eqn.field_stats()
+        # the dofs on the x axis (y = z = 0), from the source to the absorbing end
+        line = np.where((np.abs(X[:, 1]) < 1e-12) & (np.abs(X[:, 2]) < 1e-12))[0]
+        line = line[np.argsort(X[line, 0])]
+        x = X[line, 0]
+        pmax, pmin, p1, p2 = fs.pmax[line], fs.pmin[line], np.abs(fs.harmonics[0, line]), np.abs(fs.harmonics[1, line])
+        whole = fs.samples == args.stats_periods * k
+        print(f"field statistics over {fs.samples} steps ({fs.samples / k:g} periods of {k} steps"
+              f"{'' if whole else ', fewer than asked: the run is shorter than the window'}), "
+              f"t = {fs.t_first:.6e} .. {fs.t_last:.6e}")
+        if fs.samples:
+            print(f"along x: max pmax = {pmax.max():.6e} at x = {x[pmax.argmax()]:.4f}, "
+                  f"min pmin = {pmin.min():.6e} at x = {x[pmin.argmin()]:.4f}")
+            print(f"at the absorbing end (x = {x[-1]:.4f}): |p1| = {p1[-1]:.6e}, |p2|/|p1| = {p2[-1] / p1[-1]:.6e}")
+    else:
+        print(f"max |p| = {np.abs(u).max():.6e} at x = {X[np.abs(u).argmax(), 0]:.4f}")
     if args.check:
         from oracle import oracle
         G, detJ = oracle.precompute_geometric_data(mesh, degreeOfBasis)
@@ -73,13 +114,13 @@ def main():
         uo, vo = np.zeros(mesh.ndofs), np.zeros(mesh.ndofs)
         if args.model == "linear":
             oracle.rk4(mesh, degreeOfBasis, G, m, m1, m2, speedOfSound, sourceFrequency, pressureAmplitude,
-                       startTime, finalTime, timeStepSize, uo, vo, max_steps=args.steps, sumfact=True,
+                       startTime, run_tf, timeStepSize, uo, vo, max_steps=run_steps, sumfact=True,
                        nthreads=oracle.max_threads())
         else:
             from model_oracle import model_oracle
             model_oracle.rk4_westervelt(mesh, degreeOfBasis, G, m, m1, m2, speedOfSound, sourceFrequency,
-                                        pressureAmplitude, delta, beta, args.rho0, startTime, finalTime,
-                                        timeStepSize, uo, vo, max_steps=args.steps, sumfact=True,
+                                        pressureAmplitude, delta, beta, args.rho0, startTime, run_tf,
+                                        timeStepSize, uo, vo, max_steps=run_steps, sumfact=True,
                                         nthreads=oracle.max_threads())
         print(f"relative L2 difference to the CPU oracle: u {np.linalg.norm(u - uo) / np.linalg.norm(uo):.3e}"
               f"  v {np.linalg.norm(v - vo) / np.linalg.norm(vo):.3e}")

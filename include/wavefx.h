@@ -313,7 +313,7 @@ int wfx_wave_create(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass, wfx_boun
  * and c0; member m is the model LinearGLLOpt(..., c0, f0_host[m], p0_host[m]) with its own source
  * g_m(t) = window_m(t) p0_m w_m / c0 cos(w_m t), w_m = 2 pi f0_m, and its own four-period Hann ramp.
  * stiff must have been created with WFX_STIFF_ENSEMBLE.  init, set_state, get_state, state_ptrs, f0, f1,
- * rk4, set_probes, get_probe_series and destroy accept the model; their vectors are then
+ * rk4, set_probes, get_probe_series, set_field_stats, get_field_stats and destroy accept the model; their vectors are then
  * member-interleaved [ndofs][nv] (see wfx_stiffness_apply_ensemble), probe values [nrecords][nprobes][nv].
  * set_snapshot refuses an ensemble model. */
 int wfx_wave_create_ensemble(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass, wfx_boundary* bnd, int nv,
@@ -363,6 +363,30 @@ int wfx_wave_rk4(wfx_wave* wave, double t0, double tf, double dt, int64_t max_st
  * host; either pointer may be NULL.  init / set_state start a new series. */
 int wfx_wave_set_probes(wfx_wave* wave, int64_t nprobes, const int32_t* dofs_host, int64_t max_records);
 int wfx_wave_get_probe_series(wfx_wave* wave, int64_t* nrecords, double* t_host, void* values_host);
+/* Field statistics (DESIGN.md section 4.5b): maps of the pressure u over the steady-state part of a run,
+ * accumulated on the device.  After every completed time step whose reached time t_n satisfies
+ * t_n >= t_start - dt_step / 2 (dt_step: the size of that step), every local entry i (owned and ghost;
+ * every member of an ensemble) is sampled:
+ *   pmax[i] = max_n u_i(t_n), pmin[i] = min_n u_i(t_n)   (model dtype, NaN propagates)
+ *   harm_h[i] = (2 / N) sum_n u_i(t_n) exp(-i h w t_n),   h = 1..nharm, w = 2 pi f0 (member m: f0_host[m]),
+ * accumulated in fp64 for both model dtypes, N the number of sampled steps.  With whole periods in the window
+ * and whole steps per period, Re(harm_h e^{i h w t}) is the h-th Fourier component of the sampled signal.
+ * init, set_state and set_field_stats reset the accumulators; a run split across several rk4 calls keeps
+ * accumulating.  Probes and snapshots are independent of them.
+ * enable = 0 switches off and frees the accumulators.  Otherwise allocates/resets them:
+ * pmax/pmin in the model dtype, H complex fp64 accumulators, all [ndofs] or [ndofs][nv].
+ * nharm in [0, WFX_HARMONICS_MAX], t_start finite. */
+#define WFX_HARMONICS_MAX 8
+int wfx_wave_set_field_stats(wfx_wave* wave, int enable, double t_start, int nharm);
+/* Synchronises like wfx_wave_get_probe_series.  nsamples = N, t_first/t_last = first and last sampled time;
+ * pmax_host/pmin_host in the model dtype (member-interleaved for ensembles); harm_host complex128
+ * [nharm][ndofs*nv] as (re, im) pairs, already scaled by 2/N.  Any output pointer may be NULL.
+ * N = 0: pmax = -inf, pmin = +inf, harmonics 0 (t_first = t_last = 0).  Refused when the statistics are off. */
+int wfx_wave_get_field_stats(wfx_wave* wave, int64_t* nsamples, double* t_first, double* t_last,
+                             void* pmax_host, void* pmin_host, double* harm_host);
+/* The statistics' current settings: enabled (0 / 1), t_start and nharm (0 when off), e.g. to size the buffers of
+ * wfx_wave_get_field_stats.  Any output pointer may be NULL. */
+int wfx_wave_field_stats_info(wfx_wave* wave, int* enabled, double* t_start, int* nharm);
 /* Snapshots / checkpoints: every `every` completed steps (counted since init / set_state) u and v are
  * copied device -> device on the stepping stream and device -> pinned host on a separate copy stream
  * while the time stepping continues; `fn` then receives host pointers valid for the duration of the

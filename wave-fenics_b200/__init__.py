@@ -7,6 +7,6 @@ package is the Python host-side mirror of the reference's operator interface.
 from . import capi  # noqa: F401  (raises when libwavefx.so is missing: no CPU fallback)
 from .capi import WfxError  # noqa: F401
 from .mesh import HexMesh, create_box_hex, cfl_timestep, dof_coordinates  # noqa: F401
-from .operators import (BoundaryOperator, Context, Geometry, LinearGLLEnsemble, LinearGLLOpt,  # noqa: F401
+from .operators import (BoundaryOperator, Context, FieldStats, Geometry, LinearGLLEnsemble, LinearGLLOpt,  # noqa: F401
                         LossyGLLOpt, MassOperator, MassOperatorCPU, StiffnessOperator, WesterveltGLLOpt,
                         compute_jacobian_data)

@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("WFX_LIB") or os.path.join(HERE, "libwavefx.so")
 F64, F32 = 0, 1
 STIFF_AUTO, STIFF_CELL_COLOUR, STIFF_NO_SPLIT, STIFF_CELL_STREAM, STIFF_ENSEMBLE = 0, 1, 2, 4, 8
 ENSEMBLE_MAX = 8
+HARMONICS_MAX = 8
 
 _c_i32p = C.POINTER(C.c_int32)
 _c_i64p = C.POINTER(C.c_int64)
@@ -118,6 +119,9 @@ _SIG = {
     "wfx_wave_rk4": [_vp, C.c_double, C.c_double, C.c_double, C.c_int64, _c_i64p, _c_f64p, _vp],
     "wfx_wave_set_probes": [_vp, C.c_int64, _c_i32p, C.c_int64],
     "wfx_wave_get_probe_series": [_vp, _c_i64p, _c_f64p, _vp],
+    "wfx_wave_set_field_stats": [_vp, C.c_int, C.c_double, C.c_int],
+    "wfx_wave_get_field_stats": [_vp, _c_i64p, _c_f64p, _c_f64p, _vp, _vp, _c_f64p],
+    "wfx_wave_field_stats_info": [_vp, C.POINTER(C.c_int), _c_f64p, C.POINTER(C.c_int)],
     "wfx_wave_set_snapshot": [_vp, C.c_int64, _vp, _vp],
     "wfx_wave_destroy": [_vp],
     "wfx_debug_structured_coords": [C.c_int64, C.c_int64, _c_i32p, _c_i32p, C.POINTER(C.c_int)],

@@ -73,8 +73,9 @@ struct DevBuf
   void alloc(size_t n_)
   {
     release();
+    // n is set once the allocation succeeded: after a failed one the buffer is empty, not sized with p = NULL
+    if (n_) WFX_CUDA(cudaMalloc((void**)&p, n_ * sizeof(T)));
     n = n_;
-    if (n) WFX_CUDA(cudaMalloc((void**)&p, n * sizeof(T)));
   }
   void release()
   {

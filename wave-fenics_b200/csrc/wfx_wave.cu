@@ -60,6 +60,14 @@ struct wfx_wave
   DevBuf<int32_t> d_probe_idx;
   DevBuf<unsigned char> d_probe_val;
   std::vector<double> probe_t;
+  // field statistics (section 4.5b): peaks [n*nv] in the model dtype and stats_nharm double2 planes [h][n*nv] of
+  // fp64 harmonic sums, updated after every step with t_n >= stats_t_start - dt/2; reset with the probes
+  bool stats_on = false;
+  int stats_nharm = 0;
+  double stats_t_start = 0, stats_t_first = 0, stats_t_last = 0;
+  int64_t stats_n = 0;
+  DevBuf<unsigned char> stats_pmax, stats_pmin;
+  DevBuf<double2> stats_harm;
   // snapshots: every `snap_every` steps u, v are copied device -> device on the work stream, then
   // device -> pinned host on a copy stream while the time stepping goes on; the callback runs on the
   // calling thread once the copy has landed (at the next snapshot or at the end of rk4)
@@ -340,6 +348,99 @@ __global__ void probe_ens_kernel(int64_t n, int nv, const int32_t* __restrict__ 
   if (t < n * nv) out[t] = u[(int64_t)idx[t / nv] * nv + t % nv];
 }
 
+// Field statistics: e^{-i h w_m t_n} of one sampled step as (cos, -sin) pairs, [h - 1][member], passed by value
+struct StatsWeights
+{
+  double2 e[WFX_HARMONICS_MAX * WFX_ENSEMBLE_MAX];
+};
+// One sampled step, one thread per entry k (member k % nv, the mapping of rk_stage_ens_kernel): reads u once,
+// read-modify-writes the peaks and the nharm fp64 (re, im) pairs, each a coalesced 16-byte access of its plane.
+// The pairs are all loaded before any is stored so that their loads are in flight together.
+template <typename T>
+__global__ void __launch_bounds__(256)
+field_stats_kernel(int64_t n, int nv, int nharm, const T* __restrict__ u, T* __restrict__ pmax, T* __restrict__ pmin,
+                   double2* __restrict__ harm, const __grid_constant__ StatsWeights wt)
+{
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const T x = u[k];
+  double2 acc[WFX_HARMONICS_MAX];
+#pragma unroll
+  for (int h = 0; h < WFX_HARMONICS_MAX; ++h)
+    if (h < nharm) acc[h] = harm[h * n + k];
+  const T a = pmax[k], b = pmin[k];
+  // NaN propagates: a NaN sample replaces the peak, and a NaN peak stays (every comparison with it is false)
+  pmax[k] = (x > a || x != x) ? x : a;
+  pmin[k] = (x < b || x != x) ? x : b;
+  const double xd = (double)x;
+  const int m = nv == 1 ? 0 : (int)(k % nv);
+#pragma unroll
+  for (int h = 0; h < WFX_HARMONICS_MAX; ++h)
+    if (h < nharm)
+    {
+      const double2 e = wt.e[h * WFX_ENSEMBLE_MAX + m];
+      acc[h].x = fma(xd, e.x, acc[h].x);
+      acc[h].y = fma(xd, e.y, acc[h].y);
+      harm[h * n + k] = acc[h];
+    }
+}
+
+// the statistics' reset state: pmax = -inf, pmin = +inf
+template <typename T>
+__global__ void fill_peaks_kernel(int64_t n, T* __restrict__ pmax, T* __restrict__ pmin)
+{
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k < n) pmax[k] = -INFINITY, pmin[k] = INFINITY;
+}
+
+// empty accumulators (set_field_stats, init, set_state): ordered after and before all device work, since the
+// stepping may run on any of the caller's streams
+void reset_field_stats(wfx_wave* w)
+{
+  w->stats_n = 0;
+  w->stats_t_first = w->stats_t_last = 0;
+  const int64_t ne = w->n * w->nv;
+  if (ne == 0) return;
+  WFX_CUDA(cudaDeviceSynchronize());
+  const unsigned grid = (unsigned)((ne + 255) / 256);
+  if (w->dtype == WFX_F64)
+    fill_peaks_kernel<double><<<grid, 256>>>(ne, (double*)w->stats_pmax.p, (double*)w->stats_pmin.p);
+  else
+    fill_peaks_kernel<float><<<grid, 256>>>(ne, (float*)w->stats_pmax.p, (float*)w->stats_pmin.p);
+  WFX_CUDA(cudaGetLastError());
+  if (w->stats_nharm) WFX_CUDA(cudaMemsetAsync(w->stats_harm.p, 0, w->stats_harm.n * sizeof(double2), nullptr));
+  WFX_CUDA(cudaDeviceSynchronize());
+}
+
+// one sampled step at the time reached, w->t_now
+void sample_field_stats(wfx_wave* w, cudaStream_t ws)
+{
+  const double t = w->t_now;
+  if (w->stats_n == 0) w->stats_t_first = t;
+  w->stats_t_last = t;
+  w->stats_n += 1;
+  const int64_t ne = w->n * w->nv;
+  if (ne == 0) return;
+  StatsWeights wt{};
+  for (int h = 1; h <= w->stats_nharm; ++h)
+    for (int m = 0; m < w->nv; ++m)
+    {
+      const double w0 = 2.0 * M_PI * (w->ens ? w->f0s[m] : w->f0);
+      const double ph = h * w0 * t;
+      wt.e[(h - 1) * WFX_ENSEMBLE_MAX + m] = make_double2(std::cos(ph), -std::sin(ph));
+    }
+  const unsigned grid = (unsigned)((ne + 255) / 256);
+  if (w->dtype == WFX_F64)
+    field_stats_kernel<double><<<grid, 256, 0, ws>>>(ne, w->nv, w->stats_nharm, (const double*)w->u_.p,
+                                                      (double*)w->stats_pmax.p, (double*)w->stats_pmin.p,
+                                                      w->stats_harm.p, wt);
+  else
+    field_stats_kernel<float><<<grid, 256, 0, ws>>>(ne, w->nv, w->stats_nharm, (const float*)w->u_.p,
+                                                     (float*)w->stats_pmax.p, (float*)w->stats_pmin.p,
+                                                     w->stats_harm.p, wt);
+  WFX_CUDA(cudaGetLastError());
+}
+
 // the pending snapshot's copy has landed: hand it to the callback
 void flush_snapshot(wfx_wave* w)
 {
@@ -349,10 +450,12 @@ void flush_snapshot(wfx_wave* w)
   if (w->snap_fn) w->snap_fn(w->snap_user, w->snap_step, w->snap_t, w->snap_hu, w->snap_hv);
 }
 
-// after a completed step: probe record and, every snap_every steps, a snapshot
-void after_step(wfx_wave* w, cudaStream_t ws)
+// after a completed step of size dt: probe record, field statistics inside their window and, every snap_every
+// steps, a snapshot.  The half step in the window test keeps rounding in the accumulated t from moving its edge.
+void after_step(wfx_wave* w, double dt, cudaStream_t ws)
 {
   const size_t esz = w->dtype == WFX_F64 ? 8 : 4;
+  if (w->stats_on && w->t_now >= w->stats_t_start - 0.5 * dt) sample_field_stats(w, ws);
   if (w->nprobes && w->probe_rec < w->probe_cap)
   {
     const unsigned grid = (unsigned)((w->nprobes * w->nv + 255) / 256);
@@ -634,6 +737,7 @@ extern "C" int wfx_wave_init(wfx_wave* w)
   w->t_now = 0;
   w->probe_rec = 0;
   w->probe_t.clear();
+  if (w->stats_on) reset_field_stats(w);
   WFX_API_END
 }
 
@@ -648,6 +752,7 @@ extern "C" int wfx_wave_set_state(wfx_wave* w, const void* u, const void* v)
   w->t_now = 0;
   w->probe_rec = 0;
   w->probe_t.clear();
+  if (w->stats_on) reset_field_stats(w);
   // u->scatter_fwd(), v->scatter_fwd() (LinearGLL.hpp:164,167): the stage kernels update ghost
   // entries locally from then on, so the copies are made consistent once, here
   if (w->halo && w->n)
@@ -848,11 +953,11 @@ extern "C" int wfx_wave_rk4(wfx_wave* w, double t0, double tf, double dt, int64_
     step += 1;
     w->steps_done += 1;
     w->t_now = t;
-    if (w->nprobes || w->snap_every > 0)
+    if (w->nprobes || w->snap_every > 0 || w->stats_on)
     {
       if (w->snap_pending && w->snap_every > 0 && (w->steps_done % w->snap_every) == 0)
         WFX_CUDA(cudaStreamWaitEvent(ws, w->ev_snap_done, 0));
-      after_step(w, ws);
+      after_step(w, dt, ws);
     }
   }
   if (w->snap_pending)
@@ -903,6 +1008,70 @@ extern "C" int wfx_wave_get_probe_series(wfx_wave* w, int64_t* nrecords, double*
     WFX_CUDA(cudaDeviceSynchronize());
     WFX_CUDA(cudaMemcpy(values_host, w->d_probe_val.p,
                         (size_t)w->probe_rec * w->nprobes * w->nv * (w->dtype == WFX_F64 ? 8 : 4), cudaMemcpyDeviceToHost));
+  }
+  WFX_API_END
+}
+
+extern "C" int wfx_wave_set_field_stats(wfx_wave* w, int enable, double t_start, int nharm)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  if (enable && (nharm < 0 || nharm > WFX_HARMONICS_MAX))
+    fail("field statistics: nharm = %d outside [0, %d]", nharm, WFX_HARMONICS_MAX);
+  if (enable && !std::isfinite(t_start)) fail("field statistics: t_start must be finite");
+  ScopedDevice sd(w->ctx->device);
+  WFX_CUDA(cudaDeviceSynchronize()); // the buffers may still be in use by a step in flight
+  w->stats_on = false;
+  w->stats_n = 0;
+  if (!enable)
+  {
+    w->stats_nharm = 0;
+    w->stats_pmax.release();
+    w->stats_pmin.release();
+    w->stats_harm.release();
+    return 0;
+  }
+  const size_t ne = (size_t)w->n * w->nv, nb = ne * (w->dtype == WFX_F64 ? 8 : 4);
+  // each buffer on its own: after a failed allocation (out of memory) a retry allocates what is missing
+  if (w->stats_pmax.n != nb) w->stats_pmax.alloc(nb);
+  if (w->stats_pmin.n != nb) w->stats_pmin.alloc(nb);
+  if (w->stats_harm.n != ne * nharm) w->stats_harm.alloc(ne * nharm);
+  w->stats_nharm = nharm;
+  w->stats_t_start = t_start;
+  w->stats_on = true;
+  reset_field_stats(w);
+  WFX_API_END
+}
+
+extern "C" int wfx_wave_field_stats_info(wfx_wave* w, int* enabled, double* t_start, int* nharm)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  if (enabled) *enabled = w->stats_on ? 1 : 0;
+  if (t_start) *t_start = w->stats_on ? w->stats_t_start : 0.0;
+  if (nharm) *nharm = w->stats_on ? w->stats_nharm : 0;
+  WFX_API_END
+}
+
+extern "C" int wfx_wave_get_field_stats(wfx_wave* w, int64_t* nsamples, double* t_first, double* t_last,
+                                        void* pmax_host, void* pmin_host, double* harm_host)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  if (!w->stats_on) fail("field statistics are off (wfx_wave_set_field_stats)");
+  ScopedDevice sd(w->ctx->device);
+  if (nsamples) *nsamples = w->stats_n;
+  if (t_first) *t_first = w->stats_t_first;
+  if (t_last) *t_last = w->stats_t_last;
+  if (!pmax_host && !pmin_host && !harm_host) return 0;
+  WFX_CUDA(cudaDeviceSynchronize());
+  if (pmax_host) w->stats_pmax.download((unsigned char*)pmax_host, w->stats_pmax.n);
+  if (pmin_host) w->stats_pmin.download((unsigned char*)pmin_host, w->stats_pmin.n);
+  if (harm_host && w->stats_harm.n)
+  {
+    w->stats_harm.download((double2*)harm_host, w->stats_harm.n);
+    const double scale = w->stats_n ? 2.0 / (double)w->stats_n : 0.0;
+    for (size_t i = 0; i < 2 * w->stats_harm.n; ++i) harm_host[i] *= scale;
   }
   WFX_API_END
 }

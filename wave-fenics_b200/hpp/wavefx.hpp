@@ -18,6 +18,7 @@
 #include "wavefx.h"
 
 #include <array>
+#include <complex>
 #include <cstdint>
 #include <functional>
 #include <map>
@@ -308,6 +309,28 @@ private:
   wfx_halo* _h = nullptr;
 };
 
+// Field statistics of a wave model (wfx_wave_set_field_stats, DESIGN.md section 4.5b), host copies: N sampled
+// steps from t_first to t_last, peaks shaped like the state, harmonics[(h - 1) * entries + i] the amplitude
+// (2 / N) sum_n u_i(t_n) exp(-i h w t_n) of harmonic h at state entry i.
+struct FieldStats
+{
+  std::int64_t samples = 0;
+  double t_first = 0, t_last = 0;
+  std::vector<double> pmax, pmin;
+  std::vector<std::complex<double>> harmonics;
+};
+inline void read_field_stats(wfx_wave* wave, std::int64_t entries, FieldStats& out)
+{
+  int enabled = 0, nharm = 0; // the library's own setting sizes the buffers
+  check(wfx_wave_field_stats_info(wave, &enabled, nullptr, &nharm));
+  if (!enabled) throw std::runtime_error("wavefx: field statistics are off (set_field_stats)");
+  out.pmax.resize((std::size_t)entries);
+  out.pmin.resize((std::size_t)entries);
+  out.harmonics.resize((std::size_t)(entries * nharm));
+  check(wfx_wave_get_field_stats(wave, &out.samples, &out.t_first, &out.t_last, out.pmax.data(), out.pmin.data(),
+                                 reinterpret_cast<double*>(out.harmonics.data())));
+}
+
 // The wave model and its RK4 driver (common/LinearGLL.hpp:37-287), fp64 like the reference.
 class LinearGLLOpt
 {
@@ -376,6 +399,13 @@ public:
     values.resize((std::size_t)(n * _nprobes));
     check(wfx_wave_get_probe_series(_wave, &n, t.data(), values.data()));
   }
+  // peaks and harmonics 1..nharm (<= WFX_HARMONICS_MAX) of u over the steps with t_n >= t_start - dt/2, kept on
+  // the device; resets them (so do init and set_state).  enable = false switches them off.
+  void set_field_stats(bool enable, double t_start = 0.0, int nharm = 0)
+  {
+    check(wfx_wave_set_field_stats(_wave, enable ? 1 : 0, t_start, nharm));
+  }
+  void field_stats(FieldStats& out) const { read_field_stats(_wave, _ndofs, out); }
   // fn(step, t, u, v) every `every` steps with pointers into pinned host copies (ndofs entries each);
   // the device -> host copy overlaps the time stepping.  A checkpoint is a snapshot handed back to
   // set_state.
@@ -520,6 +550,12 @@ public:
     values.resize((std::size_t)(n * _nprobes * _nv));
     check(wfx_wave_get_probe_series(_wave, &n, t.data(), values.data()));
   }
+  // as LinearGLLOpt's, member m analysed at its own f0[m]; peaks [ndofs][nv], harmonics [nharm][ndofs][nv]
+  void set_field_stats(bool enable, double t_start = 0.0, int nharm = 0)
+  {
+    check(wfx_wave_set_field_stats(_wave, enable ? 1 : 0, t_start, nharm));
+  }
+  void field_stats(FieldStats& out) const { read_field_stats(_wave, _ndofs * _nv, out); }
   void set_state(const std::vector<double>& u, const std::vector<double>& v)
   {
     if ((std::int64_t)u.size() != _ndofs * _nv || (std::int64_t)v.size() != _ndofs * _nv)

@@ -18,10 +18,14 @@ stream) or numpy arrays (host path: copied to the GPU and back inside the call, 
 reference functor applied to host la::Vectors).  All compute happens in libwavefx.so.
 """
 import ctypes as C
+from collections import namedtuple
 
 import numpy as np
 
 from . import capi
+
+# field statistics of a wave model (LinearGLLOpt.field_stats, DESIGN.md section 4.5b)
+FieldStats = namedtuple("FieldStats", "samples t_first t_last pmax pmin harmonics")
 
 
 def _is_torch(x):
@@ -409,6 +413,37 @@ class LinearGLLOpt:
         capi.call("wfx_wave_get_probe_series", self.handle, C.byref(n), capi.f64p(t), C.c_void_p(vals.ctypes.data))
         return t, vals
 
+    def set_field_stats(self, t_start, harmonics=0):
+        """Accumulate field statistics (DESIGN.md section 4.5b) on the device after every completed step whose
+        reached time is >= t_start - dt/2: peak positive and negative pressure and the complex amplitudes of
+        harmonics 1..`harmonics` (<= 8) of the model's source frequency at every dof.  Resets the accumulators,
+        as do init and set_state.  set_field_stats(None) switches them off and frees them."""
+        if t_start is None:
+            capi.call("wfx_wave_set_field_stats", self.handle, 0, 0.0, 0)
+            return
+        capi.call("wfx_wave_set_field_stats", self.handle, 1, float(t_start), int(harmonics))
+
+    def _entry_shape(self):
+        return (self.ndofs,)
+
+    def field_stats(self):
+        """FieldStats(samples, t_first, t_last, pmax, pmin, harmonics) accumulated so far: pmax, pmin in the model
+        dtype, shaped like the state; harmonics complex128 [H, *state shape], harmonics[h - 1] the amplitude
+        p_h = (2 / N) sum_n u(t_n) exp(-i h w t_n) of harmonic h."""
+        shape = self._entry_shape()
+        on, nharm = C.c_int(), C.c_int()
+        capi.call("wfx_wave_field_stats_info", self.handle, C.byref(on), None, C.byref(nharm))
+        if not on.value:
+            raise capi.WfxError("field statistics are off (set_field_stats)")
+        nharm = nharm.value
+        pmax, pmin = np.empty(shape, dtype=self.dtype), np.empty(shape, dtype=self.dtype)
+        harm = np.empty((nharm, *shape), dtype=np.complex128)
+        n, t0, t1 = C.c_int64(), C.c_double(), C.c_double()
+        capi.call("wfx_wave_get_field_stats", self.handle, C.byref(n), C.byref(t0), C.byref(t1),
+                  C.c_void_p(pmax.ctypes.data), C.c_void_p(pmin.ctypes.data),
+                  C.cast(C.c_void_p(harm.ctypes.data), capi._c_f64p))
+        return FieldStats(n.value, t0.value, t1.value, pmax, pmin, harm)
+
     def set_snapshot(self, every, fn):
         """fn(step, t, u, v) with numpy views of the pinned host copies (copy them to keep them), every
         `every` completed steps; the device -> host copy overlaps the time stepping."""
@@ -500,6 +535,9 @@ class LinearGLLEnsemble(LinearGLLOpt):
         v = np.empty((self.ndofs, self.nv), dtype=self.dtype)
         capi.call("wfx_wave_get_state", self.handle, C.c_void_p(u.ctypes.data), C.c_void_p(v.ctypes.data))
         return u, v
+
+    def _entry_shape(self):
+        return (self.ndofs, self.nv)
 
     def probe_series(self):
         """(t [nrec], u [nrec, nprobes, nv]) recorded so far."""
