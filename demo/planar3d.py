@@ -11,11 +11,17 @@ section 4.5b) and prints, along the x axis, the peak positive and negative press
 fundamental's amplitude and the second harmonic's share of it.  The harmonics are exact Fourier components only
 over whole periods of whole steps, so the run then stops on the last whole step before the final time (a shortened
 last step would be a sample off the uniform grid) and exactly K * (steps per period) steps are sampled.
+--focus DEPTH focuses the source (DESIGN.md section 4.5c): per-dof delays from focus_delays for a focus at x = DEPTH
+on the axis through the centre of the source face, and the four lateral faces absorbing (tag 2) instead of rigid;
+--aperture R switches the source off outside radius R of the face centre.  With --stats-periods the field statistics
+are then reported along that axis: the position and value of the maximum of |p1| and of pmax.  For a small
+aperture (Fresnel number a^2 / (lambda DEPTH) of a few) that maximum lies short of DEPTH, as the Rayleigh integral
+predicts.
 The reference reads `../mesh.xdmf` (not in its repository); here the mesh is a structured
 n x m x m hexahedral box with tag 1 on x = 0 (source) and tag 2 on x = L (absorbing).
 
-    python demo/planar3d.py [--nx 32] [--nyz 4] [--steps N] [--check] [--model linear|lossy|westervelt]
-                            [--stats-periods K]
+    python demo/planar3d.py [--nx 32] [--nyz 4] [--length 0.1] [--steps N] [--check]
+                            [--model linear|lossy|westervelt] [--stats-periods K] [--focus DEPTH] [--aperture R]
 """
 import argparse
 import os
@@ -52,15 +58,23 @@ def main():
     ap.add_argument("--rho0", type=float, default=1000.0, help="density [kg/m^3] (westervelt)")
     ap.add_argument("--stats-periods", type=int, default=0,
                     help="field statistics (peaks, harmonics) over the last K periods of the run (0: off)")
+    ap.add_argument("--length", type=float, default=0.1, help="domain length along x [m]")
+    ap.add_argument("--focus", type=float, default=0.0,
+                    help="focal depth [m] on the axis through the centre of the source face (0: plane source)")
+    ap.add_argument("--aperture", type=float, default=0.0,
+                    help="with --focus: source radius [m] around the face centre (0: the whole face)")
     args = ap.parse_args()
 
     speedOfSound, sourceFrequency, pressureAmplitude = 1500.0, 0.5e6, 60000.0   # main.cpp:25-30
     period = 1.0 / sourceFrequency
-    domainLength = 0.1                                                           # :33
+    domainLength = args.length                                                   # :33
     degreeOfBasis = 4                                                            # :36
     side = domainLength / args.nx
-    mesh = wfx.create_box_hex((args.nx, args.nyz, args.nyz), degreeOfBasis,
-                              (domainLength, side * args.nyz, side * args.nyz))
+    width = side * args.nyz
+    tags = ((0, 0, 1), (0, 1, 2))
+    if args.focus > 0:
+        tags += ((1, 0, 2), (1, 1, 2), (2, 0, 2), (2, 1, 2))
+    mesh = wfx.create_box_hex((args.nx, args.nyz, args.nyz), degreeOfBasis, (domainLength, width, width), tags=tags)
     timeStepSize = wfx.cfl_timestep(mesh.h_min, speedOfSound, degreeOfBasis, sourceFrequency)  # :61-66
     startTime, finalTime = 0.0, domainLength / speedOfSound + 8.0 / sourceFrequency            # :63-64
     print(f"Number of step per period: {int(round(period / timeStepSize))}")
@@ -75,6 +89,17 @@ def main():
                                    delta, beta, args.rho0)
     print(f"Number of steps: {nstep}")
     print(f"Degrees of freedom: {mesh.ndofs_global}")
+    X = wfx.dof_coordinates(mesh)
+    if args.focus > 0:
+        face = np.abs(X[:, 0]) < 1e-12
+        delay = np.zeros(mesh.ndofs)
+        delay[face] = wfx.focus_delays(X[face], (args.focus, width / 2, width / 2), speedOfSound)
+        amp = None
+        if args.aperture > 0:
+            amp = (np.hypot(X[:, 1] - width / 2, X[:, 2] - width / 2) <= args.aperture).astype(np.float64)
+        eqn.set_source_profile(amp, delay)
+        print(f"focused source: focus at x = {args.focus:.4f} on the face axis, "
+              f"delays up to {delay.max():.4e} s, aperture {'whole face' if amp is None else args.aperture}")
     eqn.init()                                                                   # :83
     run_tf, run_steps = finalTime, args.steps
     if args.stats_periods > 0:
@@ -87,11 +112,11 @@ def main():
     eqn.ctx.synchronize()
     print(f"Solve time: {time.perf_counter() - t0:.6f}  ({steps} steps, t = {t_end:.6e})")   # :92
     u, v = eqn.get_state()
-    X = wfx.dof_coordinates(mesh)
     if args.stats_periods > 0:
         fs = eqn.field_stats()
-        # the dofs on the x axis (y = z = 0), from the source to the absorbing end
-        line = np.where((np.abs(X[:, 1]) < 1e-12) & (np.abs(X[:, 2]) < 1e-12))[0]
+        # the dofs on the x axis (y = z = 0; with --focus the axis through the face centre), source to absorbing end
+        yz = width / 2 if args.focus > 0 else 0.0
+        line = np.where((np.abs(X[:, 1] - yz) < 1e-9 * width) & (np.abs(X[:, 2] - yz) < 1e-9 * width))[0]
         line = line[np.argsort(X[line, 0])]
         x = X[line, 0]
         pmax, pmin, p1, p2 = fs.pmax[line], fs.pmin[line], np.abs(fs.harmonics[0, line]), np.abs(fs.harmonics[1, line])
@@ -103,6 +128,9 @@ def main():
             print(f"along x: max pmax = {pmax.max():.6e} at x = {x[pmax.argmax()]:.4f}, "
                   f"min pmin = {pmin.min():.6e} at x = {x[pmin.argmin()]:.4f}")
             print(f"at the absorbing end (x = {x[-1]:.4f}): |p1| = {p1[-1]:.6e}, |p2|/|p1| = {p2[-1] / p1[-1]:.6e}")
+            if args.focus > 0:
+                print(f"on-axis maximum: |p1| = {p1.max():.6e} at x = {x[p1.argmax()]:.5f}, "
+                      f"pmax = {pmax.max():.6e} at x = {x[pmax.argmax()]:.5f} (focus requested at x = {args.focus:.5f})")
     else:
         print(f"max |p| = {np.abs(u).max():.6e} at x = {X[np.abs(u).argmax(), 0]:.4f}")
     if args.check:
@@ -112,7 +140,13 @@ def main():
         oracle.mass_apply(mesh, degreeOfBasis, detJ, np.ones(mesh.ndofs), m)
         m1, m2 = oracle.boundary_facet_mass(mesh, degreeOfBasis)
         uo, vo = np.zeros(mesh.ndofs), np.zeros(mesh.ndofs)
-        if args.model == "linear":
+        if args.focus > 0:
+            from model_oracle import model_oracle
+            model_oracle.rk4_westervelt_profile(mesh, degreeOfBasis, G, m, m1, m2, speedOfSound, sourceFrequency,
+                                                pressureAmplitude, delta, beta, args.rho0, amp, delay, startTime,
+                                                run_tf, timeStepSize, uo, vo, max_steps=run_steps, sumfact=True,
+                                                nthreads=oracle.max_threads())
+        elif args.model == "linear":
             oracle.rk4(mesh, degreeOfBasis, G, m, m1, m2, speedOfSound, sourceFrequency, pressureAmplitude,
                        startTime, run_tf, timeStepSize, uo, vo, max_steps=run_steps, sumfact=True,
                        nthreads=oracle.max_threads())

@@ -387,6 +387,18 @@ int wfx_wave_get_field_stats(wfx_wave* wave, int64_t* nsamples, double* t_first,
 /* The statistics' current settings: enabled (0 / 1), t_start and nharm (0 when off), e.g. to size the buffers of
  * wfx_wave_get_field_stats.  Any output pointer may be NULL. */
 int wfx_wave_field_stats_info(wfx_wave* wave, int* enabled, double* t_start, int* nharm);
+/* Source profile (DESIGN.md section 4.5c): phased-array sources on the tag-1 facets.  With a profile, the
+ * boundary term of every model uses per-entry delayed sources in place of g(t):
+ *   g_i(t) = a_i g(t - tau_i),   g(s) = g'(s) = 0 for s < 0,
+ * g the model's source including its four-period ramp (lossy / Westervelt models: a_i (g + (delta / c0^2) g')
+ * (t - tau_i); ensemble member m: its own f0 / p0).  The sources are evaluated on the device in fp64 at every
+ * stage time, for both model dtypes.  amp_host and delay_host hold the model's local entries in the state
+ * layout (ndofs, or ndofs * nv member-interleaved for an ensemble); entries off tag 1 are ignored.  Either may be
+ * NULL (a = 1, tau = 0 respectively); both NULL clears the profile and restores the unprofiled path.
+ * The profile is model configuration: it survives init, set_state and snapshot restarts, and may be changed
+ * between rk4 calls.  Refused: a NULL model, a model without a boundary operator, a distributed model, a
+ * non-finite amplitude or delay, a negative delay. */
+int wfx_wave_set_source_profile(wfx_wave* wave, const double* amp_host, const double* delay_host);
 /* Snapshots / checkpoints: every `every` completed steps (counted since init / set_state) u and v are
  * copied device -> device on the stepping stream and device -> pinned host on a separate copy stream
  * while the time stepping continues; `fn` then receives host pointers valid for the duration of the

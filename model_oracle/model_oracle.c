@@ -122,3 +122,102 @@ int64_t wo_rk4_westervelt(int P, int64_t ncells, int64_t ndofs, const int32_t* d
   free(u_); free(v_); free(un); free(vn); free(u0); free(v0); free(ku); free(kv); free(b); free(bv);
   return step;
 }
+
+/* ---- source profiles (DESIGN.md section 4.5c) ----------------------------------------------------------------
+ * The same model with a per-dof source g_k(t) = amp_k g(t - delay_k), g and g' of wo_source, both zero before
+ * the delay.  model_rhs_profile is model_rhs with that source; with amp = 1 and delay = 0 it computes what
+ * model_rhs computes, bit for bit (1 * g = g, t - 0 = t). */
+static void model_rhs_profile(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                              const double* m, const double* m1, const double* m2, double c0, double freq0, double p0,
+                              double delta, double beta, double rho0, const double* amp, const double* delay, double t,
+                              const double* un, const double* vn, double* kv, double* b, double* bv, int sumfact,
+                              int nthreads)
+{
+  const size_t nb = sizeof(double) * ndofs;
+  const double kappa = beta > 0 ? 2.0 * beta / (rho0 * c0 * c0) : 0.0;
+  const double s = delta / (1500.0 * 1500.0);
+  memset(b, 0, nb);
+  memset(bv, 0, nb);
+  model_stiffness(P, ncells, ndofs, dofmap, G, un, b, sumfact, nthreads);  /* A un */
+  model_stiffness(P, ncells, ndofs, dofmap, G, vn, bv, sumfact, nthreads); /* A vn */
+  for (int64_t k = 0; k < ndofs; ++k)
+  {
+    double g = 0.0, gdot = 0.0;
+    if (m1[k] != 0.0)
+    {
+      const double sk = t - delay[k];
+      if (sk >= 0.0) wo_source(sk, freq0, p0, c0, &g, &gdot);
+      else g = gdot = 0.0; /* the source has not started at this dof yet */
+      g = amp[k] * g;
+      gdot = amp[k] * gdot;
+    }
+    double r = b[k] + s * bv[k];
+    r += (c0 * c0 * g + delta * gdot) * m1[k] - c0 * m2[k] * vn[k];
+    r += kappa * m[k] * vn[k] * vn[k];
+    kv[k] = r / (m[k] * (1.0 - kappa * un[k]) + delta / c0 * m2[k]);
+  }
+}
+
+/* wo_f1_westervelt with a source profile amp[ndofs], delay[ndofs] */
+void wo_f1_westervelt_profile(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                              const double* m, const double* m1, const double* m2, double c0, double freq0, double p0,
+                              double delta, double beta, double rho0, const double* amp, const double* delay, double t,
+                              const double* u, const double* v, double* out, int sumfact, int nthreads)
+{
+  const size_t nb = sizeof(double) * ndofs;
+  double *b = malloc(nb), *bv = malloc(nb);
+  model_rhs_profile(P, ncells, ndofs, dofmap, G, m, m1, m2, c0, freq0, p0, delta, beta, rho0, amp, delay, t, u, v,
+                    out, b, bv, sumfact, nthreads);
+  free(b);
+  free(bv);
+}
+
+/* wo_rk4_westervelt with a source profile: the same stage loop, model_rhs_profile as f1 */
+int64_t wo_rk4_westervelt_profile(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                                  const double* m, const double* m1, const double* m2, double c0, double freq0,
+                                  double p0, double delta, double beta, double rho0, const double* amp,
+                                  const double* delay, double t0, double tf, double dt, int64_t max_steps, double* u_n,
+                                  double* v_n, int sumfact, int nthreads, double* t_end)
+{
+  const double a_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  const double b_runge[4] = {1.0 / 6.0, 1.0 / 3.0, 1.0 / 3.0, 1.0 / 6.0};
+  const double c_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  const size_t nb = sizeof(double) * ndofs;
+  double *u_ = malloc(nb), *v_ = malloc(nb), *un = malloc(nb), *vn = malloc(nb);
+  double *u0 = malloc(nb), *v0 = malloc(nb), *ku = malloc(nb), *kv = malloc(nb), *b = malloc(nb), *bv = malloc(nb);
+  memcpy(u_, u_n, nb);
+  memcpy(v_, v_n, nb);
+  memcpy(ku, u_, nb);
+  memcpy(kv, v_, nb);
+  double t = t0;
+  int64_t step = 0;
+  while (t < tf)
+  {
+    if (max_steps > 0 && step >= max_steps) break;
+    dt = dt < tf - t ? dt : tf - t;
+    memcpy(u0, u_, nb);
+    memcpy(v0, v_, nb);
+    for (int i = 0; i < 4; ++i)
+    {
+      memcpy(un, u0, nb);
+      memcpy(vn, v0, nb);
+      const double adt = dt * a_runge[i];
+      for (int64_t k = 0; k < ndofs; ++k) un[k] = ku[k] * adt + un[k];
+      for (int64_t k = 0; k < ndofs; ++k) vn[k] = kv[k] * adt + vn[k];
+      const double tn = t + c_runge[i] * dt;
+      memcpy(ku, vn, nb);
+      model_rhs_profile(P, ncells, ndofs, dofmap, G, m, m1, m2, c0, freq0, p0, delta, beta, rho0, amp, delay, tn, un,
+                        vn, kv, b, bv, sumfact, nthreads);
+      const double bdt = dt * b_runge[i];
+      for (int64_t k = 0; k < ndofs; ++k) u_[k] = ku[k] * bdt + u_[k];
+      for (int64_t k = 0; k < ndofs; ++k) v_[k] = kv[k] * bdt + v_[k];
+    }
+    t += dt;
+    step += 1;
+  }
+  memcpy(u_n, u_, nb);
+  memcpy(v_n, v_, nb);
+  if (t_end) *t_end = t;
+  free(u_); free(v_); free(un); free(vn); free(u0); free(v0); free(ku); free(kv); free(b); free(bv);
+  return step;
+}

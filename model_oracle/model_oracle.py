@@ -63,6 +63,12 @@ def lib():
         L.wo_rk4_westervelt.restype = l
         L.wo_rk4_westervelt.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, d, d, d, d, d, l,
                                         _f64p, _f64p, i, i, _f64p]
+        L.wo_f1_westervelt_profile.restype = None
+        L.wo_f1_westervelt_profile.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, d, d, _f64p,
+                                               _f64p, d, _f64p, _f64p, _f64p, i, i]
+        L.wo_rk4_westervelt_profile.restype = l
+        L.wo_rk4_westervelt_profile.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, d, d, _f64p,
+                                                _f64p, d, d, d, l, _f64p, _f64p, i, i, _f64p]
         _lib.append(L)
     return _lib[0]
 
@@ -98,3 +104,35 @@ def rk4_westervelt(mesh, P, G, m, m1, m2, c0, f0, p0, delta, beta, rho0, t0, tf,
                                     _f(v), int(sumfact), nthreads, C.byref(t_end))
     return steps, t_end.value
 
+
+
+def _profile(mesh, amp, delay):
+    amp = np.ones(mesh.ndofs) if amp is None else np.ascontiguousarray(amp, dtype=np.float64)
+    delay = np.zeros(mesh.ndofs) if delay is None else np.ascontiguousarray(delay, dtype=np.float64)
+    assert amp.shape == delay.shape == (mesh.ndofs,)
+    return amp, delay
+
+
+def f1_westervelt_profile(mesh, P, G, m, m1, m2, c0, f0, p0, delta, beta, rho0, amp, delay, t, u, v, sumfact=False,
+                          nthreads=1):
+    """f1_westervelt with the source amp[i] g(t - delay[i]) at dof i (zero before the delay); None: 1 / 0."""
+    amp, delay = _profile(mesh, amp, delay)
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    out = np.empty(mesh.ndofs)
+    lib().wo_f1_westervelt_profile(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)), _f(m),
+                                   _f(m1), _f(m2), c0, f0, p0, delta, beta, rho0, _f(amp), _f(delay), t, _f(u), _f(v),
+                                   _f(out), int(sumfact), nthreads)
+    return out
+
+
+def rk4_westervelt_profile(mesh, P, G, m, m1, m2, c0, f0, p0, delta, beta, rho0, amp, delay, t0, tf, dt, u, v,
+                           max_steps=0, sumfact=False, nthreads=1):
+    """rk4_westervelt with a source profile (see f1_westervelt_profile); u, v updated in place.  -> (steps, t_end)"""
+    amp, delay = _profile(mesh, amp, delay)
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    t_end = C.c_double()
+    steps = lib().wo_rk4_westervelt_profile(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)),
+                                            _f(m), _f(m1), _f(m2), c0, f0, p0, delta, beta, rho0, _f(amp), _f(delay),
+                                            t0, tf, dt, max_steps, _f(u), _f(v), int(sumfact), nthreads,
+                                            C.byref(t_end))
+    return steps, t_end.value

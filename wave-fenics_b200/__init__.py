@@ -9,4 +9,4 @@ from .capi import WfxError  # noqa: F401
 from .mesh import HexMesh, create_box_hex, cfl_timestep, dof_coordinates  # noqa: F401
 from .operators import (BoundaryOperator, Context, FieldStats, Geometry, LinearGLLEnsemble, LinearGLLOpt,  # noqa: F401
                         LossyGLLOpt, MassOperator, MassOperatorCPU, StiffnessOperator, WesterveltGLLOpt,
-                        compute_jacobian_data)
+                        compute_jacobian_data, focus_delays)

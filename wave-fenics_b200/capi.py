@@ -122,6 +122,7 @@ _SIG = {
     "wfx_wave_set_field_stats": [_vp, C.c_int, C.c_double, C.c_int],
     "wfx_wave_get_field_stats": [_vp, _c_i64p, _c_f64p, _c_f64p, _vp, _vp, _c_f64p],
     "wfx_wave_field_stats_info": [_vp, C.POINTER(C.c_int), _c_f64p, C.POINTER(C.c_int)],
+    "wfx_wave_set_source_profile": [_vp, _c_f64p, _c_f64p],
     "wfx_wave_set_snapshot": [_vp, C.c_int64, _vp, _vp],
     "wfx_wave_destroy": [_vp],
     "wfx_debug_structured_coords": [C.c_int64, C.c_int64, _c_i32p, _c_i32p, C.POINTER(C.c_int)],

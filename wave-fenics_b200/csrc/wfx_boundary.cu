@@ -4,6 +4,7 @@
 // masses m1 (tag 1, Neumann source) and m2 (tag 2, absorbing) are reduced once on the host
 // over the tagged facets and kept compact (boundary dofs only) on the device.
 #include "wfx_internal.h"
+#include "wfx_source.h"
 
 #include <cmath>
 #include <map>
@@ -60,6 +61,39 @@ __global__ void boundary_ens_kernel(int64_t nb, int nv, const int32_t* __restric
   b[i] = (T)((double)b[i] + c02g * m1[p] - c0 * m2[p] * (double)vn[i]);
 }
 
+// A source profile (section 4.5c) on nv member-interleaved fields (nv = 1: one field), one thread per
+// (boundary dof p, member m), compact entry t = p nv + m:
+//   b[i,m] += c0^2 a_t (g_m + s_src g_m')(tn - tau_t) m1_p - c0 m2_p vn[i,m],   g_m = g_m' = 0 before tau_t,
+// with g_m member m's source (f0, p0 of SourceParams) evaluated in fp64 by source_eval for every scalar type.
+// The stage time tn comes by value or, in graph replays, from t_dev.  Entries off Gamma1 (m1 = 0) and
+// switched-off entries (a = 0) skip the trigonometry.
+template <typename T>
+__global__ void __launch_bounds__(256)
+boundary_profile_kernel(int64_t nb, int nv, const int32_t* __restrict__ idx, const double* __restrict__ m1,
+                        const double* __restrict__ m2, double c0, double s_src, const __grid_constant__ SourceParams sp,
+                        double t_host, const double* __restrict__ t_dev, const double* __restrict__ amp,
+                        const double* __restrict__ delay, const T* __restrict__ vn, T* __restrict__ b)
+{
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t >= nb * nv) return;
+  const int64_t p = t / nv;
+  const int m = (int)(t % nv);
+  const double m1p = m1[p], a = amp[t];
+  double src = 0.0;
+  if (m1p != 0.0 && a != 0.0)
+  {
+    const double s = (t_dev ? *t_dev : t_host) - delay[t];
+    if (s >= 0.0)
+    {
+      double g, gdot;
+      source_eval(sp.f0[m], sp.p0[m], c0, s, &g, &gdot);
+      src = a * (g + s_src * gdot);
+    }
+  }
+  const int64_t i = (int64_t)idx[p] * nv + m;
+  b[i] = (T)((double)b[i] + __dmul_rn(c0 * c0, src) * m1p - c0 * m2[p] * (double)vn[i]);
+}
+
 // Lossy / Westervelt models: the Gamma2 mass term q = qc m2 on the absorbing dofs only, so that the dense
 // stage update needs nothing beyond 1/m (see boundary_absorbing_mass in wfx_internal.h).  p is formed in T
 // exactly as the stage kernel forms it.
@@ -90,6 +124,24 @@ void wfx::boundary_absorbing_mass(wfx_boundary* op, const double* m64, double qc
   else
     absorbing_mass_kernel<float><<<grid, 256, 0, stream>>>(op->nb, op->d_idx.p, op->d_m2.p, m64, qc, kappa, (float)s,
                                                             (const float*)pw, (const float*)pd, (float*)b);
+  WFX_CUDA(cudaGetLastError());
+}
+
+void wfx::boundary_apply_profile(wfx_boundary* op, int nv, double c0, double s_src, const SourceParams& sp,
+                                 double t_host, const double* t_dev, const double* amp, const double* delay,
+                                 const void* vn, void* b, cudaStream_t stream)
+{
+  if (!op || op->nb == 0) return;
+  if (nv < 1 || nv > WFX_ENSEMBLE_MAX) fail("boundary: nv = %d outside [1, %d]", nv, WFX_ENSEMBLE_MAX);
+  const unsigned grid = (unsigned)((op->nb * nv + 255) / 256);
+  if (op->dtype == WFX_F64)
+    boundary_profile_kernel<double><<<grid, 256, 0, stream>>>(op->nb, nv, op->d_idx.p, op->d_m1.p, op->d_m2.p, c0,
+                                                               s_src, sp, t_host, t_dev, amp, delay,
+                                                               (const double*)vn, (double*)b);
+  else
+    boundary_profile_kernel<float><<<grid, 256, 0, stream>>>(op->nb, nv, op->d_idx.p, op->d_m1.p, op->d_m2.p, c0,
+                                                              s_src, sp, t_host, t_dev, amp, delay,
+                                                              (const float*)vn, (float*)b);
   WFX_CUDA(cudaGetLastError());
 }
 
@@ -307,6 +359,7 @@ namespace wfx
 {
 bool boundary_assembled(const wfx_boundary* op) { return op->assembled; }
 int boundary_dtype(const wfx_boundary* op) { return op->dtype; }
+const std::vector<int32_t>& boundary_dofs(const wfx_boundary* op) { return op->h_idx; }
 } // namespace wfx
 
 extern "C" int wfx_boundary_destroy(wfx_boundary* op)

@@ -119,6 +119,18 @@ void boundary_apply_dev(struct ::wfx_boundary* op, double c0, const double* g_de
 bool stiffness_has_ensemble(const struct ::wfx_stiffness* op);
 void boundary_apply_ens(struct ::wfx_boundary* op, int nv, double c0, const double* g_host, const double* g_dev,
                         const void* vn, void* b, cudaStream_t stream);
+// source profiles (wfx_wave_set_source_profile, DESIGN.md section 4.5c): the compact dof list of the boundary
+// term (the order of its amp / delay arrays), and the term with per-entry delayed sources
+//   b[i,m] += c0^2 amp[t] (g_m + s_src g_m')(tn - delay[t]) m1_i - c0 m2_i vn[i,m],  t = p nv + m, i = dofs[p],
+// g_m from member m's f0 / p0 (nv = 1: one field); tn read from t_dev when it is not NULL (graph replays)
+struct SourceParams
+{
+  double f0[WFX_ENSEMBLE_MAX], p0[WFX_ENSEMBLE_MAX];
+};
+const std::vector<int32_t>& boundary_dofs(const struct ::wfx_boundary* op);
+void boundary_apply_profile(struct ::wfx_boundary* op, int nv, double c0, double s_src, const SourceParams& sp,
+                            double t_host, const double* t_dev, const double* amp, const double* delay,
+                            const void* vn, void* b, cudaStream_t stream);
 // lossy / Westervelt models (wfx_wave_create_westervelt)
 double stiffness_c0(const struct ::wfx_stiffness* op);       // the c0 of y = -c0^2 K x
 int64_t stiffness_nshared(const struct ::wfx_stiffness* op); // rank-shared dofs (0 on one rank)

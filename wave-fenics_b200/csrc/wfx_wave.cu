@@ -5,6 +5,7 @@
 // facet dofs, one optional halo reduction of b, and ONE fused pointwise kernel that does
 // kv = b/m, both solution updates and the next stage state.
 #include "wfx_internal.h"
+#include "wfx_source.h"
 
 #include <cmath>
 #include <cstdlib>
@@ -50,6 +51,11 @@ struct wfx_wave
   cudaGraphExec_t step_graph = nullptr;
   double graph_dt = 0;
   DevBuf<double> g_dev;
+  // source profile (section 4.5c): per-entry amplitude and delay, compact over the boundary dofs [nb][nv]; the
+  // boundary term then evaluates the delayed sources on the device from the four stage times, which graph
+  // replays read from t_dev.  Setting or clearing it drops step_graph (captured with the other boundary kernel).
+  bool prof_on = false;
+  DevBuf<double> prof_amp, prof_delay, t_dev;
   cudaStream_t own_stream = nullptr; // capture needs a non-legacy stream
   cudaEvent_t ev_in = nullptr, ev_out = nullptr;
   // time-stepping position (reset by init / set_state): steps completed and the time reached
@@ -504,16 +510,20 @@ __global__ void set_source_ens_kernel(double* g_dev, const StepAmp a, int n)
   if ((int)threadIdx.x < n) g_dev[threadIdx.x] = a.g[threadIdx.x];
 }
 
+void boundary_profiled(wfx_wave* w, double tn, const double* t_dev, const void* vn, cudaStream_t st);
+
 // One time step of size dt on stream st: the four stages of LinearGLL.hpp:244-270.  g[i*nv + m] is the
 // source amplitude of stage i (of member m); with g_from_dev the boundary kernels read it from w->g_dev
-// instead (graph capture).
-void enqueue_step(wfx_wave* w, double dt, const double* g, bool g_from_dev, cudaStream_t st)
+// instead (graph capture).  With a source profile the boundary term takes the stage times tn[i] instead, or
+// reads them from w->t_dev.
+void enqueue_step(wfx_wave* w, double dt, const double* g, const double* tn, bool g_from_dev, cudaStream_t st)
 {
   const double a_runge[5] = {0.0, 0.5, 0.5, 1.0, 0.0};
   const double b_runge[4] = {1.0 / 6.0, 1.0 / 3.0, 1.0 / 3.0, 1.0 / 6.0};
   auto boundary = [&](int i, const void* vn) {
     if (!w->bnd) return;
-    if (w->ens)
+    if (w->prof_on) boundary_profiled(w, g_from_dev ? 0.0 : tn[i], g_from_dev ? w->t_dev.p + i : nullptr, vn, st);
+    else if (w->ens)
       boundary_apply_ens(w->bnd, w->nv, w->c0, g_from_dev ? nullptr : g + i * w->nv,
                          g_from_dev ? w->g_dev.p + i * w->nv : nullptr, vn, w->b.p, st);
     else if (g_from_dev) boundary_apply_dev(w->bnd, w->c0, w->g_dev.p + i, vn, w->b.p, st);
@@ -648,6 +658,7 @@ extern "C" int wfx_wave_create(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mas
   if (!halo)
   {
     w->g_dev.alloc(4);
+    w->t_dev.alloc(4);
     WFX_CUDA(cudaStreamCreateWithFlags(&w->own_stream, cudaStreamNonBlocking));
     WFX_CUDA(cudaEventCreateWithFlags(&w->ev_in, cudaEventDisableTiming));
     WFX_CUDA(cudaEventCreateWithFlags(&w->ev_out, cudaEventDisableTiming));
@@ -785,32 +796,36 @@ extern "C" int wfx_wave_state_ptrs(wfx_wave* w, void** u, void** v)
 
 namespace
 {
-// g(t) of LinearGLL.hpp:155-162: Hann ramp over the first alpha periods
+// g(t) of LinearGLL.hpp:155-162 (source_eval, wfx_source.h)
 double source_amplitude(double f0, double p0, double c0, double tn)
 {
-  const double w0 = 2.0 * M_PI * f0, T = 1.0 / f0, alpha = 4.0; // :96-99
-  const double window = tn < T * alpha ? 0.5 * (1.0 - std::cos(f0 * M_PI * tn / alpha)) : 1.0;
-  return window * p0 * w0 / c0 * std::cos(w0 * tn);
-}
-// its time derivative g'(t) = A (W' cos(w0 t) - W w0 sin(w0 t)), A = p0 w0 / c0
-double source_rate(double f0, double p0, double c0, double tn)
-{
-  const double w0 = 2.0 * M_PI * f0, T = 1.0 / f0, alpha = 4.0;
-  const bool ramp = tn < T * alpha;
-  const double window = ramp ? 0.5 * (1.0 - std::cos(f0 * M_PI * tn / alpha)) : 1.0;
-  const double rate = ramp ? f0 * M_PI / (2.0 * alpha) * std::sin(f0 * M_PI * tn / alpha) : 0.0;
-  return p0 * w0 / c0 * (rate * std::cos(w0 * tn) - window * w0 * std::sin(w0 * tn));
+  double g, gdot;
+  source_eval(f0, p0, c0, tn, &g, &gdot);
+  return g;
 }
 // the amplitude the boundary term receives: g, or g + (delta / c0^2) g' for the lossy / Westervelt models
 double source_amplitude(const wfx_wave* w, double tn)
 {
-  const double g = source_amplitude(w->f0, w->p0, w->c0, tn);
-  return w->model ? g + w->s_src * source_rate(w->f0, w->p0, w->c0, tn) : g;
+  double g, gdot;
+  source_eval(w->f0, w->p0, w->c0, tn, &g, &gdot);
+  return w->model ? g + w->s_src * gdot : g;
 }
 // g_m(t) of every member (ensemble models): g[m], m < nv
 void source_amplitudes(const wfx_wave* w, double tn, double* g)
 {
   for (int m = 0; m < w->nv; ++m) g[m] = source_amplitude(w->f0s[m], w->p0s[m], w->c0, tn);
+}
+// the boundary term with the source profile at stage time tn (t_dev: read it from there, graph capture)
+void boundary_profiled(wfx_wave* w, double tn, const double* t_dev, const void* vn, cudaStream_t st)
+{
+  SourceParams sp{};
+  for (int m = 0; m < w->nv; ++m)
+  {
+    sp.f0[m] = w->ens ? w->f0s[m] : w->f0;
+    sp.p0[m] = w->ens ? w->p0s[m] : w->p0;
+  }
+  boundary_apply_profile(w->bnd, w->nv, w->c0, w->model ? w->s_src : 0.0, sp, tn, t_dev, w->prof_amp.p,
+                         w->prof_delay.p, vn, w->b.p, st);
 }
 } // namespace
 
@@ -838,7 +853,8 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
     double g[WFX_ENSEMBLE_MAX];
     source_amplitudes(w, t, g);
     if (wfx_stiffness_apply_ensemble(w->stiff, w->nv, u, nullptr, w->b.p, 0, st)) fail("%s", wfx_last_error());
-    boundary_apply_ens(w->bnd, w->nv, w->c0, g, nullptr, v, w->b.p, st);
+    if (w->prof_on) boundary_profiled(w, t, nullptr, v, st);
+    else boundary_apply_ens(w->bnd, w->nv, w->c0, g, nullptr, v, w->b.p, st);
     const int64_t n = w->n * w->nv;
     if (n == 0) return 0;
     const unsigned grid = (unsigned)((n + 255) / 256);
@@ -857,7 +873,8 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
     if (w->f1_w.n != nb) w->f1_w.alloc(nb);
     launch_axpy(w, u, v, w->s_stiff, w->f1_w.p, st);
     if (wfx_stiffness_apply(w->stiff, w->f1_w.p, w->b.p, 0, st)) fail("%s", wfx_last_error());
-    if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());
+    if (w->prof_on) boundary_profiled(w, t, nullptr, v, st);
+    else if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());
     if (w->qc != 0) boundary_absorbing_mass(w->bnd, w->m64, w->qc, w->kappa, 0.0, u, v, w->b.p, st);
     if (w->n == 0) return 0;
     const unsigned grid = (unsigned)((w->n + 255) / 256);
@@ -872,7 +889,8 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
   }
   if (wfx_stiffness_apply(w->stiff, u, w->b.p, 0, st)) fail("%s", wfx_last_error());                     // :173-174
   if (w->halo && wfx_halo_update_rev_fwd(w->halo, w->b.p, st)) fail("%s", wfx_last_error());             // :176
-  if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());       // :175
+  if (w->prof_on) boundary_profiled(w, t, nullptr, v, st);
+  else if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());  // :175
   if (wfx_mass_apply_inverse(w->mass, w->b.p, result, st)) fail("%s", wfx_last_error());                 // :188-191
   WFX_API_END
 }
@@ -909,11 +927,13 @@ extern "C" int wfx_wave_rk4(wfx_wave* w, double t0, double tf, double dt, int64_
     NvtxRange step_range("wfx rk4 step");
     dt = std::min(dt, tf - t); // :242
     double g[4 * WFX_ENSEMBLE_MAX]; // [stage][member]
+    double tn[4];
     for (int i = 0; i < 4; ++i)
     {
-      const double tn = t + c_runge[i] * dt; // :257
-      if (w->ens) source_amplitudes(w, tn, g + i * w->nv);
-      else g[i] = source_amplitude(w, tn); // :155-162
+      tn[i] = t + c_runge[i] * dt; // :257
+      if (w->prof_on) continue;    // the boundary term evaluates the delayed sources on the device
+      if (w->ens) source_amplitudes(w, tn[i], g + i * w->nv);
+      else g[i] = source_amplitude(w, tn[i]); // :155-162
     }
     if (graph_ok && dt == dt_nominal)
     {
@@ -925,7 +945,7 @@ extern "C" int wfx_wave_rk4(wfx_wave* w, double t0, double tf, double dt, int64_
         WFX_CUDA(cudaStreamBeginCapture(ws, cudaStreamCaptureModeThreadLocal));
         try
         {
-          enqueue_step(w, dt, nullptr, true, ws);
+          enqueue_step(w, dt, nullptr, nullptr, true, ws);
         }
         catch (...)
         {
@@ -939,7 +959,8 @@ extern "C" int wfx_wave_rk4(wfx_wave* w, double t0, double tf, double dt, int64_
         WFX_CUDA(ie);
         w->graph_dt = dt;
       }
-      if (w->ens)
+      if (w->prof_on) set_source_kernel<<<1, 1, 0, ws>>>(w->t_dev.p, tn[0], tn[1], tn[2], tn[3]);
+      else if (w->ens)
       {
         StepAmp a{};
         for (int q = 0; q < 4 * w->nv; ++q) a.g[q] = g[q];
@@ -948,7 +969,7 @@ extern "C" int wfx_wave_rk4(wfx_wave* w, double t0, double tf, double dt, int64_
       else set_source_kernel<<<1, 1, 0, ws>>>(w->g_dev.p, g[0], g[1], g[2], g[3]);
       WFX_CUDA(cudaGraphLaunch(w->step_graph, ws));
     }
-    else enqueue_step(w, dt, g, false, ws);
+    else enqueue_step(w, dt, g, tn, false, ws);
     t += dt;
     step += 1;
     w->steps_done += 1;
@@ -1073,6 +1094,52 @@ extern "C" int wfx_wave_get_field_stats(wfx_wave* w, int64_t* nsamples, double* 
     const double scale = w->stats_n ? 2.0 / (double)w->stats_n : 0.0;
     for (size_t i = 0; i < 2 * w->stats_harm.n; ++i) harm_host[i] *= scale;
   }
+  WFX_API_END
+}
+
+extern "C" int wfx_wave_set_source_profile(wfx_wave* w, const double* amp_host, const double* delay_host)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  if (!w->bnd) fail("source profile: the model has no boundary operator");
+  if (w->halo) fail("source profile: one rank only (the model is distributed)");
+  const int64_t ne = w->n * w->nv;
+  for (int64_t k = 0; k < ne; ++k)
+  {
+    if (amp_host && !std::isfinite(amp_host[k])) fail("source profile: non-finite amplitude at entry %lld", (long long)k);
+    if (delay_host && !std::isfinite(delay_host[k])) fail("source profile: non-finite delay at entry %lld", (long long)k);
+    if (delay_host && delay_host[k] < 0) fail("source profile: negative delay at entry %lld", (long long)k);
+  }
+  ScopedDevice sd(w->ctx->device);
+  // a step in flight may read the buffers, and the captured step holds the other boundary kernel (or these buffers)
+  WFX_CUDA(cudaDeviceSynchronize());
+  if (w->step_graph) WFX_CUDA(cudaGraphExecDestroy(w->step_graph));
+  w->step_graph = nullptr;
+  w->prof_on = false;
+  if (!amp_host && !delay_host)
+  {
+    w->prof_amp.release();
+    w->prof_delay.release();
+    return 0;
+  }
+  // compact onto the boundary term's dof list: entry (p, m) <- state entry (dofs[p], m)
+  const std::vector<int32_t>& dofs = boundary_dofs(w->bnd);
+  const int nv = w->nv;
+  const size_t nbv = dofs.size() * (size_t)nv;
+  std::vector<double> a(nbv, 1.0), d(nbv, 0.0);
+  for (size_t p = 0; p < dofs.size(); ++p)
+    for (int m = 0; m < nv; ++m)
+    {
+      const size_t i = (size_t)dofs[p] * nv + m;
+      if (amp_host) a[p * nv + m] = amp_host[i];
+      if (delay_host) d[p * nv + m] = delay_host[i];
+    }
+  // each buffer on its own: after a failed allocation (out of memory) a retry allocates what is missing
+  if (w->prof_amp.n != nbv) w->prof_amp.alloc(nbv);
+  if (w->prof_delay.n != nbv) w->prof_delay.alloc(nbv);
+  w->prof_amp.upload(a);
+  w->prof_delay.upload(d);
+  w->prof_on = true;
   WFX_API_END
 }
 

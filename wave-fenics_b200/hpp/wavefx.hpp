@@ -330,6 +330,15 @@ inline void read_field_stats(wfx_wave* wave, std::int64_t entries, FieldStats& o
   check(wfx_wave_get_field_stats(wave, &out.samples, &out.t_first, &out.t_last, out.pmax.data(), out.pmin.data(),
                                  reinterpret_cast<double*>(out.harmonics.data())));
 }
+// wfx_wave_set_source_profile over `entries` state entries; an empty vector is passed as NULL
+inline void set_profile(wfx_wave* wave, std::int64_t entries, const std::vector<double>& amp,
+                        const std::vector<double>& delay)
+{
+  for (const auto* a : {&amp, &delay})
+    if (!a->empty() && (std::int64_t)a->size() != entries)
+      throw std::runtime_error("wavefx: source profile arrays must hold one entry per state entry (or none)");
+  check(wfx_wave_set_source_profile(wave, amp.empty() ? nullptr : amp.data(), delay.empty() ? nullptr : delay.data()));
+}
 
 // The wave model and its RK4 driver (common/LinearGLL.hpp:37-287), fp64 like the reference.
 class LinearGLLOpt
@@ -406,6 +415,12 @@ public:
     check(wfx_wave_set_field_stats(_wave, enable ? 1 : 0, t_start, nharm));
   }
   void field_stats(FieldStats& out) const { read_field_stats(_wave, _ndofs, out); }
+  // phased-array source on tag 1 (DESIGN.md section 4.5c): amp[i] g(t - delay[i]) in place of g(t), ndofs entries
+  // each; an empty vector stands for amp = 1 / delay = 0, both empty clear the profile
+  void set_source_profile(const std::vector<double>& amp, const std::vector<double>& delay)
+  {
+    set_profile(_wave, _ndofs, amp, delay);
+  }
   // fn(step, t, u, v) every `every` steps with pointers into pinned host copies (ndofs entries each);
   // the device -> host copy overlaps the time stepping.  A checkpoint is a snapshot handed back to
   // set_state.
@@ -556,6 +571,11 @@ public:
     check(wfx_wave_set_field_stats(_wave, enable ? 1 : 0, t_start, nharm));
   }
   void field_stats(FieldStats& out) const { read_field_stats(_wave, _ndofs * _nv, out); }
+  // as LinearGLLOpt's, member m with its own profile: amp, delay [ndofs][nv] (member-interleaved)
+  void set_source_profile(const std::vector<double>& amp, const std::vector<double>& delay)
+  {
+    set_profile(_wave, _ndofs * _nv, amp, delay);
+  }
   void set_state(const std::vector<double>& u, const std::vector<double>& v)
   {
     if ((std::int64_t)u.size() != _ndofs * _nv || (std::int64_t)v.size() != _ndofs * _nv)

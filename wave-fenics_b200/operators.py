@@ -342,6 +342,15 @@ class BoundaryOperator(_Operator):
             self.handle = None
 
 
+def focus_delays(points, focus, c0):
+    """Delays that focus a phased-array source at `focus`: tau_i = (max_j d_j - d_i) / c0 with d_i = |x_i - focus|,
+    for points [n, 3] (e.g. dof_coordinates(mesh)).  Every tau_i >= 0; the farthest point fires first (tau = 0), so
+    all contributions reach the focus at the same time."""
+    x = np.asarray(points, dtype=np.float64)
+    d = np.linalg.norm(x - np.asarray(focus, dtype=np.float64).reshape(1, -1), axis=1)
+    return (d.max() - d) / float(c0) if len(d) else d
+
+
 class LinearGLLOpt:
     """The wave model + RK4 driver (common/LinearGLL.hpp:37-287) on the GPU.
 
@@ -443,6 +452,25 @@ class LinearGLLOpt:
                   C.c_void_p(pmax.ctypes.data), C.c_void_p(pmin.ctypes.data),
                   C.cast(C.c_void_p(harm.ctypes.data), capi._c_f64p))
         return FieldStats(n.value, t0.value, t1.value, pmax, pmin, harm)
+
+    def set_source_profile(self, amplitude=None, delay=None):
+        """Phased-array source on tag 1 (DESIGN.md section 4.5c): the boundary term uses amplitude[i] g(t - delay[i])
+        at every entry i in place of g(t), with g(s) = g'(s) = 0 for s < 0.  Arrays shaped like the state
+        ((ndofs,), or (ndofs, nv) for an ensemble); entries off tag 1 are ignored.  None stands for 1 (amplitude)
+        or 0 (delay); set_source_profile() clears the profile.  The profile survives init, set_state and
+        restarts.  Delays are >= 0, see focus_delays."""
+        shape = self._entry_shape()
+
+        def arr(a):
+            if a is None:
+                return None
+            a = np.ascontiguousarray(a, dtype=np.float64)
+            if a.shape != shape:
+                raise capi.WfxError(f"source profile arrays must have shape {shape}")
+            return a
+
+        amplitude, delay = arr(amplitude), arr(delay)
+        capi.call("wfx_wave_set_source_profile", self.handle, capi.f64p(amplitude), capi.f64p(delay))
 
     def set_snapshot(self, every, fn):
         """fn(step, t, u, v) with numpy views of the pinned host copies (copy them to keep them), every
