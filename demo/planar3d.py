@@ -17,11 +17,17 @@ on the axis through the centre of the source face, and the four lateral faces ab
 are then reported along that axis: the position and value of the maximum of |p1| and of pmax.  For a small
 aperture (Fresnel number a^2 / (lambda DEPTH) of a few) that maximum lies short of DEPTH, as the Rayleigh integral
 predicts.
+--heat-seconds S (with --stats-periods) heats tissue with the acoustic field (DESIGN.md section 4.5d): a Pennes thermal
+model on the same mesh and operators takes its heat source Q = sum_h alpha0 (h f0 / 1 MHz)^y |p_h|^2 / (rho0 c0) from
+the harmonic maps, is heated for S seconds and cools for --cool-seconds C with the source off, and reports the peak
+temperature rise, the maximum CEM43 thermal dose, and the number of dofs and the volume at or above 240 min.
+--absorption alpha0 [Np/m at 1 MHz] and --absorption-power y set the tissue absorption.
 The reference reads `../mesh.xdmf` (not in its repository); here the mesh is a structured
 n x m x m hexahedral box with tag 1 on x = 0 (source) and tag 2 on x = L (absorbing).
 
     python demo/planar3d.py [--nx 32] [--nyz 4] [--length 0.1] [--steps N] [--check]
                             [--model linear|lossy|westervelt] [--stats-periods K] [--focus DEPTH] [--aperture R]
+                            [--heat-seconds S] [--cool-seconds C] [--absorption ALPHA0] [--absorption-power Y]
 """
 import argparse
 import os
@@ -63,7 +69,14 @@ def main():
                     help="focal depth [m] on the axis through the centre of the source face (0: plane source)")
     ap.add_argument("--aperture", type=float, default=0.0,
                     help="with --focus: source radius [m] around the face centre (0: the whole face)")
+    ap.add_argument("--heat-seconds", type=float, default=0.0,
+                    help="with --stats-periods: heat tissue with the field's harmonic maps for S seconds (0: off)")
+    ap.add_argument("--cool-seconds", type=float, default=0.0, help="cooling after the heating, source off")
+    ap.add_argument("--absorption", type=float, default=5.0, help="tissue absorption alpha0 [Np/m at 1 MHz]")
+    ap.add_argument("--absorption-power", type=float, default=1.1, help="frequency power law y of the absorption")
     args = ap.parse_args()
+    if args.heat_seconds > 0 and args.stats_periods <= 0:
+        ap.error("--heat-seconds needs --stats-periods (the heat source comes from the harmonic maps)")
 
     speedOfSound, sourceFrequency, pressureAmplitude = 1500.0, 0.5e6, 60000.0   # main.cpp:25-30
     period = 1.0 / sourceFrequency
@@ -131,6 +144,10 @@ def main():
             if args.focus > 0:
                 print(f"on-axis maximum: |p1| = {p1.max():.6e} at x = {x[p1.argmax()]:.5f}, "
                       f"pmax = {pmax.max():.6e} at x = {x[pmax.argmax()]:.5f} (focus requested at x = {args.focus:.5f})")
+        if args.heat_seconds > 0 and fs.samples == 0:
+            print("thermal: skipped, the statistics window holds no samples (no heat source without harmonics)")
+        elif args.heat_seconds > 0:
+            heat(args, eqn, speedOfSound)
     else:
         print(f"max |p| = {np.abs(u).max():.6e} at x = {X[np.abs(u).argmax(), 0]:.4f}")
     if args.check:
@@ -158,6 +175,33 @@ def main():
                                         nthreads=oracle.max_threads())
         print(f"relative L2 difference to the CPU oracle: u {np.linalg.norm(u - uo) / np.linalg.norm(uo):.3e}"
               f"  v {np.linalg.norm(v - vo) / np.linalg.norm(vo):.3e}")
+
+
+def heat(args, eqn, c0, k=0.5, rhoc=3.6e6, perfusion=2.0e3, T_art=37.0):
+    """HIFU heating from the wave model's harmonic maps: soft-tissue-like k [W/(m K)], rhoC [J/(m^3 K)] and
+    perfusion wbCb [W/(m^3 K)], all faces insulated"""
+    th = wfx.PennesGLL.from_wave(eqn, k, rhoc, perfusion, T_art)
+    th.heat_from_wave(eqn, args.absorption, args.absorption_power, args.rho0, c0)
+    dt = th.stable_dt()
+    th.init()
+    eqn.ctx.synchronize()
+    t0 = time.perf_counter()
+    th.set_heat_scale(1.0)
+    n1, t = th.rk4(0.0, args.heat_seconds, dt)
+    T_heat = th.get_state()
+    n2 = 0
+    if args.cool_seconds > 0:
+        th.set_heat_scale(0.0)
+        n2, t = th.rk4(t, args.heat_seconds + args.cool_seconds, dt)
+    eqn.ctx.synchronize()
+    d = th.dose()
+    lesion = d.cem43 >= 240.0
+    m = eqn.mass_op.diagonal().astype(np.float64)
+    print(f"thermal: Q max {th.heat_source().max():.6e} W/m^3, dt = {dt:.6e} s, {n1} heating + {n2} cooling steps "
+          f"in {time.perf_counter() - t0:.3f} s")
+    print(f"thermal: peak rise {d.T_max.max() - T_art:.6e} K (at the end of heating {T_heat.max() - T_art:.6e} K), "
+          f"max CEM43 {d.cem43.max():.6e} min, {int(lesion.sum())} dofs >= 240 min, "
+          f"volume {m[lesion].sum():.6e} m^3 >= 240 min")
 
 
 if __name__ == "__main__":

@@ -409,6 +409,64 @@ typedef void (*wfx_snapshot_fn)(void* user, int64_t step, double t, const void* 
 int wfx_wave_set_snapshot(wfx_wave* wave, int64_t every, wfx_snapshot_fn fn, void* user);
 int wfx_wave_destroy(wfx_wave* wave);
 
+/* ---- thermal model: Pennes bioheat equation + RK4 with a CEM43 thermal dose (DESIGN.md section 4.5d) ------
+ * State: the temperature rise theta = T - T_art over the arterial temperature, in the operators' dtype.
+ *   rhoC theta_t = div(k grad theta) - wbCb theta + s Q            in the domain
+ *   -k d theta / dn = h_j (theta - (T_ext_j - T_art))              on the tag-j facets, j = 1, 2
+ * all other faces insulated.  Lumped GLL system per dof i (m: lumped mass, m1 / m2: the facet masses of bnd):
+ *   theta_i' = scale_i [-cK^2 K theta]_i - r_i theta_i + f_i,   scale_i = (k / cK^2) / (rhoC_i m_i)
+ *   r_i = (wbCb_i m_i + h1 m1_i + h2 m2_i) / (rhoC_i m_i)
+ *   f_i = (h1 m1_i (T_ext1 - T_art) + h2 m2_i (T_ext2 - T_art) + s Q_i m_i) / (rhoC_i m_i)
+ * with cK the stiffness operator's c0, so that the diffusion term is one fused wfx_stiffness_apply_scaled.  A
+ * per-cell conductivity k_c is the operator's geometry scaled by wfx_geometry_scale_cells(k_c / k) before the
+ * stiffness operator is created.  The model borrows the operators (they must outlive it) and may share them with
+ * a wave model whose geometry is unscaled.  One rank only.
+ * k [W/(m K)] > 0; rhoc_host [ndofs] [J/(m^3 K)] > 0; perf_host [ndofs] (wbCb [W/(m^3 K)]) >= 0 or NULL (0);
+ * h_host[2] [W/(m^2 K)] >= 0 or NULL (insulated); T_ext_host[2] or NULL (T_art); h != 0 needs bnd.  All finite.
+ * Per-cell rhoC and wbCb enter as mass-weighted averages sum_c coeff_c (detJ w)_{c,i} / m_i (INTEGRATION.md).
+ * The heat source Q starts at 0 and the heat scale s at 1.
+ *
+ * Dose: after every completed step of size dt_n, with T_i = T_art + theta_i at its end,
+ *   CEM43_i += (dt_n / 60) R^(43 - T_i),  R = 0.5 for T_i >= 43, else 0.25   (fp64; t in s, CEM43 in min)
+ *   theta_max_i = max(theta_max_i, theta_i)                                  (model dtype, NaN propagates)
+ * init and set_state reset both (CEM43 = 0, theta_max = -inf) and the step count; a run split over several rk4
+ * calls keeps accumulating. */
+typedef struct wfx_thermal wfx_thermal;
+int wfx_thermal_create(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass, wfx_boundary* bnd, double k,
+                       const double* rhoc_host, const double* perf_host, double T_art, const double* h_host,
+                       const double* T_ext_host, wfx_thermal** th);
+int wfx_thermal_init(wfx_thermal* th); /* theta = 0 */
+int wfx_thermal_set_state(wfx_thermal* th, const void* theta_host);
+int wfx_thermal_get_state(wfx_thermal* th, void* theta_host);
+int wfx_thermal_state_ptr(wfx_thermal* th, void** theta_dev);
+/* Q [W/m^3] per dof, fp64; NULL: Q = 0.  Non-finite values are refused. */
+int wfx_thermal_set_heat_source(wfx_thermal* th, const double* q_host);
+/* Q from the harmonic maps of a wave model's field statistics (wfx_wave_set_field_stats), on the device:
+ *   Q_i = sum_{h=1..H} alpha_i(h f0_m) |p_h,i|^2 / (rho0 c0),   alpha_i(f) = alpha0_i (f / 1 MHz)^y  [Np/m]
+ * with p_h = (2 / N) times the accumulated sums (as wfx_wave_get_field_stats scales them), member m's amplitudes
+ * and source frequency f0_m (m = 0 for a single-field model).  alpha0_host [ndofs] or NULL (alpha0 everywhere).
+ * Refused: statistics off, N = 0 or H = 0, member out of range, a wave on another context or with another ndofs,
+ * alpha0 < 0, rho0 <= 0, c0 <= 0 or non-finite parameters. */
+int wfx_thermal_heat_from_wave(wfx_thermal* th, wfx_wave* wave, int member, double alpha0,
+                               const double* alpha0_host, double y, double rho0, double c0);
+int wfx_thermal_get_heat_source(wfx_thermal* th, double* q_host);
+/* s >= 0, finite: duty cycles; heating then cooling is two rk4 calls with s = 1 and s = 0 */
+int wfx_thermal_set_heat_scale(wfx_thermal* th, double s);
+/* out = theta' at theta (device vectors of ndofs entries, model dtype); out must not alias theta */
+int wfx_thermal_rhs(wfx_thermal* th, const void* theta_dev, void* out_dev, void* stream);
+/* classical RK4 from t0 to tf (loop of wfx_wave_rk4: while t < tf, dt = min(dt, tf - t)); max_steps <= 0: run
+ * to tf.  Graph replay on one rank as wfx_wave_rk4 (WFX_WAVE_GRAPH=0 switches it off). */
+int wfx_thermal_rk4(wfx_thermal* th, double t0, double tf, double dt, int64_t max_steps, int64_t* steps,
+                    double* t_end, void* stream);
+/* steps since init / set_state; cem43_host [ndofs] fp64, theta_max_host [ndofs] model dtype; any may be NULL */
+int wfx_thermal_get_dose(wfx_thermal* th, int64_t* nsteps, double* cem43_host, void* theta_max_host);
+/* Power iteration (iters >= 1 applications, deterministic) for the largest eigenvalue lambda of theta -> -theta'
+ * without its source (self-adjoint in the rhoC m inner product), estimated by the Rayleigh quotient, and
+ * dt_max = 2.785293563405282 / lambda, the RK4 stability limit on the negative real axis.  The estimate
+ * approaches lambda from below, so dt_max is an upper bound's estimate: step with a safety factor (e.g. 0.8). */
+int wfx_thermal_stable_dt(wfx_thermal* th, int iters, double* lambda, double* dt_max);
+int wfx_thermal_destroy(wfx_thermal* th);
+
 #ifdef __cplusplus
 }
 #endif

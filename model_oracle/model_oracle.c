@@ -221,3 +221,73 @@ int64_t wo_rk4_westervelt_profile(int P, int64_t ncells, int64_t ndofs, const in
   free(u_); free(v_); free(un); free(vn); free(u0); free(v0); free(ku); free(kv); free(b); free(bv);
   return step;
 }
+
+/* ---- thermal model: Pennes bioheat equation (DESIGN.md section 4.5d) ------------------------------------------
+ * State theta = T - T_art.  Lumped GLL system per dof i, written out plainly (one quotient, no precomputed scale,
+ * r or f), with A = -1500^2 K the oracle's stiffness, so that (k / 1500^2) A theta = -k K theta:
+ *   rhoC_i m_i theta_i' = (k / 1500^2) [A theta]_i - (wbCb_i m_i + h1 m1_i + h2 m2_i) theta_i
+ *                         + h1 m1_i (T_ext1 - T_art) + h2 m2_i (T_ext2 - T_art) + s Q_i m_i
+ * perf and Q may be NULL (0). */
+void wo_rhs_pennes(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G, const double* m,
+                   const double* m1, const double* m2, double k, const double* rhoc, const double* perf, double T_art,
+                   double h1, double h2, double T_ext1, double T_ext2, const double* Q, double s, const double* theta,
+                   double* out, int sumfact, int nthreads)
+{
+  memset(out, 0, sizeof(double) * ndofs);
+  model_stiffness(P, ncells, ndofs, dofmap, G, theta, out, sumfact, nthreads); /* A theta */
+  for (int64_t i = 0; i < ndofs; ++i)
+  {
+    const double wb = perf ? perf[i] : 0.0, q = Q ? Q[i] : 0.0;
+    double num = k / (1500.0 * 1500.0) * out[i];
+    num -= (wb * m[i] + h1 * m1[i] + h2 * m2[i]) * theta[i];
+    num += h1 * m1[i] * (T_ext1 - T_art) + h2 * m2[i] * (T_ext2 - T_art) + s * q * m[i];
+    out[i] = num / (rhoc[i] * m[i]);
+  }
+}
+
+/* RK4 of the thermal model: the stage loop of wo_rk4_westervelt on theta alone.  After every step of size dt,
+ * with T = T_art + theta:  cem43 += dt / 60 * R^(43 - T) (R = 0.5 for T >= 43, else 0.25) and
+ * theta_max = max(theta_max, theta) (a NaN theta replaces the maximum).  theta, cem43, theta_max: in / out.
+ * Returns the number of steps; *t_end the final time. */
+int64_t wo_rk4_pennes(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G, const double* m,
+                      const double* m1, const double* m2, double k, const double* rhoc, const double* perf,
+                      double T_art, double h1, double h2, double T_ext1, double T_ext2, const double* Q, double s,
+                      double t0, double tf, double dt, int64_t max_steps, double* theta, double* cem43,
+                      double* theta_max, int sumfact, int nthreads, double* t_end)
+{
+  const double a_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  const double b_runge[4] = {1.0 / 6.0, 1.0 / 3.0, 1.0 / 3.0, 1.0 / 6.0};
+  const size_t nb = sizeof(double) * ndofs;
+  double *u_ = malloc(nb), *un = malloc(nb), *u0 = malloc(nb), *kv = malloc(nb);
+  memcpy(u_, theta, nb);
+  memset(kv, 0, nb);
+  double t = t0;
+  int64_t step = 0;
+  while (t < tf)
+  {
+    if (max_steps > 0 && step >= max_steps) break;
+    dt = dt < tf - t ? dt : tf - t;
+    memcpy(u0, u_, nb);
+    for (int i = 0; i < 4; ++i)
+    {
+      const double adt = dt * a_runge[i];
+      for (int64_t j = 0; j < ndofs; ++j) un[j] = kv[j] * adt + u0[j];
+      wo_rhs_pennes(P, ncells, ndofs, dofmap, G, m, m1, m2, k, rhoc, perf, T_art, h1, h2, T_ext1, T_ext2, Q, s, un,
+                    kv, sumfact, nthreads);
+      const double bdt = dt * b_runge[i];
+      for (int64_t j = 0; j < ndofs; ++j) u_[j] = kv[j] * bdt + u_[j];
+    }
+    for (int64_t j = 0; j < ndofs; ++j)
+    {
+      const double T = T_art + u_[j];
+      cem43[j] += dt / 60.0 * pow(T >= 43.0 ? 0.5 : 0.25, 43.0 - T);
+      if (u_[j] > theta_max[j] || u_[j] != u_[j]) theta_max[j] = u_[j];
+    }
+    t += dt;
+    step += 1;
+  }
+  memcpy(theta, u_, nb);
+  if (t_end) *t_end = t;
+  free(u_); free(un); free(u0); free(kv);
+  return step;
+}

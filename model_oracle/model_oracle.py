@@ -1,4 +1,5 @@
-"""ctypes loader for the CPU restatement of the lossy and Westervelt models (model_oracle.c).
+"""ctypes loader for the CPU restatement of the lossy and Westervelt models and of the Pennes thermal model
+(model_oracle.c).
 
 TEST INFRASTRUCTURE ONLY -- imported by tests/, the demo's --check and tools/, never by the product package.
 Built with the strict flags of oracle/oracle.py, so that its linear part computes what the oracle computes.
@@ -69,6 +70,12 @@ def lib():
         L.wo_rk4_westervelt_profile.restype = l
         L.wo_rk4_westervelt_profile.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, d, d, _f64p,
                                                 _f64p, d, d, d, l, _f64p, _f64p, i, i, _f64p]
+        L.wo_rhs_pennes.restype = None
+        L.wo_rhs_pennes.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, d, _f64p, _f64p, d, d, d, d, d, _f64p,
+                                    d, _f64p, _f64p, i, i]
+        L.wo_rk4_pennes.restype = l
+        L.wo_rk4_pennes.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, d, _f64p, _f64p, d, d, d, d, d, _f64p,
+                                    d, d, d, d, l, _f64p, _f64p, _f64p, i, i, _f64p]
         _lib.append(L)
     return _lib[0]
 
@@ -135,4 +142,38 @@ def rk4_westervelt_profile(mesh, P, G, m, m1, m2, c0, f0, p0, delta, beta, rho0,
                                             _f(m), _f(m1), _f(m2), c0, f0, p0, delta, beta, rho0, _f(amp), _f(delay),
                                             t0, tf, dt, max_steps, _f(u), _f(v), int(sumfact), nthreads,
                                             C.byref(t_end))
+    return steps, t_end.value
+
+
+def _opt(a):
+    return None if a is None else _f(np.ascontiguousarray(a, dtype=np.float64))
+
+
+def rhs_pennes(mesh, P, G, m, m1, m2, k, rhoc, perf, T_art, h, T_ext, Q, s, theta, sumfact=False, nthreads=1):
+    """theta' of the lumped Pennes system (DESIGN.md section 4.5d) at theta = T - T_art.  rhoc [ndofs]; perf, Q
+    [ndofs] or None (0); h, T_ext: the two Robin tags' (h1, h2) and (T_ext1, T_ext2)."""
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    rhoc = np.ascontiguousarray(rhoc, dtype=np.float64)
+    perf = None if perf is None else np.ascontiguousarray(perf, dtype=np.float64)
+    Q = None if Q is None else np.ascontiguousarray(Q, dtype=np.float64)
+    out = np.empty(mesh.ndofs)
+    lib().wo_rhs_pennes(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)), _f(m), _f(m1), _f(m2),
+                        k, _f(rhoc), _opt(perf), T_art, h[0], h[1], T_ext[0], T_ext[1], _opt(Q), s,
+                        _f(np.ascontiguousarray(theta, dtype=np.float64)), _f(out), int(sumfact), nthreads)
+    return out
+
+
+def rk4_pennes(mesh, P, G, m, m1, m2, k, rhoc, perf, T_art, h, T_ext, Q, s, t0, tf, dt, theta, cem43, theta_max,
+               max_steps=0, sumfact=False, nthreads=1):
+    """RK4 of the Pennes model with the CEM43 dose and the peak rise; theta, cem43, theta_max updated in place.
+    -> (steps, t_end)"""
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    rhoc = np.ascontiguousarray(rhoc, dtype=np.float64)
+    perf = None if perf is None else np.ascontiguousarray(perf, dtype=np.float64)
+    Q = None if Q is None else np.ascontiguousarray(Q, dtype=np.float64)
+    t_end = C.c_double()
+    steps = lib().wo_rk4_pennes(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)), _f(m), _f(m1),
+                                _f(m2), k, _f(rhoc), _opt(perf), T_art, h[0], h[1], T_ext[0], T_ext[1], _opt(Q), s,
+                                t0, tf, dt, max_steps, _f(theta), _f(cem43), _f(theta_max), int(sumfact), nthreads,
+                                C.byref(t_end))
     return steps, t_end.value

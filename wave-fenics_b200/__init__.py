@@ -8,5 +8,5 @@ from . import capi  # noqa: F401  (raises when libwavefx.so is missing: no CPU f
 from .capi import WfxError  # noqa: F401
 from .mesh import HexMesh, create_box_hex, cfl_timestep, dof_coordinates  # noqa: F401
 from .operators import (BoundaryOperator, Context, FieldStats, Geometry, LinearGLLEnsemble, LinearGLLOpt,  # noqa: F401
-                        LossyGLLOpt, MassOperator, MassOperatorCPU, StiffnessOperator, WesterveltGLLOpt,
-                        compute_jacobian_data, focus_delays)
+                        LossyGLLOpt, MassOperator, MassOperatorCPU, PennesGLL, StiffnessOperator, ThermalDose,
+                        WesterveltGLLOpt, cell_to_dof_average, compute_jacobian_data, focus_delays)

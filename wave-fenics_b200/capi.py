@@ -125,6 +125,20 @@ _SIG = {
     "wfx_wave_set_source_profile": [_vp, _c_f64p, _c_f64p],
     "wfx_wave_set_snapshot": [_vp, C.c_int64, _vp, _vp],
     "wfx_wave_destroy": [_vp],
+    "wfx_thermal_create": [_vp, _vp, _vp, _vp, C.c_double, _c_f64p, _c_f64p, C.c_double, _c_f64p, _c_f64p, _vpp],
+    "wfx_thermal_init": [_vp],
+    "wfx_thermal_set_state": [_vp, _vp],
+    "wfx_thermal_get_state": [_vp, _vp],
+    "wfx_thermal_state_ptr": [_vp, _vpp],
+    "wfx_thermal_set_heat_source": [_vp, _c_f64p],
+    "wfx_thermal_heat_from_wave": [_vp, _vp, C.c_int, C.c_double, _c_f64p, C.c_double, C.c_double, C.c_double],
+    "wfx_thermal_get_heat_source": [_vp, _c_f64p],
+    "wfx_thermal_set_heat_scale": [_vp, C.c_double],
+    "wfx_thermal_rhs": [_vp, _vp, _vp, _vp],
+    "wfx_thermal_rk4": [_vp, C.c_double, C.c_double, C.c_double, C.c_int64, _c_i64p, _c_f64p, _vp],
+    "wfx_thermal_get_dose": [_vp, _c_i64p, _c_f64p, _vp],
+    "wfx_thermal_stable_dt": [_vp, C.c_int, _c_f64p, _c_f64p],
+    "wfx_thermal_destroy": [_vp],
     "wfx_debug_structured_coords": [C.c_int64, C.c_int64, _c_i32p, _c_i32p, C.POINTER(C.c_int)],
     # debug helper (not in wavefx.h): host-only plan construction + verification
     "wfx_debug_stream_plan_check": [C.c_int, C.c_int64, C.c_int64, _c_i32p, C.POINTER(C.c_float), C.c_int, C.c_int,

@@ -359,6 +359,7 @@ namespace wfx
 {
 bool boundary_assembled(const wfx_boundary* op) { return op->assembled; }
 int boundary_dtype(const wfx_boundary* op) { return op->dtype; }
+int64_t boundary_ndofs(const wfx_boundary* op) { return op->ndofs; }
 const std::vector<int32_t>& boundary_dofs(const wfx_boundary* op) { return op->h_idx; }
 } // namespace wfx
 

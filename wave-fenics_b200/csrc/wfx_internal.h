@@ -107,8 +107,10 @@ bool stiffness_graph_safe(const struct ::wfx_stiffness* op); // its launches may
 int halo_dtype(const struct ::wfx_halo* h);                // wfx_halo.cu
 bool mass_assembled(const struct ::wfx_mass* op);          // wfx_mass.cu: diagonal summed over the ranks
 int mass_dtype(const struct ::wfx_mass* op);
+int64_t mass_ndofs(const struct ::wfx_mass* op);          // length of the diagonal
 bool boundary_assembled(const struct ::wfx_boundary* op);  // wfx_boundary.cu: facet masses summed over the ranks
 int boundary_dtype(const struct ::wfx_boundary* op);
+int64_t boundary_ndofs(const struct ::wfx_boundary* op);  // length of the vectors it adds into
 // wfx_boundary_apply with the source amplitude g read from device memory at run time (CUDA-graph
 // replays of a time step change g without touching the graph), wfx_boundary.cu
 void boundary_apply_dev(struct ::wfx_boundary* op, double c0, const double* g_dev, const void* vn, void* b,
@@ -140,6 +142,21 @@ const double* mass_diagonal64(const struct ::wfx_mass* op);   // m on the device
 // kv = (b minv + kappa pd^2) / (1 - kappa p) yields it; p = pw - s pd (s = 0: pw is p itself)
 void boundary_absorbing_mass(struct ::wfx_boundary* op, const double* m64, double qc, double kappa, double s,
                              const void* pw, const void* pd, void* b, cudaStream_t stream);
+// A wave model's field statistics as the thermal model reads them (wfx_thermal_heat_from_wave, DESIGN.md section
+// 4.5d): the unscaled fp64 harmonic sums, planes [h][ndofs * nv] (entry (dof i, member m) at i nv + m), the number
+// of sampled steps N (the amplitudes are the sums times 2 / N) and every member's source frequency (wfx_wave.cu)
+struct WaveFieldStats
+{
+  wfx_ctx* ctx = nullptr;
+  int64_t ndofs = 0;
+  int nv = 1;
+  bool on = false;
+  int nharm = 0;
+  int64_t nsamples = 0;
+  const double2* harm = nullptr;
+  double f0[WFX_ENSEMBLE_MAX] = {};
+};
+WaveFieldStats wave_field_stats(const struct ::wfx_wave* w);
 
 // NVTX ranges around the phases of a time step (the reference marks its profiled regions the same
 // way: demo/gpu_scatter_mpi/main.cpp:101-121, demo/gpu_cg/CUDA/cg.hpp:74-113).  nvtx3 is header-only

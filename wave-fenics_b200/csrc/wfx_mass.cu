@@ -304,6 +304,7 @@ namespace wfx
 {
 bool mass_assembled(const wfx_mass* op) { return op->assembled; }
 int mass_dtype(const wfx_mass* op) { return op->dtype; }
+int64_t mass_ndofs(const wfx_mass* op) { return op->ndofs; }
 const double* mass_diagonal64(const wfx_mass* op) { return op->d_m64.p; }
 } // namespace wfx
 

@@ -1097,6 +1097,20 @@ extern "C" int wfx_wave_get_field_stats(wfx_wave* w, int64_t* nsamples, double* 
   WFX_API_END
 }
 
+WaveFieldStats wfx::wave_field_stats(const wfx_wave* w)
+{
+  WaveFieldStats s;
+  s.ctx = w->ctx;
+  s.ndofs = w->n;
+  s.nv = w->nv;
+  s.on = w->stats_on;
+  s.nharm = w->stats_on ? w->stats_nharm : 0;
+  s.nsamples = w->stats_n;
+  s.harm = w->stats_harm.p;
+  for (int m = 0; m < w->nv; ++m) s.f0[m] = w->ens ? w->f0s[m] : w->f0;
+  return s;
+}
+
 extern "C" int wfx_wave_set_source_profile(wfx_wave* w, const double* amp_host, const double* delay_host)
 {
   WFX_API_BEGIN

@@ -443,6 +443,8 @@ public:
 
   std::shared_ptr<MassOperator<double>> mass_op;
   std::shared_ptr<StiffnessOperator<double>> stiff_op;
+  // the C handle, e.g. for PennesGLL::heat_from_wave
+  wfx_wave* get() const { return _wave; }
 
 protected:
   // the lossy / Westervelt models (wfx_wave_create_westervelt, one rank): see WesterveltGLLOpt
@@ -600,5 +602,103 @@ private:
   std::int64_t _nprobes = 0;
   wfx_boundary* _bnd = nullptr;
   wfx_wave* _wave = nullptr;
+};
+
+// The Pennes bioheat model with a CEM43 thermal dose (wfx_thermal_create, DESIGN.md section 4.5d), one rank, fp64:
+//   rhoC T_t = div(k grad T) - wbCb (T - T_art) + s Q,   -k dT/dn = h[j] (T - T_ext[j]) on tag j + 1
+// rhoC and wbCb per dof (mass-weighted averages of per-cell values, INTEGRATION.md; an empty perfusion is 0).
+// Temperatures in and out are absolute (T = T_art + theta).  T_ext: the two Robin tags' exterior temperatures, nullptr
+// for T_art on both.
+class PennesGLL
+{
+public:
+  PennesGLL(std::shared_ptr<Context> ctx, const SpaceView& V, int degree, double k, const std::vector<double>& rhoC,
+            const std::vector<double>& perfusion, double T_art, std::array<double, 2> h = {0.0, 0.0},
+            const std::array<double, 2>* T_ext = nullptr)
+      : _ctx(std::move(ctx)), _ndofs(V.ndofs), _T_art(T_art)
+  {
+    if ((std::int64_t)rhoC.size() != _ndofs || (!perfusion.empty() && (std::int64_t)perfusion.size() != _ndofs))
+      throw std::runtime_error("wavefx: rhoC and perfusion must hold one value per dof");
+    _geom = std::make_shared<Geometry<double>>(_ctx, V);
+    mass_op = std::make_shared<MassOperator<double>>(_geom, V, degree);
+    std::map<std::string, double> params; // the stiffness operator's own c0 (1500) is folded into the scale
+    stiff_op = std::make_shared<StiffnessOperator<double>>(_geom, V, degree, params);
+    if (h[0] != 0.0 || h[1] != 0.0)
+      check(wfx_boundary_create(_ctx->get(), V.degree, WFX_F64, V.nfacets, V.facet_cell, V.facet_local, V.facet_tag,
+                                V.npoints, V.x, V.xdofs, V.ndofs, V.dofmap, &_bnd));
+    check(wfx_thermal_create(_ctx->get(), stiff_op->get(), mass_op->get(), _bnd, k, rhoC.data(),
+                             perfusion.empty() ? nullptr : perfusion.data(), T_art, h.data(), T_ext ? T_ext->data() : nullptr, &_th));
+  }
+  ~PennesGLL()
+  {
+    wfx_thermal_destroy(_th);
+    wfx_boundary_destroy(_bnd);
+  }
+  PennesGLL(const PennesGLL&) = delete;
+  PennesGLL& operator=(const PennesGLL&) = delete;
+
+  void init() { check(wfx_thermal_init(_th)); }
+  void set_temperature(const std::vector<double>& T)
+  {
+    if ((std::int64_t)T.size() != _ndofs) throw std::runtime_error("wavefx: one temperature per dof expected");
+    std::vector<double> rise(T.size());
+    for (std::size_t i = 0; i < T.size(); ++i) rise[i] = T[i] - _T_art;
+    check(wfx_thermal_set_state(_th, rise.data()));
+  }
+  void temperature(std::vector<double>& T) const
+  {
+    T.resize((std::size_t)_ndofs);
+    check(wfx_thermal_get_state(_th, T.data()));
+    for (double& x : T) x += _T_art;
+  }
+  // Q [W/m^3] per dof; empty: 0
+  void set_heat_source(const std::vector<double>& Q) { check(wfx_thermal_set_heat_source(_th, Q.empty() ? nullptr : Q.data())); }
+  void heat_source(std::vector<double>& Q) const
+  {
+    Q.resize((std::size_t)_ndofs);
+    check(wfx_thermal_get_heat_source(_th, Q.data()));
+  }
+  // Q from the harmonic maps of a wave model's field statistics, alpha(f) = alpha0 (f / 1 MHz)^y
+  void heat_from_wave(const LinearGLLOpt& wave, double alpha0, double y, double rho0, double c0)
+  {
+    check(wfx_thermal_heat_from_wave(_th, wave.get(), 0, alpha0, nullptr, y, rho0, c0));
+  }
+  void set_heat_scale(double s) { check(wfx_thermal_set_heat_scale(_th, s)); }
+  std::int64_t rk4(double startTime, double finalTime, double timeStep)
+  {
+    std::int64_t steps = 0;
+    double t_end = 0;
+    check(wfx_thermal_rk4(_th, startTime, finalTime, timeStep, 0, &steps, &t_end, nullptr));
+    _ctx->synchronize();
+    return steps;
+  }
+  // steps since init / set_temperature, CEM43 [min] and the peak temperature of every dof
+  std::int64_t dose(std::vector<double>& cem43, std::vector<double>& T_max) const
+  {
+    std::int64_t n = 0;
+    cem43.resize((std::size_t)_ndofs);
+    T_max.resize((std::size_t)_ndofs);
+    check(wfx_thermal_get_dose(_th, &n, cem43.data(), T_max.data()));
+    for (double& x : T_max) x += _T_art;
+    return n;
+  }
+  // safety * the power iteration's RK4 limit; the estimate approaches the limit from above, hence the safety factor
+  double stable_dt(double safety = 0.8, int iters = 200) const
+  {
+    double lambda = 0, dt_max = 0;
+    check(wfx_thermal_stable_dt(_th, iters, &lambda, &dt_max));
+    return safety * dt_max;
+  }
+
+  std::shared_ptr<MassOperator<double>> mass_op;
+  std::shared_ptr<StiffnessOperator<double>> stiff_op;
+
+private:
+  std::shared_ptr<Context> _ctx;
+  std::shared_ptr<Geometry<double>> _geom;
+  std::int64_t _ndofs;
+  double _T_art;
+  wfx_boundary* _bnd = nullptr;
+  wfx_thermal* _th = nullptr;
 };
 } // namespace wavefx

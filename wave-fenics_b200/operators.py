@@ -83,6 +83,13 @@ class Geometry:
         if coeff.size != self.ncells:
             raise capi.WfxError("one coefficient per cell expected")
         capi.call("wfx_geometry_scale_cells", self.handle, capi.f64p(coeff))
+        self.scaled = True
+
+    def detJw(self):
+        """detJ * w [ncells, nq] (fp64, reference layout): the lumped mass's per-point weights."""
+        detJ = np.empty((self.ncells, (self.P + 1) ** 3))
+        capi.call("wfx_geometry_get", self.handle, None, capi.f64p(detJ.reshape(-1)))
+        return detJ
 
     def get(self):
         """(G [ncells,nq,3,3], detJ [ncells,nq]) in the reference layout."""
@@ -624,3 +631,185 @@ class LossyGLLOpt(WesterveltGLLOpt):
                  diffusivityOfSound, dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO):
         super().__init__(mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
                          diffusivityOfSound, 0.0, 1.0, dtype=dtype, ctx=ctx, stiffness_mode=stiffness_mode)
+
+
+# dose of a thermal model (PennesGLL.dose): steps since init / set_state, CEM43 [min] and peak temperature per dof
+ThermalDose = namedtuple("ThermalDose", "steps cem43 T_max")
+
+
+def cell_to_dof_average(mesh, detJw, coeff):
+    """Per-dof mass-weighted average of a per-cell coefficient, sum_c coeff_c (detJ w)_{c,i} / m_i with
+    m_i = sum_c (detJ w)_{c,i}, the lumped mass: then coeff_i m_i is the GLL quadrature of the piecewise-constant
+    coefficient.  detJw [ncells, nq] in the reference layout (Geometry.detJw, oracle.precompute_geometric_data)."""
+    coeff = np.asarray(coeff, dtype=np.float64).reshape(-1)
+    if coeff.size != mesh.ncells:
+        raise capi.WfxError("one coefficient per cell expected")
+    perm = capi.compute_permutations(mesh.P)
+    dofs = np.asarray(mesh.dofmap)[:, perm].reshape(-1)
+    w = np.asarray(detJw, dtype=np.float64).reshape(mesh.ncells, -1)
+    m = np.bincount(dofs, weights=w.reshape(-1), minlength=mesh.ndofs)
+    return np.bincount(dofs, weights=(coeff[:, None] * w).reshape(-1), minlength=mesh.ndofs) / m
+
+
+class PennesGLL:
+    """The Pennes bioheat model with a CEM43 thermal dose (DESIGN.md section 4.5d), one rank:
+
+        rhoC T_t = div(k grad T) - wbCb (T - T_art) + s Q        -k dT/dn = h_j (T - T_ext_j) on tag j = 1, 2
+
+    other faces insulated.  conductivity k [W/(m K)], heat_capacity rhoC [J/(m^3 K)] and perfusion wbCb
+    [W/(m^3 K)] are scalars or one value per cell: a per-cell k scales this model's own geometry (k_c / max k), a
+    per-cell rhoC or wbCb becomes its mass-weighted per-dof average (cell_to_dof_average).  h = (h1, h2)
+    [W/(m^2 K)], T_ext = (T_ext1, T_ext2); boundary=None builds the facet operator only when h != 0.  The state is
+    held as the rise over T_art; temperatures in and out are T = T_art + rise.  The heat source Q starts at 0 and
+    the heat scale s at 1."""
+
+    def __init__(self, mesh, degree, conductivity, heat_capacity, perfusion=0.0, T_art=37.0, h=(0.0, 0.0),
+                 T_ext=None, dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO, boundary=None, _ops=None):
+        self.ctx = ctx or Context.get()
+        self.V = mesh
+        self.P = int(degree)
+        self.dtype = np.dtype(dtype)
+        self.ndofs = int(mesh.ndofs)
+        self.T_art = float(T_art)
+        k = np.asarray(conductivity, dtype=np.float64)
+        h = np.asarray(h, dtype=np.float64).reshape(2)
+        T_ext = np.full(2, self.T_art) if T_ext is None else np.asarray(T_ext, dtype=np.float64).reshape(2)
+        if boundary is None:
+            boundary = bool(np.any(h != 0))
+        if _ops is None:
+            self.geometry = Geometry(mesh, self.P, dtype, self.ctx)
+            if k.ndim:
+                self.k = float(k.max())
+                self.geometry.scale_cells(k / self.k)    # before the operators: they copy G at creation
+            else:
+                self.k = float(k)
+            self.mass_op = MassOperator(mesh, self.P, dtype, self.ctx, self.geometry)
+            self.stiff_op = StiffnessOperator(mesh, self.P, None, dtype, self.ctx, self.geometry, mode=stiffness_mode)
+            self.bnd_op = BoundaryOperator(mesh, self.P, dtype, self.ctx) if boundary else None
+        else:
+            self.geometry, self.mass_op, self.stiff_op, self.bnd_op = _ops
+            if k.ndim:
+                raise capi.WfxError("shared operators: a per-cell conductivity needs the model's own geometry")
+            self.k = float(k)
+            if not boundary:
+                self.bnd_op = None
+        detJw = None
+
+        def per_dof(c):
+            nonlocal detJw
+            c = np.asarray(c, dtype=np.float64)
+            if not c.ndim:
+                return np.full(self.ndofs, float(c))
+            if detJw is None:
+                detJw = self.geometry.detJw()
+            return cell_to_dof_average(mesh, detJw, c)
+
+        self.rhoc = per_dof(heat_capacity)
+        self.perf = per_dof(perfusion)
+        self.handle = C.c_void_p()
+        capi.call("wfx_thermal_create", self.ctx.handle, self.stiff_op.handle, self.mass_op.handle,
+                  self.bnd_op.handle if self.bnd_op is not None else None, self.k, capi.f64p(self.rhoc),
+                  capi.f64p(self.perf), self.T_art, capi.f64p(np.ascontiguousarray(h)),
+                  capi.f64p(np.ascontiguousarray(T_ext)), C.byref(self.handle))
+
+    @classmethod
+    def from_wave(cls, model, conductivity, heat_capacity, perfusion=0.0, T_art=37.0, h=(0.0, 0.0), T_ext=None,
+                  boundary=None):
+        """A thermal model on a wave model's mesh that shares its geometry, stiffness, mass and boundary operators
+        (none keeps per-apply state).  Refused when the wave model's geometry was scaled (wfx_geometry_scale_cells):
+        the diffusion term would carry the acoustic coefficient."""
+        if getattr(model.geometry, "scaled", False):
+            raise capi.WfxError("from_wave: the wave model's geometry is scaled; build the thermal model's own operators")
+        ops = (model.geometry, model.mass_op, model.stiff_op, model.bnd_op)
+        return cls(model.V, model.k_, conductivity, heat_capacity, perfusion, T_art, h, T_ext, dtype=model.dtype,
+                   ctx=model.ctx, boundary=boundary, _ops=ops)
+
+    def init(self):
+        """T = T_art everywhere; resets the dose"""
+        capi.call("wfx_thermal_init", self.handle)
+
+    def set_state(self, T):
+        """T [ndofs] (temperatures); resets the dose"""
+        rise = np.ascontiguousarray(np.asarray(T, dtype=np.float64) - self.T_art, dtype=self.dtype)
+        if rise.shape != (self.ndofs,):
+            raise capi.WfxError(f"thermal state must have shape ({self.ndofs},)")
+        capi.call("wfx_thermal_set_state", self.handle, C.c_void_p(rise.ctypes.data))
+
+    def rise(self):
+        """theta = T - T_art in the model dtype, as held on the device"""
+        out = np.empty(self.ndofs, dtype=self.dtype)
+        capi.call("wfx_thermal_get_state", self.handle, C.c_void_p(out.ctypes.data))
+        return out
+
+    def get_state(self):
+        """T = T_art + theta, fp64"""
+        return self.T_art + self.rise().astype(np.float64)
+
+    def state_ptr(self):
+        p = C.c_void_p()
+        capi.call("wfx_thermal_state_ptr", self.handle, C.byref(p))
+        return p.value
+
+    def set_heat_source(self, Q=None):
+        """Q [W/m^3] per dof (None: 0)"""
+        q = None if Q is None else np.ascontiguousarray(Q, dtype=np.float64)
+        if q is not None and q.shape != (self.ndofs,):
+            raise capi.WfxError(f"heat source must have shape ({self.ndofs},)")
+        capi.call("wfx_thermal_set_heat_source", self.handle, capi.f64p(q))
+
+    def heat_from_wave(self, model, alpha0, y, rho0, c0, member=0):
+        """Q = sum_h alpha0 (h f0 / 1 MHz)^y |p_h|^2 / (rho0 c0) from the harmonic maps of `model`'s field statistics,
+        computed on the device.  alpha0 [Np/m at 1 MHz]: a scalar or one value per dof; member: the ensemble member."""
+        a = np.asarray(alpha0, dtype=np.float64)
+        a_host = None
+        if a.ndim:
+            a_host = np.ascontiguousarray(a.reshape(-1))
+            if a_host.size != self.ndofs:
+                raise capi.WfxError(f"alpha0 must be a scalar or have shape ({self.ndofs},)")
+        capi.call("wfx_thermal_heat_from_wave", self.handle, model.handle, int(member), float(a) if not a.ndim else 0.0,
+                  capi.f64p(a_host), float(y), float(rho0), float(c0))
+
+    def heat_source(self):
+        q = np.empty(self.ndofs)
+        capi.call("wfx_thermal_get_heat_source", self.handle, capi.f64p(q))
+        return q
+
+    def set_heat_scale(self, s):
+        """s >= 0 multiplies Q (duty cycles: heating with s = 1, cooling with s = 0)"""
+        capi.call("wfx_thermal_set_heat_scale", self.handle, float(s))
+
+    def rhs(self, theta, out):
+        """out = theta' at theta (rises), CUDA tensors of the model dtype"""
+        capi.call("wfx_thermal_rhs", self.handle, C.c_void_p(theta.data_ptr()), C.c_void_p(out.data_ptr()),
+                  _stream_ptr())
+
+    def rk4(self, startTime, finalTime, timeStep, max_steps=0, stream=None):
+        steps, t_end = C.c_int64(), C.c_double()
+        capi.call("wfx_thermal_rk4", self.handle, float(startTime), float(finalTime), float(timeStep), int(max_steps),
+                  C.byref(steps), C.byref(t_end), stream if stream is not None else _stream_ptr())
+        return steps.value, t_end.value
+
+    def dose(self):
+        """ThermalDose(steps, cem43 [min], T_max = T_art + max rise) accumulated since init / set_state"""
+        n = C.c_int64()
+        cem = np.empty(self.ndofs)
+        thmax = np.empty(self.ndofs, dtype=self.dtype)
+        capi.call("wfx_thermal_get_dose", self.handle, C.byref(n), capi.f64p(cem), C.c_void_p(thmax.ctypes.data))
+        return ThermalDose(n.value, cem, self.T_art + thmax.astype(np.float64))
+
+    def max_eigenvalue(self, iters=200):
+        """(lambda, dt_max) of the power iteration (wfx_thermal_stable_dt): lambda approaches the largest eigenvalue
+        from below, so dt_max = 2.785293563405282 / lambda may lie above the true RK4 limit."""
+        lam, dtm = C.c_double(), C.c_double()
+        capi.call("wfx_thermal_stable_dt", self.handle, int(iters), C.byref(lam), C.byref(dtm))
+        return lam.value, dtm.value
+
+    def stable_dt(self, safety=0.8, iters=200):
+        """safety * dt_max: a time step inside the RK4 stability limit (the safety factor covers the estimate's
+        shortfall)"""
+        return safety * self.max_eigenvalue(iters)[1]
+
+    def __del__(self):
+        if getattr(self, "handle", None) and getattr(capi, "lib", None) is not None:
+            capi.lib.wfx_thermal_destroy(self.handle)
+            self.handle = None
