@@ -126,7 +126,11 @@ int wfx_geometry_info(wfx_geom* geom, int64_t* ncells, int64_t* n_affine);
  * (c0[c] / c0_ref)^2 so that a stiffness operator created with c0_ref applies -c0(x)^2 K with a
  * piecewise-constant speed of sound at no cost per apply.  The reference leaves this open
  * (`// TODO: Compute coefficients`, common/LinearGLL.hpp:170; `params` ignored at
- * common/operators.hpp:113-115).  The mass (detJ) is not touched.  Call before applying. */
+ * common/operators.hpp:113-115).  The mass (detJ) is not touched.  Valid at any time before the applies
+ * that should see it, on every kernel path: the private G copies stiffness operators made from this
+ * geometry are scaled with it, and captured graphs keep their pointers.  Coefficients compose by
+ * multiplication.  Synchronises the device; applies still in flight on other streams must have finished.
+ * A refused coefficient (not positive, not finite) leaves G unchanged. */
 int wfx_geometry_scale_cells(wfx_geom* geom, const double* coeff_host);
 int wfx_geometry_destroy(wfx_geom* geom);
 
@@ -210,6 +214,7 @@ int wfx_stiffness_info(wfx_stiffness* op, int64_t* num_cells, int* num_dofs_per_
  * colour). */
 int wfx_stiffness_kernel_info(wfx_stiffness* op, int* variant, int* affine, int* mixed,
                               int* regular_batches, int* batches, int64_t* smem_bytes);
+/* Destroy an operator before the geometry it was created on (it removes its G copy from the geometry). */
 int wfx_stiffness_destroy(wfx_stiffness* op);
 
 /* ---- mass: MassOperatorCPU (common/operators.hpp:43-109) / SpectralMassOperator

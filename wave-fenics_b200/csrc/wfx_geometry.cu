@@ -10,6 +10,7 @@
 #include "wfx_plan.h"
 
 #include <cmath>
+#include <utility>
 
 using namespace wfx;
 
@@ -190,7 +191,7 @@ affine_detect_kernel(int n, int64_t ncells, const T* __restrict__ G6, Tables1D t
   }
 }
 
-// G[c] *= coeff[c] for every point of cell c (and the per-cell form)
+// G[c] *= coeff[c] for every point of cell c (and the per-cell form, when Gc is not NULL)
 template <typename T>
 __global__ void __launch_bounds__(256)
 scale_cells_kernel(int64_t ncells, int per_cell, const double* __restrict__ coeff, T* __restrict__ G6,
@@ -198,7 +199,7 @@ scale_cells_kernel(int64_t ncells, int per_cell, const double* __restrict__ coef
 {
   const int64_t gid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (gid < ncells * per_cell) G6[gid] = (T)((double)G6[gid] * coeff[gid / per_cell]);
-  if (gid < ncells * 6) Gc[gid] = (T)((double)Gc[gid] * coeff[gid / 6]);
+  if (Gc && gid < ncells * 6) Gc[gid] = (T)((double)Gc[gid] * coeff[gid / 6]);
 }
 
 // common/precompute.hpp building blocks at arbitrary reference points.
@@ -330,10 +331,17 @@ extern "C" int wfx_geometry_scale_cells(wfx_geom* g, const double* coeff_host)
   const int per_cell = g->nq * 6;
   const int64_t total = g->ncells * per_cell;
   const unsigned grid = (unsigned)((total + 255) / 256);
-  if (g->dtype == WFX_F64)
-    scale_cells_kernel<double><<<grid, 256>>>(g->ncells, per_cell, d.p, (double*)g->G6, (double*)g->Gc);
-  else
-    scale_cells_kernel<float><<<grid, 256>>>(g->ncells, per_cell, d.p, (float*)g->G6, (float*)g->Gc);
+  // the operators' private copies hold the same values per cell in another order: the same scaling keeps
+  // each one bitwise equal to the reordered scaled G
+  std::vector<std::pair<void*, void*>> targets{{g->G6, g->Gc}};
+  for (void* p : g->g_copies) targets.push_back({p, nullptr});
+  for (const auto& t : targets)
+  {
+    if (g->dtype == WFX_F64)
+      scale_cells_kernel<double><<<grid, 256>>>(g->ncells, per_cell, d.p, (double*)t.first, (double*)t.second);
+    else
+      scale_cells_kernel<float><<<grid, 256>>>(g->ncells, per_cell, d.p, (float*)t.first, (float*)t.second);
+  }
   WFX_CUDA(cudaGetLastError());
   WFX_CUDA(cudaDeviceSynchronize());
   WFX_API_END

@@ -211,6 +211,11 @@ struct wfx_geom
   int64_t ncells = 0;
   void* G6 = nullptr;     // T
   std::vector<uint8_t> g_colpos; // empty: identity; else column of point (i,j) = g_colpos[i*n+j]
+  // private copies of G6 that stiffness operators made from it ([ncells][nq*6] T each, cell-major; the
+  // points inside a cell may be reordered): wfx_geometry_scale_cells scales them with G6, so a coefficient
+  // set after an operator was created reaches every path.  An operator registers its copy at creation and
+  // removes it when destroyed.
+  std::vector<void*> g_copies;
   double* dJw = nullptr;  // fp64
   // Affine cells (parallelepipeds): G[c,q] = w_q * A_c with one symmetric 3x3 A_c per cell.  Detected
   // from the computed (clamped) per-point G, so a cell counts as affine only if the per-cell form

@@ -1981,6 +1981,11 @@ struct wfx_stiffness
               ev_fy[2] = {nullptr, nullptr};
   ~wfx_stiffness()
   {
+    if (geom && d_G6perm.p)
+    {
+      auto& v = geom->g_copies;
+      v.erase(std::remove(v.begin(), v.end(), (void*)d_G6perm.p), v.end());
+    }
     for (cudaStream_t st : {bs_h2d, bs_cmp, bs_d2h})
       if (st) cudaStreamDestroy(st);
     for (int q = 0; q < 2; ++q)
@@ -2036,7 +2041,9 @@ void launch_cell2(wfx_stiffness* op, const T* x, const T* scale, T* y, int beta,
   a.scale = scale;
   a.coeff = (T)(-1.0 * op->c0 * op->c0);
   a.beta = beta;
-  a.g_order = op->geom->g_colpos.empty() ? 0 : 1;
+  // the private copy was made from G6 in its natural column order: a column reorder of the geometry by
+  // an operator created later leaves it as it is
+  a.g_order = (op->d_G6perm.n || op->geom->g_colpos.empty()) ? 0 : 1;
   a.cps = op->cell2_cps;
   a.ndofs = op->ndofs;
   a.ncells = op->ncells;
@@ -2117,7 +2124,7 @@ void launch_ens(wfx_stiffness* op, int nv, const T* x, const T* scale, T* y, int
   a.scale = scale;
   a.coeff = (T)(-1.0 * op->c0 * op->c0);
   a.beta = beta;
-  a.g_order = op->geom->g_colpos.empty() ? 0 : 1;
+  a.g_order = ((share && op->d_G6perm.n) || op->geom->g_colpos.empty()) ? 0 : 1; // (as launch_cell2)
   a.nv = nv;
   a.ndofs = op->ndofs;
   a.ncells = op->ncells;
@@ -2573,6 +2580,7 @@ extern "C" int wfx_stiffness_create_partitioned(wfx_ctx* ctx, wfx_geom* geom, in
       {
         const size_t esz = op->dtype == WFX_F64 ? 8 : 4;
         op->d_G6perm.alloc((size_t)op->ncells * nd * 6 * esz);
+        geom->g_copies.push_back(op->d_G6perm.p); // scaled with G6 from now on (wfx_geometry_scale_cells)
         const int64_t npts = op->ncells * nd;
         const unsigned grid = (unsigned)((npts + 255) / 256);
         if (op->dtype == WFX_F64)

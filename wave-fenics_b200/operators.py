@@ -78,7 +78,8 @@ class Geometry:
         return dict(ncells=nc.value, n_affine=na.value)
 
     def scale_cells(self, coeff):
-        """G[c] *= coeff[c]: a piecewise-constant coefficient, e.g. (c0[c] / c0_ref)^2."""
+        """G[c] *= coeff[c]: a piecewise-constant coefficient, e.g. (c0[c] / c0_ref)^2.  Reaches the operators and
+        models already built on this geometry (their next applies), on every kernel path."""
         coeff = np.ascontiguousarray(coeff, dtype=np.float64)
         if coeff.size != self.ncells:
             raise capi.WfxError("one coefficient per cell expected")
@@ -680,7 +681,7 @@ class PennesGLL:
             self.geometry = Geometry(mesh, self.P, dtype, self.ctx)
             if k.ndim:
                 self.k = float(k.max())
-                self.geometry.scale_cells(k / self.k)    # before the operators: they copy G at creation
+                self.geometry.scale_cells(k / self.k)
             else:
                 self.k = float(k)
             self.mass_op = MassOperator(mesh, self.P, dtype, self.ctx, self.geometry)
