@@ -22,12 +22,18 @@ model on the same mesh and operators takes its heat source Q = sum_h alpha0 (h f
 the harmonic maps, is heated for S seconds and cools for --cool-seconds C with the source off, and reports the peak
 temperature rise, the maximum CEM43 thermal dose, and the number of dofs and the volume at or above 240 min.
 --absorption alpha0 [Np/m at 1 MHz] and --absorption-power y set the tissue absorption.
+--layer X0 X1 --layer-rho R --layer-c C [--layer-beta B] puts a slab of another medium across the beam (DESIGN.md
+section 4.5e): the cells whose centres lie in X0 < x < X1 get density R, speed of sound C and, for the Westervelt
+model, coefficient of nonlinearity B (default --beta); the rest is water (1000 kg/m^3, 1500 m/s, --beta).  The time
+step comes from the largest speed of sound.  With --stats-periods the on-axis |p1| is reported before and after the
+slab; with --heat-seconds the thermal model is built on its own operators and heated with the per-dof 1 / (rho c).
 The reference reads `../mesh.xdmf` (not in its repository); here the mesh is a structured
 n x m x m hexahedral box with tag 1 on x = 0 (source) and tag 2 on x = L (absorbing).
 
     python demo/planar3d.py [--nx 32] [--nyz 4] [--length 0.1] [--steps N] [--check]
                             [--model linear|lossy|westervelt] [--stats-periods K] [--focus DEPTH] [--aperture R]
                             [--heat-seconds S] [--cool-seconds C] [--absorption ALPHA0] [--absorption-power Y]
+                            [--layer X0 X1 --layer-rho R --layer-c C [--layer-beta B]]
 """
 import argparse
 import os
@@ -74,7 +80,17 @@ def main():
     ap.add_argument("--cool-seconds", type=float, default=0.0, help="cooling after the heating, source off")
     ap.add_argument("--absorption", type=float, default=5.0, help="tissue absorption alpha0 [Np/m at 1 MHz]")
     ap.add_argument("--absorption-power", type=float, default=1.1, help="frequency power law y of the absorption")
+    ap.add_argument("--layer", type=float, nargs=2, metavar=("X0", "X1"), default=None,
+                    help="a slab of another medium across the beam between x = X0 and x = X1 [m]")
+    ap.add_argument("--layer-rho", type=float, default=1900.0, help="with --layer: the slab's density [kg/m^3]")
+    ap.add_argument("--layer-c", type=float, default=2800.0, help="with --layer: the slab's speed of sound [m/s]")
+    ap.add_argument("--layer-beta", type=float, default=None,
+                    help="with --layer: the slab's coefficient of nonlinearity (default --beta)")
     args = ap.parse_args()
+    if args.layer is not None and args.check:
+        ap.error("--check compares with the homogeneous oracle; it does not take --layer")
+    if args.layer is not None and not args.layer[0] < args.layer[1]:
+        ap.error("--layer X0 X1 needs X0 < X1")
     if args.heat_seconds > 0 and args.stats_periods <= 0:
         ap.error("--heat-seconds needs --stats-periods (the heat source comes from the harmonic maps)")
 
@@ -88,7 +104,18 @@ def main():
     if args.focus > 0:
         tags += ((1, 0, 2), (1, 1, 2), (2, 0, 2), (2, 1, 2))
     mesh = wfx.create_box_hex((args.nx, args.nyz, args.nyz), degreeOfBasis, (domainLength, width, width), tags=tags)
-    timeStepSize = wfx.cfl_timestep(mesh.h_min, speedOfSound, degreeOfBasis, sourceFrequency)  # :61-66
+    medium = None
+    if args.layer is not None:
+        xc = mesh.x[mesh.xdofs, 0].mean(axis=1)                          # cell centres along x
+        slab = (xc > args.layer[0]) & (xc < args.layer[1])
+        beta_slab = args.beta if args.layer_beta is None else args.layer_beta
+        medium = wfx.Medium(np.where(slab, args.layer_rho, 1000.0), np.where(slab, args.layer_c, speedOfSound),
+                            np.where(slab, beta_slab, args.beta))
+        print(f"layer: {int(slab.sum())} cells in {args.layer[0]:.4f} < x < {args.layer[1]:.4f} with rho = "
+              f"{args.layer_rho:g}, c = {args.layer_c:g}, beta = {beta_slab:g}; Z ratio to water "
+              f"{args.layer_rho * args.layer_c / (1000.0 * speedOfSound):.4f}")
+    c_max = speedOfSound if medium is None else medium.c_max
+    timeStepSize = wfx.cfl_timestep(mesh.h_min, c_max, degreeOfBasis, sourceFrequency)  # :61-66
     startTime, finalTime = 0.0, domainLength / speedOfSound + 8.0 / sourceFrequency            # :63-64
     print(f"Number of step per period: {int(round(period / timeStepSize))}")
     print(f"dt = {timeStepSize:.15g}")
@@ -96,10 +123,13 @@ def main():
     delta = 0.0 if args.model == "linear" else args.delta
     beta = args.beta if args.model == "westervelt" else 0.0
     if args.model == "linear":
-        eqn = wfx.LinearGLLOpt(mesh, None, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude)  # :75
+        eqn = wfx.LinearGLLOpt(mesh, None, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
+                               medium=medium)                                                              # :75
     else:
+        if medium is not None and args.model == "lossy":
+            medium = wfx.Medium(medium.rho, medium.c)                     # the lossy model stays linear
         eqn = wfx.WesterveltGLLOpt(mesh, None, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
-                                   delta, beta, args.rho0)
+                                   delta, beta, args.rho0, medium=medium)
     print(f"Number of steps: {nstep}")
     print(f"Degrees of freedom: {mesh.ndofs_global}")
     X = wfx.dof_coordinates(mesh)
@@ -141,13 +171,19 @@ def main():
             print(f"along x: max pmax = {pmax.max():.6e} at x = {x[pmax.argmax()]:.4f}, "
                   f"min pmin = {pmin.min():.6e} at x = {x[pmin.argmin()]:.4f}")
             print(f"at the absorbing end (x = {x[-1]:.4f}): |p1| = {p1[-1]:.6e}, |p2|/|p1| = {p2[-1] / p1[-1]:.6e}")
+            if args.layer is not None:
+                before, after = x < args.layer[0], x > args.layer[1]
+                for name, sel in (("before the layer", before), ("after the layer", after)):
+                    if sel.any():
+                        print(f"{name}: on-axis |p1| mean {p1[sel].mean():.6e}, max {p1[sel].max():.6e} "
+                              f"({int(sel.sum())} dofs)")
             if args.focus > 0:
                 print(f"on-axis maximum: |p1| = {p1.max():.6e} at x = {x[p1.argmax()]:.5f}, "
                       f"pmax = {pmax.max():.6e} at x = {x[pmax.argmax()]:.5f} (focus requested at x = {args.focus:.5f})")
         if args.heat_seconds > 0 and fs.samples == 0:
             print("thermal: skipped, the statistics window holds no samples (no heat source without harmonics)")
         elif args.heat_seconds > 0:
-            heat(args, eqn, speedOfSound)
+            heat(args, eqn, speedOfSound, medium)
     else:
         print(f"max |p| = {np.abs(u).max():.6e} at x = {X[np.abs(u).argmax(), 0]:.4f}")
     if args.check:
@@ -177,11 +213,15 @@ def main():
               f"  v {np.linalg.norm(v - vo) / np.linalg.norm(vo):.3e}")
 
 
-def heat(args, eqn, c0, k=0.5, rhoc=3.6e6, perfusion=2.0e3, T_art=37.0):
+def heat(args, eqn, c0, medium=None, k=0.5, rhoc=3.6e6, perfusion=2.0e3, T_art=37.0):
     """HIFU heating from the wave model's harmonic maps: soft-tissue-like k [W/(m K)], rhoC [J/(m^3 K)] and
-    perfusion wbCb [W/(m^3 K)], all faces insulated"""
-    th = wfx.PennesGLL.from_wave(eqn, k, rhoc, perfusion, T_art)
-    th.heat_from_wave(eqn, args.absorption, args.absorption_power, args.rho0, c0)
+    perfusion wbCb [W/(m^3 K)], all faces insulated.  In a layered medium the thermal model has operators of its own
+    (the wave model's geometry is scaled) and the heat source uses the per-dof 1 / (rho c)."""
+    if medium is None:
+        th = wfx.PennesGLL.from_wave(eqn, k, rhoc, perfusion, T_art)
+    else:
+        th = wfx.PennesGLL(eqn.V, eqn.k_, k, rhoc, perfusion, T_art, dtype=eqn.dtype, ctx=eqn.ctx)
+    th.heat_from_wave(eqn, args.absorption, args.absorption_power, args.rho0, c0, medium=medium)
     dt = th.stable_dt()
     th.init()
     eqn.ctx.synchronize()

@@ -130,7 +130,10 @@ int wfx_geometry_info(wfx_geom* geom, int64_t* ncells, int64_t* n_affine);
  * that should see it, on every kernel path: the private G copies stiffness operators made from this
  * geometry are scaled with it, and captured graphs keep their pointers.  Coefficients compose by
  * multiplication.  Synchronises the device; applies still in flight on other streams must have finished.
- * A refused coefficient (not positive, not finite) leaves G unchanged. */
+ * A refused coefficient (not positive, not finite) leaves G unchanged.
+ * The scaled form models p_tt = div(c^2 grad p), i.e. a density proportional to c^-2: for a medium with its own
+ * density per cell use the weights of DESIGN.md section 4.5e (stiffness rho_ref / rho_c through this call, plus
+ * wfx_mass_create_weighted, wfx_boundary_create_weighted and wfx_wave_set_nonlinearity). */
 int wfx_geometry_scale_cells(wfx_geom* geom, const double* coeff_host);
 int wfx_geometry_destroy(wfx_geom* geom);
 
@@ -224,6 +227,12 @@ int wfx_stiffness_destroy(wfx_stiffness* op);
  * (atomic-free segmented reduction). */
 int wfx_mass_create(wfx_ctx* ctx, wfx_geom* geom, int64_t ndofs, const int32_t* dofmap_host,
                     wfx_mass** op);
+/* Weighted lumped mass of a layered medium (DESIGN.md section 4.5e): m~_i = sum_c w_c (detJ w)_{c,i}, one weight per
+ * cell (e.g. rho_ref c0^2 / (rho_c c_c^2)), reduced like wfx_mass_create in the same contribution order with each
+ * product w_c * detJw rounded on its own.  cell_weight_host NULL: wfx_mass_create bit for bit.  A weight that is not
+ * positive and finite is refused. */
+int wfx_mass_create_weighted(wfx_ctx* ctx, wfx_geom* geom, int64_t ndofs, const int32_t* dofmap_host,
+                             const double* cell_weight_host, wfx_mass** op);
 int wfx_mass_apply(wfx_mass* op, const void* x_dev, void* y_dev, int beta, void* stream);
 int wfx_mass_apply_host(wfx_mass* op, const void* x_host, void* y_host, int beta);
 /* device pointers owned by the operator: m = M.1 (LinearGLL.hpp:102-110) and 1/m */
@@ -261,6 +270,14 @@ int wfx_boundary_create(wfx_ctx* ctx, int P, int dtype, int64_t nfacets,
                         const int32_t* facet_tag_host, int64_t npts, const double* x_host,
                         const int32_t* xdofs_host, int64_t ndofs, const int32_t* dofmap_host,
                         wfx_boundary** op);
+/* The same with one weight per facet triplet (DESIGN.md section 4.5e: rho_ref / rho_f on tag 1, Z_ref / Z_f on tag 2,
+ * f the facet's cell): each facet's GLL facet mass is multiplied by its weight before the host reduction, which keeps
+ * its order.  facet_weight_host NULL: wfx_boundary_create bit for bit.  A weight that is not positive and finite is
+ * refused (also on untagged facets). */
+int wfx_boundary_create_weighted(wfx_ctx* ctx, int P, int dtype, int64_t nfacets, const int32_t* facet_cell_host,
+                                 const int32_t* facet_local_host, const int32_t* facet_tag_host, int64_t npts,
+                                 const double* x_host, const int32_t* xdofs_host, int64_t ndofs,
+                                 const int32_t* dofmap_host, const double* facet_weight_host, wfx_boundary** op);
 int wfx_boundary_apply(wfx_boundary* op, double c0, double g, const void* vn_dev, void* b_dev,
                        void* stream);
 /* dense copies of m1 / m2 (length ndofs, fp64) for checks */
@@ -339,6 +356,14 @@ int wfx_wave_create_ensemble(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass,
 int wfx_wave_create_westervelt(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mass, wfx_boundary* bnd,
                                int64_t size_local, double c0, double f0, double p0, double delta, double beta,
                                double rho0, wfx_wave** wave);
+/* Per-dof nonlinearity of a layered medium (DESIGN.md section 4.5e) for a model made by wfx_wave_create_westervelt:
+ * kappa_host [ndofs], kappa_i >= 0 and finite, replaces the scalar kappa everywhere (stage update, f1, the Gamma2
+ * mass term), and the model uses the nonlinear update even if it was created with beta = 0.  With a weighted mass
+ * m~, kappa_i = sum_c kappa_c mu_c (detJ w)_{c,i} / m~_i, kappa_c = 2 beta_c / (rho_c c_c^2).  NULL restores the
+ * scalar kappa of create.  Model configuration: it survives init, set_state and restarts.  Synchronises the device
+ * and drops the captured step graph.  Refused: a NULL model, linear and ensemble models, negative or non-finite
+ * values. */
+int wfx_wave_set_nonlinearity(wfx_wave* wave, const double* kappa_host);
 int wfx_wave_init(wfx_wave* wave);                                   /* :131-134 */
 /* Copies the state to the device; on a distributed mesh the ghost entries are then overwritten by
  * their owners' values (u->scatter_fwd(), v->scatter_fwd(), :164,167). */

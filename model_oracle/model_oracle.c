@@ -291,3 +291,145 @@ int64_t wo_rk4_pennes(int P, int64_t ncells, int64_t ndofs, const int32_t* dofma
   free(u_); free(un); free(u0); free(kv);
   return step;
 }
+
+/* ---- layered media (DESIGN.md section 4.5e) ------------------------------------------------------------------
+ * Per-cell density, sound speed and nonlinearity enter the lumped system only through weights: G scaled per cell
+ * by rho_ref / rho_c (passed in as G), the weighted lumped mass m, the weighted facet masses m1, m2 (passed in as
+ * given) and a per-dof kappa.  model_rhs_medium is model_rhs with kappa[k] in place of the scalar kappa; with
+ * kappa[k] equal to that scalar it computes what model_rhs computes, bit for bit. */
+
+/* wo_boundary_facet_mass with facet f's contributions multiplied by fw[f] (written out like the oracle's loop) */
+int wo_boundary_facet_mass_weighted(int P, int64_t nfacets, const int32_t* fcell, const int32_t* flocal,
+                                    const int32_t* ftag, const double* x, const int32_t* xdofs, const int32_t* dofmap,
+                                    const double* fw, double* m1, double* m2)
+{
+  const int n = P + 1, nd = n * n * n;
+  double pts[WO_MAXN], wts[WO_MAXN];
+  static const int F_AXIS[6] = {2, 1, 0, 0, 1, 2};
+  static const int F_SIDE[6] = {0, 0, 0, 1, 1, 1};
+  int* perm = (int*)malloc(sizeof(int) * nd);
+  if (wo_gll(P, pts, wts) || wo_perm(P, perm)) { free(perm); return -1; }
+  for (int64_t f = 0; f < nfacets; ++f)
+  {
+    const int64_t c = fcell[f];
+    const int lf = flocal[f], tag = ftag[f];
+    double* m = tag == 1 ? m1 : (tag == 2 ? m2 : NULL);
+    if (!m) continue;
+    const int ax = F_AXIS[lf], side = F_SIDE[lf];
+    const int t1 = ax == 0 ? 1 : 0, t2 = ax == 2 ? 1 : 2;
+    double coords[8][3];
+    for (int v = 0; v < 8; ++v)
+      for (int a = 0; a < 3; ++a) coords[v][a] = x[3 * (int64_t)xdofs[8 * c + v] + a];
+    for (int ia = 0; ia < n; ++ia)
+      for (int ib = 0; ib < n; ++ib)
+      {
+        int idx[3];
+        idx[ax] = side;
+        idx[t1] = ia;
+        idx[t2] = ib;
+        const double X[3] = {pts[idx[0]], pts[idx[1]], pts[idx[2]]};
+        double d[3][8], J[3][3];
+        cmap_dphi(X, d, 1);
+        for (int i = 0; i < 3; ++i)
+          for (int j = 0; j < 3; ++j)
+          {
+            double s = 0.0;
+            for (int v = 0; v < 8; ++v) s += coords[v][i] * d[j][v];
+            J[i][j] = s;
+          }
+        const double a0 = J[0][t1], a1 = J[1][t1], a2 = J[2][t1];
+        const double b0 = J[0][t2], b1 = J[1][t2], b2 = J[2][t2];
+        const double cx = a1 * b2 - a2 * b1, cy = a2 * b0 - a0 * b2, cz = a0 * b1 - a1 * b0;
+        const double scale = sqrt(cx * cx + cy * cy + cz * cz);
+        const int t = (idx[0] * n + idx[1]) * n + idx[2];
+        m[dofmap[c * nd + perm[t]]] += fw[f] * (wts[ia] * wts[ib] * scale);
+      }
+  }
+  free(perm);
+  return 0;
+}
+
+static void model_rhs_medium(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                             const double* m, const double* m1, const double* m2, const double* kappa, double c0,
+                             double freq0, double p0, double delta, double t, const double* un, const double* vn,
+                             double* kv, double* b, double* bv, int sumfact, int nthreads)
+{
+  const size_t nb = sizeof(double) * ndofs;
+  const double s = delta / (1500.0 * 1500.0);
+  double g, gdot;
+  wo_source(t, freq0, p0, c0, &g, &gdot);
+  memset(b, 0, nb);
+  memset(bv, 0, nb);
+  model_stiffness(P, ncells, ndofs, dofmap, G, un, b, sumfact, nthreads);  /* A un */
+  model_stiffness(P, ncells, ndofs, dofmap, G, vn, bv, sumfact, nthreads); /* A vn */
+  for (int64_t k = 0; k < ndofs; ++k)
+  {
+    double r = b[k] + s * bv[k];
+    r += (c0 * c0 * g + delta * gdot) * m1[k] - c0 * m2[k] * vn[k];
+    r += kappa[k] * m[k] * vn[k] * vn[k];
+    kv[k] = r / (m[k] * (1.0 - kappa[k] * un[k]) + delta / c0 * m2[k]);
+  }
+}
+
+/* dv/dt = f1(t, u, v) of the lossy / Westervelt model in a layered medium (kappa [ndofs]) */
+void wo_f1_westervelt_medium(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                             const double* m, const double* m1, const double* m2, const double* kappa, double c0,
+                             double freq0, double p0, double delta, double t, const double* u, const double* v,
+                             double* out, int sumfact, int nthreads)
+{
+  const size_t nb = sizeof(double) * ndofs;
+  double *b = malloc(nb), *bv = malloc(nb);
+  model_rhs_medium(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, t, u, v, out, b, bv, sumfact,
+                   nthreads);
+  free(b);
+  free(bv);
+}
+
+/* wo_rk4_westervelt in a layered medium: the same stage loop, model_rhs_medium as f1 */
+int64_t wo_rk4_westervelt_medium(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                                 const double* m, const double* m1, const double* m2, const double* kappa, double c0,
+                                 double freq0, double p0, double delta, double t0, double tf, double dt,
+                                 int64_t max_steps, double* u_n, double* v_n, int sumfact, int nthreads, double* t_end)
+{
+  const double a_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  const double b_runge[4] = {1.0 / 6.0, 1.0 / 3.0, 1.0 / 3.0, 1.0 / 6.0};
+  const double c_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  const size_t nb = sizeof(double) * ndofs;
+  double *u_ = malloc(nb), *v_ = malloc(nb), *un = malloc(nb), *vn = malloc(nb);
+  double *u0 = malloc(nb), *v0 = malloc(nb), *ku = malloc(nb), *kv = malloc(nb), *b = malloc(nb), *bv = malloc(nb);
+  memcpy(u_, u_n, nb);
+  memcpy(v_, v_n, nb);
+  memcpy(ku, u_, nb);
+  memcpy(kv, v_, nb);
+  double t = t0;
+  int64_t step = 0;
+  while (t < tf)
+  {
+    if (max_steps > 0 && step >= max_steps) break;
+    dt = dt < tf - t ? dt : tf - t;
+    memcpy(u0, u_, nb);
+    memcpy(v0, v_, nb);
+    for (int i = 0; i < 4; ++i)
+    {
+      memcpy(un, u0, nb);
+      memcpy(vn, v0, nb);
+      const double adt = dt * a_runge[i];
+      for (int64_t k = 0; k < ndofs; ++k) un[k] = ku[k] * adt + un[k];
+      for (int64_t k = 0; k < ndofs; ++k) vn[k] = kv[k] * adt + vn[k];
+      const double tn = t + c_runge[i] * dt;
+      memcpy(ku, vn, nb);
+      model_rhs_medium(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, tn, un, vn, kv, b, bv,
+                       sumfact, nthreads);
+      const double bdt = dt * b_runge[i];
+      for (int64_t k = 0; k < ndofs; ++k) u_[k] = ku[k] * bdt + u_[k];
+      for (int64_t k = 0; k < ndofs; ++k) v_[k] = kv[k] * bdt + v_[k];
+    }
+    t += dt;
+    step += 1;
+  }
+  memcpy(u_n, u_, nb);
+  memcpy(v_n, v_, nb);
+  if (t_end) *t_end = t;
+  free(u_); free(v_); free(un); free(vn); free(u0); free(v0); free(ku); free(kv); free(b); free(bv);
+  return step;
+}

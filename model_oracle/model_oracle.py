@@ -76,6 +76,15 @@ def lib():
         L.wo_rk4_pennes.restype = l
         L.wo_rk4_pennes.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, d, _f64p, _f64p, d, d, d, d, d, _f64p,
                                     d, d, d, d, l, _f64p, _f64p, _f64p, i, i, _f64p]
+        L.wo_boundary_facet_mass_weighted.restype = i
+        L.wo_boundary_facet_mass_weighted.argtypes = [i, l, _i32p, _i32p, _i32p, _f64p, _i32p, _i32p, _f64p, _f64p,
+                                                      _f64p]
+        L.wo_f1_westervelt_medium.restype = None
+        L.wo_f1_westervelt_medium.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, d, _f64p,
+                                              _f64p, _f64p, i, i]
+        L.wo_rk4_westervelt_medium.restype = l
+        L.wo_rk4_westervelt_medium.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, d, d, d,
+                                               l, _f64p, _f64p, i, i, _f64p]
         _lib.append(L)
     return _lib[0]
 
@@ -176,4 +185,45 @@ def rk4_pennes(mesh, P, G, m, m1, m2, k, rhoc, perf, T_art, h, T_ext, Q, s, t0, 
                                 _f(m2), k, _f(rhoc), _opt(perf), T_art, h[0], h[1], T_ext[0], T_ext[1], _opt(Q), s,
                                 t0, tf, dt, max_steps, _f(theta), _f(cem43), _f(theta_max), int(sumfact), nthreads,
                                 C.byref(t_end))
+    return steps, t_end.value
+
+
+# ---- layered media (DESIGN.md section 4.5e) -------------------------------------------------------------------------
+def boundary_facet_mass_weighted(mesh, P, facet_weight):
+    """(m1, m2) of oracle.boundary_facet_mass with facet f's GLL facet mass multiplied by facet_weight[f]"""
+    x = np.ascontiguousarray(mesh.x, dtype=np.float64)
+    xd = np.ascontiguousarray(mesh.xdofs, dtype=np.int32)
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    fc = np.ascontiguousarray(mesh.facet_cells, dtype=np.int32)
+    fl = np.ascontiguousarray(mesh.facet_local, dtype=np.int32)
+    ft = np.ascontiguousarray(mesh.facet_tags, dtype=np.int32)
+    fw = np.ascontiguousarray(facet_weight, dtype=np.float64)
+    assert fw.shape == (len(fc),)
+    m1, m2 = np.zeros(mesh.ndofs), np.zeros(mesh.ndofs)
+    ip = lambda a: a.ctypes.data_as(_i32p)  # noqa: E731
+    assert lib().wo_boundary_facet_mass_weighted(P, len(fc), ip(fc), ip(fl), ip(ft), _f(x.reshape(-1)),
+                                                 ip(xd.reshape(-1)), ip(dm.reshape(-1)), _f(fw), _f(m1), _f(m2)) == 0
+    return m1, m2
+
+
+def f1_westervelt_medium(mesh, P, G, m, m1, m2, kappa, c0, f0, p0, delta, t, u, v, sumfact=False, nthreads=1):
+    """f1_westervelt in a layered medium: G, m, m1, m2 weighted as given, kappa [ndofs] per dof"""
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    out = np.empty(mesh.ndofs)
+    lib().wo_f1_westervelt_medium(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)), _f(m),
+                                  _f(m1), _f(m2), _f(np.ascontiguousarray(kappa, dtype=np.float64)), c0, f0, p0, delta,
+                                  t, _f(u), _f(v), _f(out), int(sumfact), nthreads)
+    return out
+
+
+def rk4_westervelt_medium(mesh, P, G, m, m1, m2, kappa, c0, f0, p0, delta, t0, tf, dt, u, v, max_steps=0,
+                          sumfact=False, nthreads=1):
+    """rk4_westervelt in a layered medium (see f1_westervelt_medium); u, v updated in place.  -> (steps, t_end)"""
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    kappa = np.ascontiguousarray(kappa, dtype=np.float64)
+    assert kappa.shape == (mesh.ndofs,)
+    t_end = C.c_double()
+    steps = lib().wo_rk4_westervelt_medium(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)),
+                                           _f(m), _f(m1), _f(m2), _f(kappa), c0, f0, p0, delta, t0, tf, dt, max_steps,
+                                           _f(u), _f(v), int(sumfact), nthreads, C.byref(t_end))
     return steps, t_end.value

@@ -80,6 +80,7 @@ _SIG = {
                                   C.POINTER(C.c_int), C.POINTER(C.c_int), _c_i64p],
     "wfx_stiffness_destroy": [_vp],
     "wfx_mass_create": [_vp, _vp, C.c_int64, _c_i32p, _vpp],
+    "wfx_mass_create_weighted": [_vp, _vp, C.c_int64, _c_i32p, _c_f64p, _vpp],
     "wfx_mass_apply": [_vp, _vp, _vp, C.c_int, _vp],
     "wfx_mass_apply_host": [_vp, _vp, _vp, C.c_int],
     "wfx_mass_apply_inverse": [_vp, _vp, _vp, _vp],
@@ -93,6 +94,8 @@ _SIG = {
     "wfx_scatter_plan_destroy": [_vp],
     "wfx_boundary_create": [_vp, C.c_int, C.c_int, C.c_int64, _c_i32p, _c_i32p, _c_i32p, C.c_int64,
                             _c_f64p, _c_i32p, C.c_int64, _c_i32p, _vpp],
+    "wfx_boundary_create_weighted": [_vp, C.c_int, C.c_int, C.c_int64, _c_i32p, _c_i32p, _c_i32p, C.c_int64,
+                                     _c_f64p, _c_i32p, C.c_int64, _c_i32p, _c_f64p, _vpp],
     "wfx_boundary_apply": [_vp, C.c_double, C.c_double, _vp, _vp, _vp],
     "wfx_boundary_get": [_vp, _c_f64p, _c_f64p],
     "wfx_boundary_destroy": [_vp],
@@ -110,6 +113,7 @@ _SIG = {
     "wfx_wave_create_ensemble": [_vp, _vp, _vp, _vp, C.c_int, C.c_int64, C.c_double, _c_f64p, _c_f64p, _vpp],
     "wfx_wave_create_westervelt": [_vp, _vp, _vp, _vp, C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double,
                                    C.c_double, C.c_double, _vpp],
+    "wfx_wave_set_nonlinearity": [_vp, _c_f64p],
     "wfx_wave_init": [_vp],
     "wfx_wave_set_state": [_vp, _vp, _vp],
     "wfx_wave_get_state": [_vp, _vp, _vp],

@@ -96,34 +96,46 @@ boundary_profile_kernel(int64_t nb, int nv, const int32_t* __restrict__ idx, con
 
 // Lossy / Westervelt models: the Gamma2 mass term q = qc m2 on the absorbing dofs only, so that the dense
 // stage update needs nothing beyond 1/m (see boundary_absorbing_mass in wfx_internal.h).  p is formed in T
-// exactly as the stage kernel forms it.
-template <typename T>
+// exactly as the stage kernel forms it.  KD: a per-dof kappa (wfx_wave_set_nonlinearity), read in fp64 from kd, compact
+// over the boundary dofs like m2; otherwise the scalar kappa.
+template <typename T, bool KD>
 __global__ void absorbing_mass_kernel(int64_t nb, const int32_t* __restrict__ idx, const double* __restrict__ m2,
-                                      const double* __restrict__ m, double qc, double kappa, T s,
-                                      const T* __restrict__ pw, const T* __restrict__ pd, T* __restrict__ b)
+                                      const double* __restrict__ m, double qc, double kappa,
+                                      const double* __restrict__ kd, T s, const T* __restrict__ pw,
+                                      const T* __restrict__ pd, T* __restrict__ b)
 {
   const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (t >= nb || m2[t] == 0.0) return;
   const int32_t i = idx[t];
   const T pdt = pd[i];
   const double p = (double)(pw[i] - s * pdt);
+  if (KD) kappa = kd[t];
   const double mi = m[i], a = 1.0 - kappa * p, kp2 = kappa * (double)pdt * (double)pdt;
   const double kv = ((double)b[i] + mi * kp2) / (mi * a + qc * m2[t]);
   b[i] = (T)(mi * (kv * a - kp2));
 }
 } // namespace
 
-void wfx::boundary_absorbing_mass(wfx_boundary* op, const double* m64, double qc, double kappa, double s,
-                                  const void* pw, const void* pd, void* b, cudaStream_t stream)
+void wfx::boundary_absorbing_mass(wfx_boundary* op, const double* m64, double qc, double kappa,
+                                  const double* kappa_b, double s, const void* pw, const void* pd, void* b,
+                                  cudaStream_t stream)
 {
   if (!op || op->nb == 0) return;
   const unsigned grid = (unsigned)((op->nb + 255) / 256);
+#define WFX_ABS(T, KD)                                                                                              \
+  absorbing_mass_kernel<T, KD><<<grid, 256, 0, stream>>>(op->nb, op->d_idx.p, op->d_m2.p, m64, qc, kappa, kappa_b, \
+                                                         (T)s, (const T*)pw, (const T*)pd, (T*)b)
   if (op->dtype == WFX_F64)
-    absorbing_mass_kernel<double><<<grid, 256, 0, stream>>>(op->nb, op->d_idx.p, op->d_m2.p, m64, qc, kappa, s,
-                                                             (const double*)pw, (const double*)pd, (double*)b);
+  {
+    if (kappa_b) WFX_ABS(double, true);
+    else WFX_ABS(double, false);
+  }
   else
-    absorbing_mass_kernel<float><<<grid, 256, 0, stream>>>(op->nb, op->d_idx.p, op->d_m2.p, m64, qc, kappa, (float)s,
-                                                            (const float*)pw, (const float*)pd, (float*)b);
+  {
+    if (kappa_b) WFX_ABS(float, true);
+    else WFX_ABS(float, false);
+  }
+#undef WFX_ABS
   WFX_CUDA(cudaGetLastError());
 }
 
@@ -169,8 +181,21 @@ extern "C" int wfx_boundary_create(wfx_ctx* ctx, int P, int dtype, int64_t nface
                                    const int32_t* xdofs, int64_t ndofs, const int32_t* dofmap,
                                    wfx_boundary** out)
 {
+  return wfx_boundary_create_weighted(ctx, P, dtype, nfacets, fcell, flocal, ftag, npts, x, xdofs, ndofs, dofmap,
+                                      nullptr, out);
+}
+
+extern "C" int wfx_boundary_create_weighted(wfx_ctx* ctx, int P, int dtype, int64_t nfacets, const int32_t* fcell,
+                                            const int32_t* flocal, const int32_t* ftag, int64_t npts, const double* x,
+                                            const int32_t* xdofs, int64_t ndofs, const int32_t* dofmap,
+                                            const double* facet_weight, wfx_boundary** out)
+{
   WFX_API_BEGIN
   if (!ctx || !out) fail("NULL argument");
+  if (facet_weight)
+    for (int64_t f = 0; f < nfacets; ++f)
+      if (!std::isfinite(facet_weight[f]) || !(facet_weight[f] > 0))
+        fail("weighted boundary: the weight of facet %lld must be positive and finite", (long long)f);
   if (P < 1 || P + 1 > WFX_MAXN) fail("degree %d out of range", P);
   if (dtype != WFX_F64 && dtype != WFX_F32) fail("unknown dtype %d", dtype);
   ScopedDevice sd(ctx->device);
@@ -228,7 +253,8 @@ extern "C" int wfx_boundary_create(wfx_ctx* ctx, int P, int dtype, int64_t nface
         const double cx = t1[1] * t2[2] - t1[2] * t2[1];
         const double cy = t1[2] * t2[0] - t1[0] * t2[2];
         const double cz = t1[0] * t2[1] - t1[1] * t2[0];
-        const double ds = wts[ia] * wts[ib] * std::sqrt(cx * cx + cy * cy + cz * cz);
+        double ds = wts[ia] * wts[ib] * std::sqrt(cx * cx + cy * cy + cz * cz);
+        if (facet_weight) ds *= facet_weight[f]; // the medium's weight of this facet (1.0 leaves ds as it is)
         const int32_t dof = dofmap[c * nd + perm[(id[0] * n + id[1]) * n + id[2]]];
         if (dof < 0 || dof >= ndofs) fail("dofmap entry out of range");
         auto& e = acc[dof];

@@ -139,9 +139,11 @@ int64_t stiffness_nshared(const struct ::wfx_stiffness* op); // rank-shared dofs
 const double* mass_diagonal64(const struct ::wfx_mass* op);   // m on the device, fp64 whatever the dtype
 // On the absorbing (tag 2) dofs: b_i -> m_i [kv_i (1 - kappa p_i) - kappa pd_i^2] with the exact
 // kv_i = (b_i + kappa m_i pd_i^2) / (m_i (1 - kappa p_i) + qc m2_i), so that the dense stage update
-// kv = (b minv + kappa pd^2) / (1 - kappa p) yields it; p = pw - s pd (s = 0: pw is p itself)
-void boundary_absorbing_mass(struct ::wfx_boundary* op, const double* m64, double qc, double kappa, double s,
-                             const void* pw, const void* pd, void* b, cudaStream_t stream);
+// kv = (b minv + kappa pd^2) / (1 - kappa p) yields it; p = pw - s pd (s = 0: pw is p itself).  kappa_b (nullable):
+// a per-dof kappa in fp64, compact over boundary_dofs(op), in place of the scalar kappa
+void boundary_absorbing_mass(struct ::wfx_boundary* op, const double* m64, double qc, double kappa,
+                             const double* kappa_b, double s, const void* pw, const void* pd, void* b,
+                             cudaStream_t stream);
 // A wave model's field statistics as the thermal model reads them (wfx_thermal_heat_from_wave, DESIGN.md section
 // 4.5d): the unscaled fp64 harmonic sums, planes [h][ndofs * nv] (entry (dof i, member m) at i nv + m), the number
 // of sampled steps N (the amplitudes are the sums times 2 / N) and every member's source frequency (wfx_wave.cu)

@@ -8,6 +8,7 @@
 #include "wfx_internal.h"
 
 #include <algorithm>
+#include <cmath>
 
 using namespace wfx;
 
@@ -62,6 +63,24 @@ __global__ void segsum_kernel(int64_t nout, const int64_t* __restrict__ off,
   if (j >= nout) return;
   TO s = beta ? out[j] : TO(0);
   for (int64_t p = off[j]; p < off[j + 1]; ++p) s += (TO)in[src[p]];
+  out[j] = s;
+}
+
+// the weighted lumped mass (wfx_mass_create_weighted): segsum_kernel's reduction in the same order, every
+// contribution in[p] scaled by its cell's weight w[p / nq] first.  __dmul_rn keeps nvcc from contracting the product
+// into an FMA with the running sum, so that each term is rounded on its own as in a sum over w_c * detJw.
+__global__ void segsum_weighted_kernel(int64_t nout, const int64_t* __restrict__ off, const int32_t* __restrict__ src,
+                                       const double* __restrict__ in, const double* __restrict__ w, int nq,
+                                       double* __restrict__ out)
+{
+  const int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (j >= nout) return;
+  double s = 0.0;
+  for (int64_t p = off[j]; p < off[j + 1]; ++p)
+  {
+    const int32_t q = src[p];
+    s += __dmul_rn(w[q / nq], in[q]);
+  }
   out[j] = s;
 }
 
@@ -170,10 +189,20 @@ extern "C" int wfx_scatter_plan_destroy(wfx_scatter_plan* p)
 extern "C" int wfx_mass_create(wfx_ctx* ctx, wfx_geom* geom, int64_t ndofs,
                                const int32_t* dofmap_host, wfx_mass** out)
 {
+  return wfx_mass_create_weighted(ctx, geom, ndofs, dofmap_host, nullptr, out);
+}
+
+extern "C" int wfx_mass_create_weighted(wfx_ctx* ctx, wfx_geom* geom, int64_t ndofs, const int32_t* dofmap_host,
+                                        const double* cell_weight, wfx_mass** out)
+{
   WFX_API_BEGIN
   if (!ctx || !geom || !out) fail("NULL argument");
   if (geom->ctx != ctx) fail("geometry belongs to another context");
   if (ndofs < 0) fail("negative ndofs");
+  if (cell_weight)
+    for (int64_t c = 0; c < geom->ncells; ++c)
+      if (!std::isfinite(cell_weight[c]) || !(cell_weight[c] > 0))
+        fail("weighted mass: the weight of cell %lld must be positive and finite", (long long)c);
   ScopedDevice sd(ctx->device);
   auto op = std::make_unique<wfx_mass>();
   op->ctx = ctx;
@@ -194,8 +223,18 @@ extern "C" int wfx_mass_create(wfx_ctx* ctx, wfx_geom* geom, int64_t ndofs,
     plan.ctx = ctx;
     build_scatter_plan(&plan, (int64_t)tdm.size(), tdm.data(), ndofs);
     timer.lap("scatter plan");
-    segsum_kernel<double, double><<<(unsigned)((ndofs + 255) / 256), 256>>>(
-        ndofs, plan.d_off.p, plan.d_src.p, geom->dJw, op->d_m64.p, 0);
+    // m~ = sum_c w_c (detJ w)_{c,i}: the same segments, each contribution weighted by its cell (d_w lives until
+    // the synchronisation below)
+    DevBuf<double> d_w;
+    if (cell_weight)
+    {
+      d_w.upload(cell_weight, (size_t)geom->ncells);
+      segsum_weighted_kernel<<<(unsigned)((ndofs + 255) / 256), 256>>>(ndofs, plan.d_off.p, plan.d_src.p, geom->dJw,
+                                                                       d_w.p, geom->nq, op->d_m64.p);
+    }
+    else
+      segsum_kernel<double, double><<<(unsigned)((ndofs + 255) / 256), 256>>>(
+          ndofs, plan.d_off.p, plan.d_src.p, geom->dJw, op->d_m64.p, 0);
     WFX_CUDA(cudaGetLastError());
     WFX_CUDA(cudaDeviceSynchronize());
   }

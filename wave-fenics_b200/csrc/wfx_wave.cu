@@ -36,6 +36,12 @@ struct wfx_wave
   // boundary term is g + s_src g'; q = qc m2 is the Gamma2 mass term; f1 builds its w in f1_w.
   int model = 0;
   double kappa = 0, s_stiff = 0, s_src = 0, qc = 0;
+  // per-dof nonlinearity (wfx_wave_set_nonlinearity): kd [n] in the model dtype for the stage update and f1, kd_b
+  // the same values in fp64, compact over the boundary dofs, for the Gamma2 mass term.  With kd_on the nonlinear
+  // update runs whatever beta the model was created with.
+  bool kd_on = false;
+  DevBuf<unsigned char> kd;
+  DevBuf<double> kd_b;
   const double* m64 = nullptr;
   DevBuf<unsigned char> f1_w;
   const void* minv = nullptr;
@@ -232,11 +238,13 @@ void launch_stage_ens(int stage, int64_t n, int nv, const void* b, const void* m
 // p is u_ at stage 0; at stages 1-3 it is rebuilt as w - s vn (one read of w, no un vector).
 // On the absorbing dofs b has been replaced beforehand (boundary_absorbing_mass) so that this
 // quotient is the exact kv of the lumped system with the Gamma2 mass term.
-template <typename T, int STAGE, bool NL>
+// KD: kappa per dof, read from kd[n] (a layered medium, wfx_wave_set_nonlinearity); otherwise the scalar kappa.  The
+// arithmetic is the same, so kd filled with the scalar gives the scalar path's results bit for bit.
+template <typename T, int STAGE, bool NL, bool KD>
 __global__ void __launch_bounds__(256)
 rk_stage_westervelt_kernel(int64_t n, const T* __restrict__ b, const T* __restrict__ minv, T* __restrict__ u_,
                            T* __restrict__ v_, T* __restrict__ u0, T* __restrict__ v0, T* __restrict__ w,
-                           T* __restrict__ vn, T bdt, T adt_next, T s, T kappa)
+                           T* __restrict__ vn, T bdt, T adt_next, T s, T kappa, const T* __restrict__ kd)
 {
   const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (k >= n) return;
@@ -262,6 +270,7 @@ rk_stage_westervelt_kernel(int64_t n, const T* __restrict__ b, const T* __restri
       vb = v0[k];
     }
   }
+  if (KD) kappa = kd[k];
   if (NL) kv = (kv + kappa * ku * ku) / (T(1) - kappa * p);
   const T un_ = ku * bdt + us, vn_ = kv * bdt + vs;
   u_[k] = un_;
@@ -275,27 +284,39 @@ rk_stage_westervelt_kernel(int64_t n, const T* __restrict__ b, const T* __restri
   else w[k] = un_ + s * vn_;
 }
 
+// kd (nullable): per-dof kappa in T, which implies the nonlinear update
 template <typename T>
 void launch_stage_westervelt(int stage, bool nl, int64_t n, const void* b, const void* minv, void* u_, void* v_,
                              void* u0, void* v0, void* w, void* vn, double bdt, double adt_next, double s,
-                             double kappa, cudaStream_t st)
+                             double kappa, const void* kd, cudaStream_t st)
 {
   const unsigned grid = (unsigned)((n + 255) / 256);
-#define WFX_STAGE(S, NL)                                                                                    \
-  rk_stage_westervelt_kernel<T, S, NL><<<grid, 256, 0, st>>>(n, (const T*)b, (const T*)minv, (T*)u_, (T*)v_, \
-                                                              (T*)u0, (T*)v0, (T*)w, (T*)vn, (T)bdt,          \
-                                                              (T)adt_next, (T)s, (T)kappa)
-  switch (stage * 2 + (nl ? 1 : 0))
+#define WFX_STAGE(S, NL, KD)                                                                                    \
+  rk_stage_westervelt_kernel<T, S, NL, KD><<<grid, 256, 0, st>>>(n, (const T*)b, (const T*)minv, (T*)u_, (T*)v_, \
+                                                                  (T*)u0, (T*)v0, (T*)w, (T*)vn, (T)bdt,          \
+                                                                  (T)adt_next, (T)s, (T)kappa, (const T*)kd)
+  if (kd)
   {
-  case 0: WFX_STAGE(0, false); break;
-  case 1: WFX_STAGE(0, true); break;
-  case 2: WFX_STAGE(1, false); break;
-  case 3: WFX_STAGE(1, true); break;
-  case 4: WFX_STAGE(2, false); break;
-  case 5: WFX_STAGE(2, true); break;
-  case 6: WFX_STAGE(3, false); break;
-  default: WFX_STAGE(3, true); break;
+    switch (stage)
+    {
+    case 0: WFX_STAGE(0, true, true); break;
+    case 1: WFX_STAGE(1, true, true); break;
+    case 2: WFX_STAGE(2, true, true); break;
+    default: WFX_STAGE(3, true, true); break;
+    }
   }
+  else
+    switch (stage * 2 + (nl ? 1 : 0))
+    {
+    case 0: WFX_STAGE(0, false, false); break;
+    case 1: WFX_STAGE(0, true, false); break;
+    case 2: WFX_STAGE(1, false, false); break;
+    case 3: WFX_STAGE(1, true, false); break;
+    case 4: WFX_STAGE(2, false, false); break;
+    case 5: WFX_STAGE(2, true, false); break;
+    case 6: WFX_STAGE(3, false, false); break;
+    default: WFX_STAGE(3, true, false); break;
+    }
 #undef WFX_STAGE
   WFX_CUDA(cudaGetLastError());
 }
@@ -308,13 +329,16 @@ __global__ void axpy_kernel(int64_t n, const T* __restrict__ u, const T* __restr
   if (k < n) w[k] = u[k] + s * v[k];
 }
 
-// f1 of the lossy / Westervelt models: out = (b / m + kappa v^2) / (1 - kappa u), the stage kernel's kv
-template <typename T>
+// f1 of the lossy / Westervelt models: out = (b / m + kappa v^2) / (1 - kappa u), the stage kernel's kv (KD: kappa
+// per dof from kd)
+template <typename T, bool KD>
 __global__ void westervelt_rhs_kernel(int64_t n, const T* __restrict__ b, const T* __restrict__ minv,
-                                      const T* __restrict__ u, const T* __restrict__ v, T kappa, T* __restrict__ out)
+                                      const T* __restrict__ u, const T* __restrict__ v, T kappa,
+                                      const T* __restrict__ kd, T* __restrict__ out)
 {
   const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (k >= n) return;
+  if (KD) kappa = kd[k];
   const T vk = v[k];
   out[k] = (b[k] * minv[k] + kappa * vk * vk) / (T(1) - kappa * u[k]);
 }
@@ -578,15 +602,18 @@ void enqueue_step(wfx_wave* w, double dt, const double* g, const double* tn, boo
     {
       // Gamma2 mass term (compact, absorbing dofs), then the fused update; p = u_ at stage 0, else w - s vn
       if (w->qc != 0)
-        boundary_absorbing_mass(w->bnd, w->m64, w->qc, w->kappa, i == 0 ? 0.0 : w->s_stiff,
-                                i == 0 ? w->u_.p : w->un.p, vn, w->b.p, st);
+        boundary_absorbing_mass(w->bnd, w->m64, w->qc, w->kappa, w->kd_on ? w->kd_b.p : nullptr,
+                                i == 0 ? 0.0 : w->s_stiff, i == 0 ? w->u_.p : w->un.p, vn, w->b.p, st);
       NvtxRange update_range("wfx fused stage update");
+      const void* kd = w->kd_on ? w->kd.p : nullptr;
       if (w->dtype == WFX_F64)
         launch_stage_westervelt<double>(i, w->model == 2, w->n, w->b.p, w->minv, w->u_.p, w->v_.p, w->u0.p, w->v0.p,
-                                        w->un.p, w->vn.p, dt * b_runge[i], dt * a_runge[i + 1], w->s_stiff, w->kappa, st);
+                                        w->un.p, w->vn.p, dt * b_runge[i], dt * a_runge[i + 1], w->s_stiff, w->kappa,
+                                        kd, st);
       else
         launch_stage_westervelt<float>(i, w->model == 2, w->n, w->b.p, w->minv, w->u_.p, w->v_.p, w->u0.p, w->v0.p,
-                                       w->un.p, w->vn.p, dt * b_runge[i], dt * a_runge[i + 1], w->s_stiff, w->kappa, st);
+                                       w->un.p, w->vn.p, dt * b_runge[i], dt * a_runge[i + 1], w->s_stiff, w->kappa,
+                                       kd, st);
       continue;
     }
     NvtxRange update_range("wfx fused stage update");
@@ -875,15 +902,24 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
     if (wfx_stiffness_apply(w->stiff, w->f1_w.p, w->b.p, 0, st)) fail("%s", wfx_last_error());
     if (w->prof_on) boundary_profiled(w, t, nullptr, v, st);
     else if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());
-    if (w->qc != 0) boundary_absorbing_mass(w->bnd, w->m64, w->qc, w->kappa, 0.0, u, v, w->b.p, st);
+    if (w->qc != 0)
+      boundary_absorbing_mass(w->bnd, w->m64, w->qc, w->kappa, w->kd_on ? w->kd_b.p : nullptr, 0.0, u, v, w->b.p, st);
     if (w->n == 0) return 0;
     const unsigned grid = (unsigned)((w->n + 255) / 256);
+#define WFX_RHS(T, KD)                                                                                           \
+  westervelt_rhs_kernel<T, KD><<<grid, 256, 0, st>>>(w->n, (const T*)w->b.p, (const T*)w->minv, (const T*)u,    \
+                                                     (const T*)v, (T)w->kappa, (const T*)w->kd.p, (T*)result)
     if (w->dtype == WFX_F64)
-      westervelt_rhs_kernel<double><<<grid, 256, 0, st>>>(w->n, (const double*)w->b.p, (const double*)w->minv,
-                                                           (const double*)u, (const double*)v, w->kappa, (double*)result);
+    {
+      if (w->kd_on) WFX_RHS(double, true);
+      else WFX_RHS(double, false);
+    }
     else
-      westervelt_rhs_kernel<float><<<grid, 256, 0, st>>>(w->n, (const float*)w->b.p, (const float*)w->minv,
-                                                          (const float*)u, (const float*)v, (float)w->kappa, (float*)result);
+    {
+      if (w->kd_on) WFX_RHS(float, true);
+      else WFX_RHS(float, false);
+    }
+#undef WFX_RHS
     WFX_CUDA(cudaGetLastError());
     return 0;
   }
@@ -1154,6 +1190,49 @@ extern "C" int wfx_wave_set_source_profile(wfx_wave* w, const double* amp_host, 
   w->prof_amp.upload(a);
   w->prof_delay.upload(d);
   w->prof_on = true;
+  WFX_API_END
+}
+
+extern "C" int wfx_wave_set_nonlinearity(wfx_wave* w, const double* kappa_host)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  if (!w->model || w->ens) fail("nonlinearity: needs a model made by wfx_wave_create_westervelt");
+  if (kappa_host)
+    for (int64_t k = 0; k < w->n; ++k)
+      if (!std::isfinite(kappa_host[k]) || kappa_host[k] < 0)
+        fail("nonlinearity: kappa at dof %lld must be finite and not negative", (long long)k);
+  ScopedDevice sd(w->ctx->device);
+  // a step in flight may read the buffers, and the captured step holds the scalar or the per-dof kernels
+  WFX_CUDA(cudaDeviceSynchronize());
+  if (w->step_graph) WFX_CUDA(cudaGraphExecDestroy(w->step_graph));
+  w->step_graph = nullptr;
+  w->kd_on = false;
+  if (!kappa_host)
+  {
+    w->kd.release();
+    w->kd_b.release();
+    return 0;
+  }
+  const size_t esz = w->dtype == WFX_F64 ? 8 : 4;
+  if (w->kd.n != (size_t)w->n * esz) w->kd.alloc((size_t)w->n * esz);
+  if (w->dtype == WFX_F64) w->kd.upload((const unsigned char*)kappa_host, (size_t)w->n * esz);
+  else
+  {
+    std::vector<float> k32((size_t)w->n);
+    for (int64_t k = 0; k < w->n; ++k) k32[k] = (float)kappa_host[k];
+    w->kd.upload((const unsigned char*)k32.data(), (size_t)w->n * esz);
+  }
+  if (w->bnd)
+  {
+    // the Gamma2 mass term takes kappa in fp64, as the scalar path does
+    const std::vector<int32_t>& dofs = boundary_dofs(w->bnd);
+    std::vector<double> kb(dofs.size());
+    for (size_t p = 0; p < dofs.size(); ++p) kb[p] = kappa_host[dofs[p]];
+    if (w->kd_b.n != kb.size()) w->kd_b.alloc(kb.size());
+    w->kd_b.upload(kb);
+  }
+  w->kd_on = true;
   WFX_API_END
 }
 

@@ -196,11 +196,12 @@ template <typename T>
 class MassOperator
 {
 public:
-  MassOperator(std::shared_ptr<Geometry<T>> geom, const SpaceView& V, int bdegree)
+  // cell_weight: one weight per cell (the weighted mass of a layered medium, DESIGN.md section 4.5e) or nullptr
+  MassOperator(std::shared_ptr<Geometry<T>> geom, const SpaceView& V, int bdegree, const double* cell_weight = nullptr)
       : _geom(std::move(geom)), _ndofs(V.ndofs)
   {
     if (bdegree != V.degree) throw std::runtime_error("wavefx: degree mismatch");
-    check(wfx_mass_create(_geom->context()->get(), _geom->get(), V.ndofs, V.dofmap, &_h));
+    check(wfx_mass_create_weighted(_geom->context()->get(), _geom->get(), V.ndofs, V.dofmap, cell_weight, &_h));
   }
   ~MassOperator() { wfx_mass_destroy(_h); }
   MassOperator(const MassOperator&) = delete;
@@ -340,6 +341,22 @@ inline void set_profile(wfx_wave* wave, std::int64_t entries, const std::vector<
   check(wfx_wave_set_source_profile(wave, amp.empty() ? nullptr : amp.data(), delay.empty() ? nullptr : delay.data()));
 }
 
+// A layered medium (DESIGN.md section 4.5e) as the weights of the operators, e.g. from the Python Medium class:
+//   stiffness [ncells]  rho_ref / rho_c                         (scales the model's geometry)
+//   mass      [ncells]  rho_ref c0^2 / (rho_c c_c^2)            (weighted lumped mass)
+//   facet     [nfacets] rho_ref / rho_f on tag 1, rho_ref c0 / (rho_f c_f) on tag 2, 1 elsewhere
+//   kappa     [ndofs]   the per-dof nonlinearity of the Westervelt model; empty: the model's scalar kappa
+struct Medium
+{
+  std::vector<double> stiffness, mass, facet, kappa;
+};
+inline void check_medium(const SpaceView& V, const Medium& m)
+{
+  if ((std::int64_t)m.stiffness.size() != V.ncells || (std::int64_t)m.mass.size() != V.ncells ||
+      (std::int64_t)m.facet.size() != V.nfacets)
+    throw std::runtime_error("wavefx: medium needs stiffness and mass weights per cell and a weight per facet");
+}
+
 // The wave model and its RK4 driver (common/LinearGLL.hpp:37-287), fp64 like the reference.
 class LinearGLLOpt
 {
@@ -364,6 +381,15 @@ public:
                               V.facet_tag, V.npoints, V.x, V.xdofs, V.ndofs, V.dofmap, &_bnd));  // :113-115
     check(wfx_wave_create(_ctx->get(), stiff_op->get(), mass_op->get(), _bnd, _halo ? _halo->get() : nullptr, V.size_local,
                           speedOfSound, sourceFrequency, pressureAmplitude, &_wave));
+  }
+  // the same model in a layered medium (one rank)
+  LinearGLLOpt(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
+               double sourceFrequency, double pressureAmplitude, const Medium& medium)
+      : _ctx(std::move(ctx)), _ndofs(V.ndofs)
+  {
+    make_operators(V, degreeOfBasis, speedOfSound, &medium);
+    check(wfx_wave_create(_ctx->get(), stiff_op->get(), mass_op->get(), _bnd, nullptr, V.size_local, speedOfSound,
+                          sourceFrequency, pressureAmplitude, &_wave));
   }
   ~LinearGLLOpt()
   {
@@ -449,17 +475,31 @@ public:
 protected:
   // the lossy / Westervelt models (wfx_wave_create_westervelt, one rank): see WesterveltGLLOpt
   LinearGLLOpt(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
-               double sourceFrequency, double pressureAmplitude, double delta, double beta, double rho0)
+               double sourceFrequency, double pressureAmplitude, double delta, double beta, double rho0,
+               const Medium* medium = nullptr)
       : _ctx(std::move(ctx)), _ndofs(V.ndofs)
   {
-    _geom = std::make_shared<Geometry<double>>(_ctx, V);
-    mass_op = std::make_shared<MassOperator<double>>(_geom, V, degreeOfBasis);
-    std::map<std::string, double> params{{"c0", speedOfSound}};
-    stiff_op = std::make_shared<StiffnessOperator<double>>(_geom, V, degreeOfBasis, params);
-    check(wfx_boundary_create(_ctx->get(), V.degree, WFX_F64, V.nfacets, V.facet_cell, V.facet_local,
-                              V.facet_tag, V.npoints, V.x, V.xdofs, V.ndofs, V.dofmap, &_bnd));
+    make_operators(V, degreeOfBasis, speedOfSound, medium);
     check(wfx_wave_create_westervelt(_ctx->get(), stiff_op->get(), mass_op->get(), _bnd, V.size_local, speedOfSound,
                                      sourceFrequency, pressureAmplitude, delta, beta, rho0, &_wave));
+    if (medium && !medium->kappa.empty())
+    {
+      if ((std::int64_t)medium->kappa.size() != V.ndofs) throw std::runtime_error("wavefx: medium kappa needs ndofs entries");
+      check(wfx_wave_set_nonlinearity(_wave, medium->kappa.data()));
+    }
+  }
+  // geometry (scaled by the medium's stiffness weight), mass, stiffness and boundary operators of one rank
+  void make_operators(const SpaceView& V, int degreeOfBasis, double speedOfSound, const Medium* medium)
+  {
+    _geom = std::make_shared<Geometry<double>>(_ctx, V);
+    if (medium) check_medium(V, *medium);
+    if (medium) _geom->scale_cells(medium->stiffness);
+    mass_op = std::make_shared<MassOperator<double>>(_geom, V, degreeOfBasis, medium ? medium->mass.data() : nullptr);
+    std::map<std::string, double> params{{"c0", speedOfSound}};
+    stiff_op = std::make_shared<StiffnessOperator<double>>(_geom, V, degreeOfBasis, params);
+    check(wfx_boundary_create_weighted(_ctx->get(), V.degree, WFX_F64, V.nfacets, V.facet_cell, V.facet_local,
+                                       V.facet_tag, V.npoints, V.x, V.xdofs, V.ndofs, V.dofmap,
+                                       medium ? medium->facet.data() : nullptr, &_bnd));
   }
 
 private:
@@ -490,6 +530,19 @@ public:
                      diffusivityOfSound, coefficientOfNonlinearity, density)
   {
   }
+  // in a layered medium: medium.kappa (per dof) in place of the scalar kappa when it is not empty
+  WesterveltGLLOpt(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
+                   double sourceFrequency, double pressureAmplitude, double diffusivityOfSound,
+                   double coefficientOfNonlinearity, double density, const Medium& medium)
+      : LinearGLLOpt(std::move(ctx), V, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
+                     diffusivityOfSound, coefficientOfNonlinearity, density, &medium)
+  {
+  }
+  // a per-dof kappa (ndofs entries) in place of the scalar; an empty vector restores the scalar
+  void set_nonlinearity(const std::vector<double>& kappa)
+  {
+    check(wfx_wave_set_nonlinearity(get(), kappa.empty() ? nullptr : kappa.data()));
+  }
 };
 // The lossy model: WesterveltGLLOpt with beta = 0,  p_tt - c0^2 lap p - delta lap p_t = 0
 class LossyGLLOpt : public WesterveltGLLOpt
@@ -499,6 +552,12 @@ public:
               double sourceFrequency, double pressureAmplitude, double diffusivityOfSound)
       : WesterveltGLLOpt(std::move(ctx), V, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
                          diffusivityOfSound, 0.0, 1.0)
+  {
+  }
+  LossyGLLOpt(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
+              double sourceFrequency, double pressureAmplitude, double diffusivityOfSound, const Medium& medium)
+      : WesterveltGLLOpt(std::move(ctx), V, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
+                         diffusivityOfSound, 0.0, 1.0, medium)
   {
   }
 };
@@ -512,20 +571,42 @@ class LinearGLLEnsemble
 public:
   LinearGLLEnsemble(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
                     const std::vector<double>& sourceFrequencies, const std::vector<double>& pressureAmplitudes)
+      : LinearGLLEnsemble(std::move(ctx), V, degreeOfBasis, speedOfSound, sourceFrequencies, pressureAmplitudes,
+                          static_cast<const Medium*>(nullptr))
+  {
+  }
+  // in a layered medium (its kappa is not used: the ensemble is linear)
+  LinearGLLEnsemble(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
+                    const std::vector<double>& sourceFrequencies, const std::vector<double>& pressureAmplitudes,
+                    const Medium& medium)
+      : LinearGLLEnsemble(std::move(ctx), V, degreeOfBasis, speedOfSound, sourceFrequencies, pressureAmplitudes,
+                          &medium)
+  {
+  }
+
+private:
+  LinearGLLEnsemble(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
+                    const std::vector<double>& sourceFrequencies, const std::vector<double>& pressureAmplitudes,
+                    const Medium* medium)
       : _ctx(std::move(ctx)), _ndofs(V.ndofs), _nv((int)sourceFrequencies.size())
   {
     if (pressureAmplitudes.size() != sourceFrequencies.size())
       throw std::runtime_error("wavefx: one source frequency and one pressure amplitude per member expected");
     _geom = std::make_shared<Geometry<double>>(_ctx, V);
-    mass_op = std::make_shared<MassOperator<double>>(_geom, V, degreeOfBasis);
+    if (medium) check_medium(V, *medium);
+    if (medium) _geom->scale_cells(medium->stiffness);
+    mass_op = std::make_shared<MassOperator<double>>(_geom, V, degreeOfBasis, medium ? medium->mass.data() : nullptr);
     std::map<std::string, double> params{{"c0", speedOfSound}};
     stiff_op = std::make_shared<StiffnessOperator<double>>(_geom, V, degreeOfBasis, params, std::vector<std::int32_t>{},
                                                            WFX_STIFF_ENSEMBLE);
-    check(wfx_boundary_create(_ctx->get(), V.degree, WFX_F64, V.nfacets, V.facet_cell, V.facet_local, V.facet_tag,
-                              V.npoints, V.x, V.xdofs, V.ndofs, V.dofmap, &_bnd));
+    check(wfx_boundary_create_weighted(_ctx->get(), V.degree, WFX_F64, V.nfacets, V.facet_cell, V.facet_local,
+                                       V.facet_tag, V.npoints, V.x, V.xdofs, V.ndofs, V.dofmap,
+                                       medium ? medium->facet.data() : nullptr, &_bnd));
     check(wfx_wave_create_ensemble(_ctx->get(), stiff_op->get(), mass_op->get(), _bnd, _nv, V.size_local, speedOfSound,
                                    sourceFrequencies.data(), pressureAmplitudes.data(), &_wave));
   }
+
+public:
   ~LinearGLLEnsemble()
   {
     wfx_wave_destroy(_wave);

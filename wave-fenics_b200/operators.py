@@ -10,6 +10,8 @@ Same names, argument meaning and call shape as the reference classes:
                                                 nv LinearGLLOpt models on one mesh, stepped together
   WesterveltGLLOpt(mesh, meshtags, degree, c0, f0, p0, delta, beta, rho0), LossyGLLOpt (beta = 0)
                                                 lossy and nonlinear (Westervelt) models, DESIGN.md 4.5a
+  Medium(rho, c, beta)                          layered media (per-cell density, sound speed and nonlinearity),
+                                                the `medium=` keyword of every wave model, DESIGN.md 4.5e
 
 `V` is a HexMesh (mesh.py): it carries what the reference pulls out of the DOLFINx
 FunctionSpace (geometry, geometry dofmap, cell dofmap, index-map sizes).  Vectors are
@@ -245,9 +247,10 @@ class StiffnessOperator(_Operator):
 
 
 class MassOperator(_Operator):
-    """y += M x with the collocated (diagonal) GLL mass (common/operators.hpp:86-108)."""
+    """y += M x with the collocated (diagonal) GLL mass (common/operators.hpp:86-108).  cell_weight: one positive
+    weight per cell, m_i = sum_c w_c (detJ w)_{c,i} (the weighted mass of a layered medium, Medium.mass_weight)."""
 
-    def __init__(self, V, degree, dtype=np.float64, ctx=None, geometry=None):
+    def __init__(self, V, degree, dtype=np.float64, ctx=None, geometry=None, cell_weight=None):
         self.ctx = ctx or Context.get()
         self.P = int(degree)
         self.dtype = np.dtype(dtype)
@@ -255,8 +258,12 @@ class MassOperator(_Operator):
         self.ndofs = int(V.ndofs)
         self.handle = C.c_void_p()
         dm = np.ascontiguousarray(V.dofmap, dtype=np.int32)
-        capi.call("wfx_mass_create", self.ctx.handle, self.geometry.handle, self.ndofs,
-                  capi.i32p(dm.reshape(-1)), C.byref(self.handle))
+        if cell_weight is not None:
+            cell_weight = np.ascontiguousarray(cell_weight, dtype=np.float64).reshape(-1)
+            if cell_weight.size != V.ncells:
+                raise capi.WfxError("one mass weight per cell expected")
+        capi.call("wfx_mass_create_weighted", self.ctx.handle, self.geometry.handle, self.ndofs,
+                  capi.i32p(dm.reshape(-1)), capi.f64p(cell_weight), C.byref(self.handle))
 
     def __call__(self, x, y):
         self.apply(x, y, beta=1)
@@ -312,9 +319,10 @@ MassOperatorCPU = MassOperator
 
 
 class BoundaryOperator(_Operator):
-    """b += c0^2 g m1 - c0 m2 .* v_n  (forms.ufl:21-24 via assemble_vector, LinearGLL.hpp:175)."""
+    """b += c0^2 g m1 - c0 m2 .* v_n  (forms.ufl:21-24 via assemble_vector, LinearGLL.hpp:175).  facet_weight: one
+    positive weight per facet triplet multiplying its facet mass (a layered medium, Medium.facet_weight)."""
 
-    def __init__(self, V, degree, dtype=np.float64, ctx=None):
+    def __init__(self, V, degree, dtype=np.float64, ctx=None, facet_weight=None):
         self.ctx = ctx or Context.get()
         self.P = int(degree)
         self.dtype = np.dtype(dtype)
@@ -326,9 +334,14 @@ class BoundaryOperator(_Operator):
         fc = np.ascontiguousarray(V.facet_cells, dtype=np.int32)
         fl = np.ascontiguousarray(V.facet_local, dtype=np.int32)
         ft = np.ascontiguousarray(V.facet_tags, dtype=np.int32)
-        capi.call("wfx_boundary_create", self.ctx.handle, self.P, capi.dtype_code(self.dtype), len(fc),
+        if facet_weight is not None:
+            facet_weight = np.ascontiguousarray(facet_weight, dtype=np.float64).reshape(-1)
+            if facet_weight.size != len(fc):
+                raise capi.WfxError("one facet weight per facet triplet expected")
+        capi.call("wfx_boundary_create_weighted", self.ctx.handle, self.P, capi.dtype_code(self.dtype), len(fc),
                   capi.i32p(fc), capi.i32p(fl), capi.i32p(ft), x.shape[0], capi.f64p(x.reshape(-1)),
-                  capi.i32p(xd.reshape(-1)), self.ndofs, capi.i32p(dm.reshape(-1)), C.byref(self.handle))
+                  capi.i32p(xd.reshape(-1)), self.ndofs, capi.i32p(dm.reshape(-1)), capi.f64p(facet_weight),
+                  C.byref(self.handle))
 
     def apply(self, c0, g, vn, b):
         self._check(vn, b)
@@ -363,26 +376,30 @@ class LinearGLLOpt:
     """The wave model + RK4 driver (common/LinearGLL.hpp:37-287) on the GPU.
 
     mesh carries the facet tags (`meshtags` may be None or a (cells, local, tags) triple that
-    overrides them)."""
+    overrides them).  medium: a Medium (layered media, DESIGN.md section 4.5e) or None; one rank only."""
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency,
                  pressureAmplitude, dtype=np.float64, ctx=None, halo=None, stiffness_mode=capi.STIFF_AUTO,
-                 setup_halo=None):
+                 setup_halo=None, medium=None):
         self.ctx = ctx or Context.get()
         self.V = mesh
         if meshtags is not None:
             import copy
             mesh = copy.copy(mesh)
             mesh.facet_cells, mesh.facet_local, mesh.facet_tags = meshtags
+        if medium is not None and halo is not None:
+            raise capi.WfxError("medium: distributed models are not supported (one rank only)")
         self.k_ = int(degreeOfBasis)
         self.c0_, self.freq0_, self.p0_ = float(speedOfSound), float(sourceFrequency), float(pressureAmplitude)
         self.dtype = np.dtype(dtype)
-        self.geometry = Geometry(mesh, self.k_, dtype, self.ctx)
-        self.mass_op = MassOperator(mesh, self.k_, dtype, self.ctx, self.geometry)      # :105
+        self._medium_geometry(mesh, medium)
+        self.mass_op = MassOperator(mesh, self.k_, dtype, self.ctx, self.geometry,
+                                    cell_weight=self._mass_weight)                      # :105
         params = {"c0": self.c0_}
         self.stiff_op = StiffnessOperator(mesh, self.k_, params, dtype, self.ctx, self.geometry,
                                           mode=stiffness_mode)                           # :120
-        self.bnd_op = BoundaryOperator(mesh, self.k_, dtype, self.ctx)                   # :113-115
+        self.bnd_op = BoundaryOperator(mesh, self.k_, dtype, self.ctx,
+                                       facet_weight=self._facet_weight)                  # :113-115
         self.halo = halo
         if halo is not None:
             # the masses are summed over the ranks in fp64: an fp32 model needs a second, fp64 halo
@@ -401,6 +418,20 @@ class LinearGLLOpt:
                   self.bnd_op.handle, halo.handle if halo is not None else None, int(mesh.size_local),
                   self.c0_, self.freq0_, self.p0_, C.byref(self.handle))
         self.ndofs = int(mesh.ndofs)
+
+    def _medium_geometry(self, mesh, medium):
+        """The model's geometry, scaled by the medium's stiffness weight, and the medium's mass and facet weights
+        (None without a medium)."""
+        if medium is not None and not isinstance(medium, Medium):
+            raise capi.WfxError("medium must be a Medium")
+        self.medium = medium
+        self.geometry = Geometry(mesh, self.k_, self.dtype, self.ctx)
+        self._mass_weight = self._facet_weight = None
+        if medium is None:
+            return
+        self.geometry.scale_cells(medium.stiffness_weight(mesh.ncells))
+        self._mass_weight = medium.mass_weight(mesh.ncells, self.c0_)
+        self._facet_weight = medium.facet_weight(mesh, self.c0_)
 
     def init(self):
         capi.call("wfx_wave_init", self.handle)
@@ -528,7 +559,7 @@ class LinearGLLEnsemble(LinearGLLOpt):
     available for ensembles."""
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequencies, pressureAmplitudes,
-                 dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO):
+                 dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO, medium=None):
         self.ctx = ctx or Context.get()
         self.V = mesh
         if meshtags is not None:
@@ -544,11 +575,11 @@ class LinearGLLEnsemble(LinearGLLOpt):
         self.c0_ = float(speedOfSound)
         self.freq0s_, self.p0s_ = f0s, p0s
         self.dtype = np.dtype(dtype)
-        self.geometry = Geometry(mesh, self.k_, dtype, self.ctx)
-        self.mass_op = MassOperator(mesh, self.k_, dtype, self.ctx, self.geometry)
+        self._medium_geometry(mesh, medium)
+        self.mass_op = MassOperator(mesh, self.k_, dtype, self.ctx, self.geometry, cell_weight=self._mass_weight)
         self.stiff_op = StiffnessOperator(mesh, self.k_, {"c0": self.c0_}, dtype, self.ctx, self.geometry,
                                           mode=stiffness_mode, ensemble=True)
-        self.bnd_op = BoundaryOperator(mesh, self.k_, dtype, self.ctx)
+        self.bnd_op = BoundaryOperator(mesh, self.k_, dtype, self.ctx, facet_weight=self._facet_weight)
         self.halo = None
         self.handle = C.c_void_p()
         capi.call("wfx_wave_create_ensemble", self.ctx.handle, self.stiff_op.handle, self.mass_op.handle,
@@ -596,11 +627,13 @@ class WesterveltGLLOpt(LinearGLLOpt):
     dp/dn = g(t) on tag 1 (the source of LinearGLLOpt), dp/dn = -p_t / c0 on tag 2.  diffusivityOfSound
     delta [m^2/s] >= 0, coefficientOfNonlinearity beta >= 0, density rho0 [kg/m^3] > 0 when beta > 0.
     delta = beta = 0 is LinearGLLOpt bit for bit.  A per-cell coefficient set with Geometry.scale_cells
-    multiplies the delta term too (delta_eff = delta * coeff)."""
+    multiplies the delta term too (delta_eff = delta * coeff).  With a Medium the nonlinearity is per dof
+    (set_nonlinearity), from the medium's beta, which defaults to coefficientOfNonlinearity; delta_eff = delta
+    (c / c0)^2 (DESIGN.md section 4.5e)."""
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
                  diffusivityOfSound, coefficientOfNonlinearity, density, dtype=np.float64, ctx=None,
-                 stiffness_mode=capi.STIFF_AUTO):
+                 stiffness_mode=capi.STIFF_AUTO, medium=None):
         self.ctx = ctx or Context.get()
         self.V = mesh
         if meshtags is not None:
@@ -612,44 +645,156 @@ class WesterveltGLLOpt(LinearGLLOpt):
         self.delta_, self.beta_, self.rho0_ = (float(diffusivityOfSound), float(coefficientOfNonlinearity),
                                                float(density))
         self.dtype = np.dtype(dtype)
-        self.geometry = Geometry(mesh, self.k_, dtype, self.ctx)
-        self.mass_op = MassOperator(mesh, self.k_, dtype, self.ctx, self.geometry)
+        self._medium_geometry(mesh, medium)
+        self.mass_op = MassOperator(mesh, self.k_, dtype, self.ctx, self.geometry, cell_weight=self._mass_weight)
         self.stiff_op = StiffnessOperator(mesh, self.k_, {"c0": self.c0_}, dtype, self.ctx, self.geometry,
                                           mode=stiffness_mode)
-        self.bnd_op = BoundaryOperator(mesh, self.k_, dtype, self.ctx)
+        self.bnd_op = BoundaryOperator(mesh, self.k_, dtype, self.ctx, facet_weight=self._facet_weight)
         self.halo = None
         self.handle = C.c_void_p()
         capi.call("wfx_wave_create_westervelt", self.ctx.handle, self.stiff_op.handle, self.mass_op.handle,
                   self.bnd_op.handle, int(mesh.size_local), self.c0_, self.freq0_, self.p0_, self.delta_,
                   self.beta_, self.rho0_, C.byref(self.handle))
         self.ndofs = int(mesh.ndofs)
+        self.kappa = None
+        if medium is not None:
+            kappa = medium.kappa(mesh, self.geometry.detJw(), self.c0_, self.beta_)
+            # the medium's kappa replaces the scalar one whenever either is nonzero; only a model created with
+            # beta = 0 in a medium without nonlinearity keeps the lossy update
+            if self.beta_ > 0 or np.any(kappa > 0):
+                self.set_nonlinearity(kappa)
+
+    def set_nonlinearity(self, kappa=None):
+        """kappa [ndofs] >= 0: a per-dof kappa in place of 2 beta / (rho0 c0^2) (the model then steps the nonlinear
+        update even with beta = 0); None restores the scalar.  Survives init, set_state and restarts."""
+        k = None if kappa is None else np.ascontiguousarray(kappa, dtype=np.float64)
+        if k is not None and k.shape != (self.ndofs,):
+            raise capi.WfxError(f"kappa must have shape ({self.ndofs},)")
+        capi.call("wfx_wave_set_nonlinearity", self.handle, capi.f64p(k))
+        self.kappa = k
 
 
 class LossyGLLOpt(WesterveltGLLOpt):
-    """The lossy wave model (WesterveltGLLOpt with beta = 0):  p_tt - c0^2 lap p - delta lap p_t = 0."""
+    """The lossy wave model (WesterveltGLLOpt with beta = 0):  p_tt - c0^2 lap p - delta lap p_t = 0.  In a Medium
+    that gives beta per cell the model steps the Westervelt update with the medium's per-dof kappa (the medium's
+    beta replaces the model's beta = 0, as for WesterveltGLLOpt); a Medium without beta keeps it lossy."""
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
-                 diffusivityOfSound, dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO):
+                 diffusivityOfSound, dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO, medium=None):
         super().__init__(mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
-                         diffusivityOfSound, 0.0, 1.0, dtype=dtype, ctx=ctx, stiffness_mode=stiffness_mode)
+                         diffusivityOfSound, 0.0, 1.0, dtype=dtype, ctx=ctx, stiffness_mode=stiffness_mode,
+                         medium=medium)
 
 
 # dose of a thermal model (PennesGLL.dose): steps since init / set_state, CEM43 [min] and peak temperature per dof
 ThermalDose = namedtuple("ThermalDose", "steps cem43 T_max")
 
 
-def cell_to_dof_average(mesh, detJw, coeff):
+def cell_to_dof_average(mesh, detJw, coeff, weight=None):
     """Per-dof mass-weighted average of a per-cell coefficient, sum_c coeff_c (detJ w)_{c,i} / m_i with
     m_i = sum_c (detJ w)_{c,i}, the lumped mass: then coeff_i m_i is the GLL quadrature of the piecewise-constant
-    coefficient.  detJw [ncells, nq] in the reference layout (Geometry.detJw, oracle.precompute_geometric_data)."""
+    coefficient.  detJw [ncells, nq] in the reference layout (Geometry.detJw, oracle.precompute_geometric_data).
+    weight: per-cell weights w_c of a weighted mass, sum_c coeff_c w_c (detJ w)_{c,i} / sum_c w_c (detJ w)_{c,i}."""
     coeff = np.asarray(coeff, dtype=np.float64).reshape(-1)
     if coeff.size != mesh.ncells:
         raise capi.WfxError("one coefficient per cell expected")
     perm = capi.compute_permutations(mesh.P)
     dofs = np.asarray(mesh.dofmap)[:, perm].reshape(-1)
     w = np.asarray(detJw, dtype=np.float64).reshape(mesh.ncells, -1)
+    if weight is not None:
+        weight = np.asarray(weight, dtype=np.float64).reshape(-1)
+        if weight.size != mesh.ncells:
+            raise capi.WfxError("one weight per cell expected")
+        w = weight[:, None] * w
     m = np.bincount(dofs, weights=w.reshape(-1), minlength=mesh.ndofs)
     return np.bincount(dofs, weights=(coeff[:, None] * w).reshape(-1), minlength=mesh.ndofs) / m
+
+
+class Medium:
+    """A layered acoustic medium (DESIGN.md section 4.5e): per-cell density rho [kg/m^3] > 0, speed of sound c [m/s]
+    > 0 and, optionally, coefficient of nonlinearity beta >= 0, each a scalar or one value per cell, solving
+
+        (1 / (rho c^2)) p_tt - div((1 / rho) grad p) [- loss] = (beta / (rho^2 c^4)) (p^2)_tt
+
+    with p and (1 / rho) dp/dn continuous at interfaces.  Multiplied by rho_ref c0^2 it maps onto per-cell and
+    per-facet weights of the existing operators: stiffness rho_ref / rho_c (Geometry.scale_cells), mass
+    rho_ref c0^2 / (rho_c c_c^2) (MassOperator cell_weight), facet masses rho_ref / rho_f on tag 1 and
+    rho_ref c0 / (rho_f c_f) on tag 2 (BoundaryOperator facet_weight, f the facet's cell), and a per-dof kappa for
+    the Westervelt model.  With rho = rho_ref and c = c0 every weight is exactly 1.  The loss term becomes
+    delta (c / c0)^2.  Pass it as `medium=` to a wave model; cfl_timestep(h, medium.c_max, ...) gives its step."""
+
+    def __init__(self, rho, c, beta=None, rho_ref=1000.0):
+        def arr(name, a, positive):
+            a = np.asarray(a, dtype=np.float64)
+            if a.ndim > 1:
+                raise capi.WfxError(f"medium: {name} must be a scalar or one value per cell")
+            if not np.all(np.isfinite(a)) or not np.all(a > 0 if positive else a >= 0):
+                need = "positive" if positive else "not negative"
+                raise capi.WfxError(f"medium: {name} must be finite and {need}")
+            return a
+        self.rho, self.c = arr("rho", rho, True), arr("c", c, True)
+        self.beta = None if beta is None else arr("beta", beta, False)
+        if np.ndim(rho_ref):
+            raise capi.WfxError("medium: rho_ref must be a scalar")
+        self.rho_ref = float(arr("rho_ref", rho_ref, True))
+        sizes = {a.size for a in (self.rho, self.c, self.beta) if a is not None and a.ndim == 1}
+        if len(sizes) > 1:
+            raise capi.WfxError("medium: per-cell arrays differ in length")
+        self.ncells = sizes.pop() if sizes else None
+
+    @property
+    def c_max(self):
+        """the largest speed of sound, for the CFL step"""
+        return float(np.max(self.c))
+
+    def _cells(self, a, ncells):
+        if self.ncells is not None and self.ncells != ncells:
+            raise capi.WfxError(f"medium: {self.ncells} cells given, the mesh has {ncells}")
+        return np.broadcast_to(a, (ncells,)).astype(np.float64)
+
+    def cell_impedance(self, ncells):
+        """Z_c = rho_c c_c, one value per cell"""
+        return self._cells(self.rho, ncells) * self._cells(self.c, ncells)
+
+    def stiffness_weight(self, ncells):
+        """sigma_c = rho_ref / rho_c"""
+        return self.rho_ref / self._cells(self.rho, ncells)
+
+    def mass_weight(self, ncells, c0):
+        """mu_c = rho_ref c0^2 / (rho_c c_c^2)"""
+        rho, c = self._cells(self.rho, ncells), self._cells(self.c, ncells)
+        return (self.rho_ref * c0 * c0) / (rho * c * c)
+
+    def facet_weight(self, mesh, c0):
+        """one weight per facet triplet: rho_ref / rho_f on tag 1, rho_ref c0 / (rho_f c_f) = Z_ref / Z_f on tag 2,
+        1 elsewhere (f the facet's cell)"""
+        rho, c = self._cells(self.rho, mesh.ncells), self._cells(self.c, mesh.ncells)
+        fc = np.asarray(mesh.facet_cells, dtype=np.int64)
+        tag = np.asarray(mesh.facet_tags)
+        w = np.ones(len(fc))
+        w[tag == 1] = self.rho_ref / rho[fc[tag == 1]]
+        w[tag == 2] = (self.rho_ref * c0) / (rho[fc[tag == 2]] * c[fc[tag == 2]])
+        return w
+
+    def cell_kappa(self, ncells, beta=0.0):
+        """kappa_c = 2 beta_c / (rho_c c_c^2); beta: the value where the medium has none"""
+        b = self._cells(beta if self.beta is None else self.beta, ncells)
+        rho, c = self._cells(self.rho, ncells), self._cells(self.c, ncells)
+        return 2.0 * b / (rho * c * c)
+
+    def kappa(self, mesh, detJw, c0, beta=0.0):
+        """kappa_i = sum_c kappa_c mu_c (detJ w)_{c,i} / m~_i with m~ the weighted mass (host set-up).  A dof whose
+        cells all carry the same kappa_c gets that value exactly, so that a homogeneous region (the reference medium
+        in particular) steps with the scalar kappa bit for bit."""
+        kc = self.cell_kappa(mesh.ncells, beta)
+        avg = cell_to_dof_average(mesh, detJw, kc, self.mass_weight(mesh.ncells, c0))
+        perm = capi.compute_permutations(mesh.P)
+        dofs = np.asarray(mesh.dofmap)[:, perm].reshape(-1)
+        kpt = np.repeat(kc, len(perm))
+        lo, hi = np.full(mesh.ndofs, np.inf), np.full(mesh.ndofs, -np.inf)
+        np.minimum.at(lo, dofs, kpt)
+        np.maximum.at(hi, dofs, kpt)
+        return np.where(lo == hi, lo, avg)
 
 
 class PennesGLL:
@@ -758,15 +903,23 @@ class PennesGLL:
             raise capi.WfxError(f"heat source must have shape ({self.ndofs},)")
         capi.call("wfx_thermal_set_heat_source", self.handle, capi.f64p(q))
 
-    def heat_from_wave(self, model, alpha0, y, rho0, c0, member=0):
+    def heat_from_wave(self, model, alpha0, y, rho0, c0, member=0, medium=None):
         """Q = sum_h alpha0 (h f0 / 1 MHz)^y |p_h|^2 / (rho0 c0) from the harmonic maps of `model`'s field statistics,
-        computed on the device.  alpha0 [Np/m at 1 MHz]: a scalar or one value per dof; member: the ensemble member."""
+        computed on the device.  alpha0 [Np/m at 1 MHz]: a scalar or one value per dof; member: the ensemble member.
+        medium: a Medium on this mesh; 1 / (rho0 c0) is then the per-dof mass-weighted average of 1 / (rho_c c_c),
+        folded into alpha0 (rho0 and c0 are not used)."""
         a = np.asarray(alpha0, dtype=np.float64)
         a_host = None
         if a.ndim:
             a_host = np.ascontiguousarray(a.reshape(-1))
             if a_host.size != self.ndofs:
                 raise capi.WfxError(f"alpha0 must be a scalar or have shape ({self.ndofs},)")
+        if medium is not None:
+            nc = self.V.ncells
+            inv_z = 1.0 / medium.cell_impedance(nc)
+            a_host = np.ascontiguousarray(np.broadcast_to(a, (self.ndofs,)) *
+                                          cell_to_dof_average(self.V, self.geometry.detJw(), inv_z))
+            a, rho0, c0 = np.asarray(0.0), 1.0, 1.0
         capi.call("wfx_thermal_heat_from_wave", self.handle, model.handle, int(member), float(a) if not a.ndim else 0.0,
                   capi.f64p(a_host), float(y), float(rho0), float(c0))
 
