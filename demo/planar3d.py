@@ -27,6 +27,10 @@ section 4.5e): the cells whose centres lie in X0 < x < X1 get density R, speed o
 model, coefficient of nonlinearity B (default --beta); the rest is water (1000 kg/m^3, 1500 m/s, --beta).  The time
 step comes from the largest speed of sound.  With --stats-periods the on-axis |p1| is reported before and after the
 slab; with --heat-seconds the thermal model is built on its own operators and heated with the per-dof 1 / (rho c).
+--relaxation M [--band F_LO F_HI] (lossy / westervelt) makes the wave itself lose energy with the same power law that
+heats (DESIGN.md section 4.5f): M relaxation processes fitted to --absorption (f / 1 MHz)^--absorption-power over the
+band (default f0 / 2 .. 3 f0) in the tissue -- the slab with --layer (water keeps delta), else the whole domain.  It
+reports the fit error and the phase speed at f0; the time step is also kept below the relaxation's bound.
 The reference reads `../mesh.xdmf` (not in its repository); here the mesh is a structured
 n x m x m hexahedral box with tag 1 on x = 0 (source) and tag 2 on x = L (absorbing).
 
@@ -34,6 +38,7 @@ n x m x m hexahedral box with tag 1 on x = 0 (source) and tag 2 on x = L (absorb
                             [--model linear|lossy|westervelt] [--stats-periods K] [--focus DEPTH] [--aperture R]
                             [--heat-seconds S] [--cool-seconds C] [--absorption ALPHA0] [--absorption-power Y]
                             [--layer X0 X1 --layer-rho R --layer-c C [--layer-beta B]]
+                            [--relaxation M [--band F_LO F_HI]]
 """
 import argparse
 import os
@@ -86,7 +91,15 @@ def main():
     ap.add_argument("--layer-c", type=float, default=2800.0, help="with --layer: the slab's speed of sound [m/s]")
     ap.add_argument("--layer-beta", type=float, default=None,
                     help="with --layer: the slab's coefficient of nonlinearity (default --beta)")
+    ap.add_argument("--relaxation", type=int, default=0, choices=(0, 1, 2, 3),
+                    help="absorb the wave in the tissue with M relaxation processes (lossy, westervelt; 0: off)")
+    ap.add_argument("--band", type=float, nargs=2, metavar=("F_LO", "F_HI"), default=None,
+                    help="with --relaxation: the fitted band [Hz] (default f0 / 2 .. 3 f0)")
     args = ap.parse_args()
+    if args.relaxation and args.model == "linear":
+        ap.error("--relaxation needs --model lossy or westervelt (for linear tissue: --model lossy --delta 0)")
+    if args.relaxation and args.check:
+        ap.error("--check compares with the oracle without relaxation; it does not take --relaxation")
     if args.layer is not None and args.check:
         ap.error("--check compares with the homogeneous oracle; it does not take --layer")
     if args.layer is not None and not args.layer[0] < args.layer[1]:
@@ -114,8 +127,25 @@ def main():
         print(f"layer: {int(slab.sum())} cells in {args.layer[0]:.4f} < x < {args.layer[1]:.4f} with rho = "
               f"{args.layer_rho:g}, c = {args.layer_c:g}, beta = {beta_slab:g}; Z ratio to water "
               f"{args.layer_rho * args.layer_c / (1000.0 * speedOfSound):.4f}")
+    relaxation = None
+    if args.relaxation:
+        # the tissue: the slab (water elsewhere keeps delta), else every cell
+        tissue = slab if args.layer is not None else np.ones(mesh.ncells, dtype=bool)
+        rho = medium.rho if medium is not None else 1000.0
+        c = medium.c if medium is not None else speedOfSound
+        medium = wfx.Medium(rho, c, None if medium is None else medium.beta, alpha0=np.where(tissue, args.absorption, 0.0),
+                            y=args.absorption_power)
+        band = args.band or (0.5 * sourceFrequency, 3.0 * sourceFrequency)
+        relaxation = medium.relaxation(band[0], band[1], args.relaxation)
+        cell = int(np.argmax(tissue))
+        print(f"relaxation: {relaxation.M} processes fitted to {args.absorption:g} (f / 1 MHz)^{args.absorption_power:g}"
+              f" Np/m over {band[0]:.4g} .. {band[1]:.4g} Hz, fit error {relaxation.fit_error:.3e}; in the tissue "
+              f"alpha(f0) = {relaxation.alpha(sourceFrequency)[cell]:.6e} Np/m, phase speed at f0 "
+              f"{relaxation.phase_speed(sourceFrequency)[cell]:.4f} m/s (c = {np.broadcast_to(c, (mesh.ncells,))[cell]:g})")
     c_max = speedOfSound if medium is None else medium.c_max
     timeStepSize = wfx.cfl_timestep(mesh.h_min, c_max, degreeOfBasis, sourceFrequency)  # :61-66
+    if relaxation is not None and timeStepSize >= relaxation.max_dt():
+        timeStepSize = period / np.ceil(period / relaxation.max_dt())                  # whole steps per period
     startTime, finalTime = 0.0, domainLength / speedOfSound + 8.0 / sourceFrequency            # :63-64
     print(f"Number of step per period: {int(round(period / timeStepSize))}")
     print(f"dt = {timeStepSize:.15g}")
@@ -127,9 +157,10 @@ def main():
                                medium=medium)                                                              # :75
     else:
         if medium is not None and args.model == "lossy":
-            medium = wfx.Medium(medium.rho, medium.c)                     # the lossy model stays linear
+            # the lossy model stays linear
+            medium = wfx.Medium(medium.rho, medium.c, alpha0=medium.alpha0, y=medium.y)
         eqn = wfx.WesterveltGLLOpt(mesh, None, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
-                                   delta, beta, args.rho0, medium=medium)
+                                   delta, beta, args.rho0, medium=medium, relaxation=relaxation)
     print(f"Number of steps: {nstep}")
     print(f"Degrees of freedom: {mesh.ndofs_global}")
     X = wfx.dof_coordinates(mesh)
@@ -221,7 +252,10 @@ def heat(args, eqn, c0, medium=None, k=0.5, rhoc=3.6e6, perfusion=2.0e3, T_art=3
         th = wfx.PennesGLL.from_wave(eqn, k, rhoc, perfusion, T_art)
     else:
         th = wfx.PennesGLL(eqn.V, eqn.k_, k, rhoc, perfusion, T_art, dtype=eqn.dtype, ctx=eqn.ctx)
-    th.heat_from_wave(eqn, args.absorption, args.absorption_power, args.rho0, c0, medium=medium)
+    if medium is not None and medium.alpha0 is not None:
+        th.heat_from_wave(eqn, None, medium=medium)       # the absorption the wave relaxes with (--relaxation)
+    else:
+        th.heat_from_wave(eqn, args.absorption, args.absorption_power, args.rho0, c0, medium=medium)
     dt = th.stable_dt()
     th.init()
     eqn.ctx.synchronize()

@@ -364,6 +364,26 @@ int wfx_wave_create_westervelt(wfx_ctx* ctx, wfx_stiffness* stiff, wfx_mass* mas
  * and drops the captured step graph.  Refused: a NULL model, linear and ensemble models, negative or non-finite
  * values. */
 int wfx_wave_set_nonlinearity(wfx_wave* wave, const double* kappa_host);
+/* Relaxation absorption (power-law tissue absorption, DESIGN.md section 4.5f) for a model made by
+ * wfx_wave_create_westervelt: M <= WFX_RELAX_MAX processes with relaxation times tau_host[M] > 0 [s] and per-dof
+ * strengths eps_host[M][ndofs] >= 0 (dimensionless), each with a memory variable q_nu per dof:
+ *   (m_i (1 - kappa p_i) + q_i) p_tt,i = b_i + m_i (kappa p_t,i^2 - sum_nu q_nu,i'')
+ *   tau_nu q_nu' + q_nu = eps_nu p
+ * (b: the right-hand side of wfx_wave_create_westervelt's lumped system).  In a medium with per-cell eps_nu,c
+ * and a weighted mass m~, eps_nu,i = sum_c eps_nu,c mu_c (detJ w)_{c,i} / m~_i is exact.  The memory variables are
+ * RK4 state like u and v: they start at 0 here, init and set_state zero them, and wfx_wave_get/set_relaxation_state
+ * carry them through a checkpoint.  M = 0 or tau_host / eps_host NULL clears it: the model without relaxation, bit
+ * for bit.  Model configuration: it survives init, set_state and restarts.  Synchronises the device and drops the
+ * captured step graph.  rk4 then refuses dt (1 + sum_nu max_i eps_nu,i) / min_nu tau_nu >= 2.5 (RK4 is unstable
+ * beyond 2.785 on a lone dof).  The absorbing boundary (tag 2) stays the first-order condition and reflects
+ * O(eps).  Refused: a NULL model, linear and ensemble models, M < 0 or M > WFX_RELAX_MAX, tau <= 0, eps < 0,
+ * non-finite values, a model with snapshots on (a snapshot carries u and v only). */
+#define WFX_RELAX_MAX 3
+int wfx_wave_set_relaxation(wfx_wave* wave, int M, const double* tau_host, const double* eps_host);
+/* The memory variables q [M][ndofs] in the model dtype, for checkpoints: get after get_state, set after
+ * set_state (which zeroes them).  Refused without relaxation. */
+int wfx_wave_get_relaxation_state(wfx_wave* wave, void* q_host);
+int wfx_wave_set_relaxation_state(wfx_wave* wave, const void* q_host);
 int wfx_wave_init(wfx_wave* wave);                                   /* :131-134 */
 /* Copies the state to the device; on a distributed mesh the ghost entries are then overwritten by
  * their owners' values (u->scatter_fwd(), v->scatter_fwd(), :164,167). */
@@ -434,7 +454,8 @@ int wfx_wave_set_source_profile(wfx_wave* wave, const double* amp_host, const do
  * while the time stepping continues; `fn` then receives host pointers valid for the duration of the
  * call (step number, time reached, u, v in the model dtype, ndofs entries each).  It runs on the
  * thread that called wfx_wave_rk4, at the next snapshot or before rk4 returns.  A checkpoint is a
- * snapshot fed back through wfx_wave_set_state.  every = 0 or fn = NULL switches snapshots off. */
+ * snapshot fed back through wfx_wave_set_state.  every = 0 or fn = NULL switches snapshots off.  Refused for a
+ * model with relaxation (wfx_wave_set_relaxation), whose state includes the memory variables. */
 typedef void (*wfx_snapshot_fn)(void* user, int64_t step, double t, const void* u_host, const void* v_host);
 int wfx_wave_set_snapshot(wfx_wave* wave, int64_t every, wfx_snapshot_fn fn, void* user);
 int wfx_wave_destroy(wfx_wave* wave);

@@ -433,3 +433,122 @@ int64_t wo_rk4_westervelt_medium(int P, int64_t ncells, int64_t ndofs, const int
   free(u_); free(v_); free(un); free(vn); free(u0); free(v0); free(ku); free(kv); free(b); free(bv);
   return step;
 }
+
+/* ---- relaxation absorption (DESIGN.md section 4.5f) ----------------------------------------------------------
+ * M relaxation processes with times tau[nu] and per-dof strengths eps[nu * ndofs + k], memory variables
+ * q[nu * ndofs + k], on the lumped system of model_rhs_medium:
+ *   (m (1 - kappa p) + (delta / c0) m2) p_tt = r - m sum_nu q_nu'',   tau_nu q_nu' + q_nu = eps_nu p
+ * with r the numerator of model_rhs_medium and q_nu'' = (eps_nu p_t - q_nu') / tau_nu.  Written out plainly: q_nu'
+ * and q_nu'' divide by tau (no reciprocal), the sum is subtracted from the numerator, not folded into the quotient.
+ * With M = 0 the stage loop and the quotient are those of wo_rk4_westervelt_medium, bit for bit. */
+static void model_rhs_relax(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                            const double* m, const double* m1, const double* m2, const double* kappa, double c0,
+                            double freq0, double p0, double delta, int M, const double* tau, const double* eps, double t,
+                            const double* un, const double* vn, const double* qn, double* kv, double* kq, double* b,
+                            double* bv, int sumfact, int nthreads)
+{
+  const size_t nb = sizeof(double) * ndofs;
+  const double s = delta / (1500.0 * 1500.0);
+  double g, gdot;
+  wo_source(t, freq0, p0, c0, &g, &gdot);
+  memset(b, 0, nb);
+  memset(bv, 0, nb);
+  model_stiffness(P, ncells, ndofs, dofmap, G, un, b, sumfact, nthreads);  /* A un */
+  model_stiffness(P, ncells, ndofs, dofmap, G, vn, bv, sumfact, nthreads); /* A vn */
+  for (int64_t k = 0; k < ndofs; ++k)
+  {
+    double r = b[k] + s * bv[k];
+    r += (c0 * c0 * g + delta * gdot) * m1[k] - c0 * m2[k] * vn[k];
+    r += kappa[k] * m[k] * vn[k] * vn[k];
+    if (M > 0)
+    {
+      double qdd = 0.0;
+      for (int nu = 0; nu < M; ++nu)
+      {
+        const int64_t o = nu * ndofs + k;
+        kq[o] = (eps[o] * un[k] - qn[o]) / tau[nu];
+        qdd += (eps[o] * vn[k] - kq[o]) / tau[nu];
+      }
+      r -= m[k] * qdd;
+    }
+    kv[k] = r / (m[k] * (1.0 - kappa[k] * un[k]) + delta / c0 * m2[k]);
+  }
+}
+
+/* dv/dt = f1(t, u, v; q) of the lossy / Westervelt model with relaxation at the memory variables q [M][ndofs] */
+void wo_f1_westervelt_relax(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                            const double* m, const double* m1, const double* m2, const double* kappa, double c0,
+                            double freq0, double p0, double delta, int M, const double* tau, const double* eps, double t,
+                            const double* u, const double* v, const double* q, double* out, int sumfact, int nthreads)
+{
+  const size_t nb = sizeof(double) * ndofs;
+  double *b = malloc(nb), *bv = malloc(nb), *kq = malloc(nb * (M > 0 ? M : 1));
+  model_rhs_relax(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, M, tau, eps, t, u, v, q, out, kq,
+                  b, bv, sumfact, nthreads);
+  free(b);
+  free(bv);
+  free(kq);
+}
+
+/* wo_rk4_westervelt_medium with relaxation: the same stage loop, with q [M][ndofs] (in / out) stepped by the same
+ * tableau as u and v */
+int64_t wo_rk4_westervelt_relax(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                                const double* m, const double* m1, const double* m2, const double* kappa, double c0,
+                                double freq0, double p0, double delta, int M, const double* tau, const double* eps,
+                                double t0, double tf, double dt, int64_t max_steps, double* u_n, double* v_n,
+                                double* q_n, int sumfact, int nthreads, double* t_end)
+{
+  const double a_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  const double b_runge[4] = {1.0 / 6.0, 1.0 / 3.0, 1.0 / 3.0, 1.0 / 6.0};
+  const double c_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  const size_t nb = sizeof(double) * ndofs, nq = nb * (M > 0 ? M : 1);
+  const int64_t nqe = (int64_t)M * ndofs;
+  double *u_ = malloc(nb), *v_ = malloc(nb), *un = malloc(nb), *vn = malloc(nb);
+  double *u0 = malloc(nb), *v0 = malloc(nb), *ku = malloc(nb), *kv = malloc(nb), *b = malloc(nb), *bv = malloc(nb);
+  double *q_ = malloc(nq), *qn = malloc(nq), *q0 = malloc(nq), *kq = malloc(nq);
+  memcpy(u_, u_n, nb);
+  memcpy(v_, v_n, nb);
+  memcpy(ku, u_, nb);
+  memcpy(kv, v_, nb);
+  if (M > 0)
+  {
+    memcpy(q_, q_n, sizeof(double) * nqe);
+    memset(kq, 0, sizeof(double) * nqe);
+  }
+  double t = t0;
+  int64_t step = 0;
+  while (t < tf)
+  {
+    if (max_steps > 0 && step >= max_steps) break;
+    dt = dt < tf - t ? dt : tf - t;
+    memcpy(u0, u_, nb);
+    memcpy(v0, v_, nb);
+    if (M > 0) memcpy(q0, q_, sizeof(double) * nqe);
+    for (int i = 0; i < 4; ++i)
+    {
+      memcpy(un, u0, nb);
+      memcpy(vn, v0, nb);
+      const double adt = dt * a_runge[i];
+      for (int64_t k = 0; k < ndofs; ++k) un[k] = ku[k] * adt + un[k];
+      for (int64_t k = 0; k < ndofs; ++k) vn[k] = kv[k] * adt + vn[k];
+      for (int64_t k = 0; k < nqe; ++k) qn[k] = i == 0 ? q0[k] : kq[k] * adt + q0[k];
+      const double tn = t + c_runge[i] * dt;
+      memcpy(ku, vn, nb);
+      model_rhs_relax(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, M, tau, eps, tn, un, vn, qn,
+                      kv, kq, b, bv, sumfact, nthreads);
+      const double bdt = dt * b_runge[i];
+      for (int64_t k = 0; k < ndofs; ++k) u_[k] = ku[k] * bdt + u_[k];
+      for (int64_t k = 0; k < ndofs; ++k) v_[k] = kv[k] * bdt + v_[k];
+      for (int64_t k = 0; k < nqe; ++k) q_[k] = kq[k] * bdt + q_[k];
+    }
+    t += dt;
+    step += 1;
+  }
+  memcpy(u_n, u_, nb);
+  memcpy(v_n, v_, nb);
+  if (M > 0) memcpy(q_n, q_, sizeof(double) * nqe);
+  if (t_end) *t_end = t;
+  free(u_); free(v_); free(un); free(vn); free(u0); free(v0); free(ku); free(kv); free(b); free(bv);
+  free(q_); free(qn); free(q0); free(kq);
+  return step;
+}

@@ -85,6 +85,12 @@ def lib():
         L.wo_rk4_westervelt_medium.restype = l
         L.wo_rk4_westervelt_medium.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, d, d, d,
                                                l, _f64p, _f64p, i, i, _f64p]
+        L.wo_f1_westervelt_relax.restype = None
+        L.wo_f1_westervelt_relax.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, i, _f64p,
+                                             _f64p, d, _f64p, _f64p, _f64p, _f64p, i, i]
+        L.wo_rk4_westervelt_relax.restype = l
+        L.wo_rk4_westervelt_relax.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, i, _f64p,
+                                              _f64p, d, d, d, l, _f64p, _f64p, _f64p, i, i, _f64p]
         _lib.append(L)
     return _lib[0]
 
@@ -226,4 +232,43 @@ def rk4_westervelt_medium(mesh, P, G, m, m1, m2, kappa, c0, f0, p0, delta, t0, t
     steps = lib().wo_rk4_westervelt_medium(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)),
                                            _f(m), _f(m1), _f(m2), _f(kappa), c0, f0, p0, delta, t0, tf, dt, max_steps,
                                            _f(u), _f(v), int(sumfact), nthreads, C.byref(t_end))
+    return steps, t_end.value
+
+
+# ---- relaxation absorption (DESIGN.md section 4.5f) -----------------------------------------------------------------
+def _relax(mesh, tau, eps, q):
+    tau = np.ascontiguousarray(tau, dtype=np.float64).reshape(-1)
+    M = len(tau)
+    eps = np.ascontiguousarray(eps, dtype=np.float64).reshape(M, mesh.ndofs)
+    q = np.zeros((M, mesh.ndofs)) if q is None else q
+    assert q.dtype == np.float64 and q.shape == (M, mesh.ndofs) and q.flags["C_CONTIGUOUS"]
+    p = lambda a: _f(a.reshape(-1)) if a.size else _f(np.zeros(1))  # noqa: E731
+    return M, p(tau), p(eps), q, p(q)
+
+
+def f1_westervelt_relax(mesh, P, G, m, m1, m2, kappa, c0, f0, p0, delta, tau, eps, t, u, v, q=None, sumfact=False,
+                        nthreads=1):
+    """f1_westervelt_medium with M relaxation processes: tau [M], eps [M, ndofs], memory variables q [M, ndofs]
+    (None: 0)"""
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    M, tp, ep, _, qp = _relax(mesh, tau, eps, q)
+    out = np.empty(mesh.ndofs)
+    lib().wo_f1_westervelt_relax(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)), _f(m),
+                                 _f(m1), _f(m2), _f(np.ascontiguousarray(kappa, dtype=np.float64)), c0, f0, p0, delta,
+                                 M, tp, ep, t, _f(u), _f(v), qp, _f(out), int(sumfact), nthreads)
+    return out
+
+
+def rk4_westervelt_relax(mesh, P, G, m, m1, m2, kappa, c0, f0, p0, delta, tau, eps, t0, tf, dt, u, v, q, max_steps=0,
+                         sumfact=False, nthreads=1):
+    """rk4_westervelt_medium with relaxation (see f1_westervelt_relax); u, v and q [M, ndofs] updated in place.
+    -> (steps, t_end)"""
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    kappa = np.ascontiguousarray(kappa, dtype=np.float64)
+    assert kappa.shape == (mesh.ndofs,)
+    M, tp, ep, q, qp = _relax(mesh, tau, eps, q)
+    t_end = C.c_double()
+    steps = lib().wo_rk4_westervelt_relax(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)),
+                                          _f(m), _f(m1), _f(m2), _f(kappa), c0, f0, p0, delta, M, tp, ep, t0, tf, dt,
+                                          max_steps, _f(u), _f(v), qp, int(sumfact), nthreads, C.byref(t_end))
     return steps, t_end.value

@@ -15,6 +15,7 @@ F64, F32 = 0, 1
 STIFF_AUTO, STIFF_CELL_COLOUR, STIFF_NO_SPLIT, STIFF_CELL_STREAM, STIFF_ENSEMBLE = 0, 1, 2, 4, 8
 ENSEMBLE_MAX = 8
 HARMONICS_MAX = 8
+RELAX_MAX = 3
 
 _c_i32p = C.POINTER(C.c_int32)
 _c_i64p = C.POINTER(C.c_int64)
@@ -114,6 +115,9 @@ _SIG = {
     "wfx_wave_create_westervelt": [_vp, _vp, _vp, _vp, C.c_int64, C.c_double, C.c_double, C.c_double, C.c_double,
                                    C.c_double, C.c_double, _vpp],
     "wfx_wave_set_nonlinearity": [_vp, _c_f64p],
+    "wfx_wave_set_relaxation": [_vp, C.c_int, _c_f64p, _c_f64p],
+    "wfx_wave_get_relaxation_state": [_vp, _vp],
+    "wfx_wave_set_relaxation_state": [_vp, _vp],
     "wfx_wave_init": [_vp],
     "wfx_wave_set_state": [_vp, _vp, _vp],
     "wfx_wave_get_state": [_vp, _vp, _vp],

@@ -114,7 +114,70 @@ __global__ void absorbing_mass_kernel(int64_t nb, const int32_t* __restrict__ id
   const double kv = ((double)b[i] + mi * kp2) / (mi * a + qc * m2[t]);
   b[i] = (T)(mi * (kv * a - kp2));
 }
+
+// absorbing_mass_kernel with M relaxation processes (a separate template, so that the kernels above keep their code):
+// R = sum_nu (eps_nu pd - kq_nu) / tau_nu, kq_nu = (eps_nu p - q_nu) / tau_nu, in fp64 from eps_b [M][nb] and the
+// stage's q [M][n]
+template <typename T, bool KD, int M>
+__global__ void absorbing_mass_relax_kernel(int64_t nb, int64_t n, const int32_t* __restrict__ idx,
+                                            const double* __restrict__ m2, const double* __restrict__ m, double qc,
+                                            double kappa, const double* __restrict__ kd, const RelaxTau rt,
+                                            const double* __restrict__ eps_b, const T* __restrict__ q, T s,
+                                            const T* __restrict__ pw, const T* __restrict__ pd, T* __restrict__ b)
+{
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t >= nb || m2[t] == 0.0) return;
+  const int32_t i = idx[t];
+  const T pdt = pd[i];
+  const double p = (double)(pw[i] - s * pdt), pdd = (double)pdt;
+  double R = 0.0;
+#pragma unroll
+  for (int j = 0; j < M; ++j)
+  {
+    const double e = eps_b[j * nb + t];
+    const double kq = (e * p - (double)q[j * n + i]) * rt.inv_tau[j];
+    R += (e * pdd - kq) * rt.inv_tau[j];
+  }
+  if (KD) kappa = kd[t];
+  const double mi = m[i], a = 1.0 - kappa * p, kp2 = kappa * pdd * pdd;
+  const double kv = ((double)b[i] + mi * (kp2 - R)) / (mi * a + qc * m2[t]);
+  b[i] = (T)(mi * (kv * a - kp2 + R));
+}
 } // namespace
+
+void wfx::boundary_absorbing_mass_relax(wfx_boundary* op, const double* m64, double qc, double kappa,
+                                        const double* kappa_b, int M, const RelaxTau& rt, const double* eps_b,
+                                        const void* q, double s, const void* pw, const void* pd, void* b,
+                                        cudaStream_t stream)
+{
+  if (!op || op->nb == 0) return;
+  const unsigned grid = (unsigned)((op->nb + 255) / 256);
+  const int64_t n = op->ndofs;
+#define WFX_ABS(T, KD, MM)                                                                                            \
+  absorbing_mass_relax_kernel<T, KD, MM><<<grid, 256, 0, stream>>>(op->nb, n, op->d_idx.p, op->d_m2.p, m64, qc, kappa, \
+                                                                   kappa_b, rt, eps_b, (const T*)q, (T)s,            \
+                                                                   (const T*)pw, (const T*)pd, (T*)b)
+#define WFX_ABS_M(T, KD)                                                                                              \
+  switch (M)                                                                                                          \
+  {                                                                                                                   \
+  case 1: WFX_ABS(T, KD, 1); break;                                                                                   \
+  case 2: WFX_ABS(T, KD, 2); break;                                                                                   \
+  default: WFX_ABS(T, KD, 3); break;                                                                                  \
+  }
+  if (op->dtype == WFX_F64)
+  {
+    if (kappa_b) { WFX_ABS_M(double, true) }
+    else { WFX_ABS_M(double, false) }
+  }
+  else
+  {
+    if (kappa_b) { WFX_ABS_M(float, true) }
+    else { WFX_ABS_M(float, false) }
+  }
+#undef WFX_ABS_M
+#undef WFX_ABS
+  WFX_CUDA(cudaGetLastError());
+}
 
 void wfx::boundary_absorbing_mass(wfx_boundary* op, const double* m64, double qc, double kappa,
                                   const double* kappa_b, double s, const void* pw, const void* pd, void* b,

@@ -144,6 +144,17 @@ const double* mass_diagonal64(const struct ::wfx_mass* op);   // m on the device
 void boundary_absorbing_mass(struct ::wfx_boundary* op, const double* m64, double qc, double kappa,
                              const double* kappa_b, double s, const void* pw, const void* pd, void* b,
                              cudaStream_t stream);
+// Relaxation processes (wfx_wave_set_relaxation, DESIGN.md section 4.5f): 1 / tau_nu of the M processes
+struct RelaxTau
+{
+  double inv_tau[WFX_RELAX_MAX];
+};
+// boundary_absorbing_mass with M relaxation processes: b_i -> m_i [kv_i (1 - kappa p_i) - kappa pd_i^2 + R_i] with
+// the exact kv_i = (b_i + m_i (kappa pd_i^2 - R_i)) / (m_i (1 - kappa p_i) + qc m2_i), R_i = sum_nu q_nu,i'' from the
+// stage's memory variables q [M][ndofs] (model dtype) and eps_b [M][nb] (fp64, compact over boundary_dofs(op))
+void boundary_absorbing_mass_relax(struct ::wfx_boundary* op, const double* m64, double qc, double kappa,
+                                   const double* kappa_b, int M, const RelaxTau& rt, const double* eps_b, const void* q,
+                                   double s, const void* pw, const void* pd, void* b, cudaStream_t stream);
 // A wave model's field statistics as the thermal model reads them (wfx_thermal_heat_from_wave, DESIGN.md section
 // 4.5d): the unscaled fp64 harmonic sums, planes [h][ndofs * nv] (entry (dof i, member m) at i nv + m), the number
 // of sampled steps N (the amplitudes are the sums times 2 / N) and every member's source frequency (wfx_wave.cu)

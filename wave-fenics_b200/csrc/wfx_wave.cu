@@ -7,6 +7,7 @@
 #include "wfx_internal.h"
 #include "wfx_source.h"
 
+#include <algorithm>
 #include <cmath>
 #include <cstdlib>
 
@@ -42,6 +43,14 @@ struct wfx_wave
   bool kd_on = false;
   DevBuf<unsigned char> kd;
   DevBuf<double> kd_b;
+  // relaxation processes (wfx_wave_set_relaxation, section 4.5f): relax_m processes, eps [M][n] in the model dtype,
+  // eps_b the same in fp64 compact over the boundary dofs for the Gamma2 mass term; memory variables q_ (solution),
+  // q0 (start of step), qn (stage state), each [M][n] in the model dtype.  relax_rate = (1 + sum max eps) / tau_min
+  int relax_m = 0;
+  RelaxTau relax_tau{};
+  double relax_rate = 0;
+  DevBuf<unsigned char> relax_eps, rq_, rq0, rqn;
+  DevBuf<double> relax_eps_b;
   const double* m64 = nullptr;
   DevBuf<unsigned char> f1_w;
   const void* minv = nullptr;
@@ -321,6 +330,135 @@ void launch_stage_westervelt(int stage, bool nl, int64_t n, const void* b, const
   WFX_CUDA(cudaGetLastError());
 }
 
+// rk_stage_westervelt_kernel with M relaxation processes (section 4.5f; a separate template, so that the kernel above
+// keeps its code).  The memory variables q_nu are RK4 state with the tableau of u and v: q_ (solution), q0 (start of
+// step), qn (stage state), each plane nu at [nu * n].  At the stage state (p, pd, q):
+//   kq_nu = (eps_nu p - q_nu) / tau_nu,   R = sum_nu (eps_nu pd - kq_nu) / tau_nu   (= sum_nu q_nu'')
+//   kv = b / m - R  (lossy),   kv = (b / m + kappa pd^2 - R) / (1 - kappa p)  (Westervelt)
+// p = w - s vn at stages 1-3 on both paths.  The Gamma2 kernel (boundary_absorbing_mass_relax) has replaced b on the
+// absorbing dofs so that this quotient is exact there too.
+template <typename T, int STAGE, bool NL, bool KD, int M>
+__global__ void __launch_bounds__(256)
+rk_stage_relax_kernel(int64_t n, const T* __restrict__ b, const T* __restrict__ minv, T* __restrict__ u_,
+                      T* __restrict__ v_, T* __restrict__ u0, T* __restrict__ v0, T* __restrict__ w,
+                      T* __restrict__ vn, T bdt, T adt_next, T s, T kappa, const T* __restrict__ kd,
+                      const T* __restrict__ eps, T* __restrict__ q_, T* __restrict__ q0, T* __restrict__ qn,
+                      const RelaxTau rt)
+{
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  T kv = b[k] * minv[k];
+  T us = u_[k], vs = v_[k];
+  T ku, ub, vb, p;
+  if (STAGE == 0)
+  {
+    ku = vs;
+    ub = us;
+    vb = vs;
+    p = us;
+    u0[k] = ub;
+    v0[k] = vb;
+  }
+  else
+  {
+    ku = vn[k];
+    p = w[k] - s * ku;
+    if (STAGE < 3)
+    {
+      ub = u0[k];
+      vb = v0[k];
+    }
+  }
+  T R = T(0);
+#pragma unroll
+  for (int j = 0; j < M; ++j)
+  {
+    const int64_t o = j * n + k;
+    const T e = eps[o], it = (T)rt.inv_tau[j], qs = q_[o];
+    T qst, qb;
+    if (STAGE == 0)
+    {
+      qst = qs;
+      qb = qs;
+      q0[o] = qs;
+    }
+    else
+    {
+      qst = qn[o];
+      if (STAGE < 3) qb = q0[o];
+    }
+    const T kq = (e * p - qst) * it;
+    R += (e * ku - kq) * it;
+    q_[o] = kq * bdt + qs;
+    if (STAGE < 3) qn[o] = kq * adt_next + qb;
+  }
+  if (KD) kappa = kd[k];
+  // R is subtracted after the numerator of rk_stage_westervelt_kernel, written the same way, so that eps = 0 (R = 0)
+  // reproduces its rounding bit for bit
+  if (NL) kv = ((kv + kappa * ku * ku) - R) / (T(1) - kappa * p);
+  else kv = kv - R;
+  const T un_ = ku * bdt + us, vn_ = kv * bdt + vs;
+  u_[k] = un_;
+  v_[k] = vn_;
+  if (STAGE < 3)
+  {
+    const T ui = ku * adt_next + ub, vi = kv * adt_next + vb;
+    w[k] = ui + s * vi;
+    vn[k] = vi;
+  }
+  else w[k] = un_ + s * vn_;
+}
+
+template <typename T, int STAGE, bool NL, bool KD>
+void launch_stage_relax_m(unsigned grid, int M, int64_t n, const void* b, const void* minv, void* u_, void* v_,
+                          void* u0, void* v0, void* w, void* vn, double bdt, double adt_next, double s, double kappa,
+                          const void* kd, const void* eps, void* q_, void* q0, void* qn, const RelaxTau& rt,
+                          cudaStream_t st)
+{
+#define WFX_STAGE(MM)                                                                                                 \
+  rk_stage_relax_kernel<T, STAGE, NL, KD, MM><<<grid, 256, 0, st>>>(                                                \
+      n, (const T*)b, (const T*)minv, (T*)u_, (T*)v_, (T*)u0, (T*)v0, (T*)w, (T*)vn, (T)bdt, (T)adt_next, (T)s,      \
+      (T)kappa, (const T*)kd, (const T*)eps, (T*)q_, (T*)q0, (T*)qn, rt)
+  switch (M)
+  {
+  case 1: WFX_STAGE(1); break;
+  case 2: WFX_STAGE(2); break;
+  default: WFX_STAGE(3); break;
+  }
+#undef WFX_STAGE
+}
+
+// kd (nullable): per-dof kappa in T, which implies the nonlinear update
+template <typename T>
+void launch_stage_relax(int stage, bool nl, int M, int64_t n, const void* b, const void* minv, void* u_, void* v_,
+                        void* u0, void* v0, void* w, void* vn, double bdt, double adt_next, double s, double kappa,
+                        const void* kd, const void* eps, void* q_, void* q0, void* qn, const RelaxTau& rt,
+                        cudaStream_t st)
+{
+  const unsigned grid = (unsigned)((n + 255) / 256);
+#define WFX_STAGE(S, NL, KD)                                                                                          \
+  launch_stage_relax_m<T, S, NL, KD>(grid, M, n, b, minv, u_, v_, u0, v0, w, vn, bdt, adt_next, s, kappa, kd, eps,    \
+                                     q_, q0, qn, rt, st)
+  const int path = kd ? 2 : (nl ? 1 : 0);
+  switch (stage * 3 + path)
+  {
+  case 0: WFX_STAGE(0, false, false); break;
+  case 1: WFX_STAGE(0, true, false); break;
+  case 2: WFX_STAGE(0, true, true); break;
+  case 3: WFX_STAGE(1, false, false); break;
+  case 4: WFX_STAGE(1, true, false); break;
+  case 5: WFX_STAGE(1, true, true); break;
+  case 6: WFX_STAGE(2, false, false); break;
+  case 7: WFX_STAGE(2, true, false); break;
+  case 8: WFX_STAGE(2, true, true); break;
+  case 9: WFX_STAGE(3, false, false); break;
+  case 10: WFX_STAGE(3, true, false); break;
+  default: WFX_STAGE(3, true, true); break;
+  }
+#undef WFX_STAGE
+  WFX_CUDA(cudaGetLastError());
+}
+
 // w = u + s v: the stiffness input of the lossy / Westervelt models
 template <typename T>
 __global__ void axpy_kernel(int64_t n, const T* __restrict__ u, const T* __restrict__ v, T s, T* __restrict__ w)
@@ -341,6 +479,29 @@ __global__ void westervelt_rhs_kernel(int64_t n, const T* __restrict__ b, const 
   if (KD) kappa = kd[k];
   const T vk = v[k];
   out[k] = (b[k] * minv[k] + kappa * vk * vk) / (T(1) - kappa * u[k]);
+}
+
+// westervelt_rhs_kernel with M relaxation processes: out = (b / m + kappa v^2 - R) / (1 - kappa u), R from the model's
+// current memory variables q [M][n] (rk_stage_relax_kernel's R at the state (u, v, q))
+template <typename T, bool KD, int M>
+__global__ void westervelt_rhs_relax_kernel(int64_t n, const T* __restrict__ b, const T* __restrict__ minv,
+                                            const T* __restrict__ u, const T* __restrict__ v, T kappa,
+                                            const T* __restrict__ kd, const T* __restrict__ eps,
+                                            const T* __restrict__ q, const RelaxTau rt, T* __restrict__ out)
+{
+  const int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  if (KD) kappa = kd[k];
+  const T uk = u[k], vk = v[k];
+  T R = T(0);
+#pragma unroll
+  for (int j = 0; j < M; ++j)
+  {
+    const T e = eps[j * n + k], it = (T)rt.inv_tau[j];
+    const T kq = (e * uk - q[j * n + k]) * it;
+    R += (e * vk - kq) * it;
+  }
+  out[k] = ((b[k] * minv[k] + kappa * vk * vk) - R) / (T(1) - kappa * uk);
 }
 
 void launch_axpy(const wfx_wave* w, const void* u, const void* v, double s, void* out, cudaStream_t st)
@@ -601,6 +762,25 @@ void enqueue_step(wfx_wave* w, double dt, const double* g, const double* tn, boo
     if (w->model)
     {
       // Gamma2 mass term (compact, absorbing dofs), then the fused update; p = u_ at stage 0, else w - s vn
+      if (w->relax_m)
+      {
+        const void* kd = w->kd_on ? w->kd.p : nullptr;
+        void* qs = i == 0 ? w->rq_.p : w->rqn.p; // the stage's memory variables
+        if (w->qc != 0)
+          boundary_absorbing_mass_relax(w->bnd, w->m64, w->qc, w->kappa, w->kd_on ? w->kd_b.p : nullptr, w->relax_m,
+                                        w->relax_tau, w->relax_eps_b.p, qs, i == 0 ? 0.0 : w->s_stiff,
+                                        i == 0 ? w->u_.p : w->un.p, vn, w->b.p, st);
+        NvtxRange update_range("wfx fused stage update");
+        if (w->dtype == WFX_F64)
+          launch_stage_relax<double>(i, w->model == 2, w->relax_m, w->n, w->b.p, w->minv, w->u_.p, w->v_.p, w->u0.p,
+                                     w->v0.p, w->un.p, w->vn.p, dt * b_runge[i], dt * a_runge[i + 1], w->s_stiff,
+                                     w->kappa, kd, w->relax_eps.p, w->rq_.p, w->rq0.p, w->rqn.p, w->relax_tau, st);
+        else
+          launch_stage_relax<float>(i, w->model == 2, w->relax_m, w->n, w->b.p, w->minv, w->u_.p, w->v_.p, w->u0.p,
+                                    w->v0.p, w->un.p, w->vn.p, dt * b_runge[i], dt * a_runge[i + 1], w->s_stiff,
+                                    w->kappa, kd, w->relax_eps.p, w->rq_.p, w->rq0.p, w->rqn.p, w->relax_tau, st);
+        continue;
+      }
       if (w->qc != 0)
         boundary_absorbing_mass(w->bnd, w->m64, w->qc, w->kappa, w->kd_on ? w->kd_b.p : nullptr,
                                 i == 0 ? 0.0 : w->s_stiff, i == 0 ? w->u_.p : w->un.p, vn, w->b.p, st);
@@ -761,6 +941,15 @@ extern "C" int wfx_wave_create_westervelt(wfx_ctx* ctx, wfx_stiffness* stiff, wf
   WFX_API_END
 }
 
+namespace
+{
+// the memory variables start from rest (init, set_state, set_relaxation); synchronous like the state copies
+void zero_relaxation_state(wfx_wave* w)
+{
+  if (w->rq_.n) WFX_CUDA(cudaMemset(w->rq_.p, 0, w->rq_.n));
+}
+} // namespace
+
 extern "C" int wfx_wave_init(wfx_wave* w)
 {
   WFX_API_BEGIN
@@ -771,6 +960,7 @@ extern "C" int wfx_wave_init(wfx_wave* w)
     WFX_CUDA(cudaMemset(w->u_.p, 0, w->u_.n));
     WFX_CUDA(cudaMemset(w->v_.p, 0, w->v_.n));
   }
+  zero_relaxation_state(w);
   w->steps_done = 0;
   w->t_now = 0;
   w->probe_rec = 0;
@@ -786,6 +976,7 @@ extern "C" int wfx_wave_set_state(wfx_wave* w, const void* u, const void* v)
   ScopedDevice sd(w->ctx->device);
   if (u && w->u_.n) WFX_CUDA(cudaMemcpy(w->u_.p, u, w->u_.n, cudaMemcpyHostToDevice));
   if (v && w->v_.n) WFX_CUDA(cudaMemcpy(w->v_.p, v, w->v_.n, cudaMemcpyHostToDevice));
+  zero_relaxation_state(w);
   w->steps_done = 0;
   w->t_now = 0;
   w->probe_rec = 0;
@@ -902,10 +1093,42 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
     if (wfx_stiffness_apply(w->stiff, w->f1_w.p, w->b.p, 0, st)) fail("%s", wfx_last_error());
     if (w->prof_on) boundary_profiled(w, t, nullptr, v, st);
     else if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());
-    if (w->qc != 0)
+    if (w->qc != 0 && w->relax_m)
+      boundary_absorbing_mass_relax(w->bnd, w->m64, w->qc, w->kappa, w->kd_on ? w->kd_b.p : nullptr, w->relax_m,
+                                    w->relax_tau, w->relax_eps_b.p, w->rq_.p, 0.0, u, v, w->b.p, st);
+    else if (w->qc != 0)
       boundary_absorbing_mass(w->bnd, w->m64, w->qc, w->kappa, w->kd_on ? w->kd_b.p : nullptr, 0.0, u, v, w->b.p, st);
     if (w->n == 0) return 0;
     const unsigned grid = (unsigned)((w->n + 255) / 256);
+    if (w->relax_m)
+    {
+#define WFX_RHS(T, KD, MM)                                                                                          \
+  westervelt_rhs_relax_kernel<T, KD, MM><<<grid, 256, 0, st>>>(w->n, (const T*)w->b.p, (const T*)w->minv,         \
+                                                               (const T*)u, (const T*)v, (T)w->kappa,             \
+                                                               (const T*)w->kd.p, (const T*)w->relax_eps.p,       \
+                                                               (const T*)w->rq_.p, w->relax_tau, (T*)result)
+#define WFX_RHS_M(T, KD)                                                                                            \
+  switch (w->relax_m)                                                                                               \
+  {                                                                                                                 \
+  case 1: WFX_RHS(T, KD, 1); break;                                                                                 \
+  case 2: WFX_RHS(T, KD, 2); break;                                                                                 \
+  default: WFX_RHS(T, KD, 3); break;                                                                                \
+  }
+      if (w->dtype == WFX_F64)
+      {
+        if (w->kd_on) { WFX_RHS_M(double, true) }
+        else { WFX_RHS_M(double, false) }
+      }
+      else
+      {
+        if (w->kd_on) { WFX_RHS_M(float, true) }
+        else { WFX_RHS_M(float, false) }
+      }
+#undef WFX_RHS_M
+#undef WFX_RHS
+      WFX_CUDA(cudaGetLastError());
+      return 0;
+    }
 #define WFX_RHS(T, KD)                                                                                           \
   westervelt_rhs_kernel<T, KD><<<grid, 256, 0, st>>>(w->n, (const T*)w->b.p, (const T*)w->minv, (const T*)u,    \
                                                      (const T*)v, (T)w->kappa, (const T*)w->kd.p, (T*)result)
@@ -939,6 +1162,11 @@ extern "C" int wfx_wave_rk4(wfx_wave* w, double t0, double tf, double dt, int64_
   ScopedDevice sd(w->ctx->device);
   cudaStream_t st = (cudaStream_t)stream;
   const double c_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  // a lone relaxing dof has the eigenvalue -(1 + sum eps) / tau; RK4's real-axis limit is 2.785
+  if (w->relax_m && tf > t0 && !(dt * w->relax_rate < 2.5))
+    fail("rk4: dt (1 + sum_nu max eps_nu) / tau_min = %g must stay below 2.5 (relaxation; RK4 is unstable beyond "
+         "2.785): dt must be below %g",
+         dt * w->relax_rate, 2.5 / w->relax_rate);
   // Graph replay (one rank only: the distributed step spans two streams and NCCL).  A capture
   // cannot run on the legacy default stream: such callers are moved to an internal stream that
   // is ordered after and before the caller's stream by events.
@@ -1236,12 +1464,109 @@ extern "C" int wfx_wave_set_nonlinearity(wfx_wave* w, const double* kappa_host)
   WFX_API_END
 }
 
+extern "C" int wfx_wave_set_relaxation(wfx_wave* w, int M, const double* tau_host, const double* eps_host)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  if (!w->model || w->ens) fail("relaxation: needs a model made by wfx_wave_create_westervelt");
+  if (M < 0 || M > WFX_RELAX_MAX) fail("relaxation: M = %d outside [0, %d]", M, WFX_RELAX_MAX);
+  const bool on = M > 0 && tau_host && eps_host;
+  if (on && w->snap_every > 0) fail("relaxation: switch snapshots off first (a snapshot carries u and v only)");
+  double eps_max_sum = 0, tau_min = 0;
+  if (on)
+  {
+    for (int j = 0; j < M; ++j)
+    {
+      if (!std::isfinite(tau_host[j]) || !(tau_host[j] > 0))
+        fail("relaxation: tau[%d] must be finite and positive", j);
+      double emax = 0;
+      for (int64_t k = 0; k < w->n; ++k)
+      {
+        const double e = eps_host[(size_t)j * w->n + k];
+        if (!std::isfinite(e) || e < 0)
+          fail("relaxation: eps[%d] at dof %lld must be finite and not negative", j, (long long)k);
+        emax = std::max(emax, e);
+      }
+      eps_max_sum += emax;
+      tau_min = j == 0 ? tau_host[j] : std::min(tau_min, tau_host[j]);
+    }
+  }
+  ScopedDevice sd(w->ctx->device);
+  // a step in flight may read the buffers, and the captured step holds the kernels without relaxation
+  WFX_CUDA(cudaDeviceSynchronize());
+  if (w->step_graph) WFX_CUDA(cudaGraphExecDestroy(w->step_graph));
+  w->step_graph = nullptr;
+  w->relax_m = 0;
+  w->relax_rate = 0;
+  if (!on)
+  {
+    for (auto* b : {&w->relax_eps, &w->rq_, &w->rq0, &w->rqn}) b->release();
+    w->relax_eps_b.release();
+    return 0;
+  }
+  const size_t esz = w->dtype == WFX_F64 ? 8 : 4, ne = (size_t)M * w->n, nb = ne * esz;
+  // each buffer on its own: after a failed allocation (out of memory) a retry allocates what is missing
+  for (auto* b : {&w->relax_eps, &w->rq_, &w->rq0, &w->rqn})
+    if (b->n != nb) b->alloc(nb);
+  if (w->dtype == WFX_F64) w->relax_eps.upload((const unsigned char*)eps_host, nb);
+  else
+  {
+    std::vector<float> e32(ne);
+    for (size_t k = 0; k < ne; ++k) e32[k] = (float)eps_host[k];
+    w->relax_eps.upload((const unsigned char*)e32.data(), nb);
+  }
+  if (w->bnd)
+  {
+    // the Gamma2 mass term takes eps in fp64, compact over the boundary dofs [M][nb]
+    const std::vector<int32_t>& dofs = boundary_dofs(w->bnd);
+    std::vector<double> eb((size_t)M * dofs.size());
+    for (int j = 0; j < M; ++j)
+      for (size_t p = 0; p < dofs.size(); ++p) eb[j * dofs.size() + p] = eps_host[(size_t)j * w->n + dofs[p]];
+    if (w->relax_eps_b.n != eb.size()) w->relax_eps_b.alloc(eb.size());
+    w->relax_eps_b.upload(eb);
+  }
+  if (nb)
+    for (auto* b : {&w->rq_, &w->rq0, &w->rqn}) WFX_CUDA(cudaMemset(b->p, 0, nb));
+  w->relax_tau = RelaxTau{};
+  for (int j = 0; j < M; ++j) w->relax_tau.inv_tau[j] = 1.0 / tau_host[j];
+  w->relax_rate = (1.0 + eps_max_sum) / tau_min;
+  w->relax_m = M;
+  WFX_API_END
+}
+
+extern "C" int wfx_wave_get_relaxation_state(wfx_wave* w, void* q_host)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  if (!w->relax_m) fail("relaxation state: the model has no relaxation (wfx_wave_set_relaxation)");
+  if (!q_host) fail("relaxation state: NULL buffer");
+  ScopedDevice sd(w->ctx->device);
+  WFX_CUDA(cudaDeviceSynchronize()); // the stepping may run on any of the caller's streams
+  w->rq_.download((unsigned char*)q_host, w->rq_.n);
+  WFX_API_END
+}
+
+extern "C" int wfx_wave_set_relaxation_state(wfx_wave* w, const void* q_host)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  if (!w->relax_m) fail("relaxation state: the model has no relaxation (wfx_wave_set_relaxation)");
+  if (!q_host) fail("relaxation state: NULL buffer");
+  ScopedDevice sd(w->ctx->device);
+  WFX_CUDA(cudaDeviceSynchronize());
+  w->rq_.upload((const unsigned char*)q_host, w->rq_.n);
+  WFX_API_END
+}
+
 extern "C" int wfx_wave_set_snapshot(wfx_wave* w, int64_t every, wfx_snapshot_fn fn, void* user)
 {
   WFX_API_BEGIN
   if (!w) fail("wave model is NULL");
   if (every < 0) fail("snapshot interval must not be negative");
   if (w->ens) fail("wave: snapshots are not available for ensemble models");
+  if (w->relax_m && fn && every > 0)
+    fail("wave: snapshots carry u and v only; a model with relaxation checkpoints through "
+         "wfx_wave_get_relaxation_state");
   ScopedDevice sd(w->ctx->device);
   flush_snapshot(w);
   w->snap_every = fn ? every : 0;

@@ -471,6 +471,7 @@ public:
   std::shared_ptr<StiffnessOperator<double>> stiff_op;
   // the C handle, e.g. for PennesGLL::heat_from_wave
   wfx_wave* get() const { return _wave; }
+  std::int64_t ndofs() const { return _ndofs; }
 
 protected:
   // the lossy / Westervelt models (wfx_wave_create_westervelt, one rank): see WesterveltGLLOpt
@@ -543,6 +544,31 @@ public:
   {
     check(wfx_wave_set_nonlinearity(get(), kappa.empty() ? nullptr : kappa.data()));
   }
+  // relaxation absorption (wavefx.h wfx_wave_set_relaxation, DESIGN.md section 4.5f): tau [M] > 0, eps [M][ndofs] >= 0
+  // per dof (the Python Relaxation.eps_dofs); an empty tau switches it off.  The memory variables start at 0.
+  void set_relaxation(const std::vector<double>& tau, const std::vector<double>& eps)
+  {
+    if (!tau.empty() && eps.size() != tau.size() * (std::size_t)ndofs())
+      throw std::runtime_error("wavefx: relaxation eps needs M * ndofs entries");
+    check(wfx_wave_set_relaxation(get(), (int)tau.size(), tau.empty() ? nullptr : tau.data(),
+                                  tau.empty() ? nullptr : eps.data()));
+    _relax_m = (int)tau.size();
+  }
+  // the memory variables q [M][ndofs], for checkpoints: get after solution(), set after set_state()
+  void relaxation_state(std::vector<double>& q) const
+  {
+    q.resize((std::size_t)_relax_m * (std::size_t)ndofs());
+    check(wfx_wave_get_relaxation_state(get(), q.data()));
+  }
+  void set_relaxation_state(const std::vector<double>& q)
+  {
+    if (q.size() != (std::size_t)_relax_m * (std::size_t)ndofs())
+      throw std::runtime_error("wavefx: relaxation state needs M * ndofs entries");
+    check(wfx_wave_set_relaxation_state(get(), q.data()));
+  }
+
+private:
+  int _relax_m = 0;
 };
 // The lossy model: WesterveltGLLOpt with beta = 0,  p_tt - c0^2 lap p - delta lap p_t = 0
 class LossyGLLOpt : public WesterveltGLLOpt

@@ -12,6 +12,8 @@ Same names, argument meaning and call shape as the reference classes:
                                                 lossy and nonlinear (Westervelt) models, DESIGN.md 4.5a
   Medium(rho, c, beta)                          layered media (per-cell density, sound speed and nonlinearity),
                                                 the `medium=` keyword of every wave model, DESIGN.md 4.5e
+  Relaxation(tau, eps, c), Medium.relaxation   power-law absorption by relaxation processes, the `relaxation=`
+                                                keyword of LossyGLLOpt / WesterveltGLLOpt, DESIGN.md 4.5f
 
 `V` is a HexMesh (mesh.py): it carries what the reference pulls out of the DOLFINx
 FunctionSpace (geometry, geometry dofmap, cell dofmap, index-map sizes).  Vectors are
@@ -372,6 +374,12 @@ def focus_delays(points, focus, c0):
     return (d.max() - d) / float(c0) if len(d) else d
 
 
+def _refuse_relaxation(relaxation):
+    if relaxation is not None:
+        raise capi.WfxError("relaxation: needs LossyGLLOpt or WesterveltGLLOpt (for linear tissue, LossyGLLOpt with "
+                            "delta = 0)")
+
+
 class LinearGLLOpt:
     """The wave model + RK4 driver (common/LinearGLL.hpp:37-287) on the GPU.
 
@@ -380,7 +388,8 @@ class LinearGLLOpt:
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency,
                  pressureAmplitude, dtype=np.float64, ctx=None, halo=None, stiffness_mode=capi.STIFF_AUTO,
-                 setup_halo=None, medium=None):
+                 setup_halo=None, medium=None, relaxation=None):
+        _refuse_relaxation(relaxation)
         self.ctx = ctx or Context.get()
         self.V = mesh
         if meshtags is not None:
@@ -559,7 +568,8 @@ class LinearGLLEnsemble(LinearGLLOpt):
     available for ensembles."""
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequencies, pressureAmplitudes,
-                 dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO, medium=None):
+                 dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO, medium=None, relaxation=None):
+        _refuse_relaxation(relaxation)
         self.ctx = ctx or Context.get()
         self.V = mesh
         if meshtags is not None:
@@ -629,11 +639,12 @@ class WesterveltGLLOpt(LinearGLLOpt):
     delta = beta = 0 is LinearGLLOpt bit for bit.  A per-cell coefficient set with Geometry.scale_cells
     multiplies the delta term too (delta_eff = delta * coeff).  With a Medium the nonlinearity is per dof
     (set_nonlinearity), from the medium's beta, which defaults to coefficientOfNonlinearity; delta_eff = delta
-    (c / c0)^2 (DESIGN.md section 4.5e)."""
+    (c / c0)^2 (DESIGN.md section 4.5e).  relaxation: a Relaxation (power-law absorption, DESIGN.md section 4.5f),
+    see set_relaxation."""
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
                  diffusivityOfSound, coefficientOfNonlinearity, density, dtype=np.float64, ctx=None,
-                 stiffness_mode=capi.STIFF_AUTO, medium=None):
+                 stiffness_mode=capi.STIFF_AUTO, medium=None, relaxation=None):
         self.ctx = ctx or Context.get()
         self.V = mesh
         if meshtags is not None:
@@ -663,6 +674,9 @@ class WesterveltGLLOpt(LinearGLLOpt):
             # beta = 0 in a medium without nonlinearity keeps the lossy update
             if self.beta_ > 0 or np.any(kappa > 0):
                 self.set_nonlinearity(kappa)
+        self.relaxation = None
+        if relaxation is not None:
+            self.set_relaxation(relaxation)
 
     def set_nonlinearity(self, kappa=None):
         """kappa [ndofs] >= 0: a per-dof kappa in place of 2 beta / (rho0 c0^2) (the model then steps the nonlinear
@@ -673,6 +687,42 @@ class WesterveltGLLOpt(LinearGLLOpt):
         capi.call("wfx_wave_set_nonlinearity", self.handle, capi.f64p(k))
         self.kappa = k
 
+    def set_relaxation(self, relaxation=None):
+        """Relaxation absorption (DESIGN.md section 4.5f): a Relaxation whose per-cell strengths become per-dof ones
+        with this model's mass weights (Relaxation.eps_dofs); None switches it off.  Model configuration: it survives
+        init, set_state and restarts.  The memory variables start at 0 here, at init and at set_state; a checkpoint
+        restores them with set_relaxation_state after set_state.  rk4 then refuses steps of Relaxation.max_dt and
+        above; snapshots are refused (they carry u and v only)."""
+        if relaxation is None:
+            capi.call("wfx_wave_set_relaxation", self.handle, 0, None, None)
+            self.relaxation, self.relaxation_eps = None, None
+            return
+        if not isinstance(relaxation, Relaxation):
+            raise capi.WfxError("relaxation must be a Relaxation")
+        eps = relaxation.eps_dofs(self.V, self.geometry.detJw(), self._mass_weight)
+        capi.call("wfx_wave_set_relaxation", self.handle, relaxation.M, capi.f64p(relaxation.tau),
+                  capi.f64p(np.ascontiguousarray(eps)))
+        self.relaxation, self.relaxation_eps = relaxation, eps
+
+    def _relax_shape(self):
+        if self.relaxation is None:
+            raise capi.WfxError("relaxation state: the model has no relaxation (set_relaxation)")
+        return (self.relaxation.M, self.ndofs)
+
+    def relaxation_state(self):
+        """the memory variables q [M, ndofs] in the model dtype"""
+        q = np.empty(self._relax_shape(), dtype=self.dtype)
+        capi.call("wfx_wave_get_relaxation_state", self.handle, C.c_void_p(q.ctypes.data))
+        return q
+
+    def set_relaxation_state(self, q):
+        """q [M, ndofs]: the memory variables of a checkpoint (after set_state, which zeroes them)"""
+        shape = self._relax_shape()
+        q = np.ascontiguousarray(q, dtype=self.dtype)
+        if q.shape != shape:
+            raise capi.WfxError(f"relaxation state must have shape {shape}")
+        capi.call("wfx_wave_set_relaxation_state", self.handle, C.c_void_p(q.ctypes.data))
+
 
 class LossyGLLOpt(WesterveltGLLOpt):
     """The lossy wave model (WesterveltGLLOpt with beta = 0):  p_tt - c0^2 lap p - delta lap p_t = 0.  In a Medium
@@ -680,10 +730,11 @@ class LossyGLLOpt(WesterveltGLLOpt):
     beta replaces the model's beta = 0, as for WesterveltGLLOpt); a Medium without beta keeps it lossy."""
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
-                 diffusivityOfSound, dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO, medium=None):
+                 diffusivityOfSound, dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO, medium=None,
+                 relaxation=None):
         super().__init__(mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
                          diffusivityOfSound, 0.0, 1.0, dtype=dtype, ctx=ctx, stiffness_mode=stiffness_mode,
-                         medium=medium)
+                         medium=medium, relaxation=relaxation)
 
 
 # dose of a thermal model (PennesGLL.dose): steps since init / set_state, CEM43 [min] and peak temperature per dof
@@ -721,9 +772,12 @@ class Medium:
     rho_ref c0^2 / (rho_c c_c^2) (MassOperator cell_weight), facet masses rho_ref / rho_f on tag 1 and
     rho_ref c0 / (rho_f c_f) on tag 2 (BoundaryOperator facet_weight, f the facet's cell), and a per-dof kappa for
     the Westervelt model.  With rho = rho_ref and c = c0 every weight is exactly 1.  The loss term becomes
-    delta (c / c0)^2.  Pass it as `medium=` to a wave model; cfl_timestep(h, medium.c_max, ...) gives its step."""
+    delta (c / c0)^2.  Pass it as `medium=` to a wave model; cfl_timestep(h, medium.c_max, ...) gives its step.
+    alpha0 [Np/m at 1 MHz] >= 0 and y > 0 (scalars or per cell, given together): the tissue's power-law absorption
+    alpha0 (f / 1 MHz)^y, which Medium.relaxation fits with relaxation processes (DESIGN.md section 4.5f) and
+    PennesGLL.heat_from_wave(..., medium=) heats with."""
 
-    def __init__(self, rho, c, beta=None, rho_ref=1000.0):
+    def __init__(self, rho, c, beta=None, rho_ref=1000.0, alpha0=None, y=None):
         def arr(name, a, positive):
             a = np.asarray(a, dtype=np.float64)
             if a.ndim > 1:
@@ -737,7 +791,11 @@ class Medium:
         if np.ndim(rho_ref):
             raise capi.WfxError("medium: rho_ref must be a scalar")
         self.rho_ref = float(arr("rho_ref", rho_ref, True))
-        sizes = {a.size for a in (self.rho, self.c, self.beta) if a is not None and a.ndim == 1}
+        if (alpha0 is None) != (y is None):
+            raise capi.WfxError("medium: alpha0 and y go together")
+        self.alpha0 = None if alpha0 is None else arr("alpha0", alpha0, False)
+        self.y = None if y is None else arr("y", y, True)
+        sizes = {a.size for a in (self.rho, self.c, self.beta, self.alpha0, self.y) if a is not None and a.ndim == 1}
         if len(sizes) > 1:
             raise capi.WfxError("medium: per-cell arrays differ in length")
         self.ncells = sizes.pop() if sizes else None
@@ -786,15 +844,142 @@ class Medium:
         """kappa_i = sum_c kappa_c mu_c (detJ w)_{c,i} / m~_i with m~ the weighted mass (host set-up).  A dof whose
         cells all carry the same kappa_c gets that value exactly, so that a homogeneous region (the reference medium
         in particular) steps with the scalar kappa bit for bit."""
-        kc = self.cell_kappa(mesh.ncells, beta)
-        avg = cell_to_dof_average(mesh, detJw, kc, self.mass_weight(mesh.ncells, c0))
-        perm = capi.compute_permutations(mesh.P)
-        dofs = np.asarray(mesh.dofmap)[:, perm].reshape(-1)
-        kpt = np.repeat(kc, len(perm))
-        lo, hi = np.full(mesh.ndofs, np.inf), np.full(mesh.ndofs, -np.inf)
-        np.minimum.at(lo, dofs, kpt)
-        np.maximum.at(hi, dofs, kpt)
-        return np.where(lo == hi, lo, avg)
+        return _shared_exact_average(mesh, detJw, self.cell_kappa(mesh.ncells, beta), self.mass_weight(mesh.ncells, c0))
+
+    def relaxation(self, f_lo, f_hi, mechanisms=3):
+        """Relaxation processes that reproduce alpha0 (f / 1 MHz)^y over the band [f_lo, f_hi] [Hz] in every cell
+        (DESIGN.md section 4.5f).  The `mechanisms` (1..3) relaxation frequencies are log-spaced over
+        [f_lo / s, s f_hi] and shared by all cells, with the spread s in 1.5..3 that fits best.  Per cell, eps >= 0 is
+        the minimax fit of the first-order attenuation (a linear program), refined on the exact alpha from
+        k(w) = (w / c) sqrt(1 + sum eps / (1 + i w tau)).  Returns a Relaxation whose fit_error is the largest
+        relative error of the exact alpha over the band, over all cells."""
+        if self.alpha0 is None:
+            raise capi.WfxError("relaxation: the medium has no absorption (alpha0, y)")
+        if not (0 < f_lo < f_hi and np.isfinite(f_hi)):
+            raise capi.WfxError("relaxation: the band needs 0 < f_lo < f_hi")
+        if mechanisms not in (1, 2, 3):
+            raise capi.WfxError("relaxation: 1 to 3 mechanisms")
+        n = self.ncells or 1
+        a0, y, c = (np.broadcast_to(a, (n,)) for a in (self.alpha0, self.y, self.c))
+        groups, inv = np.unique(np.stack([a0, y, c], 1), axis=0, return_inverse=True)
+        best = None
+        for spread in (1.5, 2.0, 2.5, 3.0):
+            fr = np.geomspace(f_lo / spread, spread * f_hi, mechanisms) if mechanisms > 1 else np.array(
+                [np.sqrt(f_lo * f_hi)])
+            tau = 1.0 / (2.0 * np.pi * fr)
+            fits = [_fit_relaxation(tau, g[0], g[1], g[2], f_lo, f_hi) for g in groups]
+            err = max(e for _, e in fits)
+            if best is None or err < best[0]:
+                best = (err, tau, np.stack([e for e, _ in fits], 1))
+        err, tau, eps_groups = best
+        return Relaxation(tau, eps_groups[:, inv.reshape(-1)], c, fit_error=err)
+
+
+def _shared_exact_average(mesh, detJw, coeff, weight):
+    """cell_to_dof_average with `weight`, except that a dof whose cells all carry the same value gets it exactly"""
+    avg = cell_to_dof_average(mesh, detJw, coeff, weight)
+    perm = capi.compute_permutations(mesh.P)
+    dofs = np.asarray(mesh.dofmap)[:, perm].reshape(-1)
+    cpt = np.repeat(coeff, len(perm))
+    lo, hi = np.full(mesh.ndofs, np.inf), np.full(mesh.ndofs, -np.inf)
+    np.minimum.at(lo, dofs, cpt)
+    np.maximum.at(hi, dofs, cpt)
+    return np.where(lo == hi, lo, avg)
+
+
+def _relax_k(f, tau, eps, c):
+    """k(w) = (w / c) sqrt(1 + sum_nu eps_nu / (1 + i w tau_nu)), shape f.shape + (ncells,); eps [M, ncells]"""
+    w = 2.0 * np.pi * np.asarray(f, dtype=np.float64)[..., None]
+    x = sum(eps[j] / (1.0 + 1j * w * tau[j]) for j in range(len(tau)))
+    return w / c * np.sqrt(1.0 + x)
+
+
+def _fit_relaxation(tau, a0, y, c, f_lo, f_hi, iters=8):
+    """(eps [M], max relative error of the exact alpha) for alpha0 (f / 1 MHz)^y over [f_lo, f_hi] at speed c"""
+    from scipy.optimize import linprog
+    M = len(tau)
+    if a0 == 0:
+        return np.zeros(M), 0.0
+    f = np.geomspace(f_lo, f_hi, 96)
+    w = 2.0 * np.pi * f
+    target = a0 * (f / 1e6) ** y
+    A = (w / (2.0 * c))[:, None] * (w[:, None] * tau[None, :]) / (1.0 + (w[:, None] * tau[None, :]) ** 2)
+    exact = lambda e: -_relax_k(f, tau, e[:, None], c)[:, 0].imag  # noqa: E731
+    goal = target.copy()
+    eps = np.zeros(M)
+    for _ in range(iters):
+        # minimise t subject to |A eps / goal - 1| <= t, eps >= 0
+        Ar = A / goal[:, None]
+        one = np.ones((len(f), 1))
+        res = linprog(np.r_[np.zeros(M), 1.0], A_ub=np.block([[Ar, -one], [-Ar, -one]]),
+                      b_ub=np.r_[np.ones(len(f)), -np.ones(len(f))], bounds=[(0, None)] * (M + 1), method="highs")
+        if res.status != 0:
+            raise capi.WfxError(f"relaxation: the fit failed ({res.message})")
+        eps = res.x[:M]
+        # the exact alpha differs from the first-order one by a smooth factor: aim the first-order fit past it
+        goal = target * (A @ eps) / exact(eps)
+    fd = np.geomspace(f_lo, f_hi, 1024)
+    return eps, float(np.abs(-_relax_k(fd, tau, eps[:, None], c)[:, 0].imag / (a0 * (fd / 1e6) ** y) - 1.0).max())
+
+
+class Relaxation:
+    """M = 1..3 relaxation processes (DESIGN.md section 4.5f) with shared relaxation times tau [M] > 0 [s] and
+    strengths eps [M, ncells] >= 0 (or [M]: the same in every cell), in cells with the high-frequency sound speed c
+    (scalar or per cell):  tau_nu q_nu' + q_nu = eps_nu p,  (1 / (rho c^2)) (p + sum_nu q_nu)_tt - ... .  For
+    p ~ e^{i w t}:  k(w) = (w / c) sqrt(1 + sum_nu eps_nu / (1 + i w tau_nu)),  alpha = -Im k,  phase speed w / Re k
+    (below c, rising to c at high frequency).  fit_error: Medium.relaxation's largest relative error of alpha."""
+
+    def __init__(self, tau, eps, c, fit_error=None):
+        tau = np.asarray(tau, dtype=np.float64).reshape(-1)
+        if not 1 <= tau.size <= capi.RELAX_MAX:
+            raise capi.WfxError(f"relaxation: 1 to {capi.RELAX_MAX} processes")
+        if not np.all(np.isfinite(tau)) or not np.all(tau > 0):
+            raise capi.WfxError("relaxation: tau must be finite and positive")
+        eps = np.asarray(eps, dtype=np.float64)
+        if eps.ndim == 1:
+            eps = eps[:, None]
+        if eps.ndim != 2 or eps.shape[0] != tau.size:
+            raise capi.WfxError("relaxation: eps must have shape [M] or [M, ncells]")
+        if not np.all(np.isfinite(eps)) or not np.all(eps >= 0):
+            raise capi.WfxError("relaxation: eps must be finite and not negative")
+        c = np.asarray(c, dtype=np.float64)
+        if c.ndim > 1 or not np.all(np.isfinite(c)) or not np.all(c > 0):
+            raise capi.WfxError("relaxation: c must be finite and positive, a scalar or one value per cell")
+        if c.ndim and eps.shape[1] not in (1, c.size):
+            raise capi.WfxError("relaxation: eps and c differ in the number of cells")
+        self.tau, self.eps, self.c = np.ascontiguousarray(tau), np.ascontiguousarray(eps), c
+        self.fit_error = fit_error
+
+    @property
+    def M(self):
+        return self.tau.size
+
+    def eps_cells(self, ncells):
+        """eps [M, ncells]"""
+        if self.eps.shape[1] not in (1, ncells):
+            raise capi.WfxError(f"relaxation: {self.eps.shape[1]} cells given, the mesh has {ncells}")
+        return np.ascontiguousarray(np.broadcast_to(self.eps, (self.M, ncells)))
+
+    def alpha(self, f):
+        """attenuation [Np/m] per cell at frequency f [Hz] (shape f.shape + (ncells,)), from the exact k(w)"""
+        return -_relax_k(f, self.tau, self.eps, self.c).imag
+
+    def phase_speed(self, f):
+        """phase speed w / Re k [m/s] per cell at frequency f [Hz]"""
+        return 2.0 * np.pi * np.asarray(f, dtype=np.float64)[..., None] / _relax_k(f, self.tau, self.eps, self.c).real
+
+    def max_dt(self):
+        """just below the step at which rk4 refuses: dt (1 + sum_nu max eps_nu) / tau_min = 2.5 (a lone dof's
+        eigenvalue -(1 + eps) / tau; RK4 is unstable beyond 2.785).  The per-dof eps are averages of the per-cell
+        ones, so this bound holds for every mesh."""
+        return 2.5 * (1.0 - 1e-9) * self.tau.min() / (1.0 + self.eps.max(axis=1).sum())
+
+    def eps_dofs(self, mesh, detJw, mass_weight=None):
+        """eps_nu,i = sum_c eps_nu,c mu_c (detJ w)_{c,i} / m~_i [M, ndofs] with the weighted mass m~ (mass_weight: mu_c,
+        None for 1), exact for the lumped system; a dof whose cells share one eps gets it exactly"""
+        e = self.eps_cells(mesh.ncells)
+        return np.ascontiguousarray(np.stack([_shared_exact_average(mesh, detJw, e[j], mass_weight)
+                                              for j in range(self.M)]))
 
 
 class PennesGLL:
@@ -903,11 +1088,27 @@ class PennesGLL:
             raise capi.WfxError(f"heat source must have shape ({self.ndofs},)")
         capi.call("wfx_thermal_set_heat_source", self.handle, capi.f64p(q))
 
-    def heat_from_wave(self, model, alpha0, y, rho0, c0, member=0, medium=None):
+    def heat_from_wave(self, model, alpha0, y=None, rho0=None, c0=None, member=0, medium=None):
         """Q = sum_h alpha0 (h f0 / 1 MHz)^y |p_h|^2 / (rho0 c0) from the harmonic maps of `model`'s field statistics,
         computed on the device.  alpha0 [Np/m at 1 MHz]: a scalar or one value per dof; member: the ensemble member.
         medium: a Medium on this mesh; 1 / (rho0 c0) is then the per-dof mass-weighted average of 1 / (rho_c c_c),
-        folded into alpha0 (rho0 and c0 are not used)."""
+        folded into alpha0 (rho0 and c0 are not used).  alpha0 = None takes alpha0 from the medium, as its per-dof
+        mass-weighted average, and y from the medium too when y is None; the medium must then have one y everywhere
+        (a per-cell y is refused)."""
+        if alpha0 is None:
+            if medium is None or medium.alpha0 is None:
+                raise capi.WfxError("heat_from_wave: alpha0 = None needs a medium with alpha0 and y")
+            ys = np.unique(medium.y)
+            if ys.size != 1:
+                raise capi.WfxError("heat_from_wave: the medium's y varies per cell; pass alpha0 and y")
+            if y is None:
+                y = float(ys[0])
+            elif float(y) != float(ys[0]):
+                raise capi.WfxError("heat_from_wave: y differs from the medium's")
+            nc = self.V.ncells
+            alpha0 = cell_to_dof_average(self.V, self.geometry.detJw(), np.broadcast_to(medium.alpha0, (nc,)))
+        if y is None or (medium is None and (rho0 is None or c0 is None)):
+            raise capi.WfxError("heat_from_wave: needs y, and rho0 and c0 without a medium")
         a = np.asarray(alpha0, dtype=np.float64)
         a_host = None
         if a.ndim:
