@@ -31,6 +31,10 @@ slab; with --heat-seconds the thermal model is built on its own operators and he
 heats (DESIGN.md section 4.5f): M relaxation processes fitted to --absorption (f / 1 MHz)^--absorption-power over the
 band (default f0 / 2 .. 3 f0) in the tissue -- the slab with --layer (water keeps delta), else the whole domain.  It
 reports the fit error and the phase speed at f0; the time step is also kept below the relaxation's bound.
+--pml WIDTH replaces every absorbing face -- the far end and, with --focus, the four lateral faces -- by a perfectly
+matched layer (DESIGN.md section 4.5g) WIDTH deep inside the domain (PML.box, R0 = 1e-4) with rigid outer faces, so
+that a focused beam's side lobes leave the domain instead of coming back into the maps; it prints the layer's cells,
+dofs and largest damping, and keeps the time step below the layer's bound.
 The reference reads `../mesh.xdmf` (not in its repository); here the mesh is a structured
 n x m x m hexahedral box with tag 1 on x = 0 (source) and tag 2 on x = L (absorbing).
 
@@ -38,7 +42,7 @@ n x m x m hexahedral box with tag 1 on x = 0 (source) and tag 2 on x = L (absorb
                             [--model linear|lossy|westervelt] [--stats-periods K] [--focus DEPTH] [--aperture R]
                             [--heat-seconds S] [--cool-seconds C] [--absorption ALPHA0] [--absorption-power Y]
                             [--layer X0 X1 --layer-rho R --layer-c C [--layer-beta B]]
-                            [--relaxation M [--band F_LO F_HI]]
+                            [--relaxation M [--band F_LO F_HI]] [--pml WIDTH]
 """
 import argparse
 import os
@@ -95,7 +99,13 @@ def main():
                     help="absorb the wave in the tissue with M relaxation processes (lossy, westervelt; 0: off)")
     ap.add_argument("--band", type=float, nargs=2, metavar=("F_LO", "F_HI"), default=None,
                     help="with --relaxation: the fitted band [Hz] (default f0 / 2 .. 3 f0)")
+    ap.add_argument("--pml", type=float, default=0.0, metavar="WIDTH",
+                    help="a perfectly matched layer WIDTH [m] deep in place of the absorbing faces (0: off)")
     args = ap.parse_args()
+    if args.pml < 0:
+        ap.error("--pml WIDTH needs WIDTH > 0")
+    if args.pml > 0 and args.check:
+        ap.error("--check compares with the oracle without a layer; it does not take --pml")
     if args.relaxation and args.model == "linear":
         ap.error("--relaxation needs --model lossy or westervelt (for linear tissue: --model lossy --delta 0)")
     if args.relaxation and args.check:
@@ -113,10 +123,13 @@ def main():
     degreeOfBasis = 4                                                            # :36
     side = domainLength / args.nx
     width = side * args.nyz
-    tags = ((0, 0, 1), (0, 1, 2))
+    absorbing = [(0, 1)]
     if args.focus > 0:
-        tags += ((1, 0, 2), (1, 1, 2), (2, 0, 2), (2, 1, 2))
+        absorbing += [(1, 0), (1, 1), (2, 0), (2, 1)]
+    # with --pml the absorbing faces are rigid and the layer takes their place
+    tags = ((0, 0, 1),) + (() if args.pml > 0 else tuple((a, s, 2) for a, s in absorbing))
     mesh = wfx.create_box_hex((args.nx, args.nyz, args.nyz), degreeOfBasis, (domainLength, width, width), tags=tags)
+    pml = wfx.PML.box(mesh, args.pml, absorbing, speedOfSound) if args.pml > 0 else None
     medium = None
     if args.layer is not None:
         xc = mesh.x[mesh.xdofs, 0].mean(axis=1)                          # cell centres along x
@@ -146,6 +159,8 @@ def main():
     timeStepSize = wfx.cfl_timestep(mesh.h_min, c_max, degreeOfBasis, sourceFrequency)  # :61-66
     if relaxation is not None and timeStepSize >= relaxation.max_dt():
         timeStepSize = period / np.ceil(period / relaxation.max_dt())                  # whole steps per period
+    if pml is not None and timeStepSize >= pml.max_dt():
+        timeStepSize = period / np.ceil(period / pml.max_dt())
     startTime, finalTime = 0.0, domainLength / speedOfSound + 8.0 / sourceFrequency            # :63-64
     print(f"Number of step per period: {int(round(period / timeStepSize))}")
     print(f"dt = {timeStepSize:.15g}")
@@ -154,14 +169,18 @@ def main():
     beta = args.beta if args.model == "westervelt" else 0.0
     if args.model == "linear":
         eqn = wfx.LinearGLLOpt(mesh, None, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
-                               medium=medium)                                                              # :75
+                               medium=medium, pml=pml)                                                     # :75
     else:
         if medium is not None and args.model == "lossy":
             # the lossy model stays linear
             medium = wfx.Medium(medium.rho, medium.c, alpha0=medium.alpha0, y=medium.y)
         eqn = wfx.WesterveltGLLOpt(mesh, None, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
-                                   delta, beta, args.rho0, medium=medium, relaxation=relaxation)
+                                   delta, beta, args.rho0, medium=medium, relaxation=relaxation, pml=pml)
     print(f"Number of steps: {nstep}")
+    if pml is not None:
+        info = eqn.pml_info()
+        print(f"pml: {info['cells']} cells, {info['dofs']} dofs, {args.pml:.4f} m deep on {len(absorbing)} faces, "
+              f"zeta_max = {info['zeta_max']:.6e} 1/s")
     print(f"Degrees of freedom: {mesh.ndofs_global}")
     X = wfx.dof_coordinates(mesh)
     if args.focus > 0:

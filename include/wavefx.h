@@ -62,6 +62,7 @@ typedef struct wfx_scatter_plan wfx_scatter_plan;
 typedef struct wfx_comm wfx_comm;
 typedef struct wfx_halo wfx_halo;
 typedef struct wfx_wave wfx_wave;
+typedef struct wfx_pml wfx_pml;
 
 const char* wfx_last_error(void);
 int wfx_version(void);
@@ -384,6 +385,35 @@ int wfx_wave_set_relaxation(wfx_wave* wave, int M, const double* tau_host, const
  * set_state (which zeroes them).  Refused without relaxation. */
 int wfx_wave_get_relaxation_state(wfx_wave* wave, void* q_host);
 int wfx_wave_set_relaxation_state(wfx_wave* wave, const void* q_host);
+/* Perfectly matched layer (DESIGN.md section 4.5g): the second-order PML of Grote and Sim (2010) on the cells where a
+ * per-dof damping profile zeta_host[3][ndofs] (zeta_j >= 0 [1/s] along physical axis j, finite) is positive at any of
+ * their points.  With a = cK^2 coeff_c (cK the stiffness operator's c0, coeff_c the cell's composed
+ * wfx_geometry_scale_cells coefficient, which reaches the layer whether it is set before or after create):
+ *   m~ (p_tt + sum zeta p_t + sum_{j<k} zeta_j zeta_k p + zeta1 zeta2 zeta3 psi) = b + div phi,   psi_t = p
+ *   phi_t = -Z phi + a Gamma1 grad w + a Gamma2 grad(psi + s p),   Z = diag(zeta_j)
+ *   Gamma1 = diag(zeta2 + zeta3 - zeta1, ..), Gamma2 = diag(zeta2 zeta3, zeta1 zeta3, zeta1 zeta2)
+ * (b: the model's right-hand side, w = p + s p_t its stiffness input, s = delta / cK^2, 0 for the linear model).
+ * psi lives on the layer's dofs, phi (3 components) at the GLL points of its cells; the layer's outer boundary term
+ * is dropped (the natural condition).  The Westervelt and relaxation terms are not stretched: the layer reflects
+ * O(kappa p) and O(eps).  geom, dofmap_host [ncells][(P+1)^3] (DOLFINx order), x_host [npts][3] and xdofs_host
+ * [ncells][8] are those of the wave model's stiffness operator.  The geometry must outlive the layer.  P <= 8. */
+int wfx_pml_create(wfx_ctx* ctx, wfx_geom* geom, int64_t ndofs, const int32_t* dofmap_host, int64_t npts,
+                   const double* x_host, const int32_t* xdofs_host, const double* zeta_host, wfx_pml** pml);
+/* The layer's cells, dofs and largest zeta.  Any output pointer may be NULL. */
+int wfx_pml_info(wfx_pml* pml, int64_t* ncells, int64_t* ndofs, double* zeta_max);
+int wfx_pml_destroy(wfx_pml* pml);
+/* Gives a one-rank linear, lossy or Westervelt model the layer (NULL clears it; a layer without cells launches
+ * nothing).  Model configuration: it survives init and set_state, which zero psi and phi, as does this call.  psi and
+ * phi are RK4 state with the tableau of u and v; rk4 then refuses dt max zeta >= 2.5.  The layer's kernels run after
+ * the boundary term of every stage and in f1 (at the model's current psi and phi).  Synchronises the device and
+ * drops the captured step graph.  The layer must outlive its use by the model.  Refused: ensemble and distributed
+ * models, a layer on another geometry, context, dof count or dtype, a model with snapshots on. */
+int wfx_wave_set_pml(wfx_wave* wave, wfx_pml* pml);
+/* The layer's state for checkpoints: psi [npml_dofs] and phi [npml_cells][(P+1)^3][3] in the model dtype (points
+ * in the tensor order of the reference's dof permutation); get after get_state, set after set_state.  Refused
+ * without a layer. */
+int wfx_wave_get_pml_state(wfx_wave* wave, void* psi_host, void* phi_host);
+int wfx_wave_set_pml_state(wfx_wave* wave, const void* psi_host, const void* phi_host);
 int wfx_wave_init(wfx_wave* wave);                                   /* :131-134 */
 /* Copies the state to the device; on a distributed mesh the ghost entries are then overwritten by
  * their owners' values (u->scatter_fwd(), v->scatter_fwd(), :164,167). */
@@ -455,7 +485,8 @@ int wfx_wave_set_source_profile(wfx_wave* wave, const double* amp_host, const do
  * call (step number, time reached, u, v in the model dtype, ndofs entries each).  It runs on the
  * thread that called wfx_wave_rk4, at the next snapshot or before rk4 returns.  A checkpoint is a
  * snapshot fed back through wfx_wave_set_state.  every = 0 or fn = NULL switches snapshots off.  Refused for a
- * model with relaxation (wfx_wave_set_relaxation), whose state includes the memory variables. */
+ * model with relaxation (wfx_wave_set_relaxation) or a perfectly matched layer (wfx_wave_set_pml), whose state
+ * includes the memory variables or the layer's fields. */
 typedef void (*wfx_snapshot_fn)(void* user, int64_t step, double t, const void* u_host, const void* v_host);
 int wfx_wave_set_snapshot(wfx_wave* wave, int64_t every, wfx_snapshot_fn fn, void* user);
 int wfx_wave_destroy(wfx_wave* wave);

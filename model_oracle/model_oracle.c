@@ -552,3 +552,285 @@ int64_t wo_rk4_westervelt_relax(int P, int64_t ncells, int64_t ndofs, const int3
   free(q_); free(qn); free(q0); free(kq);
   return step;
 }
+
+/* ---- perfectly matched layer (DESIGN.md section 4.5g) --------------------------------------------------------
+ * The second-order PML of Grote and Sim (2010) on the lumped system of model_rhs_relax, with damping zeta[j * ndofs
+ * + k] along physical axis j, psi [ndofs] and phi [ncells][nq][3] (points in tensor order t = (i0 n + i1) n + i2,
+ * dof dofmap[c nq + perm[t]]).  PML cells: zeta > 0 at any of their dofs; PML dofs: the dofs of PML cells.  At the
+ * stage state (p, p_t, psi, phi), with w = p + s p_t, chi = psi + s p, a_c = 1500^2 coeff[c] and the clamped 1-D
+ * derivative table D of the stiffness:
+ *   r_k += [D^T phi]_k - m_k (sum zeta p_t + sum zeta zeta p + zeta1 zeta2 zeta3 psi)_k   (PML dofs, before kappa)
+ *   [D^T phi]_k = -sum_c sum_q grad^ l_k(xi_q) . (dJw_q K_q phi_q)
+ *   psi' = p,   phi_l' = a_c (Gamma1_l (K^T grad^ w)_l + Gamma2_l (K^T grad^ chi)_l) - zeta_l phi_l
+ * K = J^-1 [ncells][nq][3][3] (K[a][l] = dX_a / dx_l) and dJw = |detJ| w [ncells][nq], both in tensor order.  With
+ * no PML cell every step is wo_rk4_westervelt_relax's, bit for bit. */
+typedef struct
+{
+  const double *zeta, *K, *dJw, *coeff;
+  int64_t ncells_pml;
+  uint8_t *cell_on, *dof_on; /* [ncells], [ndofs] */
+} pml_t;
+
+static void pml_setup(pml_t* L, int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* zeta,
+                      const double* K, const double* dJw, const double* coeff)
+{
+  const int nd = (P + 1) * (P + 1) * (P + 1);
+  L->zeta = zeta, L->K = K, L->dJw = dJw, L->coeff = coeff;
+  L->cell_on = calloc(ncells > 0 ? ncells : 1, 1);
+  L->dof_on = calloc(ndofs > 0 ? ndofs : 1, 1);
+  L->ncells_pml = 0;
+  for (int64_t c = 0; c < ncells; ++c)
+  {
+    int on = 0;
+    for (int t = 0; t < nd; ++t)
+    {
+      const int32_t d = dofmap[c * nd + t];
+      on |= zeta[d] > 0 || zeta[ndofs + d] > 0 || zeta[2 * ndofs + d] > 0;
+    }
+    if (!on) continue;
+    L->cell_on[c] = 1;
+    L->ncells_pml += 1;
+    for (int t = 0; t < nd; ++t) L->dof_on[dofmap[c * nd + t]] = 1;
+  }
+}
+
+static void pml_free(pml_t* L)
+{
+  free(L->cell_on);
+  free(L->dof_on);
+}
+
+/* tp[k] = the PML terms of dof k (PML dofs), kpsi, kphi: the layer's rates (0 off the layer) */
+static void pml_terms(const pml_t* L, int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* m,
+                      double s, const double* un, const double* vn, const double* psin, const double* phin, double* tp,
+                      double* kpsi, double* kphi)
+{
+  const int n = P + 1, nd = n * n * n;
+  double D[WO_MAXN * WO_MAXN];
+  int* perm = malloc(sizeof(int) * nd);
+  double* buf = malloc(sizeof(double) * nd * 5);
+  double *W = buf, *X = buf + nd, *F = buf + 2 * nd; /* F [nd][3] */
+  wo_deriv_1d(P, D, 1);
+  wo_perm(P, perm);
+  memset(tp, 0, sizeof(double) * ndofs);
+  memset(kpsi, 0, sizeof(double) * ndofs);
+  memset(kphi, 0, sizeof(double) * ncells * nd * 3);
+  for (int64_t c = 0; c < ncells; ++c)
+  {
+    if (!L->cell_on[c]) continue;
+    const int32_t* cd = dofmap + c * nd;
+    const double a = 1500.0 * 1500.0 * L->coeff[c];
+    for (int t = 0; t < nd; ++t)
+    {
+      const int32_t d = cd[perm[t]];
+      W[t] = un[d] + s * vn[d];
+      X[t] = psin[d] + s * un[d];
+    }
+    for (int i0 = 0; i0 < n; ++i0)
+      for (int i1 = 0; i1 < n; ++i1)
+        for (int i2 = 0; i2 < n; ++i2)
+        {
+          const int t = (i0 * n + i1) * n + i2;
+          double gw[3] = {0, 0, 0}, gx[3] = {0, 0, 0};
+          for (int q = 0; q < n; ++q)
+          {
+            gw[0] += D[i0 * n + q] * W[(q * n + i1) * n + i2];
+            gw[1] += D[i1 * n + q] * W[(i0 * n + q) * n + i2];
+            gw[2] += D[i2 * n + q] * W[(i0 * n + i1) * n + q];
+            gx[0] += D[i0 * n + q] * X[(q * n + i1) * n + i2];
+            gx[1] += D[i1 * n + q] * X[(i0 * n + q) * n + i2];
+            gx[2] += D[i2 * n + q] * X[(i0 * n + i1) * n + q];
+          }
+          const double* k = L->K + (c * nd + t) * 9;
+          const double* ph = phin + (c * nd + t) * 3;
+          const double dj = L->dJw[c * nd + t];
+          for (int d = 0; d < 3; ++d) F[t * 3 + d] = dj * (k[3 * d] * ph[0] + k[3 * d + 1] * ph[1] + k[3 * d + 2] * ph[2]);
+          const int32_t dof = cd[perm[t]];
+          const double z[3] = {L->zeta[dof], L->zeta[ndofs + dof], L->zeta[2 * ndofs + dof]};
+          const double g1[3] = {z[1] + z[2] - z[0], z[0] + z[2] - z[1], z[0] + z[1] - z[2]};
+          const double g2[3] = {z[1] * z[2], z[0] * z[2], z[0] * z[1]};
+          for (int l = 0; l < 3; ++l)
+          {
+            const double pw = k[l] * gw[0] + k[3 + l] * gw[1] + k[6 + l] * gw[2];
+            const double px = k[l] * gx[0] + k[3 + l] * gx[1] + k[6 + l] * gx[2];
+            kphi[(c * nd + t) * 3 + l] = a * (g1[l] * pw + g2[l] * px) - z[l] * ph[l];
+          }
+        }
+    for (int i0 = 0; i0 < n; ++i0)
+      for (int i1 = 0; i1 < n; ++i1)
+        for (int i2 = 0; i2 < n; ++i2)
+        {
+          double acc = 0.0;
+          for (int q = 0; q < n; ++q)
+            acc += D[q * n + i0] * F[((q * n + i1) * n + i2) * 3 + 0] + D[q * n + i1] * F[((i0 * n + q) * n + i2) * 3 + 1]
+                   + D[q * n + i2] * F[((i0 * n + i1) * n + q) * 3 + 2];
+          tp[cd[perm[(i0 * n + i1) * n + i2]]] -= acc;
+        }
+  }
+  for (int64_t k = 0; k < ndofs; ++k)
+  {
+    if (!L->dof_on[k]) continue;
+    const double z0 = L->zeta[k], z1 = L->zeta[ndofs + k], z2 = L->zeta[2 * ndofs + k];
+    tp[k] -= m[k] * ((z0 + z1 + z2) * vn[k] + (z0 * z1 + z0 * z2 + z1 * z2) * un[k] + z0 * z1 * z2 * psin[k]);
+    kpsi[k] = un[k];
+  }
+  free(buf);
+  free(perm);
+}
+
+/* model_rhs_relax with the layer's terms tp added to the numerator (PML dofs) */
+static void model_rhs_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                          const double* m, const double* m1, const double* m2, const double* kappa, double c0,
+                          double freq0, double p0, double delta, int M, const double* tau, const double* eps, double t,
+                          const double* un, const double* vn, const double* qn, const pml_t* L, const double* psin,
+                          const double* phin, double* kv, double* kq, double* kpsi, double* kphi, double* tp, double* b,
+                          double* bv, int sumfact, int nthreads)
+{
+  const size_t nb = sizeof(double) * ndofs;
+  const double s = delta / (1500.0 * 1500.0);
+  double g, gdot;
+  wo_source(t, freq0, p0, c0, &g, &gdot);
+  memset(b, 0, nb);
+  memset(bv, 0, nb);
+  model_stiffness(P, ncells, ndofs, dofmap, G, un, b, sumfact, nthreads);  /* A un */
+  model_stiffness(P, ncells, ndofs, dofmap, G, vn, bv, sumfact, nthreads); /* A vn */
+  if (L->ncells_pml) pml_terms(L, P, ncells, ndofs, dofmap, m, s, un, vn, psin, phin, tp, kpsi, kphi);
+  for (int64_t k = 0; k < ndofs; ++k)
+  {
+    double r = b[k] + s * bv[k];
+    r += (c0 * c0 * g + delta * gdot) * m1[k] - c0 * m2[k] * vn[k];
+    if (L->ncells_pml && L->dof_on[k]) r += tp[k];
+    r += kappa[k] * m[k] * vn[k] * vn[k];
+    if (M > 0)
+    {
+      double qdd = 0.0;
+      for (int nu = 0; nu < M; ++nu)
+      {
+        const int64_t o = nu * ndofs + k;
+        kq[o] = (eps[o] * un[k] - qn[o]) / tau[nu];
+        qdd += (eps[o] * vn[k] - kq[o]) / tau[nu];
+      }
+      r -= m[k] * qdd;
+    }
+    kv[k] = r / (m[k] * (1.0 - kappa[k] * un[k]) + delta / c0 * m2[k]);
+  }
+}
+
+/* dv/dt = f1(t, u, v; q, psi, phi) of the lossy / Westervelt model with relaxation and a perfectly matched layer */
+void wo_f1_westervelt_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G, const double* m,
+                          const double* m1, const double* m2, const double* kappa, double c0, double freq0, double p0,
+                          double delta, int M, const double* tau, const double* eps, const double* zeta,
+                          const double* K, const double* dJw, const double* coeff, double t, const double* u,
+                          const double* v, const double* q, const double* psi, const double* phi, double* out,
+                          int sumfact, int nthreads)
+{
+  const int nd = (P + 1) * (P + 1) * (P + 1);
+  const size_t nb = sizeof(double) * ndofs, nphi = sizeof(double) * (ncells * nd * 3 + 1);
+  double *b = malloc(nb), *bv = malloc(nb), *kq = malloc(nb * (M > 0 ? M : 1));
+  double *tp = malloc(nb + 8), *kpsi = malloc(nb + 8), *kphi = malloc(nphi);
+  pml_t L;
+  pml_setup(&L, P, ncells, ndofs, dofmap, zeta, K, dJw, coeff);
+  model_rhs_pml(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, M, tau, eps, t, u, v, q, &L, psi,
+                phi, out, kq, kpsi, kphi, tp, b, bv, sumfact, nthreads);
+  pml_free(&L);
+  free(b); free(bv); free(kq); free(tp); free(kpsi); free(kphi);
+}
+
+/* wo_rk4_westervelt_relax with a perfectly matched layer: psi [ndofs] and phi [ncells][nq][3] (in / out) are stepped
+ * by the same tableau as u, v and q */
+int64_t wo_rk4_westervelt_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                              const double* m, const double* m1, const double* m2, const double* kappa, double c0,
+                              double freq0, double p0, double delta, int M, const double* tau, const double* eps,
+                              const double* zeta, const double* K, const double* dJw, const double* coeff, double t0,
+                              double tf, double dt, int64_t max_steps, double* u_n, double* v_n, double* q_n,
+                              double* psi_n, double* phi_n, int sumfact, int nthreads, double* t_end)
+{
+  const double a_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  const double b_runge[4] = {1.0 / 6.0, 1.0 / 3.0, 1.0 / 3.0, 1.0 / 6.0};
+  const double c_runge[4] = {0.0, 0.5, 0.5, 1.0};
+  const int nd = (P + 1) * (P + 1) * (P + 1);
+  const size_t nb = sizeof(double) * ndofs, nq = nb * (M > 0 ? M : 1);
+  const int64_t nqe = (int64_t)M * ndofs, nph = ncells * nd * 3;
+  double *u_ = malloc(nb), *v_ = malloc(nb), *un = malloc(nb), *vn = malloc(nb);
+  double *u0 = malloc(nb), *v0 = malloc(nb), *ku = malloc(nb), *kv = malloc(nb), *b = malloc(nb), *bv = malloc(nb);
+  double *q_ = malloc(nq), *qn = malloc(nq), *q0 = malloc(nq), *kq = malloc(nq);
+  double *ps_ = malloc(nb + 8), *psn = malloc(nb + 8), *ps0 = malloc(nb + 8), *kps = malloc(nb + 8), *tp = malloc(nb + 8);
+  const size_t nphb = sizeof(double) * (nph + 1);
+  double *ph_ = malloc(nphb), *phn = malloc(nphb), *ph0 = malloc(nphb), *kph = malloc(nphb);
+  pml_t L;
+  pml_setup(&L, P, ncells, ndofs, dofmap, zeta, K, dJw, coeff);
+  const int on = L.ncells_pml > 0;
+  memcpy(u_, u_n, nb);
+  memcpy(v_, v_n, nb);
+  memcpy(ku, u_, nb);
+  memcpy(kv, v_, nb);
+  if (M > 0)
+  {
+    memcpy(q_, q_n, sizeof(double) * nqe);
+    memset(kq, 0, sizeof(double) * nqe);
+  }
+  if (on)
+  {
+    memcpy(ps_, psi_n, nb);
+    memcpy(ph_, phi_n, sizeof(double) * nph);
+  }
+  double t = t0;
+  int64_t step = 0;
+  while (t < tf)
+  {
+    if (max_steps > 0 && step >= max_steps) break;
+    dt = dt < tf - t ? dt : tf - t;
+    memcpy(u0, u_, nb);
+    memcpy(v0, v_, nb);
+    if (M > 0) memcpy(q0, q_, sizeof(double) * nqe);
+    if (on)
+    {
+      memcpy(ps0, ps_, nb);
+      memcpy(ph0, ph_, sizeof(double) * nph);
+    }
+    for (int i = 0; i < 4; ++i)
+    {
+      memcpy(un, u0, nb);
+      memcpy(vn, v0, nb);
+      const double adt = dt * a_runge[i];
+      for (int64_t k = 0; k < ndofs; ++k) un[k] = ku[k] * adt + un[k];
+      for (int64_t k = 0; k < ndofs; ++k) vn[k] = kv[k] * adt + vn[k];
+      for (int64_t k = 0; k < nqe; ++k) qn[k] = i == 0 ? q0[k] : kq[k] * adt + q0[k];
+      if (on)
+      {
+        for (int64_t k = 0; k < ndofs; ++k) psn[k] = i == 0 ? ps0[k] : kps[k] * adt + ps0[k];
+        for (int64_t k = 0; k < nph; ++k) phn[k] = i == 0 ? ph0[k] : kph[k] * adt + ph0[k];
+      }
+      const double tn = t + c_runge[i] * dt;
+      memcpy(ku, vn, nb);
+      model_rhs_pml(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, M, tau, eps, tn, un, vn, qn, &L,
+                    psn, phn, kv, kq, kps, kph, tp, b, bv, sumfact, nthreads);
+      const double bdt = dt * b_runge[i];
+      for (int64_t k = 0; k < ndofs; ++k) u_[k] = ku[k] * bdt + u_[k];
+      for (int64_t k = 0; k < ndofs; ++k) v_[k] = kv[k] * bdt + v_[k];
+      for (int64_t k = 0; k < nqe; ++k) q_[k] = kq[k] * bdt + q_[k];
+      if (on)
+      {
+        for (int64_t k = 0; k < ndofs; ++k) ps_[k] = kps[k] * bdt + ps_[k];
+        for (int64_t k = 0; k < nph; ++k) ph_[k] = kph[k] * bdt + ph_[k];
+      }
+    }
+    t += dt;
+    step += 1;
+  }
+  memcpy(u_n, u_, nb);
+  memcpy(v_n, v_, nb);
+  if (M > 0) memcpy(q_n, q_, sizeof(double) * nqe);
+  if (on)
+  {
+    memcpy(psi_n, ps_, nb);
+    memcpy(phi_n, ph_, sizeof(double) * nph);
+  }
+  if (t_end) *t_end = t;
+  pml_free(&L);
+  free(u_); free(v_); free(un); free(vn); free(u0); free(v0); free(ku); free(kv); free(b); free(bv);
+  free(q_); free(qn); free(q0); free(kq);
+  free(ps_); free(psn); free(ps0); free(kps); free(tp);
+  free(ph_); free(phn); free(ph0); free(kph);
+  return step;
+}

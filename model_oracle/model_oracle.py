@@ -91,6 +91,14 @@ def lib():
         L.wo_rk4_westervelt_relax.restype = l
         L.wo_rk4_westervelt_relax.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, i, _f64p,
                                               _f64p, d, d, d, l, _f64p, _f64p, _f64p, i, i, _f64p]
+        L.wo_f1_westervelt_pml.restype = None
+        L.wo_f1_westervelt_pml.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, i, _f64p,
+                                           _f64p, _f64p, _f64p, _f64p, _f64p, d, _f64p, _f64p, _f64p, _f64p, _f64p,
+                                           _f64p, i, i]
+        L.wo_rk4_westervelt_pml.restype = l
+        L.wo_rk4_westervelt_pml.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, i, _f64p,
+                                            _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, l, _f64p, _f64p, _f64p, _f64p,
+                                            _f64p, i, i, _f64p]
         _lib.append(L)
     return _lib[0]
 
@@ -271,4 +279,63 @@ def rk4_westervelt_relax(mesh, P, G, m, m1, m2, kappa, c0, f0, p0, delta, tau, e
     steps = lib().wo_rk4_westervelt_relax(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)),
                                           _f(m), _f(m1), _f(m2), _f(kappa), c0, f0, p0, delta, M, tp, ep, t0, tf, dt,
                                           max_steps, _f(u), _f(v), qp, int(sumfact), nthreads, C.byref(t_end))
+    return steps, t_end.value
+
+
+# ---- perfectly matched layer (DESIGN.md section 4.5g) --------------------------------------------------------------
+class PMLInputs:
+    """The layer's inputs of the restatement: zeta [3, ndofs], K = J^-1 [ncells, nq, 3, 3] and dJw = |detJ| w
+    [ncells, nq] at the GLL points in tensor order (the reference layout of oracle.precompute_geometric_data), and the
+    cells' composed stiffness coefficient coeff [ncells] (a_c = 1500^2 coeff_c)."""
+
+    def __init__(self, mesh, P, zeta, K, dJw, coeff=None):
+        nq = (P + 1) ** 3
+        self.zeta = np.ascontiguousarray(zeta, dtype=np.float64).reshape(3, mesh.ndofs)
+        self.K = np.ascontiguousarray(K, dtype=np.float64).reshape(mesh.ncells, nq, 3, 3)
+        self.dJw = np.ascontiguousarray(dJw, dtype=np.float64).reshape(mesh.ncells, nq)
+        self.coeff = (np.ones(mesh.ncells) if coeff is None
+                      else np.ascontiguousarray(coeff, dtype=np.float64).reshape(mesh.ncells))
+
+    def args(self):
+        return (_f(self.zeta.reshape(-1)), _f(self.K.reshape(-1)), _f(self.dJw.reshape(-1)), _f(self.coeff))
+
+
+def pml_state(mesh, P):
+    """zero (psi [ndofs], phi [ncells, nq, 3])"""
+    return np.zeros(mesh.ndofs), np.zeros((mesh.ncells, (P + 1) ** 3, 3))
+
+
+def f1_westervelt_pml(mesh, P, G, m, m1, m2, kappa, c0, f0, p0, delta, tau, eps, pml, t, u, v, q=None, psi=None,
+                      phi=None, sumfact=False, nthreads=1):
+    """f1_westervelt_relax with a perfectly matched layer (pml: PMLInputs) at psi [ndofs], phi [ncells, nq, 3]
+    (None: 0)"""
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    M, tp, ep, _, qp = _relax(mesh, tau, eps, q)
+    z_psi, z_phi = pml_state(mesh, P)
+    psi = z_psi if psi is None else np.ascontiguousarray(psi, dtype=np.float64)
+    phi = z_phi if phi is None else np.ascontiguousarray(phi, dtype=np.float64)
+    out = np.empty(mesh.ndofs)
+    lib().wo_f1_westervelt_pml(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)), _f(m), _f(m1),
+                               _f(m2), _f(np.ascontiguousarray(kappa, dtype=np.float64)), c0, f0, p0, delta, M, tp, ep,
+                               *pml.args(), t, _f(u), _f(v), qp, _f(psi), _f(phi.reshape(-1)), _f(out), int(sumfact),
+                               nthreads)
+    return out
+
+
+def rk4_westervelt_pml(mesh, P, G, m, m1, m2, kappa, c0, f0, p0, delta, tau, eps, pml, t0, tf, dt, u, v, q, psi, phi,
+                       max_steps=0, sumfact=False, nthreads=1):
+    """rk4_westervelt_relax with a perfectly matched layer (see f1_westervelt_pml); u, v, q, psi [ndofs] and phi
+    [ncells, nq, 3] updated in place.  -> (steps, t_end)"""
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    kappa = np.ascontiguousarray(kappa, dtype=np.float64)
+    assert kappa.shape == (mesh.ndofs,)
+    M, tp, ep, q, qp = _relax(mesh, tau, eps, q)
+    for a in (psi, phi):
+        assert a.dtype == np.float64 and a.flags["C_CONTIGUOUS"]
+    assert psi.shape == (mesh.ndofs,) and phi.shape == (mesh.ncells, (P + 1) ** 3, 3)
+    t_end = C.c_double()
+    steps = lib().wo_rk4_westervelt_pml(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)),
+                                        _f(m), _f(m1), _f(m2), _f(kappa), c0, f0, p0, delta, M, tp, ep, *pml.args(),
+                                        t0, tf, dt, max_steps, _f(u), _f(v), qp, _f(psi), _f(phi.reshape(-1)),
+                                        int(sumfact), nthreads, C.byref(t_end))
     return steps, t_end.value

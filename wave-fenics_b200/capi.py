@@ -118,6 +118,12 @@ _SIG = {
     "wfx_wave_set_relaxation": [_vp, C.c_int, _c_f64p, _c_f64p],
     "wfx_wave_get_relaxation_state": [_vp, _vp],
     "wfx_wave_set_relaxation_state": [_vp, _vp],
+    "wfx_pml_create": [_vp, _vp, C.c_int64, _c_i32p, C.c_int64, _c_f64p, _c_i32p, _c_f64p, _vpp],
+    "wfx_pml_info": [_vp, _c_i64p, _c_i64p, _c_f64p],
+    "wfx_pml_destroy": [_vp],
+    "wfx_wave_set_pml": [_vp, _vp],
+    "wfx_wave_get_pml_state": [_vp, _vp, _vp],
+    "wfx_wave_set_pml_state": [_vp, _vp, _vp],
     "wfx_wave_init": [_vp],
     "wfx_wave_set_state": [_vp, _vp, _vp],
     "wfx_wave_get_state": [_vp, _vp, _vp],

@@ -344,6 +344,9 @@ extern "C" int wfx_geometry_scale_cells(wfx_geom* g, const double* coeff_host)
   }
   WFX_CUDA(cudaGetLastError());
   WFX_CUDA(cudaDeviceSynchronize());
+  if (g->cell_coeff.empty()) g->cell_coeff.assign((size_t)g->ncells, 1.0);
+  for (int64_t c = 0; c < g->ncells; ++c) g->cell_coeff[c] *= coeff_host[c];
+  for (wfx_pml* p : g->pmls) pml_scale_cells(p, coeff_host);
   WFX_API_END
 }
 

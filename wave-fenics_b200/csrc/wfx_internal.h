@@ -171,6 +171,35 @@ struct WaveFieldStats
 };
 WaveFieldStats wave_field_stats(const struct ::wfx_wave* w);
 
+// Perfectly matched layer (wfx_pml_create, DESIGN.md section 4.5g), wfx_pml.cu.  One RK4 stage (update = true) or the
+// right-hand side of f1 (update = false, stage 0): adds the layer's terms to b and steps psi and phi.  Vectors in the
+// model dtype: w the stiffness input, p = u_ at stage 0 (v_ its rate) and w - s vn at stages 1-3; psi [npd] and phi
+// [cells][3][nq] (solution _, start of step 0, stage state n), r [cells][nq] scratch, m the mass m~ compact [npd].
+struct PmlStage
+{
+  int stage = 0;
+  bool update = true;
+  double cK2 = 0, s = 0, bdt = 0, adt = 0;
+  const void *w = nullptr, *u_ = nullptr, *v_ = nullptr, *vn = nullptr, *m = nullptr;
+  void *psi_ = nullptr, *psi0 = nullptr, *psin = nullptr, *phi_ = nullptr, *phi0 = nullptr, *phin = nullptr;
+  void *r = nullptr, *b = nullptr;
+};
+void pml_stage(const struct ::wfx_pml* pm, const PmlStage& q, cudaStream_t st);
+// wfx_geometry_scale_cells on a registered layer: its per-cell coefficients times coeff_host[geometry cell]
+void pml_scale_cells(struct ::wfx_pml* pm, const double* coeff_host);
+// what a wave model needs to know of a layer to take it (wfx_wave_set_pml)
+struct PmlShape
+{
+  wfx_ctx* ctx = nullptr;
+  const struct ::wfx_geom* geom = nullptr;
+  int dtype = 0, nq = 0;
+  int64_t ndofs = 0, ncells = 0, npd = 0;
+  double zeta_max = 0;
+  const std::vector<int32_t>* dofs = nullptr; // global dof of each PML dof
+};
+PmlShape pml_shape(const struct ::wfx_pml* pm);
+const struct ::wfx_geom* stiffness_geom(const struct ::wfx_stiffness* op); // wfx_stiffness.cu
+
 // NVTX ranges around the phases of a time step (the reference marks its profiled regions the same
 // way: demo/gpu_scatter_mpi/main.cpp:101-121, demo/gpu_cg/CUDA/cg.hpp:74-113).  nvtx3 is header-only
 // and costs a few nanoseconds when no tool is attached.
@@ -229,6 +258,10 @@ struct wfx_geom
   // set after an operator was created reaches every path.  An operator registers its copy at creation and
   // removes it when destroyed.
   std::vector<void*> g_copies;
+  // the composed wfx_geometry_scale_cells coefficient per cell (empty: never scaled), and the perfectly matched
+  // layers built on this geometry, which it scales the same way (a layer reads it at creation and registers itself)
+  std::vector<double> cell_coeff;
+  std::vector<struct ::wfx_pml*> pmls;
   double* dJw = nullptr;  // fp64
   // Affine cells (parallelepipeds): G[c,q] = w_q * A_c with one symmetric 3x3 A_c per cell.  Detected
   // from the computed (clamped) per-point G, so a cell counts as affine only if the per-cell form

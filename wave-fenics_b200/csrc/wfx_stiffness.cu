@@ -2425,6 +2425,7 @@ bool stiffness_graph_safe(const wfx_stiffness* op) { return !op->persistent; }
 bool stiffness_has_ensemble(const wfx_stiffness* op) { return op->ens; }
 double stiffness_c0(const wfx_stiffness* op) { return op->c0; }
 int64_t stiffness_nshared(const wfx_stiffness* op) { return op->nshared; }
+const wfx_geom* stiffness_geom(const wfx_stiffness* op) { return op->geom; }
 
 // tensor-ordered dofmap in the kernels' k-major point order
 void build_tensor_dofmap(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap,

@@ -51,6 +51,11 @@ struct wfx_wave
   double relax_rate = 0;
   DevBuf<unsigned char> relax_eps, rq_, rq0, rqn;
   DevBuf<double> relax_eps_b;
+  // perfectly matched layer (wfx_wave_set_pml, section 4.5g): psi [npd] and phi [cells][3][nq] in the model dtype,
+  // each as solution _, start of step 0 and stage state n; pml_r the cell kernel's scratch, pml_m m~ compact [npd]
+  wfx_pml* pml = nullptr;
+  double pml_zeta_max = 0;
+  DevBuf<unsigned char> psi_, psi0, psin, phi_, phi0, phin, pml_r, pml_m;
   const double* m64 = nullptr;
   DevBuf<unsigned char> f1_w;
   const void* minv = nullptr;
@@ -697,6 +702,35 @@ __global__ void set_source_ens_kernel(double* g_dev, const StepAmp a, int n)
 
 void boundary_profiled(wfx_wave* w, double tn, const double* t_dev, const void* vn, cudaStream_t st);
 
+// The layer's terms of one stage (update) or of f1 (stage 0, no update): wi the stiffness input, u / v the state at
+// stage 0, vn the stage's v at stages 1-3
+void pml_terms(wfx_wave* w, int stage, bool update, double bdt, double adt, const void* wi, const void* u,
+               const void* v, const void* vn, cudaStream_t st)
+{
+  PmlStage q;
+  q.stage = stage;
+  q.update = update;
+  const double cK = stiffness_c0(w->stiff);
+  q.cK2 = cK * cK;
+  q.s = w->model ? w->s_stiff : 0.0;
+  q.bdt = bdt;
+  q.adt = adt;
+  q.w = wi;
+  q.u_ = u;
+  q.v_ = v;
+  q.vn = vn;
+  q.m = w->pml_m.p;
+  q.psi_ = w->psi_.p;
+  q.psi0 = w->psi0.p;
+  q.psin = w->psin.p;
+  q.phi_ = w->phi_.p;
+  q.phi0 = w->phi0.p;
+  q.phin = w->phin.p;
+  q.r = w->pml_r.p;
+  q.b = w->b.p;
+  pml_stage(w->pml, q, st);
+}
+
 // One time step of size dt on stream st: the four stages of LinearGLL.hpp:244-270.  g[i*nv + m] is the
 // source amplitude of stage i (of member m); with g_from_dev the boundary kernels read it from w->g_dev
 // instead (graph capture).  With a source profile the boundary term takes the stage times tn[i] instead, or
@@ -759,6 +793,7 @@ void enqueue_step(wfx_wave* w, double dt, const double* g, const double* tn, boo
       WFX_CUDA(cudaStreamWaitEvent(st, w->ev_halo, 0));
       boundary(i, vn);
     }
+    if (w->pml) pml_terms(w, i, true, dt * b_runge[i], dt * a_runge[i + 1], un, w->u_.p, w->v_.p, w->vn.p, st);
     if (w->model)
     {
       // Gamma2 mass term (compact, absorbing dofs), then the fused update; p = u_ at stage 0, else w - s vn
@@ -948,6 +983,12 @@ void zero_relaxation_state(wfx_wave* w)
 {
   if (w->rq_.n) WFX_CUDA(cudaMemset(w->rq_.p, 0, w->rq_.n));
 }
+// the layer's psi and phi start from rest as well (init, set_state, set_pml)
+void zero_pml_state(wfx_wave* w)
+{
+  if (w->psi_.n) WFX_CUDA(cudaMemset(w->psi_.p, 0, w->psi_.n));
+  if (w->phi_.n) WFX_CUDA(cudaMemset(w->phi_.p, 0, w->phi_.n));
+}
 } // namespace
 
 extern "C" int wfx_wave_init(wfx_wave* w)
@@ -961,6 +1002,7 @@ extern "C" int wfx_wave_init(wfx_wave* w)
     WFX_CUDA(cudaMemset(w->v_.p, 0, w->v_.n));
   }
   zero_relaxation_state(w);
+  zero_pml_state(w);
   w->steps_done = 0;
   w->t_now = 0;
   w->probe_rec = 0;
@@ -977,6 +1019,7 @@ extern "C" int wfx_wave_set_state(wfx_wave* w, const void* u, const void* v)
   if (u && w->u_.n) WFX_CUDA(cudaMemcpy(w->u_.p, u, w->u_.n, cudaMemcpyHostToDevice));
   if (v && w->v_.n) WFX_CUDA(cudaMemcpy(w->v_.p, v, w->v_.n, cudaMemcpyHostToDevice));
   zero_relaxation_state(w);
+  zero_pml_state(w);
   w->steps_done = 0;
   w->t_now = 0;
   w->probe_rec = 0;
@@ -1093,6 +1136,7 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
     if (wfx_stiffness_apply(w->stiff, w->f1_w.p, w->b.p, 0, st)) fail("%s", wfx_last_error());
     if (w->prof_on) boundary_profiled(w, t, nullptr, v, st);
     else if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());
+    if (w->pml) pml_terms(w, 0, false, 0.0, 0.0, w->f1_w.p, u, v, nullptr, st);
     if (w->qc != 0 && w->relax_m)
       boundary_absorbing_mass_relax(w->bnd, w->m64, w->qc, w->kappa, w->kd_on ? w->kd_b.p : nullptr, w->relax_m,
                                     w->relax_tau, w->relax_eps_b.p, w->rq_.p, 0.0, u, v, w->b.p, st);
@@ -1150,6 +1194,7 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
   if (w->halo && wfx_halo_update_rev_fwd(w->halo, w->b.p, st)) fail("%s", wfx_last_error());             // :176
   if (w->prof_on) boundary_profiled(w, t, nullptr, v, st);
   else if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());  // :175
+  if (w->pml) pml_terms(w, 0, false, 0.0, 0.0, u, u, v, nullptr, st);
   if (wfx_mass_apply_inverse(w->mass, w->b.p, result, st)) fail("%s", wfx_last_error());                 // :188-191
   WFX_API_END
 }
@@ -1167,6 +1212,11 @@ extern "C" int wfx_wave_rk4(wfx_wave* w, double t0, double tf, double dt, int64_
     fail("rk4: dt (1 + sum_nu max eps_nu) / tau_min = %g must stay below 2.5 (relaxation; RK4 is unstable beyond "
          "2.785): dt must be below %g",
          dt * w->relax_rate, 2.5 / w->relax_rate);
+  // a lone dof of the layer has the eigenvalues -zeta_j
+  if (w->pml && tf > t0 && !(dt * w->pml_zeta_max < 2.5))
+    fail("rk4: dt max zeta = %g must stay below 2.5 (perfectly matched layer; RK4 is unstable beyond 2.785): dt must "
+         "be below %g",
+         dt * w->pml_zeta_max, 2.5 / w->pml_zeta_max);
   // Graph replay (one rank only: the distributed step spans two streams and NCCL).  A capture
   // cannot run on the legacy default stream: such callers are moved to an internal stream that
   // is ordered after and before the caller's stream by events.
@@ -1558,6 +1608,122 @@ extern "C" int wfx_wave_set_relaxation_state(wfx_wave* w, const void* q_host)
   WFX_API_END
 }
 
+extern "C" int wfx_wave_set_pml(wfx_wave* w, wfx_pml* pml)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  PmlShape ps;
+  if (pml)
+  {
+    ps = pml_shape(pml);
+    if (w->ens) fail("pml: ensemble models are not supported");
+    if (w->halo || stiffness_nshared(w->stiff) > 0) fail("pml: one rank only (the model is distributed)");
+    if (ps.ctx != w->ctx) fail("pml: the layer belongs to another context");
+    if (ps.geom != stiffness_geom(w->stiff)) fail("pml: the layer was built on another geometry than the model's");
+    if (ps.ndofs != w->n) fail("pml: the layer has %lld dofs, the model %lld", (long long)ps.ndofs, (long long)w->n);
+    if (ps.dtype != w->dtype) fail("pml: the layer's dtype differs from the model's");
+    if (w->snap_every > 0) fail("pml: switch snapshots off first (a snapshot carries u and v only)");
+  }
+  ScopedDevice sd(w->ctx->device);
+  // a step in flight may read the buffers, and the captured step holds the launches without the layer
+  WFX_CUDA(cudaDeviceSynchronize());
+  if (w->step_graph) WFX_CUDA(cudaGraphExecDestroy(w->step_graph));
+  w->step_graph = nullptr;
+  w->pml = nullptr;
+  w->pml_zeta_max = 0;
+  if (!pml)
+  {
+    for (auto* b : {&w->psi_, &w->psi0, &w->psin, &w->phi_, &w->phi0, &w->phin, &w->pml_r, &w->pml_m}) b->release();
+    return 0;
+  }
+  const size_t esz = w->dtype == WFX_F64 ? 8 : 4;
+  const size_t npsi = (size_t)ps.npd * esz, nphi = (size_t)ps.ncells * ps.nq * 3 * esz;
+  // each buffer on its own: after a failed allocation (out of memory) a retry allocates what is missing
+  for (auto* b : {&w->psi_, &w->psi0, &w->psin, &w->pml_m})
+    if (b->n != npsi) b->alloc(npsi);
+  for (auto* b : {&w->phi_, &w->phi0, &w->phin})
+    if (b->n != nphi) b->alloc(nphi);
+  if (w->pml_r.n != nphi / 3) w->pml_r.alloc(nphi / 3);
+  // m~ compact over the layer's dofs, in the model dtype
+  std::vector<double> m((size_t)w->n);
+  if (w->n) WFX_CUDA(cudaMemcpy(m.data(), mass_diagonal64(w->mass), m.size() * sizeof(double), cudaMemcpyDeviceToHost));
+  const std::vector<int32_t>& dofs = *ps.dofs;
+  if (w->dtype == WFX_F64)
+  {
+    std::vector<double> mc(dofs.size());
+    for (size_t j = 0; j < dofs.size(); ++j) mc[j] = m[dofs[j]];
+    if (npsi) WFX_CUDA(cudaMemcpy(w->pml_m.p, mc.data(), npsi, cudaMemcpyHostToDevice));
+  }
+  else
+  {
+    std::vector<float> mc(dofs.size());
+    for (size_t j = 0; j < dofs.size(); ++j) mc[j] = (float)m[dofs[j]];
+    if (npsi) WFX_CUDA(cudaMemcpy(w->pml_m.p, mc.data(), npsi, cudaMemcpyHostToDevice));
+  }
+  for (auto* b : {&w->psi_, &w->psi0, &w->psin, &w->phi_, &w->phi0, &w->phin})
+    if (b->n) WFX_CUDA(cudaMemset(b->p, 0, b->n));
+  w->pml = pml;
+  w->pml_zeta_max = ps.zeta_max;
+  WFX_API_END
+}
+
+namespace
+{
+// phi in the caller's layout [cells][nq][3] <-> the device's [cells][3][nq]
+template <typename T>
+void phi_transpose(const T* in, T* out, int64_t ncells, int nq, bool to_device)
+{
+  for (int64_t c = 0; c < ncells; ++c)
+    for (int q = 0; q < nq; ++q)
+      for (int l = 0; l < 3; ++l)
+      {
+        const int64_t h = (c * nq + q) * 3 + l, d = (c * 3 + l) * nq + q;
+        if (to_device) out[d] = in[h];
+        else out[h] = in[d];
+      }
+}
+void pml_state_io(wfx_wave* w, void* psi_host, void* phi_host, bool to_device)
+{
+  if (!w->pml) fail("pml state: the model has no perfectly matched layer (wfx_wave_set_pml)");
+  if (!psi_host || !phi_host) fail("pml state: NULL buffer");
+  const PmlShape ps = pml_shape(w->pml);
+  ScopedDevice sd(w->ctx->device);
+  WFX_CUDA(cudaDeviceSynchronize()); // the stepping may run on any of the caller's streams
+  const size_t nphi = w->phi_.n;
+  std::vector<unsigned char> tmp(nphi);
+  if (to_device)
+  {
+    w->psi_.upload((const unsigned char*)psi_host, w->psi_.n);
+    if (w->dtype == WFX_F64) phi_transpose((const double*)phi_host, (double*)tmp.data(), ps.ncells, ps.nq, true);
+    else phi_transpose((const float*)phi_host, (float*)tmp.data(), ps.ncells, ps.nq, true);
+    w->phi_.upload(tmp.data(), nphi);
+  }
+  else
+  {
+    w->psi_.download((unsigned char*)psi_host, w->psi_.n);
+    w->phi_.download(tmp.data(), nphi);
+    if (w->dtype == WFX_F64) phi_transpose((const double*)tmp.data(), (double*)phi_host, ps.ncells, ps.nq, false);
+    else phi_transpose((const float*)tmp.data(), (float*)phi_host, ps.ncells, ps.nq, false);
+  }
+}
+} // namespace
+
+extern "C" int wfx_wave_get_pml_state(wfx_wave* w, void* psi_host, void* phi_host)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  pml_state_io(w, psi_host, phi_host, false);
+  WFX_API_END
+}
+
+extern "C" int wfx_wave_set_pml_state(wfx_wave* w, const void* psi_host, const void* phi_host)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  pml_state_io(w, const_cast<void*>(psi_host), const_cast<void*>(phi_host), true);
+  WFX_API_END
+}
+
 extern "C" int wfx_wave_set_snapshot(wfx_wave* w, int64_t every, wfx_snapshot_fn fn, void* user)
 {
   WFX_API_BEGIN
@@ -1567,6 +1733,9 @@ extern "C" int wfx_wave_set_snapshot(wfx_wave* w, int64_t every, wfx_snapshot_fn
   if (w->relax_m && fn && every > 0)
     fail("wave: snapshots carry u and v only; a model with relaxation checkpoints through "
          "wfx_wave_get_relaxation_state");
+  if (w->pml && fn && every > 0)
+    fail("wave: snapshots carry u and v only; a model with a perfectly matched layer checkpoints through "
+         "wfx_wave_get_pml_state");
   ScopedDevice sd(w->ctx->device);
   flush_snapshot(w);
   w->snap_every = fn ? every : 0;

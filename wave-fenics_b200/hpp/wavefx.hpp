@@ -357,6 +357,13 @@ inline void check_medium(const SpaceView& V, const Medium& m)
     throw std::runtime_error("wavefx: medium needs stiffness and mass weights per cell and a weight per facet");
 }
 
+// A perfectly matched layer (DESIGN.md section 4.5g) as its damping profile, e.g. the Python PML.zeta:
+//   zeta [3][ndofs]  >= 0 [1/s] along physical axis j; the layer is the cells where some zeta_j > 0 at a point
+struct PML
+{
+  std::vector<double> zeta;
+};
+
 // The wave model and its RK4 driver (common/LinearGLL.hpp:37-287), fp64 like the reference.
 class LinearGLLOpt
 {
@@ -365,7 +372,7 @@ public:
   LinearGLLOpt(std::shared_ptr<Context> ctx, const SpaceView& V, int& degreeOfBasis, double& speedOfSound,
                double& sourceFrequency, double& pressureAmplitude,
                std::shared_ptr<VectorUpdater<double>> halo = nullptr, const HaloSpec* spec = nullptr)
-      : _ctx(std::move(ctx)), _halo(std::move(halo)), _ndofs(V.ndofs)
+      : _ctx(std::move(ctx)), _halo(std::move(halo)), _ndofs(V.ndofs), _nq((std::int64_t)(V.degree + 1) * (V.degree + 1) * (V.degree + 1))
   {
     std::vector<std::int32_t> shared;
     if (spec)
@@ -385,7 +392,7 @@ public:
   // the same model in a layered medium (one rank)
   LinearGLLOpt(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
                double sourceFrequency, double pressureAmplitude, const Medium& medium)
-      : _ctx(std::move(ctx)), _ndofs(V.ndofs)
+      : _ctx(std::move(ctx)), _ndofs(V.ndofs), _nq((std::int64_t)(V.degree + 1) * (V.degree + 1) * (V.degree + 1))
   {
     make_operators(V, degreeOfBasis, speedOfSound, &medium);
     check(wfx_wave_create(_ctx->get(), stiff_op->get(), mass_op->get(), _bnd, nullptr, V.size_local, speedOfSound,
@@ -394,6 +401,7 @@ public:
   ~LinearGLLOpt()
   {
     wfx_wave_destroy(_wave);
+    wfx_pml_destroy(_pml);
     wfx_boundary_destroy(_bnd);
   }
   LinearGLLOpt(const LinearGLLOpt&) = delete;
@@ -467,6 +475,43 @@ public:
     check(wfx_wave_get_state(_wave, u_n.data(), v_n.data()));
   }
 
+  // perfectly matched layer (wavefx.h wfx_wave_set_pml, one rank): the layer of pml.zeta, built on the model's own
+  // geometry from V (the space the model was made on); an empty zeta removes it.  psi and phi start at 0, as after
+  // init and set_state.
+  void set_pml(const SpaceView& V, const PML& pml)
+  {
+    if (!pml.zeta.empty() && (std::int64_t)pml.zeta.size() != 3 * _ndofs)
+      throw std::runtime_error("wavefx: pml zeta needs 3 * ndofs entries");
+    check(wfx_wave_set_pml(_wave, nullptr));
+    wfx_pml_destroy(_pml);
+    _pml = nullptr;
+    _pml_cells = _pml_dofs = 0;
+    if (pml.zeta.empty()) return;
+    wfx_pml* h = nullptr;
+    check(wfx_pml_create(_ctx->get(), _geom->get(), V.ndofs, V.dofmap, V.npoints, V.x, V.xdofs, pml.zeta.data(), &h));
+    if (wfx_wave_set_pml(_wave, h))
+    {
+      wfx_pml_destroy(h);
+      check(1);
+    }
+    _pml = h;
+    check(wfx_pml_info(_pml, &_pml_cells, &_pml_dofs, nullptr));
+  }
+  // the layer's psi [layer dofs] and phi [layer cells][(P+1)^3][3] for checkpoints: get after solution(), set after
+  // set_state()
+  void pml_state(std::vector<double>& psi, std::vector<double>& phi) const
+  {
+    psi.resize((std::size_t)_pml_dofs);
+    phi.resize((std::size_t)_pml_cells * _nq * 3);
+    check(wfx_wave_get_pml_state(_wave, psi.data(), phi.data()));
+  }
+  void set_pml_state(const std::vector<double>& psi, const std::vector<double>& phi)
+  {
+    if ((std::int64_t)psi.size() != _pml_dofs || (std::int64_t)phi.size() != _pml_cells * _nq * 3)
+      throw std::runtime_error("wavefx: pml state needs psi [layer dofs] and phi [layer cells][nq][3]");
+    check(wfx_wave_set_pml_state(_wave, psi.data(), phi.data()));
+  }
+
   std::shared_ptr<MassOperator<double>> mass_op;
   std::shared_ptr<StiffnessOperator<double>> stiff_op;
   // the C handle, e.g. for PennesGLL::heat_from_wave
@@ -478,7 +523,7 @@ protected:
   LinearGLLOpt(std::shared_ptr<Context> ctx, const SpaceView& V, int degreeOfBasis, double speedOfSound,
                double sourceFrequency, double pressureAmplitude, double delta, double beta, double rho0,
                const Medium* medium = nullptr)
-      : _ctx(std::move(ctx)), _ndofs(V.ndofs)
+      : _ctx(std::move(ctx)), _ndofs(V.ndofs), _nq((std::int64_t)(V.degree + 1) * (V.degree + 1) * (V.degree + 1))
   {
     make_operators(V, degreeOfBasis, speedOfSound, medium);
     check(wfx_wave_create_westervelt(_ctx->get(), stiff_op->get(), mass_op->get(), _bnd, V.size_local, speedOfSound,
@@ -517,6 +562,8 @@ private:
   std::int64_t _ndofs;
   wfx_boundary* _bnd = nullptr;
   wfx_wave* _wave = nullptr;
+  wfx_pml* _pml = nullptr;
+  std::int64_t _pml_cells = 0, _pml_dofs = 0, _nq = 0;
 };
 // The Westervelt model, one rank, fp64, with the interface of LinearGLLOpt (wavefx.h, DESIGN.md section 4.5a):
 //   (1 - kappa p) p_tt - c0^2 lap p - delta lap p_t = kappa p_t^2,  kappa = 2 beta / (rho0 c0^2),

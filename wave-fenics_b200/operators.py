@@ -14,6 +14,8 @@ Same names, argument meaning and call shape as the reference classes:
                                                 the `medium=` keyword of every wave model, DESIGN.md 4.5e
   Relaxation(tau, eps, c), Medium.relaxation   power-law absorption by relaxation processes, the `relaxation=`
                                                 keyword of LossyGLLOpt / WesterveltGLLOpt, DESIGN.md 4.5f
+  PML(mesh, zeta), PML.box                      perfectly matched layers, the `pml=` keyword of the single-field
+                                                wave models, DESIGN.md 4.5g
 
 `V` is a HexMesh (mesh.py): it carries what the reference pulls out of the DOLFINx
 FunctionSpace (geometry, geometry dofmap, cell dofmap, index-map sizes).  Vectors are
@@ -374,6 +376,11 @@ def focus_delays(points, focus, c0):
     return (d.max() - d) / float(c0) if len(d) else d
 
 
+def _refuse_pml(pml):
+    if pml is not None:
+        raise capi.WfxError("pml: ensemble models are not supported (LinearGLLOpt, LossyGLLOpt, WesterveltGLLOpt)")
+
+
 def _refuse_relaxation(relaxation):
     if relaxation is not None:
         raise capi.WfxError("relaxation: needs LossyGLLOpt or WesterveltGLLOpt (for linear tissue, LossyGLLOpt with "
@@ -388,8 +395,10 @@ class LinearGLLOpt:
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency,
                  pressureAmplitude, dtype=np.float64, ctx=None, halo=None, stiffness_mode=capi.STIFF_AUTO,
-                 setup_halo=None, medium=None, relaxation=None):
+                 setup_halo=None, medium=None, relaxation=None, pml=None):
         _refuse_relaxation(relaxation)
+        if pml is not None and halo is not None:
+            raise capi.WfxError("pml: distributed models are not supported (one rank only)")
         self.ctx = ctx or Context.get()
         self.V = mesh
         if meshtags is not None:
@@ -427,6 +436,9 @@ class LinearGLLOpt:
                   self.bnd_op.handle, halo.handle if halo is not None else None, int(mesh.size_local),
                   self.c0_, self.freq0_, self.p0_, C.byref(self.handle))
         self.ndofs = int(mesh.ndofs)
+        self.pml = None
+        if pml is not None:
+            self.set_pml(pml)
 
     def _medium_geometry(self, mesh, medium):
         """The model's geometry, scaled by the medium's stiffness weight, and the medium's mass and facet weights
@@ -554,10 +566,77 @@ class LinearGLLOpt:
                   int(max_steps), C.byref(steps), C.byref(t_end), stream if stream is not None else _stream_ptr())
         return steps.value, t_end.value
 
+    def set_pml(self, pml=None):
+        """A perfectly matched layer (DESIGN.md section 4.5g): a PML built on this model's mesh, whose layer is then
+        built on the device on the model's own geometry (so a medium's stiffness weight reaches it); None removes it.
+        Model configuration: it survives init, set_state and restarts.  psi and phi start at 0 here, at init and at
+        set_state; a checkpoint restores them with set_pml_state after set_state.  rk4 then refuses steps of
+        PML.max_dt and above; snapshots are refused (they carry u and v only)."""
+        if pml is not None:
+            if not isinstance(pml, PML):
+                raise capi.WfxError("pml must be a PML")
+            if pml.zeta.shape != (3, self.ndofs):
+                raise capi.WfxError(f"pml: the profile has {pml.zeta.shape[1]} dofs, the model {self.ndofs}")
+        capi.call("wfx_wave_set_pml", self.handle, None)
+        self._destroy_pml()
+        self.pml = None
+        if pml is None:
+            return
+        V = self.V
+        x = np.ascontiguousarray(V.x, dtype=np.float64)
+        h = C.c_void_p()
+        capi.call("wfx_pml_create", self.ctx.handle, self.geometry.handle, self.ndofs,
+                  capi.i32p(np.ascontiguousarray(V.dofmap, dtype=np.int32).reshape(-1)), x.shape[0],
+                  capi.f64p(x.reshape(-1)), capi.i32p(np.ascontiguousarray(V.xdofs, dtype=np.int32).reshape(-1)),
+                  capi.f64p(pml.zeta.reshape(-1)), C.byref(h))
+        try:
+            capi.call("wfx_wave_set_pml", self.handle, h)
+        except capi.WfxError:
+            capi.lib.wfx_pml_destroy(h)
+            raise
+        self._pml_handle = h
+        self.pml = pml
+
+    def pml_info(self):
+        """dict(cells, dofs, zeta_max) of the model's layer (the cells where zeta > 0 at a point, their dofs)"""
+        if self.pml is None:
+            raise capi.WfxError("pml: the model has no perfectly matched layer (set_pml)")
+        nc, nd, zm = C.c_int64(), C.c_int64(), C.c_double()
+        capi.call("wfx_pml_info", self._pml_handle, C.byref(nc), C.byref(nd), C.byref(zm))
+        return dict(cells=nc.value, dofs=nd.value, zeta_max=zm.value)
+
+    def _pml_shapes(self):
+        info = self.pml_info()
+        return (info["dofs"],), (info["cells"], (self.k_ + 1) ** 3, 3)
+
+    def pml_state(self):
+        """(psi [layer dofs], phi [layer cells, (P+1)^3, 3]) in the model dtype; the layer's dofs ascending, its cells
+        in mesh order, points in the tensor order of the reference's dof permutation"""
+        sp, sf = self._pml_shapes()
+        psi, phi = np.empty(sp, dtype=self.dtype), np.empty(sf, dtype=self.dtype)
+        capi.call("wfx_wave_get_pml_state", self.handle, C.c_void_p(psi.ctypes.data), C.c_void_p(phi.ctypes.data))
+        return psi, phi
+
+    def set_pml_state(self, psi, phi):
+        """psi, phi of a checkpoint (after set_state, which zeroes them), shaped as pml_state returns them"""
+        sp, sf = self._pml_shapes()
+        psi = np.ascontiguousarray(psi, dtype=self.dtype)
+        phi = np.ascontiguousarray(phi, dtype=self.dtype)
+        if psi.shape != sp or phi.shape != sf:
+            raise capi.WfxError(f"pml state must have shapes {sp} and {sf}")
+        capi.call("wfx_wave_set_pml_state", self.handle, C.c_void_p(psi.ctypes.data), C.c_void_p(phi.ctypes.data))
+
+    def _destroy_pml(self):
+        h = getattr(self, "_pml_handle", None)
+        if h and getattr(capi, "lib", None) is not None:
+            capi.lib.wfx_pml_destroy(h)
+        self._pml_handle = None
+
     def __del__(self):
         if getattr(self, "handle", None) and getattr(capi, "lib", None) is not None:
             capi.lib.wfx_wave_destroy(self.handle)
             self.handle = None
+        self._destroy_pml()
 
 
 class LinearGLLEnsemble(LinearGLLOpt):
@@ -568,8 +647,9 @@ class LinearGLLEnsemble(LinearGLLOpt):
     available for ensembles."""
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequencies, pressureAmplitudes,
-                 dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO, medium=None, relaxation=None):
+                 dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO, medium=None, relaxation=None, pml=None):
         _refuse_relaxation(relaxation)
+        _refuse_pml(pml)
         self.ctx = ctx or Context.get()
         self.V = mesh
         if meshtags is not None:
@@ -628,6 +708,9 @@ class LinearGLLEnsemble(LinearGLLOpt):
     def set_snapshot(self, every, fn):
         capi.call("wfx_wave_set_snapshot", self.handle, int(every), None, None)
 
+    def set_pml(self, pml=None):
+        _refuse_pml(pml)
+
 
 class WesterveltGLLOpt(LinearGLLOpt):
     """The Westervelt model on one rank, with the surface of LinearGLLOpt (DESIGN.md section 4.5a):
@@ -640,11 +723,11 @@ class WesterveltGLLOpt(LinearGLLOpt):
     multiplies the delta term too (delta_eff = delta * coeff).  With a Medium the nonlinearity is per dof
     (set_nonlinearity), from the medium's beta, which defaults to coefficientOfNonlinearity; delta_eff = delta
     (c / c0)^2 (DESIGN.md section 4.5e).  relaxation: a Relaxation (power-law absorption, DESIGN.md section 4.5f),
-    see set_relaxation."""
+    see set_relaxation.  pml: a PML (perfectly matched layer, DESIGN.md section 4.5g), see set_pml."""
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
                  diffusivityOfSound, coefficientOfNonlinearity, density, dtype=np.float64, ctx=None,
-                 stiffness_mode=capi.STIFF_AUTO, medium=None, relaxation=None):
+                 stiffness_mode=capi.STIFF_AUTO, medium=None, relaxation=None, pml=None):
         self.ctx = ctx or Context.get()
         self.V = mesh
         if meshtags is not None:
@@ -677,6 +760,9 @@ class WesterveltGLLOpt(LinearGLLOpt):
         self.relaxation = None
         if relaxation is not None:
             self.set_relaxation(relaxation)
+        self.pml = None
+        if pml is not None:
+            self.set_pml(pml)
 
     def set_nonlinearity(self, kappa=None):
         """kappa [ndofs] >= 0: a per-dof kappa in place of 2 beta / (rho0 c0^2) (the model then steps the nonlinear
@@ -731,10 +817,10 @@ class LossyGLLOpt(WesterveltGLLOpt):
 
     def __init__(self, mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
                  diffusivityOfSound, dtype=np.float64, ctx=None, stiffness_mode=capi.STIFF_AUTO, medium=None,
-                 relaxation=None):
+                 relaxation=None, pml=None):
         super().__init__(mesh, meshtags, degreeOfBasis, speedOfSound, sourceFrequency, pressureAmplitude,
                          diffusivityOfSound, 0.0, 1.0, dtype=dtype, ctx=ctx, stiffness_mode=stiffness_mode,
-                         medium=medium, relaxation=relaxation)
+                         medium=medium, relaxation=relaxation, pml=pml)
 
 
 # dose of a thermal model (PennesGLL.dose): steps since init / set_state, CEM43 [min] and peak temperature per dof
@@ -980,6 +1066,64 @@ class Relaxation:
         e = self.eps_cells(mesh.ncells)
         return np.ascontiguousarray(np.stack([_shared_exact_average(mesh, detJw, e[j], mass_weight)
                                               for j in range(self.M)]))
+
+
+class PML:
+    """A perfectly matched layer (DESIGN.md section 4.5g): damping profiles zeta [3, ndofs] >= 0 [1/s], zeta[j] along
+    physical axis j, on the dofs of `mesh`.  The layer is the cells where some zeta_j > 0 at one of their points; a
+    wave model given it (`pml=`, set_pml) stretches its stiffness term there with the second-order PML of Grote and
+    Sim (2010).  The Westervelt and relaxation terms are not stretched: the layer reflects O(kappa p) and O(eps)."""
+
+    def __init__(self, mesh, zeta):
+        z = np.array(zeta, dtype=np.float64)
+        if z.shape != (3, mesh.ndofs):
+            raise capi.WfxError(f"pml: zeta must have shape (3, {mesh.ndofs})")
+        if not np.all(np.isfinite(z)) or np.any(z < 0):
+            raise capi.WfxError("pml: zeta must be finite and not negative")
+        self.zeta = np.ascontiguousarray(z)
+
+    @classmethod
+    def box(cls, mesh, thickness, faces, c, R0=1e-4, order=2):
+        """A layer `thickness` deep inside the mesh from each named face (axis 0..2, side 0 (low) or 1 (high)) of the
+        bounding box of the dof coordinates: zeta_j = zeta_max (d_j / L)^order at depth d_j into a layer on axis j,
+        zeta_max = (order + 1) c ln(1 / R0) / (2 L), the normal-incidence reflection R0 of the continuous layer with a
+        rigid end for waves of speed c.  Edges and corners get two or three nonzero zeta_j."""
+        from .mesh import dof_coordinates
+        L = float(thickness)
+        if not (np.isfinite(L) and L > 0):
+            raise capi.WfxError("pml: thickness must be finite and positive")
+        if not (np.isfinite(c) and c > 0):
+            raise capi.WfxError("pml: c must be finite and positive")
+        if not (0 < R0 < 1):
+            raise capi.WfxError("pml: R0 must lie in (0, 1)")
+        if not (np.isfinite(order) and order >= 0):
+            raise capi.WfxError("pml: order must be finite and not negative")
+        faces = [tuple(int(v) for v in f) for f in faces]
+        if not faces or any(len(f) != 2 or f[0] not in (0, 1, 2) or f[1] not in (0, 1) for f in faces) \
+                or len(set(faces)) != len(faces):
+            raise capi.WfxError("pml: faces must be distinct (axis 0..2, side 0 or 1) pairs")
+        x = dof_coordinates(mesh)
+        lo, hi = x.min(axis=0), x.max(axis=0)
+        zmax = (order + 1) * float(c) * np.log(1.0 / R0) / (2.0 * L)
+        zeta = np.zeros((3, mesh.ndofs))
+        for axis, side in faces:
+            sides = sum(1 for a, _ in faces if a == axis)
+            if sides * L > hi[axis] - lo[axis]:
+                raise capi.WfxError("pml: the layers are thicker than the mesh")
+            d = (lo[axis] + L - x[:, axis]) if side == 0 else (x[:, axis] - (hi[axis] - L))
+            d = np.clip(d, 0.0, L)
+            zeta[axis] = np.maximum(zeta[axis], zmax * (d / L) ** order * (d > 0))
+        return cls(mesh, zeta)
+
+    @property
+    def zeta_max(self):
+        return float(self.zeta.max()) if self.zeta.size else 0.0
+
+    def max_dt(self):
+        """The largest time step rk4 accepts with this layer: dt max zeta < 2.5 (a lone dof has the eigenvalues
+        -zeta_j; RK4 is stable on the real axis to 2.785)"""
+        zm = self.zeta_max
+        return 2.5 / zm if zm > 0 else np.inf
 
 
 class PennesGLL:
