@@ -35,6 +35,11 @@ reports the fit error and the phase speed at f0; the time step is also kept belo
 matched layer (DESIGN.md section 4.5g) WIDTH deep inside the domain (PML.box, R0 = 1e-4) with rigid outer faces, so
 that a focused beam's side lobes leave the domain instead of coming back into the maps; it prints the layer's cells,
 dofs and largest damping, and keeps the time step below the layer's bound.
+--time-reversal (with --focus and --stats-periods; linear or lossy model) focuses by time reversal (DESIGN.md section
+4.5h): an emission run from a point source at the focus with the array silent (profile amplitude 0), the first
+harmonic on tag 1 conjugated (phase_conjugate_delays), then a treatment run with those delays and one with the
+geometric delays of --focus.  It prints the focal |p1| (the point source's weights as a sensor) of both treatments and
+the reciprocity prediction of each from the emission, sum_i m1_i a_i exp(-i w tau_i) (1 + i w delta / c0^2) p1_i.
 The reference reads `../mesh.xdmf` (not in its repository); here the mesh is a structured
 n x m x m hexahedral box with tag 1 on x = 0 (source) and tag 2 on x = L (absorbing).
 
@@ -42,7 +47,7 @@ n x m x m hexahedral box with tag 1 on x = 0 (source) and tag 2 on x = L (absorb
                             [--model linear|lossy|westervelt] [--stats-periods K] [--focus DEPTH] [--aperture R]
                             [--heat-seconds S] [--cool-seconds C] [--absorption ALPHA0] [--absorption-power Y]
                             [--layer X0 X1 --layer-rho R --layer-c C [--layer-beta B]]
-                            [--relaxation M [--band F_LO F_HI]] [--pml WIDTH]
+                            [--relaxation M [--band F_LO F_HI]] [--pml WIDTH] [--time-reversal]
 """
 import argparse
 import os
@@ -101,7 +106,13 @@ def main():
                     help="with --relaxation: the fitted band [Hz] (default f0 / 2 .. 3 f0)")
     ap.add_argument("--pml", type=float, default=0.0, metavar="WIDTH",
                     help="a perfectly matched layer WIDTH [m] deep in place of the absorbing faces (0: off)")
+    ap.add_argument("--time-reversal", action="store_true",
+                    help="with --focus and --stats-periods: time-reversal delays from a point source at the focus")
     args = ap.parse_args()
+    if args.time_reversal and (args.focus <= 0 or args.stats_periods <= 0):
+        ap.error("--time-reversal needs --focus (the target) and --stats-periods (the harmonic maps)")
+    if args.time_reversal and (args.model == "westervelt" or args.check or args.heat_seconds > 0):
+        ap.error("--time-reversal needs a linear model (--model linear or lossy) and takes no --check or --heat-seconds")
     if args.pml < 0:
         ap.error("--pml WIDTH needs WIDTH > 0")
     if args.pml > 0 and args.check:
@@ -193,6 +204,12 @@ def main():
         eqn.set_source_profile(amp, delay)
         print(f"focused source: focus at x = {args.focus:.4f} on the face axis, "
               f"delays up to {delay.max():.4e} s, aperture {'whole face' if amp is None else args.aperture}")
+    if args.time_reversal:
+        k = int(round(period / timeStepSize))
+        window = stats_window(startTime, finalTime, timeStepSize, k, args.stats_periods, args.steps)
+        time_reversal(eqn, mesh, X, (args.focus, width / 2, width / 2), amp, delay, delta / speedOfSound ** 2,
+                      sourceFrequency, startTime, timeStepSize, window)
+        return
     eqn.init()                                                                   # :83
     run_tf, run_steps = finalTime, args.steps
     if args.stats_periods > 0:
@@ -261,6 +278,40 @@ def main():
                                         nthreads=oracle.max_threads())
         print(f"relative L2 difference to the CPU oracle: u {np.linalg.norm(u - uo) / np.linalg.norm(uo):.3e}"
               f"  v {np.linalg.norm(v - vo) / np.linalg.norm(vo):.3e}")
+
+
+def time_reversal(eqn, mesh, X, focus, amp, delay, s_src, f0, t0, dt, window):
+    """Emission from a point source at `focus` with the array silent, then treatments with the geometric delays and
+    with the conjugate delays of the emission's first harmonic on tag 1; prints each focal |p1| and its reciprocity
+    prediction from the emission (DESIGN.md section 4.5h)."""
+    run_tf, run_steps, t_start = window
+    fdofs, fq = wfx.point_source(mesh, focus)
+    m1 = eqn.bnd_op.facet_masses()[0]
+    face = m1 > 0
+    a = np.ones(mesh.ndofs) if amp is None else amp
+
+    def first_harmonic():
+        eqn.init()
+        eqn.set_field_stats(t_start, harmonics=1)
+        eqn.rk4(t0, run_tf, dt, max_steps=run_steps)
+        return eqn.field_stats().harmonics[0]
+
+    eqn.set_source_profile(np.zeros(mesh.ndofs))
+    eqn.set_volume_source(fdofs, fq)
+    emission = first_harmonic()
+    eqn.set_volume_source()
+    w = 2.0 * np.pi * f0
+    print(f"time reversal: emission from a point source at x = {focus[0]:.5f} ({len(fdofs)} dofs), "
+          f"|p1| on tag 1 up to {np.abs(emission[face]).max():.6e}")
+    conjugate = np.where(face, wfx.phase_conjugate_delays(emission, f0), 0.0)
+    focal = {}
+    for name, tau in (("geometric", delay), ("time-reversal", conjugate)):
+        eqn.set_source_profile(amp, tau)
+        focal[name] = fq @ first_harmonic()[fdofs]
+        pred = np.sum(m1 * a * np.exp(-1j * w * tau) * (1.0 + 1j * w * s_src) * emission)
+        print(f"time reversal: {name} delays: focal |p1| = {abs(focal[name]):.6e}, reciprocity prediction "
+              f"{abs(pred):.6e} (difference {abs(focal[name] - pred):.3e})")
+    print(f"time reversal: gain over the geometric delays {abs(focal['time-reversal']) / abs(focal['geometric']):.4f}")
 
 
 def heat(args, eqn, c0, medium=None, k=0.5, rhoc=3.6e6, perfusion=2.0e3, T_art=37.0):

@@ -479,6 +479,17 @@ int wfx_wave_field_stats_info(wfx_wave* wave, int* enabled, double* t_start, int
  * between rk4 calls.  Refused: a NULL model, a model without a boundary operator, a distributed model, a
  * non-finite amplitude or delay, a negative delay. */
 int wfx_wave_set_source_profile(wfx_wave* wave, const double* amp_host, const double* delay_host);
+/* Volume source (DESIGN.md section 4.5h): an additive pressure source on any dofs.  At every stage, after the
+ * boundary term and before the layer, Gamma2 and stage-quotient terms,
+ *   b[j,m] += c0^2 q[p,m] g_m(t - tau[p,m]),   j = dofs_host[p],   g_m(s) = 0 for s < 0,
+ * g_m the model's source of member m (its four-period ramp, f0 and p0; g only, also in the lossy / Westervelt models),
+ * evaluated on the device in fp64 for both model dtypes.  For a point source at x0, q_j = phi_j(x0).  dofs_host holds
+ * n distinct local dofs; q_host and delay_host hold n * nv entries [n][nv] (nv = 1 for a single field).  delay_host
+ * may be NULL (tau = 0); n = 0 clears the source.  Model configuration, like the profile: it survives init, set_state
+ * and restarts, and may be changed between rk4 calls.  Refused: a NULL model, a distributed model, a dof out of range,
+ * a duplicate dof, a non-finite weight or delay, a negative delay. */
+int wfx_wave_set_volume_source(wfx_wave* wave, int64_t n, const int32_t* dofs_host, const double* q_host,
+                               const double* delay_host);
 /* Snapshots / checkpoints: every `every` completed steps (counted since init / set_state) u and v are
  * copied device -> device on the stepping stream and device -> pinned host on a separate copy stream
  * while the time stepping continues; `fn` then receives host pointers valid for the duration of the

@@ -678,13 +678,23 @@ static void pml_terms(const pml_t* L, int P, int64_t ncells, int64_t ndofs, cons
   free(perm);
 }
 
-/* model_rhs_relax with the layer's terms tp added to the numerator (PML dofs) */
+/* A volume source (DESIGN.md section 4.5h): n distinct dofs with weights q and delays, the term
+ *   r_j += c0^2 q_j g(t - delay_j),   g of wo_source, g = 0 before the delay,
+ * added after the boundary term, before the layer's, kappa and relaxation terms.  NULL or n = 0: no term. */
+typedef struct
+{
+  int64_t n;
+  const int32_t* dofs;
+  const double *q, *delay;
+} vsrc_t;
+
+/* model_rhs_relax with the layer's terms tp added to the numerator (PML dofs), and a volume source S (nullable) */
 static void model_rhs_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
                           const double* m, const double* m1, const double* m2, const double* kappa, double c0,
                           double freq0, double p0, double delta, int M, const double* tau, const double* eps, double t,
                           const double* un, const double* vn, const double* qn, const pml_t* L, const double* psin,
-                          const double* phin, double* kv, double* kq, double* kpsi, double* kphi, double* tp, double* b,
-                          double* bv, int sumfact, int nthreads)
+                          const double* phin, const vsrc_t* S, double* kv, double* kq, double* kpsi, double* kphi,
+                          double* tp, double* b, double* bv, int sumfact, int nthreads)
 {
   const size_t nb = sizeof(double) * ndofs;
   const double s = delta / (1500.0 * 1500.0);
@@ -695,10 +705,23 @@ static void model_rhs_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* d
   model_stiffness(P, ncells, ndofs, dofmap, G, un, b, sumfact, nthreads);  /* A un */
   model_stiffness(P, ncells, ndofs, dofmap, G, vn, bv, sumfact, nthreads); /* A vn */
   if (L->ncells_pml) pml_terms(L, P, ncells, ndofs, dofmap, m, s, un, vn, psin, phin, tp, kpsi, kphi);
+  double* vs = NULL; /* the volume source's term at every dof, 0 off its dofs */
+  if (S && S->n > 0)
+  {
+    vs = calloc(ndofs, sizeof(double));
+    for (int64_t p = 0; p < S->n; ++p)
+    {
+      const double sp = t - S->delay[p];
+      double gs = 0.0, gsdot;
+      if (sp >= 0.0) wo_source(sp, freq0, p0, c0, &gs, &gsdot); /* g only: the term sits in the PDE */
+      vs[S->dofs[p]] = (c0 * c0 * gs) * S->q[p];
+    }
+  }
   for (int64_t k = 0; k < ndofs; ++k)
   {
     double r = b[k] + s * bv[k];
     r += (c0 * c0 * g + delta * gdot) * m1[k] - c0 * m2[k] * vn[k];
+    if (vs) r += vs[k];
     if (L->ncells_pml && L->dof_on[k]) r += tp[k];
     r += kappa[k] * m[k] * vn[k] * vn[k];
     if (M > 0)
@@ -714,15 +737,15 @@ static void model_rhs_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* d
     }
     kv[k] = r / (m[k] * (1.0 - kappa[k] * un[k]) + delta / c0 * m2[k]);
   }
+  free(vs);
 }
 
 /* dv/dt = f1(t, u, v; q, psi, phi) of the lossy / Westervelt model with relaxation and a perfectly matched layer */
-void wo_f1_westervelt_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G, const double* m,
-                          const double* m1, const double* m2, const double* kappa, double c0, double freq0, double p0,
-                          double delta, int M, const double* tau, const double* eps, const double* zeta,
-                          const double* K, const double* dJw, const double* coeff, double t, const double* u,
-                          const double* v, const double* q, const double* psi, const double* phi, double* out,
-                          int sumfact, int nthreads)
+static void f1_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G, const double* m,
+                   const double* m1, const double* m2, const double* kappa, double c0, double freq0, double p0,
+                   double delta, int M, const double* tau, const double* eps, const double* zeta, const double* K,
+                   const double* dJw, const double* coeff, const vsrc_t* S, double t, const double* u, const double* v,
+                   const double* q, const double* psi, const double* phi, double* out, int sumfact, int nthreads)
 {
   const int nd = (P + 1) * (P + 1) * (P + 1);
   const size_t nb = sizeof(double) * ndofs, nphi = sizeof(double) * (ncells * nd * 3 + 1);
@@ -731,19 +754,19 @@ void wo_f1_westervelt_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* d
   pml_t L;
   pml_setup(&L, P, ncells, ndofs, dofmap, zeta, K, dJw, coeff);
   model_rhs_pml(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, M, tau, eps, t, u, v, q, &L, psi,
-                phi, out, kq, kpsi, kphi, tp, b, bv, sumfact, nthreads);
+                phi, S, out, kq, kpsi, kphi, tp, b, bv, sumfact, nthreads);
   pml_free(&L);
   free(b); free(bv); free(kq); free(tp); free(kpsi); free(kphi);
 }
 
 /* wo_rk4_westervelt_relax with a perfectly matched layer: psi [ndofs] and phi [ncells][nq][3] (in / out) are stepped
  * by the same tableau as u, v and q */
-int64_t wo_rk4_westervelt_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
-                              const double* m, const double* m1, const double* m2, const double* kappa, double c0,
-                              double freq0, double p0, double delta, int M, const double* tau, const double* eps,
-                              const double* zeta, const double* K, const double* dJw, const double* coeff, double t0,
-                              double tf, double dt, int64_t max_steps, double* u_n, double* v_n, double* q_n,
-                              double* psi_n, double* phi_n, int sumfact, int nthreads, double* t_end)
+static int64_t rk4_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G, const double* m,
+                       const double* m1, const double* m2, const double* kappa, double c0, double freq0, double p0,
+                       double delta, int M, const double* tau, const double* eps, const double* zeta, const double* K,
+                       const double* dJw, const double* coeff, const vsrc_t* S, double t0, double tf, double dt,
+                       int64_t max_steps, double* u_n, double* v_n, double* q_n, double* psi_n, double* phi_n,
+                       int sumfact, int nthreads, double* t_end)
 {
   const double a_runge[4] = {0.0, 0.5, 0.5, 1.0};
   const double b_runge[4] = {1.0 / 6.0, 1.0 / 3.0, 1.0 / 3.0, 1.0 / 6.0};
@@ -804,7 +827,7 @@ int64_t wo_rk4_westervelt_pml(int P, int64_t ncells, int64_t ndofs, const int32_
       const double tn = t + c_runge[i] * dt;
       memcpy(ku, vn, nb);
       model_rhs_pml(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, M, tau, eps, tn, un, vn, qn, &L,
-                    psn, phn, kv, kq, kps, kph, tp, b, bv, sumfact, nthreads);
+                    psn, phn, S, kv, kq, kps, kph, tp, b, bv, sumfact, nthreads);
       const double bdt = dt * b_runge[i];
       for (int64_t k = 0; k < ndofs; ++k) u_[k] = ku[k] * bdt + u_[k];
       for (int64_t k = 0; k < ndofs; ++k) v_[k] = kv[k] * bdt + v_[k];
@@ -833,4 +856,55 @@ int64_t wo_rk4_westervelt_pml(int P, int64_t ncells, int64_t ndofs, const int32_
   free(ps_); free(psn); free(ps0); free(kps); free(tp);
   free(ph_); free(phn); free(ph0); free(kph);
   return step;
+}
+
+void wo_f1_westervelt_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G, const double* m,
+                          const double* m1, const double* m2, const double* kappa, double c0, double freq0, double p0,
+                          double delta, int M, const double* tau, const double* eps, const double* zeta,
+                          const double* K, const double* dJw, const double* coeff, double t, const double* u,
+                          const double* v, const double* q, const double* psi, const double* phi, double* out,
+                          int sumfact, int nthreads)
+{
+  f1_pml(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, M, tau, eps, zeta, K, dJw, coeff, NULL, t,
+         u, v, q, psi, phi, out, sumfact, nthreads);
+}
+
+int64_t wo_rk4_westervelt_pml(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                              const double* m, const double* m1, const double* m2, const double* kappa, double c0,
+                              double freq0, double p0, double delta, int M, const double* tau, const double* eps,
+                              const double* zeta, const double* K, const double* dJw, const double* coeff, double t0,
+                              double tf, double dt, int64_t max_steps, double* u_n, double* v_n, double* q_n,
+                              double* psi_n, double* phi_n, int sumfact, int nthreads, double* t_end)
+{
+  return rk4_pml(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, M, tau, eps, zeta, K, dJw, coeff,
+                 NULL, t0, tf, dt, max_steps, u_n, v_n, q_n, psi_n, phi_n, sumfact, nthreads, t_end);
+}
+
+/* ---- volume sources (DESIGN.md section 4.5h) ------------------------------------------------------------------
+ * wo_f1 / wo_rk4_westervelt_pml with a volume source: ns distinct dofs sdofs [ns], weights sq [ns] and delays
+ * sdelay [ns] (see vsrc_t).  With ns = 0 they compute what wo_f1 / wo_rk4_westervelt_pml compute, bit for bit. */
+void wo_f1_westervelt_source(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                             const double* m, const double* m1, const double* m2, const double* kappa, double c0,
+                             double freq0, double p0, double delta, int M, const double* tau, const double* eps,
+                             const double* zeta, const double* K, const double* dJw, const double* coeff, int64_t ns,
+                             const int32_t* sdofs, const double* sq, const double* sdelay, double t, const double* u,
+                             const double* v, const double* q, const double* psi, const double* phi, double* out,
+                             int sumfact, int nthreads)
+{
+  const vsrc_t S = {ns, sdofs, sq, sdelay};
+  f1_pml(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, M, tau, eps, zeta, K, dJw, coeff, &S, t,
+         u, v, q, psi, phi, out, sumfact, nthreads);
+}
+
+int64_t wo_rk4_westervelt_source(int P, int64_t ncells, int64_t ndofs, const int32_t* dofmap, const double* G,
+                                 const double* m, const double* m1, const double* m2, const double* kappa, double c0,
+                                 double freq0, double p0, double delta, int M, const double* tau, const double* eps,
+                                 const double* zeta, const double* K, const double* dJw, const double* coeff,
+                                 int64_t ns, const int32_t* sdofs, const double* sq, const double* sdelay, double t0,
+                                 double tf, double dt, int64_t max_steps, double* u_n, double* v_n, double* q_n,
+                                 double* psi_n, double* phi_n, int sumfact, int nthreads, double* t_end)
+{
+  const vsrc_t S = {ns, sdofs, sq, sdelay};
+  return rk4_pml(P, ncells, ndofs, dofmap, G, m, m1, m2, kappa, c0, freq0, p0, delta, M, tau, eps, zeta, K, dJw, coeff,
+                 &S, t0, tf, dt, max_steps, u_n, v_n, q_n, psi_n, phi_n, sumfact, nthreads, t_end);
 }

@@ -99,6 +99,14 @@ def lib():
         L.wo_rk4_westervelt_pml.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, i, _f64p,
                                             _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, l, _f64p, _f64p, _f64p, _f64p,
                                             _f64p, i, i, _f64p]
+        L.wo_f1_westervelt_source.restype = None
+        L.wo_f1_westervelt_source.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, i, _f64p,
+                                              _f64p, _f64p, _f64p, _f64p, _f64p, l, _i32p, _f64p, _f64p, d, _f64p,
+                                              _f64p, _f64p, _f64p, _f64p, _f64p, i, i]
+        L.wo_rk4_westervelt_source.restype = l
+        L.wo_rk4_westervelt_source.argtypes = [i, l, l, _i32p, _f64p, _f64p, _f64p, _f64p, _f64p, d, d, d, d, i, _f64p,
+                                               _f64p, _f64p, _f64p, _f64p, _f64p, l, _i32p, _f64p, _f64p, d, d, d, l,
+                                               _f64p, _f64p, _f64p, _f64p, _f64p, i, i, _f64p]
         _lib.append(L)
     return _lib[0]
 
@@ -338,4 +346,50 @@ def rk4_westervelt_pml(mesh, P, G, m, m1, m2, kappa, c0, f0, p0, delta, tau, eps
                                         _f(m), _f(m1), _f(m2), _f(kappa), c0, f0, p0, delta, M, tp, ep, *pml.args(),
                                         t0, tf, dt, max_steps, _f(u), _f(v), qp, _f(psi), _f(phi.reshape(-1)),
                                         int(sumfact), nthreads, C.byref(t_end))
+    return steps, t_end.value
+
+
+# ---- volume sources (DESIGN.md section 4.5h) -----------------------------------------------------------------------
+def _vsrc(dofs, q, delay):
+    dofs = np.ascontiguousarray(np.zeros(0) if dofs is None else dofs, dtype=np.int32).reshape(-1)
+    q = np.ascontiguousarray(np.zeros(0) if q is None else q, dtype=np.float64).reshape(-1)
+    delay = np.zeros(len(dofs)) if delay is None else np.ascontiguousarray(delay, dtype=np.float64).reshape(-1)
+    assert len(dofs) == len(q) == len(delay)
+    return len(dofs), dofs.ctypes.data_as(_i32p), _f(q), _f(delay), (dofs, q, delay)
+
+
+def f1_westervelt_source(mesh, P, G, m, m1, m2, kappa, c0, f0, p0, delta, tau, eps, pml, dofs, q_src, delay, t, u, v,
+                         q=None, psi=None, phi=None, sumfact=False, nthreads=1):
+    """f1_westervelt_pml with a volume source: c0^2 q_src[p] g(t - delay[p]) added at dof dofs[p] (delay None: 0)"""
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    M, tp, ep, _, qp = _relax(mesh, tau, eps, q)
+    z_psi, z_phi = pml_state(mesh, P)
+    psi = z_psi if psi is None else np.ascontiguousarray(psi, dtype=np.float64)
+    phi = z_phi if phi is None else np.ascontiguousarray(phi, dtype=np.float64)
+    ns, sd, sq, sl, _keep = _vsrc(dofs, q_src, delay)
+    out = np.empty(mesh.ndofs)
+    lib().wo_f1_westervelt_source(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)), _f(m),
+                                  _f(m1), _f(m2), _f(np.ascontiguousarray(kappa, dtype=np.float64)), c0, f0, p0, delta,
+                                  M, tp, ep, *pml.args(), ns, sd, sq, sl, t, _f(u), _f(v), qp, _f(psi),
+                                  _f(phi.reshape(-1)), _f(out), int(sumfact), nthreads)
+    return out
+
+
+def rk4_westervelt_source(mesh, P, G, m, m1, m2, kappa, c0, f0, p0, delta, tau, eps, pml, dofs, q_src, delay, t0, tf,
+                          dt, u, v, q, psi, phi, max_steps=0, sumfact=False, nthreads=1):
+    """rk4_westervelt_pml with a volume source (see f1_westervelt_source); u, v, q, psi and phi updated in place.
+    -> (steps, t_end)"""
+    dm = np.ascontiguousarray(mesh.dofmap, dtype=np.int32)
+    kappa = np.ascontiguousarray(kappa, dtype=np.float64)
+    assert kappa.shape == (mesh.ndofs,)
+    M, tp, ep, q, qp = _relax(mesh, tau, eps, q)
+    for a in (psi, phi):
+        assert a.dtype == np.float64 and a.flags["C_CONTIGUOUS"]
+    assert psi.shape == (mesh.ndofs,) and phi.shape == (mesh.ncells, (P + 1) ** 3, 3)
+    ns, sd, sq, sl, _keep = _vsrc(dofs, q_src, delay)
+    t_end = C.c_double()
+    steps = lib().wo_rk4_westervelt_source(P, mesh.ncells, mesh.ndofs, dm.ctypes.data_as(_i32p), _f(G.reshape(-1)),
+                                           _f(m), _f(m1), _f(m2), _f(kappa), c0, f0, p0, delta, M, tp, ep, *pml.args(),
+                                           ns, sd, sq, sl, t0, tf, dt, max_steps, _f(u), _f(v), qp, _f(psi),
+                                           _f(phi.reshape(-1)), int(sumfact), nthreads, C.byref(t_end))
     return steps, t_end.value

@@ -9,4 +9,5 @@ from .capi import WfxError  # noqa: F401
 from .mesh import HexMesh, create_box_hex, cfl_timestep, dof_coordinates  # noqa: F401
 from .operators import (BoundaryOperator, Context, FieldStats, Geometry, LinearGLLEnsemble, LinearGLLOpt,  # noqa: F401
                         LossyGLLOpt, MassOperator, MassOperatorCPU, Medium, PML, PennesGLL, Relaxation,
-                        StiffnessOperator, ThermalDose, WesterveltGLLOpt, cell_to_dof_average, compute_jacobian_data, focus_delays)
+                        StiffnessOperator, ThermalDose, WesterveltGLLOpt, cell_to_dof_average, compute_jacobian_data, focus_delays,
+                        phase_conjugate_delays, point_source)

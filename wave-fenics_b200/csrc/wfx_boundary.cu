@@ -94,6 +94,31 @@ boundary_profile_kernel(int64_t nb, int nv, const int32_t* __restrict__ idx, con
   b[i] = (T)((double)b[i] + __dmul_rn(c0 * c0, src) * m1p - c0 * m2[p] * (double)vn[i]);
 }
 
+// A volume source (section 4.5h) on nv member-interleaved fields (nv = 1: one field), one thread per (source dof p,
+// member m), compact entry t = p nv + m:
+//   b[i,m] += c0^2 q_t g_m(tn - tau_t),   i = idx[p],   g_m = 0 before tau_t,
+// g_m member m's source evaluated in fp64 by source_eval for every scalar type (g only: the term sits in the PDE, not
+// in Neumann data on w = p + s p_t).  The stage time tn comes by value or, in graph replays, from t_dev.  The dofs are
+// distinct, so each entry writes its b once without atomics; q = 0 and entries before their delay leave b untouched.
+template <typename T>
+__global__ void __launch_bounds__(256)
+volume_source_kernel(int64_t ns, int nv, const int32_t* __restrict__ idx, const double* __restrict__ q,
+                     const double* __restrict__ delay, double c0, const __grid_constant__ SourceParams sp,
+                     double t_host, const double* __restrict__ t_dev, T* __restrict__ b)
+{
+  const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  if (t >= ns * nv) return;
+  const double qt = q[t];
+  if (qt == 0.0) return;
+  const double s = (t_dev ? *t_dev : t_host) - delay[t];
+  if (s < 0.0) return;
+  const int m = (int)(t % nv);
+  double g, gdot;
+  source_eval(sp.f0[m], sp.p0[m], c0, s, &g, &gdot);
+  const int64_t i = (int64_t)idx[t / nv] * nv + m;
+  b[i] = (T)((double)b[i] + __dmul_rn(c0 * c0, g) * qt);
+}
+
 // Lossy / Westervelt models: the Gamma2 mass term q = qc m2 on the absorbing dofs only, so that the dense
 // stage update needs nothing beyond 1/m (see boundary_absorbing_mass in wfx_internal.h).  p is formed in T
 // exactly as the stage kernel forms it.  KD: a per-dof kappa (wfx_wave_set_nonlinearity), read in fp64 from kd, compact
@@ -217,6 +242,20 @@ void wfx::boundary_apply_profile(wfx_boundary* op, int nv, double c0, double s_s
     boundary_profile_kernel<float><<<grid, 256, 0, stream>>>(op->nb, nv, op->d_idx.p, op->d_m1.p, op->d_m2.p, c0,
                                                               s_src, sp, t_host, t_dev, amp, delay,
                                                               (const float*)vn, (float*)b);
+  WFX_CUDA(cudaGetLastError());
+}
+
+void wfx::volume_source_apply(int dtype, int64_t ns, int nv, const int32_t* idx, const double* q, const double* delay,
+                              double c0, const SourceParams& sp, double t_host, const double* t_dev, void* b,
+                              cudaStream_t stream)
+{
+  if (ns == 0) return;
+  if (nv < 1 || nv > WFX_ENSEMBLE_MAX) fail("volume source: nv = %d outside [1, %d]", nv, WFX_ENSEMBLE_MAX);
+  const unsigned grid = (unsigned)((ns * nv + 255) / 256);
+  if (dtype == WFX_F64)
+    volume_source_kernel<double><<<grid, 256, 0, stream>>>(ns, nv, idx, q, delay, c0, sp, t_host, t_dev, (double*)b);
+  else
+    volume_source_kernel<float><<<grid, 256, 0, stream>>>(ns, nv, idx, q, delay, c0, sp, t_host, t_dev, (float*)b);
   WFX_CUDA(cudaGetLastError());
 }
 

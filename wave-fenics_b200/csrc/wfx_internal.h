@@ -133,6 +133,13 @@ const std::vector<int32_t>& boundary_dofs(const struct ::wfx_boundary* op);
 void boundary_apply_profile(struct ::wfx_boundary* op, int nv, double c0, double s_src, const SourceParams& sp,
                             double t_host, const double* t_dev, const double* amp, const double* delay,
                             const void* vn, void* b, cudaStream_t stream);
+// volume sources (wfx_wave_set_volume_source, DESIGN.md section 4.5h): ns distinct dofs idx [ns] (device), weights q and
+// delays [ns][nv] (device, fp64),
+//   b[idx[p],m] += c0^2 q[t] g_m(tn - delay[t]),  t = p nv + m,  g_m = 0 before the delay,
+// g_m from member m's f0 / p0 (nv = 1: one field); tn read from t_dev when it is not NULL (graph replays)
+void volume_source_apply(int dtype, int64_t ns, int nv, const int32_t* idx, const double* q, const double* delay,
+                         double c0, const SourceParams& sp, double t_host, const double* t_dev, void* b,
+                         cudaStream_t stream);
 // lossy / Westervelt models (wfx_wave_create_westervelt)
 double stiffness_c0(const struct ::wfx_stiffness* op);       // the c0 of y = -c0^2 K x
 int64_t stiffness_nshared(const struct ::wfx_stiffness* op); // rank-shared dofs (0 on one rank)

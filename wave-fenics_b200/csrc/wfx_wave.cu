@@ -76,6 +76,11 @@ struct wfx_wave
   // replays read from t_dev.  Setting or clearing it drops step_graph (captured with the other boundary kernel).
   bool prof_on = false;
   DevBuf<double> prof_amp, prof_delay, t_dev;
+  // volume source (section 4.5h): vs_n distinct dofs vs_idx, weights and delays [vs_n][nv]; evaluated on the device
+  // from the stage times like the profile (graph replays read t_dev).  Setting or clearing it drops step_graph.
+  int64_t vs_n = 0;
+  DevBuf<int32_t> vs_idx;
+  DevBuf<double> vs_q, vs_delay;
   cudaStream_t own_stream = nullptr; // capture needs a non-legacy stream
   cudaEvent_t ev_in = nullptr, ev_out = nullptr;
   // time-stepping position (reset by init / set_state): steps completed and the time reached
@@ -699,8 +704,17 @@ __global__ void set_source_ens_kernel(double* g_dev, const StepAmp a, int n)
 {
   if ((int)threadIdx.x < n) g_dev[threadIdx.x] = a.g[threadIdx.x];
 }
+// a volume source without a profile: the four stage times (volume source) and the n amplitudes (boundary term) of a
+// step in one launch
+__global__ void set_times_and_source_kernel(double* t_dev, double t0, double t1, double t2, double t3, double* g_dev,
+                                            const StepAmp a, int n)
+{
+  if ((int)threadIdx.x < n) g_dev[threadIdx.x] = a.g[threadIdx.x];
+  if (threadIdx.x == 0) t_dev[0] = t0, t_dev[1] = t1, t_dev[2] = t2, t_dev[3] = t3;
+}
 
 void boundary_profiled(wfx_wave* w, double tn, const double* t_dev, const void* vn, cudaStream_t st);
+void volume_sourced(wfx_wave* w, double tn, const double* t_dev, cudaStream_t st);
 
 // The layer's terms of one stage (update) or of f1 (stage 0, no update): wi the stiffness input, u / v the state at
 // stage 0, vn the stage's v at stages 1-3
@@ -734,7 +748,7 @@ void pml_terms(wfx_wave* w, int stage, bool update, double bdt, double adt, cons
 // One time step of size dt on stream st: the four stages of LinearGLL.hpp:244-270.  g[i*nv + m] is the
 // source amplitude of stage i (of member m); with g_from_dev the boundary kernels read it from w->g_dev
 // instead (graph capture).  With a source profile the boundary term takes the stage times tn[i] instead, or
-// reads them from w->t_dev.
+// reads them from w->t_dev; so does a volume source, added to b right after the boundary term.
 void enqueue_step(wfx_wave* w, double dt, const double* g, const double* tn, bool g_from_dev, cudaStream_t st)
 {
   const double a_runge[5] = {0.0, 0.5, 0.5, 1.0, 0.0};
@@ -793,6 +807,7 @@ void enqueue_step(wfx_wave* w, double dt, const double* g, const double* tn, boo
       WFX_CUDA(cudaStreamWaitEvent(st, w->ev_halo, 0));
       boundary(i, vn);
     }
+    if (w->vs_n) volume_sourced(w, g_from_dev ? 0.0 : tn[i], g_from_dev ? w->t_dev.p + i : nullptr, st);
     if (w->pml) pml_terms(w, i, true, dt * b_runge[i], dt * a_runge[i + 1], un, w->u_.p, w->v_.p, w->vn.p, st);
     if (w->model)
     {
@@ -1076,8 +1091,8 @@ void source_amplitudes(const wfx_wave* w, double tn, double* g)
 {
   for (int m = 0; m < w->nv; ++m) g[m] = source_amplitude(w->f0s[m], w->p0s[m], w->c0, tn);
 }
-// the boundary term with the source profile at stage time tn (t_dev: read it from there, graph capture)
-void boundary_profiled(wfx_wave* w, double tn, const double* t_dev, const void* vn, cudaStream_t st)
+// every member's f0 / p0 (one field: the model's)
+SourceParams source_params(const wfx_wave* w)
 {
   SourceParams sp{};
   for (int m = 0; m < w->nv; ++m)
@@ -1085,8 +1100,19 @@ void boundary_profiled(wfx_wave* w, double tn, const double* t_dev, const void* 
     sp.f0[m] = w->ens ? w->f0s[m] : w->f0;
     sp.p0[m] = w->ens ? w->p0s[m] : w->p0;
   }
-  boundary_apply_profile(w->bnd, w->nv, w->c0, w->model ? w->s_src : 0.0, sp, tn, t_dev, w->prof_amp.p,
+  return sp;
+}
+// the boundary term with the source profile at stage time tn (t_dev: read it from there, graph capture)
+void boundary_profiled(wfx_wave* w, double tn, const double* t_dev, const void* vn, cudaStream_t st)
+{
+  boundary_apply_profile(w->bnd, w->nv, w->c0, w->model ? w->s_src : 0.0, source_params(w), tn, t_dev, w->prof_amp.p,
                          w->prof_delay.p, vn, w->b.p, st);
+}
+// the volume source at stage time tn (t_dev: read it from there, graph capture)
+void volume_sourced(wfx_wave* w, double tn, const double* t_dev, cudaStream_t st)
+{
+  volume_source_apply(w->dtype, w->vs_n, w->nv, w->vs_idx.p, w->vs_q.p, w->vs_delay.p, w->c0, source_params(w), tn,
+                      t_dev, w->b.p, st);
 }
 } // namespace
 
@@ -1116,6 +1142,7 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
     if (wfx_stiffness_apply_ensemble(w->stiff, w->nv, u, nullptr, w->b.p, 0, st)) fail("%s", wfx_last_error());
     if (w->prof_on) boundary_profiled(w, t, nullptr, v, st);
     else boundary_apply_ens(w->bnd, w->nv, w->c0, g, nullptr, v, w->b.p, st);
+    if (w->vs_n) volume_sourced(w, t, nullptr, st);
     const int64_t n = w->n * w->nv;
     if (n == 0) return 0;
     const unsigned grid = (unsigned)((n + 255) / 256);
@@ -1136,6 +1163,7 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
     if (wfx_stiffness_apply(w->stiff, w->f1_w.p, w->b.p, 0, st)) fail("%s", wfx_last_error());
     if (w->prof_on) boundary_profiled(w, t, nullptr, v, st);
     else if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());
+    if (w->vs_n) volume_sourced(w, t, nullptr, st);
     if (w->pml) pml_terms(w, 0, false, 0.0, 0.0, w->f1_w.p, u, v, nullptr, st);
     if (w->qc != 0 && w->relax_m)
       boundary_absorbing_mass_relax(w->bnd, w->m64, w->qc, w->kappa, w->kd_on ? w->kd_b.p : nullptr, w->relax_m,
@@ -1194,6 +1222,7 @@ extern "C" int wfx_wave_f1(wfx_wave* w, double t, const void* u, const void* v, 
   if (w->halo && wfx_halo_update_rev_fwd(w->halo, w->b.p, st)) fail("%s", wfx_last_error());             // :176
   if (w->prof_on) boundary_profiled(w, t, nullptr, v, st);
   else if (w->bnd && wfx_boundary_apply(w->bnd, w->c0, g, v, w->b.p, st)) fail("%s", wfx_last_error());  // :175
+  if (w->vs_n) volume_sourced(w, t, nullptr, st);
   if (w->pml) pml_terms(w, 0, false, 0.0, 0.0, u, u, v, nullptr, st);
   if (wfx_mass_apply_inverse(w->mass, w->b.p, result, st)) fail("%s", wfx_last_error());                 // :188-191
   WFX_API_END
@@ -1273,7 +1302,15 @@ extern "C" int wfx_wave_rk4(wfx_wave* w, double t0, double tf, double dt, int64_
         WFX_CUDA(ie);
         w->graph_dt = dt;
       }
-      if (w->prof_on) set_source_kernel<<<1, 1, 0, ws>>>(w->t_dev.p, tn[0], tn[1], tn[2], tn[3]);
+      // the profiled boundary term and the volume source read the stage times, the plain boundary term the amplitudes
+      if (w->vs_n && !w->prof_on)
+      {
+        StepAmp a{};
+        for (int q = 0; q < 4 * w->nv; ++q) a.g[q] = g[q];
+        set_times_and_source_kernel<<<1, 4 * WFX_ENSEMBLE_MAX, 0, ws>>>(w->t_dev.p, tn[0], tn[1], tn[2], tn[3],
+                                                                        w->g_dev.p, a, 4 * w->nv);
+      }
+      else if (w->prof_on) set_source_kernel<<<1, 1, 0, ws>>>(w->t_dev.p, tn[0], tn[1], tn[2], tn[3]);
       else if (w->ens)
       {
         StepAmp a{};
@@ -1468,6 +1505,58 @@ extern "C" int wfx_wave_set_source_profile(wfx_wave* w, const double* amp_host, 
   w->prof_amp.upload(a);
   w->prof_delay.upload(d);
   w->prof_on = true;
+  WFX_API_END
+}
+
+extern "C" int wfx_wave_set_volume_source(wfx_wave* w, int64_t n, const int32_t* dofs_host, const double* q_host,
+                                          const double* delay_host)
+{
+  WFX_API_BEGIN
+  if (!w) fail("wave model is NULL");
+  if (w->halo) fail("volume source: one rank only (the model is distributed)");
+  if (n < 0) fail("volume source: n = %lld is negative", (long long)n);
+  if (n > 0 && (!dofs_host || !q_host)) fail("volume source: NULL dofs or weights");
+  const int nv = w->nv;
+  // the kernel adds each entry into b without atomics: the dofs must be distinct
+  std::vector<unsigned char> seen(n > 0 ? (size_t)w->n : 0, 0);
+  for (int64_t p = 0; p < n; ++p)
+  {
+    const int32_t d = dofs_host[p];
+    if (d < 0 || d >= w->n) fail("volume source: dof %d at entry %lld outside [0, %lld)", d, (long long)p, (long long)w->n);
+    if (seen[d]) fail("volume source: duplicate dof %d at entry %lld", d, (long long)p);
+    seen[d] = 1;
+    for (int m = 0; m < nv; ++m)
+    {
+      const int64_t k = p * nv + m;
+      if (!std::isfinite(q_host[k])) fail("volume source: non-finite weight at entry %lld", (long long)k);
+      if (delay_host && !std::isfinite(delay_host[k])) fail("volume source: non-finite delay at entry %lld", (long long)k);
+      if (delay_host && delay_host[k] < 0) fail("volume source: negative delay at entry %lld", (long long)k);
+    }
+  }
+  ScopedDevice sd(w->ctx->device);
+  // a step in flight may read the buffers, and the captured step holds the kernel (or lacks it)
+  WFX_CUDA(cudaDeviceSynchronize());
+  if (w->step_graph) WFX_CUDA(cudaGraphExecDestroy(w->step_graph));
+  w->step_graph = nullptr;
+  w->vs_n = 0;
+  if (n == 0)
+  {
+    w->vs_idx.release();
+    w->vs_q.release();
+    w->vs_delay.release();
+    return 0;
+  }
+  const size_t ne = (size_t)n * nv;
+  std::vector<double> d(ne, 0.0);
+  if (delay_host) d.assign(delay_host, delay_host + ne);
+  // each buffer on its own: after a failed allocation (out of memory) a retry allocates what is missing
+  if (w->vs_idx.n != (size_t)n) w->vs_idx.alloc((size_t)n);
+  if (w->vs_q.n != ne) w->vs_q.alloc(ne);
+  if (w->vs_delay.n != ne) w->vs_delay.alloc(ne);
+  w->vs_idx.upload(dofs_host, (size_t)n);
+  w->vs_q.upload(q_host, ne);
+  w->vs_delay.upload(d);
+  w->vs_n = n;
   WFX_API_END
 }
 

@@ -340,6 +340,16 @@ inline void set_profile(wfx_wave* wave, std::int64_t entries, const std::vector<
       throw std::runtime_error("wavefx: source profile arrays must hold one entry per state entry (or none)");
   check(wfx_wave_set_source_profile(wave, amp.empty() ? nullptr : amp.data(), delay.empty() ? nullptr : delay.data()));
 }
+// wfx_wave_set_volume_source with nv weights / delays per dof; an empty delay vector is passed as NULL
+inline void set_volume(wfx_wave* wave, int nv, const std::vector<std::int32_t>& dofs, const std::vector<double>& q,
+                       const std::vector<double>& delay)
+{
+  const std::size_t ne = dofs.size() * (std::size_t)nv;
+  if (q.size() != ne || (!delay.empty() && delay.size() != ne))
+    throw std::runtime_error("wavefx: volume source weights and delays must hold nv entries per dof");
+  check(wfx_wave_set_volume_source(wave, (std::int64_t)dofs.size(), dofs.data(), q.data(),
+                                   delay.empty() ? nullptr : delay.data()));
+}
 
 // A layered medium (DESIGN.md section 4.5e) as the weights of the operators, e.g. from the Python Medium class:
 //   stiffness [ncells]  rho_ref / rho_c                         (scales the model's geometry)
@@ -454,6 +464,13 @@ public:
   void set_source_profile(const std::vector<double>& amp, const std::vector<double>& delay)
   {
     set_profile(_wave, _ndofs, amp, delay);
+  }
+  // volume source (DESIGN.md section 4.5h): c0^2 q[p] g(t - delay[p]) added at dof dofs[p] (distinct dofs; an empty
+  // delay stands for 0, empty dofs clear the source); a point source's weights are the basis functions at the point
+  void set_volume_source(const std::vector<std::int32_t>& dofs, const std::vector<double>& q,
+                         const std::vector<double>& delay)
+  {
+    set_volume(_wave, 1, dofs, q, delay);
   }
   // fn(step, t, u, v) every `every` steps with pointers into pinned host copies (ndofs entries each);
   // the device -> host copy overlaps the time stepping.  A checkpoint is a snapshot handed back to
@@ -731,6 +748,12 @@ public:
   void set_source_profile(const std::vector<double>& amp, const std::vector<double>& delay)
   {
     set_profile(_wave, _ndofs * _nv, amp, delay);
+  }
+  // as LinearGLLOpt's, a column per member: q, delay [dofs][nv] (member-interleaved)
+  void set_volume_source(const std::vector<std::int32_t>& dofs, const std::vector<double>& q,
+                         const std::vector<double>& delay)
+  {
+    set_volume(_wave, _nv, dofs, q, delay);
   }
   void set_state(const std::vector<double>& u, const std::vector<double>& v)
   {

@@ -376,6 +376,96 @@ def focus_delays(points, focus, c0):
     return (d.max() - d) / float(c0) if len(d) else d
 
 
+def _trilinear(xv, xi):
+    """x(xi) and dx/dxi [3, 3] of the cell with vertices xv [8, 3] (vertex v = ix + 2 iy + 4 iz) at xi in [0, 1]^3"""
+    f = [(1.0 - xi[a], xi[a]) for a in range(3)]
+    x, J = np.zeros(3), np.zeros((3, 3))
+    for v in range(8):
+        b = (v & 1, (v >> 1) & 1, (v >> 2) & 1)
+        w = [f[a][b[a]] for a in range(3)]
+        x += w[0] * w[1] * w[2] * xv[v]
+        for a in range(3):
+            d = (1.0 if b[a] else -1.0) * w[(a + 1) % 3] * w[(a + 2) % 3]
+            J[:, a] += d * xv[v]
+    return x, J
+
+
+def _locate_in_cell(mesh, c, point, tol=1e-10):
+    """xi in [0, 1]^3 with x_c(xi) = point by Newton iteration on cell c's trilinear map, or None when the point lies
+    outside the cell.  Reference coordinates within 1e-14 of a GLL node are put on it, so that a point at a dof or on a
+    face, edge or vertex gives exact zeros at the dofs whose basis functions vanish there."""
+    xv = mesh.x[mesh.xdofs[c]]
+    x0 = np.asarray(point, dtype=np.float64)
+    xi = np.full(3, 0.5)
+    for _ in range(60):
+        x, J = _trilinear(xv, xi)
+        try:
+            step = np.linalg.solve(J, x - x0)
+        except np.linalg.LinAlgError:
+            return None
+        xi = xi - step
+        if np.any(np.abs(xi - 0.5) > 10.0):
+            return None
+        if np.abs(step).max() < 1e-15:
+            break
+    if np.any(xi < -tol) or np.any(xi > 1.0 + tol):
+        return None
+    nodes, _ = capi.gll(mesh.P)
+    for a in range(3):
+        k = np.argmin(np.abs(nodes - xi[a]))
+        if abs(nodes[k] - xi[a]) < 1e-14:
+            xi[a] = nodes[k]
+    return np.clip(xi, 0.0, 1.0)
+
+
+def _cell_weights(mesh, c, xi):
+    """(dofs, phi_dofs(x(xi))) of cell c: the GLL Lagrange basis at reference point xi, in the cell's dof order"""
+    P = mesh.P
+    nodes, _ = capi.gll(P)
+    perm = capi.compute_permutations(P)
+    L = np.ones((3, P + 1))
+    for a in range(3):
+        for i in range(P + 1):
+            for j in range(P + 1):
+                if j != i:
+                    L[a, i] *= (xi[a] - nodes[j]) / (nodes[i] - nodes[j])
+    phi = np.einsum("a,b,c->abc", L[0], L[1], L[2]).reshape(-1)   # tensor order t = (i0 n + i1) n + i2
+    return np.asarray(mesh.dofmap[c])[perm], phi
+
+
+def point_source(mesh, point):
+    """(dofs, q) of a point source at a physical point: q_j = phi_j(point), the GLL basis functions of the cell that
+    holds the point (located by Newton iteration on its trilinear map), at the dofs where they do not vanish, dofs
+    ascending.  On a shared face, edge or vertex either cell gives the same weights.  The same weights make the
+    interpolating sensor p(point) = sum_j q_j p_j.  Feed them to set_volume_source (DESIGN.md section 4.5h).  A point
+    outside the mesh raises WfxError."""
+    x0 = np.asarray(point, dtype=np.float64).reshape(3)
+    xc = mesh.x[mesh.xdofs]
+    lo, hi = xc.min(axis=1), xc.max(axis=1)
+    pad = 1e-10 * (hi - lo).max(axis=1, keepdims=True)
+    for c in np.nonzero(np.all((x0 >= lo - pad) & (x0 <= hi + pad), axis=1))[0]:
+        xi = _locate_in_cell(mesh, int(c), x0)
+        if xi is None:
+            continue
+        dofs, phi = _cell_weights(mesh, int(c), xi)
+        keep = phi != 0.0
+        order = np.argsort(dofs[keep])
+        return dofs[keep][order].astype(np.int32), phi[keep][order]
+    raise capi.WfxError(f"point_source: the point {tuple(x0)} lies outside the mesh")
+
+
+def phase_conjugate_delays(p_hat, f0):
+    """Time-reversal delays for a source profile: tau = mod(arg p_hat, 2 pi) / (2 pi f0), in [0, 1 / f0), shaped like
+    p_hat.  p_hat: the first-harmonic map (field_stats().harmonics[0]) of an emission from a point source at the
+    target; f0: the model's source frequency, or the members' frequencies [nv] for an ensemble's (ndofs, nv) map.
+    Firing every element with these delays aligns the phases of all contributions at the target (DESIGN.md section
+    4.5h)."""
+    p = np.asarray(p_hat)
+    f = np.broadcast_to(np.asarray(f0, dtype=np.float64), p.shape[-1:] if p.ndim > 1 else ())
+    tau = np.mod(np.angle(p), 2.0 * np.pi) / (2.0 * np.pi * f)
+    return np.where(tau * f < 1.0, tau, 0.0)
+
+
 def _refuse_pml(pml):
     if pml is not None:
         raise capi.WfxError("pml: ensemble models are not supported (LinearGLLOpt, LossyGLLOpt, WesterveltGLLOpt)")
@@ -531,6 +621,41 @@ class LinearGLLOpt:
 
         amplitude, delay = arr(amplitude), arr(delay)
         capi.call("wfx_wave_set_source_profile", self.handle, capi.f64p(amplitude), capi.f64p(delay))
+
+    def set_volume_source(self, dofs=None, q=None, delay=None):
+        """Volume source (DESIGN.md section 4.5h): at every stage b_j += c0^2 q_j g(t - delay_j) on the n distinct dofs
+        `dofs`, g the model's source (g = 0 before the delay), added before the layer, Gamma2 and quotient terms.
+        q and delay have shape (n,), or (n, nv) for an ensemble (a column per member); delay None stands for 0.  A
+        point source at x0 is point_source(mesh, x0).  set_volume_source() clears the source.  Model configuration:
+        it survives init, set_state and restarts."""
+        d = np.asarray([] if dofs is None else dofs)
+        if d.ndim != 1 or (d.size and not np.issubdtype(d.dtype, np.integer)):
+            raise capi.WfxError("volume source: dofs must be a 1-D array of integers")
+        if d.size == 0:
+            if any(a is not None and np.size(a) for a in (q, delay)):
+                raise capi.WfxError("volume source: weights or delays without dofs (set_volume_source() clears)")
+            capi.call("wfx_wave_set_volume_source", self.handle, 0, None, None, None)
+            return
+        # checked before the int32 conversion, which would wrap indices of 2^31 and above
+        bad = np.nonzero((d < 0) | (d >= self.ndofs))[0]
+        if len(bad):
+            raise capi.WfxError(f"volume source: dof {int(d[bad[0]])} at entry {int(bad[0])} outside [0, {self.ndofs})")
+        dofs = np.ascontiguousarray(d, dtype=np.int32)
+        shape = (len(dofs),) + self._entry_shape()[1:]
+
+        def arr(a):
+            if a is None:
+                return None
+            a = np.ascontiguousarray(a, dtype=np.float64)
+            if a.shape != shape:
+                raise capi.WfxError(f"volume source weights and delays must have shape {shape}")
+            return a
+
+        q, delay = arr(q), arr(delay)
+        if q is None:
+            raise capi.WfxError("volume source: weights q are required")
+        capi.call("wfx_wave_set_volume_source", self.handle, len(dofs), capi.i32p(dofs), capi.f64p(q),
+                  capi.f64p(delay))
 
     def set_snapshot(self, every, fn):
         """fn(step, t, u, v) with numpy views of the pinned host copies (copy them to keep them), every
